@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/s of the Hough-forest prediction path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path (HoughPrediction::predict_parameter_parallel semantics, seeds
@@ -33,6 +33,10 @@ JSON format), patch stride 5.
            this box's host cores on a bounded sample of the same workload
 --impl reference times that CPU restatement only (the reference is pure Rust + an un-vendored
 crate and cannot be built in this image; see DESIGN.md).
+--dump-outputs DIR writes the results of the last timed step of `value` (every frame of every rank,
+in rank order) as DIR/mid_point.npy (float32), DIR/rotation.npy and DIR/bounding_box.npy (float64).
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
+Above 64 MB a fixed seeded sample of frames is written, with their indices in DIR/frame_index.npy.
 """
 from __future__ import annotations
 
@@ -245,6 +249,25 @@ def _K():
     return synth.KINECT_K
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(res: np.ndarray, out_dir: str) -> None:
+    """--dump-outputs: the fields of capi.RESULT_DTYPE a caller receives, one .npy per field; the
+    padding word is not an output.  Over DUMP_LIMIT_BYTES, a sample of frames fixed by a seed."""
+    fields = {"mid_point": np.float32, "rotation": np.float64, "bounding_box": np.float64}
+    out = {k: np.ascontiguousarray(res[k], dt) for k, dt in fields.items()}
+    row_bytes = sum(a[:1].nbytes for a in out.values()) + 8
+    keep = (DUMP_LIMIT_BYTES - 4096) // row_bytes          # 4 kB for the .npy headers
+    if len(res) > keep:
+        idx = np.sort(np.random.default_rng(0).choice(len(res), keep, replace=False))
+        out = {k: a[idx] for k, a in out.items()}
+        out["frame_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_reference(args):
     """--impl reference: the CPU restatement on the host cores (rank 0 only)."""
     rank = int(os.environ.get("RANK", "0"))
@@ -341,7 +364,10 @@ def main():
     ap.add_argument("--forest-from", default="json", choices=["json", "arrays"],
                     help="load the model through the reference JSON document (default) or the flat arrays")
     ap.add_argument("--chunk", type=int, default=0, help="frames per pipeline pass (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -484,6 +510,10 @@ def main():
     clocks = sampler.stop()
     assert np.array_equal(out_dev["mid_point"], out_host["mid_point"]) and np.array_equal(out_dev["rotation"], out_host["rotation"])
     assert np.array_equal(out_dev["mid_point"], out_biwi["mid_point"]) and np.array_equal(out_dev["rotation"], out_biwi["rotation"])
+    if args.dump_outputs:
+        res_all = shard.gather_results(out_dev, n * world, dist)
+        if rank == 0:
+            dump_outputs(res_all, args.dump_outputs)
 
     # ---- strong scaling, configs[2]: one 15 000-frame sequence sharded by frame over the ranks
     strong = None
