@@ -184,6 +184,28 @@ def _as_depth(img) -> np.ndarray:
     return np.ascontiguousarray(a)
 
 
+def _as_frames(frames, device_ptr, n, w, h):
+    """(keep-alive array, pointer, location, n, w, h) of a [n,h,w] uint16 host batch or a device pointer."""
+    if device_ptr is None:
+        a = np.asarray(frames)
+        if a.dtype != np.uint16 or a.ndim != 3:
+            raise ValueError("frames must be [n,h,w] uint16")
+        a = np.ascontiguousarray(a)
+        n, h, w = a.shape
+        return a, capi.ptr(a), capi.DH_DEPTH_HOST, int(n), int(w), int(h)
+    if n is None or w is None or h is None:
+        raise ValueError("device_ptr needs n, w and h")
+    return None, C.c_void_p(int(device_ptr)), capi.DH_DEPTH_DEVICE, int(n), int(w), int(h)
+
+
+def _image_out(out_device_ptr, shape, dtype):
+    """(host array or None, pointer, location) of a batch of images: a new host array, or the caller's device memory."""
+    if out_device_ptr is None:
+        out = np.zeros(shape, dtype)
+        return out, capi.ptr(out), capi.DH_DEPTH_HOST
+    return None, C.c_void_p(int(out_device_ptr)), capi.DH_DEPTH_DEVICE
+
+
 class HoughPrediction:
     """prediction.rs:239-256 — the model plus the prediction entry points."""
 
@@ -390,6 +412,53 @@ class HoughPrediction:
         capi.check(capi.load().dh_predict_from2dhough(ctx._h, self._h, capi.ptr(depth), w, h, intrinsic._ptr(), C.byref(res)))
         return PredictionResult(np.array(res.mid_point[:], np.float32), np.array(res.rotation[:], np.float64),
                                 tuple(res.bounding_box[:]))
+
+    # ---- the 2-D entry points over n frames.  Frames: a [n,h,w] uint16 host array, or device_ptr +
+    # (n, w, h) for frames resident in HBM.  Images: returned as host arrays, or written to the
+    # caller's device memory at out_device_ptr ([n,h,w], nothing returned on the host).
+    def predict_mask_batch(self, frames, ctx: Context | None = None, device_ptr: int | None = None, n: int | None = None,
+                           w: int | None = None, h: int | None = None, out_device_ptr: int | None = None) -> np.ndarray | None:
+        """predict_mask (prediction.rs:850-905) per frame: uint8 [n,h,w]."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        ctx = ctx or default_context()
+        out, op, oloc = _image_out(out_device_ptr, (n, h, w), np.uint8)
+        capi.check(capi.load().dh_predict_mask_batch(ctx._h, self._h, p, n, w, h, loc, op, oloc))
+        return out
+
+    def hough_image_raw_batch(self, frames, intrinsic: IntrinsicMatrix, ctx: Context | None = None, device_ptr: int | None = None,
+                              n: int | None = None, w: int | None = None, h: int | None = None,
+                              out_device_ptr: int | None = None) -> np.ndarray | None:
+        """build_hough_image before its gaussian blur (prediction.rs:760-841) per frame: uint16 [n,h,w]."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        ctx = ctx or default_context()
+        out, op, oloc = _image_out(out_device_ptr, (n, h, w), np.uint16)
+        capi.check(capi.load().dh_build_hough_image_batch(ctx._h, self._h, p, n, w, h, intrinsic._ptr(), loc, 0, op, oloc, None))
+        return out
+
+    def build_hough_image_batch(self, frames, intrinsic: IntrinsicMatrix, ctx: Context | None = None, device_ptr: int | None = None,
+                                n: int | None = None, w: int | None = None, h: int | None = None, out_device_ptr: int | None = None,
+                                from2d: bool = False):
+        """build_hough_image (prediction.rs:760-845) per frame: uint16 [n,h,w] (None with out_device_ptr).
+        from2d=True: returns (images, capi.RESULT_DTYPE[n] of predict_parameter_from2dhough) from the same pass."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        ctx = ctx or default_context()
+        out, op, oloc = _image_out(out_device_ptr, (n, h, w), np.uint16)
+        res = np.zeros(n, capi.RESULT_DTYPE) if from2d else None
+        capi.check(capi.load().dh_build_hough_image_batch(ctx._h, self._h, p, n, w, h, intrinsic._ptr(), loc, 1, op, oloc,
+                                                          capi.ptr(res)))
+        return (out, res) if from2d else out
+
+    def predict_parameter_from2dhough_batch(self, frames, intrinsic: IntrinsicMatrix, ctx: Context | None = None,
+                                            device_ptr: int | None = None, n: int | None = None, w: int | None = None,
+                                            h: int | None = None) -> np.ndarray:
+        """predict_parameter_from2dhough (prediction.rs:343-367) per frame, without copying any image out:
+        capi.RESULT_DTYPE[n] (shards with shard.shard_range / gather_results like predict_batch)."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        ctx = ctx or default_context()
+        res = np.zeros(n, capi.RESULT_DTYPE)
+        capi.check(capi.load().dh_build_hough_image_batch(ctx._h, self._h, p, n, w, h, intrinsic._ptr(), loc, 1, None,
+                                                          capi.DH_DEPTH_HOST, capi.ptr(res)))
+        return res
 
     def debug_leaf_static(self, ctx: Context | None = None):
         ctx = ctx or default_context()

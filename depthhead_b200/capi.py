@@ -111,6 +111,8 @@ SIGNATURES = {
     "dh_hough_image_raw": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "dh_build_hough_image": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "dh_predict_from2dhough": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, C.POINTER(dh_result)]),
+    "dh_predict_mask_batch": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, C.c_int, _vp, C.c_int]),
+    "dh_build_hough_image_batch": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, _vp, C.c_int, C.c_int, _vp, C.c_int, _vp]),
     "dh_ctx_enable_stage_timing": (C.c_int, [_vp, C.c_int]),
     "dh_ctx_stage_ms": (C.c_int, [_vp, _vp]),
     "dh_ctx_counters": (C.c_int, [_vp, _vp]),

@@ -381,6 +381,28 @@ int dh_predict_from2dhough(dh_ctx* c, const dh_forest* f, const uint16_t* depth,
     });
 }
 
+int dh_predict_mask_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                          int depth_loc, uint8_t* mask, int mask_loc) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_mask_batch: bad depth_loc");
+        REQUIRE(mask_loc == DH_DEPTH_HOST || mask_loc == DH_DEPTH_DEVICE, "dh_predict_mask_batch: bad mask_loc");
+        REQUIRE(c && f && (n == 0 || (depth && mask)), "dh_predict_mask_batch: NULL argument");
+        c->cx->predict_mask_batch(*f->hf, depth, n, w, h, depth_loc, mask, mask_loc);
+    });
+}
+int dh_build_hough_image_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                               const float K[9], int depth_loc, int blur, uint16_t* hough, int hough_loc, dh_result* from2d) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_build_hough_image_batch: bad depth_loc");
+        REQUIRE(hough_loc == DH_DEPTH_HOST || hough_loc == DH_DEPTH_DEVICE, "dh_build_hough_image_batch: bad hough_loc");
+        REQUIRE(blur == 0 || blur == 1, "dh_build_hough_image_batch: blur must be 0 or 1");
+        REQUIRE(hough || from2d, "dh_build_hough_image_batch: hough and from2d are both NULL");
+        REQUIRE(blur || !from2d, "dh_build_hough_image_batch: from2d needs blur = 1 (the arg-max of the blurred image)");
+        REQUIRE(c && f && K && (n == 0 || depth), "dh_build_hough_image_batch: NULL argument");
+        c->cx->hough_image_batch(*f->hf, depth, n, w, h, K, depth_loc, blur != 0, hough, hough_loc, from2d);
+    });
+}
+
 int dh_ctx_enable_stage_timing(dh_ctx* c, int on) {
     return guarded([&] {
         REQUIRE(c, "NULL ctx");

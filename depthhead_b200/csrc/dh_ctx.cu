@@ -50,6 +50,11 @@ PFN_encodeTiled get_encode_fn() {
     return fn;
 }
 
+// frames per chunk of the image back ends: kImageScratchBytes of u32 sums and two u16 planes per lane
+uint32_t image_chunk_cap(uint32_t w, uint32_t h) {
+    return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(1u << 30, kImageScratchBytes / (8ull * w * h + 8)));
+}
+
 uint32_t env_u32(const char* name, uint32_t dflt) {
     const char* v = std::getenv(name);
     if (!v || !*v) return dflt;
@@ -123,9 +128,6 @@ Context::~Context() {
     dev_free(d_offsets_);
     dev_free(d_status_);
     if (h_status_) cudaFreeHost(h_status_);
-    dev_free(d_aux32_);
-    dev_free(d_aux16_);
-    dev_free(d_aux8_);
     if (h_fs_) cudaFreeHost(h_fs_);
     if (h_counters_) cudaFreeHost(h_counters_);
     if (h_results_) cudaFreeHost(h_results_);
@@ -188,6 +190,8 @@ void Context::free_forest() {
     dev_free(df_leaf_box_);
     dev_free(df_kernel_);
     df_serial_ = 0;
+    dev_free(d_blur_taps_);
+    blur_serial_ = 0;
 }
 
 // PairRec topology (dh_types.hpp): every internal node at an even depth below its root becomes a
@@ -433,6 +437,11 @@ void Context::free_lane(Lane& L) {
     dev_free(L.fs);
     dev_free(L.results);
     dev_free(L.ms_trace);
+    dev_free(L.img32);
+    dev_free(L.img16);
+    dev_free(L.img_keys);
+    L.img_px = 0;
+    L.pending_bytes = 0;
     L.allocated = false;
     L.cubes_clean = false;
 }
@@ -757,6 +766,7 @@ void Context::begin_call() {
     DH_CUDA(cudaSetDevice(device_));
     lanes_[0].stream = stream_;
     for (int i = 1; i < kMaxLanes; ++i) lanes_[i].stream = lanes_[i].own;
+    for (int i = 0; i < kMaxLanes; ++i) lanes_[i].pending_bytes = 0;  // (left behind by a call that failed)
     launches_ = 0;
     ev_used_ = 0;
     marks_.clear();
@@ -868,12 +878,16 @@ void Context::predict(const HostForest& hf, const uint16_t* depth, uint32_t w, u
 
 void Context::predict_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
                             const float K[9], int depth_loc, dh_result* out) {
-    run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, out);
+    BackEnd be;
+    be.results = out;
+    run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, be);
 }
 
 void Context::predict_batch_biwi(const HostForest& hf, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
                                  uint32_t h, const float K[9], dh_result* out) {
-    run_batch(hf, nullptr, blob, offsets, n, w, h, K, DH_DEPTH_HOST, out);
+    BackEnd be;
+    be.results = out;
+    run_batch(hf, nullptr, blob, offsets, n, w, h, K, DH_DEPTH_HOST, be);
 }
 
 // Device copies of the file offsets and room for the compressed bytes of one chunk per slot.
@@ -965,7 +979,7 @@ void Context::biwi_decode(const uint8_t* blob, const uint64_t* offsets, uint32_t
 }
 
 void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
-                        uint32_t w, uint32_t h, const float K[9], int depth_loc, dh_result* out) {
+                        uint32_t w, uint32_t h, const float K[9], int depth_loc, const BackEnd& be) {
     begin_call();
     have_debug_ = false;
     if (n == 0) {
@@ -976,27 +990,24 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     last_encoded_chunks_ = 0;
     last_h2d_bytes_ = 0;
     if (!blob && depth_loc != DH_DEPTH_DEVICE && want_encode(n, w, h)) {
-        run_batch_encoded(hf, depth, n, w, h, K, out);
+        run_batch_encoded(hf, depth, n, w, h, K, be);
         return;
     }
     // Chunks go round-robin over the lanes.  Stage timing needs the kernels of a pass back to
     // back on one stream, so it runs single-lane.
     // Biwi input: the run-length expansion is latency-bound (one thread per frame walks the run
     // headers), so its chunks are larger: more frames in flight per launch
-    const uint32_t want_chunk = (blob && !chunk_frames_) ? std::min<uint32_t>(512u, n) : pick_chunk(n, depth_loc);
+    uint32_t want_chunk = (blob && !chunk_frames_) ? std::min<uint32_t>(512u, n) : pick_chunk(n, depth_loc);
+    if (be.kind != BackEnd::kPose) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
     const int n_lanes = timing_ ? 1 : (int)std::max<uint32_t>(1u, std::min<uint32_t>((uint32_t)max_lanes_, (n + want_chunk - 1) / want_chunk));
     ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
+    if (be.kind != BackEnd::kPose) ensure_image_scratch(n_lanes);
+    if (be.kind == BackEnd::kBlurred) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
-    // pinned staging for the results
-    if (h_results_cap_ < n) {
-        if (h_results_) cudaFreeHost(h_results_);
-        h_results_ = nullptr;
-        DH_CUDA(cudaHostAlloc((void**)&h_results_, sizeof(dh_result) * n, cudaHostAllocDefault));
-        h_results_cap_ = n;
-    }
+    ensure_results(n);  // pinned staging for the results
     if (depth_loc != DH_DEPTH_DEVICE) ensure_staging(2);
     if (blob) ensure_biwi(offsets, n, F, 2);
     // fork: the other lanes (and the copy stream) start after everything already queued on the caller's stream
@@ -1006,9 +1017,9 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
         Lane& L = lanes_[c % (uint32_t)n_lanes];
         const uint32_t f0 = c * F, nc = std::min<uint32_t>(F, n - f0);
         FrameBuffers b = buffers(L, d_depth);
+        flush_pending(L);
         run_front(L, b, nc, nullptr);
-        run_back(L, b, nc, iterations);
-        DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * nc, cudaMemcpyDeviceToHost, L.stream));
+        run_chunk_back(L, b, f0, nc, iterations, be);
     };
     if (depth_loc == DH_DEPTH_DEVICE) {
         for (uint32_t c = 0; c < n_chunks; ++c) enqueue_chunk(c, depth + (size_t)c * F * frame_px);
@@ -1052,6 +1063,7 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
             DH_CUDA(cudaEventRecord(ev_consumed_[slot], L.stream));
         }
     }
+    for (int i = 0; i < n_lanes; ++i) flush_pending(lanes_[i]);
     if (n_lanes > 1) {  // join: the caller's stream continues after every lane
         for (int i = 1; i < n_lanes; ++i) {
             DH_CUDA(cudaEventRecord(lanes_[i].done, lanes_[i].stream));
@@ -1062,7 +1074,16 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     DH_CUDA(cudaStreamSynchronize(stream_));
     end_call();
     if (blob) check_biwi_status(n);
-    std::memcpy(out, h_results_, sizeof(dh_result) * n);
+    if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
+}
+
+void Context::ensure_results(uint32_t n) {
+    if (h_results_cap_ < n) {
+        if (h_results_) cudaFreeHost(h_results_);
+        h_results_ = nullptr;
+        DH_CUDA(cudaHostAlloc((void**)&h_results_, sizeof(dh_result) * n, cudaHostAllocDefault));
+        h_results_cap_ = n;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ compressed host input
@@ -1129,7 +1150,7 @@ void Context::ensure_encode(uint32_t n, uint32_t F) {
 }
 
 void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
-                                dh_result* out) {
+                                const BackEnd& be) {
     // Two streams of chunks meet inside the batch.  FRONT: the workers rewrite chunks 0, 1, 2, .. as
     // run-length files (two chunks in flight, pinned slots 0..2); a finished chunk's bytes go over
     // the first copy stream into device slots 0 / 1 and are expanded and predicted on lane 0.
@@ -1139,19 +1160,17 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     // The host cores and the copy engines therefore work all the time, on different chunks, and
     // the split adapts to how dense the frames are and how many cores the caller gave the workers.
     const bool hybrid = env_flag("DH_HOST_HYBRID", true) && !timing_ && max_lanes_ >= 2;
-    const uint32_t want_chunk = pick_chunk(n, DH_DEPTH_HOST);
+    uint32_t want_chunk = pick_chunk(n, DH_DEPTH_HOST);
+    if (be.kind != BackEnd::kPose) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
     const int n_lanes = hybrid ? 2 : 1;
     ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
+    if (be.kind != BackEnd::kPose) ensure_image_scratch(n_lanes);
+    if (be.kind == BackEnd::kBlurred) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
-    if (h_results_cap_ < n) {
-        if (h_results_) cudaFreeHost(h_results_);
-        h_results_ = nullptr;
-        DH_CUDA(cudaHostAlloc((void**)&h_results_, sizeof(dh_result) * n, cudaHostAllocDefault));
-        h_results_cap_ = n;
-    }
+    ensure_results(n);
     ensure_staging(hybrid ? 4 : 2);
     ensure_encode(n, F);
     const size_t bound = enc_frame_bound_;
@@ -1203,9 +1222,9 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     auto run_chunk = [&](Lane& L, int slot, uint32_t c) {
         const uint32_t f0 = c * F, nc = std::min<uint32_t>(F, n - f0);
         FrameBuffers b = buffers(L, d_depth_[slot]);
+        flush_pending(L);
         run_front(L, b, nc, nullptr);
-        run_back(L, b, nc, iterations);
-        DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * nc, cudaMemcpyDeviceToHost, L.stream));
+        run_chunk_back(L, b, f0, nc, iterations, be);
         DH_CUDA(cudaEventRecord(ev_consumed_[slot], L.stream));
         ++done_chunks;
     };
@@ -1324,6 +1343,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
         for (int i = 0; i < n_lanes; ++i) cudaStreamSynchronize(lanes_[i].stream);
         throw;
     }
+    for (int i = 0; i < n_lanes; ++i) flush_pending(lanes_[i]);
     if (n_lanes > 1) {
         for (int i = 1; i < n_lanes; ++i) {
             DH_CUDA(cudaEventRecord(lanes_[i].done, lanes_[i].stream));
@@ -1339,7 +1359,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
         for (uint32_t i = 0; i < n; ++i)
             if (h_status_[i]) throw ModelError(DH_E_STATE, "internal error: frame " + std::to_string(i) + " did not survive the compressed host->device path");
     }
-    std::memcpy(out, h_results_, sizeof(dh_result) * n);
+    if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
 }
 
 // ------------------------------------------------------------------------------------------------ seeded sequences
@@ -1409,30 +1429,12 @@ void Context::predict_sequences(const HostForest& hf, const uint16_t* depth, uin
     end_call();
 }
 
+// ------------------------------------------------------------------------------------------------ 2-D back ends
+// predict_mask, build_hough_image (raw or blurred) and predict_parameter_from2dhough share the
+// batch pipeline of the pose path: the same chunks, lanes, staging and front end; only the back
+// end of a chunk differs (run_image_back).  The single-frame entry points are batches of one frame.
 void Context::predict_mask(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, uint8_t* mask) {
-    begin_call();
-    have_debug_ = false;
-    ensure_forest(hf);
-    const float K[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
-    ensure_scratch(hf, w, h, 1, K);
-    ensure_staging(1);
-    DH_CUDA(cudaMemcpyAsync(d_depth_[0], depth, (size_t)w * h * sizeof(uint16_t), cudaMemcpyHostToDevice, stream_));
-    FrameBuffers b = buffers(lanes_[0], d_depth_[0]);
-    run_front(lanes_[0], b, 1, nullptr);
-    if (aux8_cap_ < (size_t)w * h) {
-        dev_free(d_aux8_);
-        dev_alloc(d_aux8_, (size_t)w * h);
-        aux8_cap_ = (size_t)w * h;
-    }
-    DH_CUDA(cudaMemsetAsync(d_aux8_, 0, (size_t)w * h, stream_));
-    if (geom_.P) {
-        launch_mask(b, geom_, fdev_, d_aux8_, stream_);
-        launches_ += 1;
-    }
-    DH_CUDA(cudaGetLastError());
-    DH_CUDA(cudaMemcpyAsync(mask, d_aux8_, (size_t)w * h, cudaMemcpyDeviceToHost, stream_));
-    mark(-1);
-    end_call();
+    predict_mask_batch(hf, depth, 1, w, h, DH_DEPTH_HOST, mask, DH_DEPTH_HOST);
 }
 
 void Context::hough_image_raw(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9],
@@ -1444,60 +1446,130 @@ void Context::hough_image_raw(const HostForest& hf, const uint16_t* depth, uint3
 // `votes` (host, may be NULL); from2d != NULL: predict_parameter_from2dhough (prediction.rs:343-367).
 void Context::hough_image(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9], uint16_t* votes,
                           bool blur, dh_result* from2d) {
-    begin_call();
-    have_debug_ = false;
-    ensure_forest(hf);
-    ensure_scratch(hf, w, h, 1, K);
-    ensure_staging(1);
-    std::vector<float> kern;
-    if (blur) kern = build_gaussian_blur_kernel(hf.gaussian_sigma);
-    DH_CUDA(cudaMemcpyAsync(d_depth_[0], depth, (size_t)w * h * sizeof(uint16_t), cudaMemcpyHostToDevice, stream_));
-    FrameBuffers b = buffers(lanes_[0], d_depth_[0]);
-    run_front(lanes_[0], b, 1, nullptr);
-    const size_t px = (size_t)w * h;
-    if (aux32_cap_ < px) {
-        dev_free(d_aux32_);
-        dev_free(d_aux16_);
-        dev_alloc(d_aux32_, px);          // u32 vote sums; reused as two u16 planes by the blur
-        dev_alloc(d_aux16_, px);
-        aux32_cap_ = px;
+    hough_image_batch(hf, depth, 1, w, h, K, DH_DEPTH_HOST, blur, votes, DH_DEPTH_HOST, from2d);
+}
+
+void Context::predict_mask_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                                 uint8_t* mask, int mask_loc) {
+    const float K[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};  // predict_mask does not project anything
+    BackEnd be;
+    be.kind = BackEnd::kMask;
+    be.image = mask;
+    be.image_on_device = mask_loc == DH_DEPTH_DEVICE;
+    run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, be);
+}
+
+void Context::hough_image_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
+                                int depth_loc, bool blur, uint16_t* votes, int votes_loc, dh_result* from2d) {
+    if (from2d && !blur) throw ModelError(DH_E_ARG, "predict_parameter_from2dhough takes the arg-max of the BLURRED vote image");
+    if (!votes && !from2d) throw ModelError(DH_E_ARG, "neither a vote image nor from2d results are asked for");
+    BackEnd be;
+    be.kind = blur ? BackEnd::kBlurred : BackEnd::kVotes;
+    be.results = from2d;
+    be.image = votes;
+    be.image_on_device = votes_loc == DH_DEPTH_DEVICE;
+    run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, be);
+}
+
+// u32 sums + two u16 planes per frame of a chunk, and the arg-max keys, on every lane of the call
+void Context::ensure_image_scratch(int n_lanes) {
+    const size_t frame_px = (size_t)sk_.w * sk_.h, need = (size_t)call_chunk_ * frame_px;
+    for (int i = 0; i < std::max(1, std::min(n_lanes, kMaxLanes)); ++i) {
+        Lane& L = lanes_[i];
+        if (L.img_px >= need) continue;
+        DH_CUDA(cudaStreamSynchronize(stream_));
+        dev_free(L.img32);
+        dev_free(L.img16);
+        dev_free(L.img_keys);
+        L.img_px = 0;
+        dev_alloc(L.img32, need);
+        dev_alloc(L.img16, 2 * need);
+        dev_alloc(L.img_keys, (size_t)call_chunk_);
+        L.img_px = need;
     }
-    DH_CUDA(cudaMemsetAsync(d_aux32_, 0, px * sizeof(uint32_t), stream_));
-    if (geom_.P) {
-        launch_hough_image(b, geom_, fdev_, d_aux32_, d_aux16_, stream_);
-        launches_ += 2;
-    } else {
-        DH_CUDA(cudaMemsetAsync(d_aux16_, 0, px * sizeof(uint16_t), stream_));
+}
+
+// taps of the blur (imageproc gaussian_kernel_f32), once per model and sigma
+void Context::ensure_blur_taps(const HostForest& hf) {
+    const uint64_t sv = hf.sigma_version.load();
+    if (d_blur_taps_ && blur_serial_ == hf.serial && blur_sigma_version_ == sv) return;
+    const std::vector<float> k = build_gaussian_blur_kernel(hf.gaussian_sigma);
+    DH_CUDA(cudaStreamSynchronize(stream_));
+    dev_free(d_blur_taps_);
+    dev_alloc(d_blur_taps_, k.size());
+    DH_CUDA(cudaMemcpy(d_blur_taps_, k.data(), k.size() * sizeof(float), cudaMemcpyHostToDevice));
+    blur_radius_ = (int)(k.size() / 2);
+    blur_serial_ = hf.serial;
+    blur_sigma_version_ = sv;
+}
+
+void Context::flush_pending(Lane& L) {
+    if (!L.pending_bytes) return;
+    DH_CUDA(cudaMemcpyAsync(L.pending_dst, L.pending_src, L.pending_bytes, cudaMemcpyDeviceToHost, L.stream));
+    L.pending_bytes = 0;
+}
+
+void Context::run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be) {
+    if (be.kind != BackEnd::kPose) {
+        run_image_back(L, b, f0, n, be);
+        return;
     }
-    const uint16_t* result = d_aux16_;
-    if (blur) {
-        float* d_k = nullptr;
-        dev_alloc(d_k, kern.size());
-        try {
-            DH_CUDA(cudaMemcpyAsync(d_k, kern.data(), kern.size() * sizeof(float), cudaMemcpyHostToDevice, stream_));
-            uint16_t* tmp = reinterpret_cast<uint16_t*>(d_aux32_);  // the u32 sums have been narrowed into d_aux16_
-            launches_ += (uint64_t)launch_gaussian_blur(d_aux16_, tmp, tmp + px, w, h, d_k, (int)(kern.size() / 2), stream_);
-            result = tmp + px;
-            DH_CUDA(cudaGetLastError());
-            DH_CUDA(cudaStreamSynchronize(stream_));  // kern / d_k go away
-        } catch (...) {
-            cudaStreamSynchronize(stream_);
-            dev_free(d_k);
-            throw;
+    run_back(L, b, n, iterations);
+    DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
+}
+
+// The 2-D back end of one chunk; the launches do not depend on the number of frames.  Images the
+// caller wants in device memory are written there by the kernels; host-bound images are left in
+// the lane's scratch and copied out before the lane's next chunk (flush_pending).
+void Context::run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be) {
+    const Geometry& g = geom_;
+    cudaStream_t st = L.stream;
+    const size_t frame_px = (size_t)g.w * g.h, px = frame_px * n;
+    uint16_t* plane0 = L.img16;
+    uint16_t* plane1 = L.img16 + L.img_px;
+    mark(DH_STAGE_VOTE);  // the whole 2-D back end is booked here
+    void* image = nullptr;  // this chunk's image in device memory
+    size_t elem = sizeof(uint16_t);
+    if (be.kind == BackEnd::kMask) {
+        elem = 1;
+        uint8_t* mask = be.image_on_device ? static_cast<uint8_t*>(be.image) + (size_t)f0 * frame_px : reinterpret_cast<uint8_t*>(plane1);
+        DH_CUDA(cudaMemsetAsync(mask, 0, px, st));
+        if (g.P) {
+            launch_mask(b, g, fdev_, n, mask, st);
+            launches_ += 1;
         }
-        dev_free(d_k);
+        image = mask;
+    } else {
+        DH_CUDA(cudaMemsetAsync(L.img32, 0, px * sizeof(uint32_t), st));
+        if (g.P) {
+            launch_hough_votes(b, g, fdev_, n, L.img32, st);
+            launches_ += 1;
+        }
+        if (be.image) image = be.image_on_device ? static_cast<uint16_t*>(be.image) + (size_t)f0 * frame_px : plane1;
+        if (be.kind == BackEnd::kVotes) {
+            launch_narrow_u16(L.img32, static_cast<uint16_t*>(image), px, st);
+            launches_ += 1;
+        } else {
+            if (be.results) DH_CUDA(cudaMemsetAsync(L.img_keys, 0, sizeof(unsigned long long) * n, st));
+            launches_ += (uint64_t)launch_gaussian_blur(L.img32, plane0, static_cast<uint16_t*>(image), be.results ? L.img_keys : nullptr,
+                                                        g.w, g.h, n, d_blur_taps_, blur_radius_, st);
+            if (be.results) {
+                launch_hough2d_pose(L.img_keys, b.depth, g, n, L.results, st);
+                launches_ += 1;
+            }
+        }
     }
-    if (from2d) {
-        if (px == 0) throw ModelError(DH_E_SHAPE, "predict_parameter_from2dhough on an empty image (the reference unwraps None)");
-        launch_hough2d_argmax(result, d_depth_[0], w, h, geom_, lanes_[0].results, stream_);
-        launches_ += 1;
-        DH_CUDA(cudaMemcpyAsync(h_result1_, lanes_[0].results, sizeof(dh_result), cudaMemcpyDeviceToHost, stream_));
+    stage_check("2-D back end");
+    mark(DH_STAGE_D2H);
+    launch_counters(b, g, n, d_counters_, st);
+    launches_ += 1;
+    if (be.results) DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, st));
+    if (image && !be.image_on_device) {
+        L.pending_dst = static_cast<char*>(be.image) + (size_t)f0 * frame_px * elem;
+        L.pending_src = image;
+        L.pending_bytes = px * elem;
     }
     DH_CUDA(cudaGetLastError());
-    if (votes) DH_CUDA(cudaMemcpyAsync(votes, result, px * sizeof(uint16_t), cudaMemcpyDeviceToHost, stream_));
-    mark(-1);
-    end_call();
-    if (from2d) *from2d = *h_result1_;
 }
 
 // ------------------------------------------------------------------------------------------------ debug exports

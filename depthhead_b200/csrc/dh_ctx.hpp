@@ -35,11 +35,32 @@ struct Lane {
     dh_result* results = nullptr;   // [F]
     int32_t* ms_trace = nullptr;    // [F][2][iters][3] (debug export)
     uint32_t* cubes = nullptr;      // [F][2][kBox^3]
+    // 2-D back ends (predict_mask, build_hough_image, from2d): allocated by the first such call
+    uint32_t* img32 = nullptr;      // [F][h][w] u32 vote sums
+    uint16_t* img16 = nullptr;      // [2][F][h][w] horizontal blur, then the image handed out (mask: u8 in the second plane)
+    unsigned long long* img_keys = nullptr;  // [F] arg-max keys of the from2d pass
+    size_t img_px = 0;              // F * h * w the image scratch holds
+    // a host-bound image copy of this lane's last chunk, issued before the lane's next chunk (a copy
+    // to pageable memory blocks the host: deferred, it overlaps the other lane's kernels)
+    void* pending_dst = nullptr;
+    const void* pending_src = nullptr;
+    size_t pending_bytes = 0;
     CUtensorMap sat_map{};
     bool allocated = false;
     bool cubes_clean = false;       // every cube is zero (meanshift_kernel cleared behind itself)
 };
 constexpr int kMaxLanes = 4;
+
+// What a batch computes after the front end (SAT + traversal) of every chunk.
+struct BackEnd {
+    enum Kind { kPose, kMask, kVotes, kBlurred } kind = kPose;
+    dh_result* results = nullptr;  // kPose: poses [n]; kBlurred: from2d poses [n] or nullptr (host memory)
+    void* image = nullptr;         // kMask: u8 [n][h][w]; kVotes / kBlurred: u16 [n][h][w] (kBlurred: may be nullptr)
+    bool image_on_device = false;  // image points to device memory on the context's GPU
+};
+// Image back ends keep a u32 accumulator and two u16 planes per frame of a chunk (8 bytes per
+// pixel, 2.4 MB per VGA frame): their chunks hold at most this much image scratch per lane.
+constexpr size_t kImageScratchBytes = 256ull << 20;
 
 struct TrainSet;  // dh_train.cu
 void trainset_free(TrainSet* t);
@@ -97,6 +118,11 @@ public:
     void train_split_level(const TrainSet& ts, const uint32_t* sample_idx, const uint64_t* node_off, uint32_t n_nodes,
                            const int32_t* rects, const double* thr, uint8_t* bits);
     void predict_mask(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, uint8_t* mask);
+    // batched 2-D back ends: depth [n][h][w] at depth_loc, images [n][h][w] at image_loc (DH_DEPTH_HOST / DH_DEPTH_DEVICE)
+    void predict_mask_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                            uint8_t* mask, int mask_loc);
+    void hough_image_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
+                           int depth_loc, bool blur, uint16_t* votes, int votes_loc, dh_result* from2d);
     void hough_image_raw(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9],
                          uint16_t* votes);
     void hough_image(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9], uint16_t* votes,
@@ -123,11 +149,19 @@ private:
     void ensure_biwi(const uint64_t* offsets, uint32_t n, uint32_t chunk, int slots);
     void check_biwi_status(uint32_t n);
     void run_batch(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
-                   uint32_t h, const float K[9], int depth_loc, dh_result* out);
+                   uint32_t h, const float K[9], int depth_loc, const BackEnd& be);
     uint32_t pick_chunk(uint32_t n_frames, int depth_loc) const;
     bool want_encode(uint32_t n, uint32_t w, uint32_t h) const;
     void ensure_encode(uint32_t n, uint32_t F);
-    void run_batch_encoded(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9], dh_result* out);
+    void run_batch_encoded(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
+                           const BackEnd& be);
+    void ensure_results(uint32_t n);
+    void ensure_image_scratch(int n_lanes);
+    void ensure_blur_taps(const HostForest& hf);
+    // after run_front: the chunk's back end and the copies of its results (frames f0 .. f0 + n - 1 of the batch)
+    void run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be);
+    void run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be);
+    void flush_pending(Lane& L);
     void free_scratch();
     TilePlan plan_tiles(const Geometry& g) const;
     FrameBuffers buffers(const Lane& L, const uint16_t* depth) const;
@@ -175,6 +209,10 @@ private:
     LeafBox* df_leaf_box_ = nullptr;
     float* df_kernel_ = nullptr;
     ForestDev fdev_{};
+    // taps of build_hough_image's gaussian blur for (blur_serial_, blur_sigma_version_)
+    float* d_blur_taps_ = nullptr;
+    int blur_radius_ = 0;
+    uint64_t blur_serial_ = 0, blur_sigma_version_ = 0;
 
     // scratch for one chunk of frames
     ScratchKey sk_;
@@ -195,10 +233,6 @@ private:
     uint32_t* d_status_ = nullptr;
     uint32_t* h_status_ = nullptr;
     size_t biwi_frames_cap_ = 0;
-    uint32_t* d_aux32_ = nullptr;
-    uint16_t* d_aux16_ = nullptr;
-    uint8_t* d_aux8_ = nullptr;
-    size_t aux32_cap_ = 0, aux8_cap_ = 0;
 
     // Compressed host->device path (run_batch_encoded): worker threads write the frames of a chunk
     // as Biwi run-length files into a pinned slot, in groups of kEncGroup frames; a group owns a

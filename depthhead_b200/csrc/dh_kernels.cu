@@ -2048,18 +2048,23 @@ __global__ void __launch_bounds__(128) leaf_gate_kernel(const double* __restrict
 }
 
 // ================================================================ next-row back-ends on the same front-end
+// The 2-D back ends work on a chunk of F frames per launch: the frame index comes from the grid and
+// every per-frame buffer is [F][h][w] (leaf ids [F][T][P], as the traversal writes them).
+//
 // predict_mask (prediction.rs:850-905): per non-background patch, mean prob -> u8, splat to a
 // stepwidth^2 block.  Patches are visited in raster order by the reference and later patches
 // overwrite earlier ones; blocks of distinct patches never overlap (block origin = centre - s/2,
-// size s, centres s apart), so the order is irrelevant.
+// size s, centres s apart), so the order is irrelevant.  One thread per (frame, patch).
 __global__ void __launch_bounds__(256) mask_kernel(FrameBuffers b, Geometry g, const double* __restrict__ leaf_prob,
                                                    uint8_t* __restrict__ mask) {
-    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x, frame = blockIdx.y;
     if (p >= g.P) return;
     const int T = (int)g.n_trees;
-    if (b.leaf[p] < 0) return;
+    const int32_t* leaf = b.leaf + (size_t)frame * g.n_trees * g.P;
+    mask += (size_t)frame * g.w * g.h;
+    if (leaf[p] < 0) return;
     double s = 0.0;
-    for (int t = 0; t < T; ++t) s = __dadd_rn(s, __ldg(leaf_prob + ((uint32_t)b.leaf[(size_t)t * g.P + p] & b.leaf_mask)));
+    for (int t = 0; t < T; ++t) s = __dadd_rn(s, __ldg(leaf_prob + ((uint32_t)leaf[(size_t)t * g.P + p] & b.leaf_mask)));
     const double prob = __ddiv_rn(s, (double)T);
     const double scaled = __dmul_rn(prob, 255.0);
     // `as u8`: saturating, NaN -> 0
@@ -2076,14 +2081,16 @@ __global__ void __launch_bounds__(256) mask_kernel(FrameBuffers b, Geometry g, c
 }
 
 // build_hough_image before the blur (prediction.rs:760-841).  u16 wrap-around adds are done as
-// u32 atomics and truncated afterwards (sum mod 2^16 is the same either way).
+// u32 atomics into the frame's accumulator and truncated by the reader (sum mod 2^16 is the same
+// either way).  One thread per (frame, tree, patch).
 __global__ void __launch_bounds__(256) hough_image_kernel(FrameBuffers b, Geometry g, ForestDev f, uint32_t* __restrict__ acc) {
-    const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x, frame = blockIdx.y;
     const uint32_t T = g.n_trees;
     if (idx >= g.P * T) return;
     const uint32_t p = idx % g.P, t = idx / g.P;
-    if (b.leaf[p] < 0) return;  // background patch: decided on the slice of tree 0 (the only one prefilled with -1)
-    const int32_t L = (int32_t)((uint32_t)b.leaf[(size_t)t * g.P + p] & b.leaf_mask);
+    const int32_t* leaf = b.leaf + (size_t)frame * T * g.P;
+    if (leaf[p] < 0) return;  // background patch: decided on the slice of tree 0 (the only one prefilled with -1)
+    const int32_t L = (int32_t)((uint32_t)leaf[(size_t)t * g.P + p] & b.leaf_mask);
     const double lp = f.leaf_prob[L];
     if (!(lp >= 0.95)) return;                                             // :805
     const uint32_t v0 = f.leaf_info[L].vote_start, n = f.leaf_info[L].n_votes;
@@ -2091,8 +2098,10 @@ __global__ void __launch_bounds__(256) hough_image_kernel(FrameBuffers b, Geomet
     const uint32_t valtoadd = (uint32_t)(uint16_t)(__double2ull_rz(__dmul_rn(255.0, lp)) / n);  // :807-808
     const uint32_t gx = p % g.npx, gy = p / g.npx;
     const uint32_t x = g.left_w + gx * g.stride, y = g.left_h + gy * g.stride;
+    const size_t frame_px = (size_t)g.w * g.h;
+    acc += (size_t)frame * frame_px;
     float p3[3];
-    img_to_space(g.Kinv, (float)x, (float)y, (float)b.depth[(size_t)y * g.w + x], p3);
+    img_to_space(g.Kinv, (float)x, (float)y, (float)b.depth[(size_t)frame * frame_px + (size_t)y * g.w + x], p3);
     for (uint32_t k = 0; k < n; ++k) {
         float np[3], p2[2];
         const float4 o = f.offsets[v0 + k];
@@ -2105,8 +2114,9 @@ __global__ void __launch_bounds__(256) hough_image_kernel(FrameBuffers b, Geomet
         atomicAdd(&acc[(size_t)ny * g.w + nx], valtoadd);
     }
 }
-__global__ void narrow_u16_kernel(const uint32_t* __restrict__ in, uint16_t* __restrict__ out, uint32_t n) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+// the raw vote image: the low 16 bits of the u32 sums
+__global__ void narrow_u16_kernel(const uint32_t* __restrict__ in, uint16_t* __restrict__ out, size_t n) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = (uint16_t)(in[i] & 0xffffu);
 }
 
@@ -2116,22 +2126,27 @@ __global__ void narrow_u16_kernel(const uint32_t* __restrict__ in, uint16_t* __r
 // coordinate is clamped to the image; the result is stored as u16 by truncation with saturation
 // (Clamp<f32> for u16).  One thread per output pixel; the pixels a block's outputs need are staged
 // in shared memory (a row segment of 128 + 2r pixels, or a column segment of 32 + 2r rows x 32 columns).
+// The frame is blockIdx.z.  The horizontal pass reads the u32 vote sums and narrows them to u16 on
+// the load, so the blurred path has no separate narrowing pass.
 __device__ __forceinline__ uint16_t clamp_f32_u16(float x) {
     if (x < 65535.0f) return x > 0.0f ? (uint16_t)__float2uint_rz(x) : (uint16_t)0;
     return 65535;
 }
 constexpr int kBlurHx = 128, kBlurHy = 4;   // horizontal pass: outputs per block
 constexpr int kBlurVx = 32, kBlurVy = 32;   // vertical pass
-__global__ void __launch_bounds__(kBlurHx * kBlurHy) blur_h_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, uint32_t w,
+__global__ void __launch_bounds__(kBlurHx * kBlurHy) blur_h_kernel(const uint32_t* __restrict__ in, uint16_t* __restrict__ out, uint32_t w,
                                                                     uint32_t h, const float* __restrict__ k, int radius) {
     extern __shared__ uint16_t s_px[];  // [kBlurHy][kBlurHx + 2 radius]
     const int span = kBlurHx + 2 * radius;
     const int x0 = (int)blockIdx.x * kBlurHx, y = (int)(blockIdx.y * kBlurHy + threadIdx.y);
+    const size_t frame_px = (size_t)w * h;
+    in += blockIdx.z * frame_px;
+    out += blockIdx.z * frame_px;
     uint16_t* row = s_px + threadIdx.y * span;
     if (y < (int)h)
         for (int i = threadIdx.x; i < span; i += kBlurHx) {
             const int xs = min(max(x0 + i - radius, 0), (int)w - 1);
-            row[i] = in[(size_t)y * w + xs];
+            row[i] = (uint16_t)(in[(size_t)y * w + xs] & 0xffffu);
         }
     __syncthreads();
     const int x = x0 + (int)threadIdx.x;
@@ -2140,11 +2155,20 @@ __global__ void __launch_bounds__(kBlurHx * kBlurHy) blur_h_kernel(const uint16_
     for (int i = 0; i <= 2 * radius; ++i) acc = __fadd_rn(acc, __fmul_rn((float)row[threadIdx.x + i], __ldg(k + i)));
     out[(size_t)y * w + x] = clamp_f32_u16(acc);
 }
+// out: the blurred image (nullptr: not written).  keys != nullptr: the arg-max of
+// predict_parameter_from2dhough (prediction.rs:343-367) rides along: Iterator::max_by_key over the
+// pixels in index order returns the LAST of equal maxima, which is the largest
+// (value << 32) | pixel index; every block folds its pixels to one such key and the frame's key is
+// the 64-bit atomicMax over the blocks (keys[frame] starts at 0, below every pixel's key).
 __global__ void __launch_bounds__(kBlurVx * kBlurVy) blur_v_kernel(const uint16_t* __restrict__ in, uint16_t* __restrict__ out, uint32_t w,
-                                                                    uint32_t h, const float* __restrict__ k, int radius) {
+                                                                    uint32_t h, const float* __restrict__ k, int radius,
+                                                                    unsigned long long* __restrict__ keys) {
     extern __shared__ uint16_t s_px[];  // [kBlurVy + 2 radius][kBlurVx]
+    __shared__ unsigned long long s_key[kBlurVx * kBlurVy / 32];
     const int span = kBlurVy + 2 * radius;
     const int x = (int)(blockIdx.x * kBlurVx + threadIdx.x), y0 = (int)blockIdx.y * kBlurVy;
+    const size_t frame_px = (size_t)w * h;
+    in += blockIdx.z * frame_px;
     if (x < (int)w)
         for (int i = threadIdx.y; i < span; i += kBlurVy) {
             const int ys = min(max(y0 + i - radius, 0), (int)h - 1);
@@ -2152,41 +2176,50 @@ __global__ void __launch_bounds__(kBlurVx * kBlurVy) blur_v_kernel(const uint16_
         }
     __syncthreads();
     const int y = y0 + (int)threadIdx.y;
-    if (y >= (int)h || x >= (int)w) return;
-    float acc = 0.0f;
-    for (int i = 0; i <= 2 * radius; ++i) acc = __fadd_rn(acc, __fmul_rn((float)s_px[(threadIdx.y + i) * kBlurVx + threadIdx.x], __ldg(k + i)));
-    out[(size_t)y * w + x] = clamp_f32_u16(acc);
-}
-// predict_parameter_from2dhough (prediction.rs:343-367): Iterator::max_by_key over the pixels in
-// index order — the LAST of equal maxima wins — then z = the depth at that pixel and the
-// back-projection of (x, y, z); rotation 0, bounding box 0.
-__global__ void __launch_bounds__(1024) hough2d_argmax_kernel(const uint16_t* __restrict__ hough, const uint16_t* __restrict__ depth,
-                                                              uint32_t w, uint32_t h, Geometry g, dh_result* __restrict__ out) {
-    __shared__ uint32_t s_val[32], s_idx[32];
-    const uint32_t n = w * h, tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    uint32_t bv = 0, bi = 0;  // every pixel compares >= against pixel 0, as the fold does
-    for (uint32_t i = tid; i < n; i += 1024u) {
-        const uint32_t v = hough[i];
-        if (v > bv || (v == bv && i > bi)) { bv = v; bi = i; }
+    const bool inside = y < (int)h && x < (int)w;
+    unsigned long long key = 0;
+    if (inside) {
+        float acc = 0.0f;
+        for (int i = 0; i <= 2 * radius; ++i) acc = __fadd_rn(acc, __fmul_rn((float)s_px[(threadIdx.y + i) * kBlurVx + threadIdx.x], __ldg(k + i)));
+        const uint16_t v = clamp_f32_u16(acc);
+        const uint32_t idx = (uint32_t)y * w + (uint32_t)x;
+        if (out) out[blockIdx.z * frame_px + idx] = v;
+        key = ((unsigned long long)v << 32) | idx;
     }
+    if (!keys) return;
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) {
-        const uint32_t ov = __shfl_xor_sync(0xffffffffu, bv, d), oi = __shfl_xor_sync(0xffffffffu, bi, d);
-        if (ov > bv || (ov == bv && oi > bi)) { bv = ov; bi = oi; }
+        const unsigned long long o = __shfl_xor_sync(0xffffffffu, key, d);
+        key = o > key ? o : key;
     }
-    if (lane == 0) { s_val[warp] = bv; s_idx[warp] = bi; }
+    const uint32_t tid = threadIdx.y * kBlurVx + threadIdx.x;
+    if ((tid & 31u) == 0) s_key[tid >> 5] = key;
     __syncthreads();
-    if (tid == 0) {
-        for (int i = 1; i < 32; ++i)
-            if (s_val[i] > bv || (s_val[i] == bv && s_idx[i] > bi)) { bv = s_val[i]; bi = s_idx[i]; }
-        const uint32_t x = bi % w, y = bi / w;
-        float p[3];
-        img_to_space(g.Kinv, (float)x, (float)y, (float)depth[(size_t)y * w + x], p);
-        out->mid_point[0] = p[0]; out->mid_point[1] = p[1]; out->mid_point[2] = p[2];
-        out->_pad = 0;
-        out->rotation[0] = out->rotation[1] = out->rotation[2] = 0.0;
-        out->bounding_box[0] = out->bounding_box[1] = out->bounding_box[2] = out->bounding_box[3] = 0;
+    if (tid < 32) {
+        key = s_key[tid];
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            const unsigned long long o = __shfl_xor_sync(0xffffffffu, key, d);
+            key = o > key ? o : key;
+        }
+        if (tid == 0) atomicMax(keys + blockIdx.z, key);
     }
+}
+// predict_parameter_from2dhough (prediction.rs:343-367) from the frames' arg-max keys: z = the
+// depth at that pixel and the back-projection of (x, y, z); rotation 0, bounding box 0.  One thread per frame.
+__global__ void hough2d_pose_kernel(const unsigned long long* __restrict__ keys, const uint16_t* __restrict__ depth, Geometry g,
+                                    uint32_t n_frames, dh_result* __restrict__ out) {
+    const uint32_t frame = blockIdx.x * blockDim.x + threadIdx.x;
+    if (frame >= n_frames) return;
+    const uint32_t w = g.w, bi = (uint32_t)(keys[frame] & 0xffffffffull);
+    const uint32_t x = bi % w, y = bi / w;
+    float p[3];
+    img_to_space(g.Kinv, (float)x, (float)y, (float)depth[(size_t)frame * w * g.h + (size_t)y * w + x], p);
+    dh_result& r = out[frame];
+    r.mid_point[0] = p[0]; r.mid_point[1] = p[1]; r.mid_point[2] = p[2];
+    r._pad = 0;
+    r.rotation[0] = r.rotation[1] = r.rotation[2] = 0.0;
+    r.bounding_box[0] = r.bounding_box[1] = r.bounding_box[2] = r.bounding_box[3] = 0;
 }
 
 // ================================================================ Biwi run-length decode
@@ -2689,31 +2722,34 @@ void launch_leaf_gates(const double* leaf_prob, const uint32_t* vote_start, cons
                                                            box_out, rot_cells, n_leaves);
 }
 
-void launch_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint8_t* mask, cudaStream_t s) {
-    mask_kernel<<<(g.P + 255) / 256, 256, 0, s>>>(b, g, f.leaf_prob, mask);
+void launch_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint8_t* mask, cudaStream_t s) {
+    mask_kernel<<<dim3((g.P + 255) / 256, n_frames), 256, 0, s>>>(b, g, f.leaf_prob, mask);
 }
 
-void launch_hough_image(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t* acc32,
-                        uint16_t* out16, cudaStream_t s) {
+void launch_hough_votes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t* acc32, cudaStream_t s) {
     const uint32_t n = g.P * g.n_trees;
-    hough_image_kernel<<<(n + 255) / 256, 256, 0, s>>>(b, g, f, acc32);
-    const uint32_t px = g.w * g.h;
-    narrow_u16_kernel<<<(px + 255) / 256, 256, 0, s>>>(acc32, out16, px);
+    hough_image_kernel<<<dim3((n + 255) / 256, n_frames), 256, 0, s>>>(b, g, f, acc32);
 }
 
-// gaussian blur of a w x h u16 image: in -> tmp (horizontal) -> out (vertical); k: 2 * radius + 1 taps on the device
-int launch_gaussian_blur(const uint16_t* in, uint16_t* tmp, uint16_t* out, uint32_t w, uint32_t h, const float* k, int radius, cudaStream_t s) {
+void launch_narrow_u16(const uint32_t* acc32, uint16_t* out16, size_t n, cudaStream_t s) {
+    narrow_u16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(acc32, out16, n);
+}
+
+int launch_gaussian_blur(const uint32_t* in, uint16_t* tmp, uint16_t* out, unsigned long long* keys, uint32_t w, uint32_t h,
+                         uint32_t n_frames, const float* k, int radius, cudaStream_t s) {
     const uint32_t smem_h = (uint32_t)(kBlurHy * (kBlurHx + 2 * radius)) * 2u, smem_v = (uint32_t)((kBlurVy + 2 * radius) * kBlurVx) * 2u;
     static SmemConfig ch, cv;
     if (ch.raise(smem_h)) cudaFuncSetAttribute(blur_h_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h);
     if (cv.raise(smem_v)) cudaFuncSetAttribute(blur_v_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_v);
-    blur_h_kernel<<<dim3((w + kBlurHx - 1) / kBlurHx, (h + kBlurHy - 1) / kBlurHy), dim3(kBlurHx, kBlurHy), smem_h, s>>>(in, tmp, w, h, k, radius);
-    blur_v_kernel<<<dim3((w + kBlurVx - 1) / kBlurVx, (h + kBlurVy - 1) / kBlurVy), dim3(kBlurVx, kBlurVy), smem_v, s>>>(tmp, out, w, h, k, radius);
+    blur_h_kernel<<<dim3((w + kBlurHx - 1) / kBlurHx, (h + kBlurHy - 1) / kBlurHy, n_frames), dim3(kBlurHx, kBlurHy), smem_h, s>>>(
+        in, tmp, w, h, k, radius);
+    blur_v_kernel<<<dim3((w + kBlurVx - 1) / kBlurVx, (h + kBlurVy - 1) / kBlurVy, n_frames), dim3(kBlurVx, kBlurVy), smem_v, s>>>(
+        tmp, out, w, h, k, radius, keys);
     return 2;
 }
-void launch_hough2d_argmax(const uint16_t* hough, const uint16_t* depth, uint32_t w, uint32_t h, const Geometry& g, dh_result* out,
-                           cudaStream_t s) {
-    hough2d_argmax_kernel<<<1, 1024, 0, s>>>(hough, depth, w, h, g, out);
+void launch_hough2d_pose(const unsigned long long* keys, const uint16_t* depth, const Geometry& g, uint32_t n_frames, dh_result* out,
+                         cudaStream_t s) {
+    hough2d_pose_kernel<<<(n_frames + 127) / 128, 128, 0, s>>>(keys, depth, g, n_frames, out);
 }
 
 void launch_seq_guess(FrameState* fs, const dh_result* prev, uint32_t n, float min_seed_z, cudaStream_t s) {

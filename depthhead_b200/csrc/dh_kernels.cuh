@@ -138,12 +138,16 @@ uint32_t vote_box_dim();
 void launch_leaf_gates(const double* leaf_prob, const uint32_t* vote_start, const uint32_t* n_votes,
                        const float* offsets, const double* rotations, const uint32_t* rot_bins, LeafInfo* out,
                        LeafBox* box_out, uint32_t* rot_cells, uint32_t n_leaves, cudaStream_t s);
-void launch_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint8_t* mask, cudaStream_t s);
-void launch_hough_image(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t* acc32,
-                        uint16_t* out16, cudaStream_t s);
-int launch_gaussian_blur(const uint16_t* in, uint16_t* tmp, uint16_t* out, uint32_t w, uint32_t h, const float* k, int radius, cudaStream_t s);
-void launch_hough2d_argmax(const uint16_t* hough, const uint16_t* depth, uint32_t w, uint32_t h, const Geometry& g, dh_result* out,
-                           cudaStream_t s);
+// 2-D back ends over n_frames frames (grids carry the frame; per-frame images are [F][h][w])
+void launch_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint8_t* mask, cudaStream_t s);
+void launch_hough_votes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t* acc32, cudaStream_t s);
+void launch_narrow_u16(const uint32_t* acc32, uint16_t* out16, size_t n, cudaStream_t s);
+// gaussian blur of u32 vote sums narrowed to u16: in -> tmp (horizontal) -> out (vertical; nullptr = not written);
+// k: 2 * radius + 1 taps on the device; keys != nullptr: per-frame arg-max keys (zeroed by the caller)
+int launch_gaussian_blur(const uint32_t* in, uint16_t* tmp, uint16_t* out, unsigned long long* keys, uint32_t w, uint32_t h,
+                         uint32_t n_frames, const float* k, int radius, cudaStream_t s);
+void launch_hough2d_pose(const unsigned long long* keys, const uint16_t* depth, const Geometry& g, uint32_t n_frames, dh_result* out,
+                         cudaStream_t s);
 void launch_seq_guess(FrameState* fs, const dh_result* prev, uint32_t n, float min_seed_z, cudaStream_t s);
 void launch_counters(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, unsigned long long* out,
                      cudaStream_t s);

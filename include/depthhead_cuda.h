@@ -18,6 +18,8 @@
  *   src/hough/prediction.rs:760-841   build_hough_image (votes, before blur)   -> dh_hough_image_raw
  *   src/hough/prediction.rs:760-845   build_hough_image (with its blur)        -> dh_build_hough_image
  *   src/hough/prediction.rs:343-367   predict_parameter_from2dhough            -> dh_predict_from2dhough
+ *   the three above over n frames                                              -> dh_predict_mask_batch,
+ *                                                                                 dh_build_hough_image_batch
  *   src/db_reader/biwi.rs:81-103      read_depth (run-length coded depth file)  -> dh_biwi_depth_dims,
  *                                                                                 dh_biwi_decode_depth, dh_predict_batch_biwi
  *   src/db_reader/biwi.rs:27-60       read_cal (depth.cal -> IntrinsicMatrix)   -> dh_biwi_parse_cal
@@ -171,6 +173,18 @@ int dh_build_hough_image(dh_ctx* c, const dh_forest* f, const uint16_t* depth, u
 int dh_predict_from2dhough(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9],
                            dh_result* out);
 
+/* The three calls above over n independent frames [n][h][w] at depth_loc, through the same chunked
+ * pipeline as dh_predict_batch (device-resident or host frames; results equal to calling the
+ * single-frame entry points frame by frame).  Images go to [n][h][w] at mask_loc / hough_loc
+ * (DH_DEPTH_HOST or DH_DEPTH_DEVICE).  Synchronous; n = 0 is a successful no-op. */
+int dh_predict_mask_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                          int depth_loc, uint8_t* mask, int mask_loc);
+/* blur = 0: the raw vote image (dh_hough_image_raw); blur = 1: build_hough_image.  hough may be NULL
+ * (no image copied out); from2d (n results, host memory) may be NULL: predict_parameter_from2dhough
+ * per frame.  from2d needs blur = 1; hough and from2d both NULL is DH_E_ARG. */
+int dh_build_hough_image_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                               const float K[9], int depth_loc, int blur, uint16_t* hough, int hough_loc, dh_result* from2d);
+
 /* ------------------------------------------------------------------ Biwi Kinect Head Pose wire formats */
 /* read_depth (biwi.rs:81-103): u32 width, u32 height, then until width*height pixels are covered
  * [u32 n_empty][u32 n_full][n_full x u16], all little-endian; pixels of empty runs are 0.  The
@@ -274,7 +288,10 @@ int dh_forest_to_json(const dh_forest* f, char* buf, size_t cap, size_t* needed)
 
 /* ------------------------------------------------------------------ measurement */
 /* Per-stage device time (CUDA events on the context's stream) of the LAST dh_predict_batch call,
- * summed over its chunks, in milliseconds.  Order of stages: see DH_STAGE_*. */
+ * summed over its chunks, in milliseconds.  Order of stages: see DH_STAGE_*.  After the 2-D calls
+ * (dh_predict_mask*, dh_hough_image_raw, dh_build_hough_image*, dh_predict_from2dhough) H2D, SAT,
+ * TRAVERSE and D2H mean the same, and their whole back end (mask or vote image, blur, arg-max) is
+ * booked under DH_STAGE_VOTE; GATE and MEANSHIFT stay 0. */
 #define DH_STAGE_H2D 0
 #define DH_STAGE_SAT 1
 #define DH_STAGE_TRAVERSE 2
@@ -289,7 +306,8 @@ int dh_ctx_stage_ms(dh_ctx* c, float ms[DH_N_STAGES]);
  * [0] frames, [1] patches (all), [2] valid (non-background) patches, [3] patch*tree evals,
  * [4] node visits, [5] gate-passing patches, [6] hits (voting patch*tree pairs, both lists), [7] centre
  * votes cast, [8] rotation votes cast, [9] kernel launches, [10] mean-shift rounds run (both
- * accumulators), [11] accumulator-cube rebuilds. */
+ * accumulators), [11] accumulator-cube rebuilds.  After a 2-D call [0]-[4] and [9] are filled and
+ * the others are 0. */
 #define DH_N_COUNTERS 12
 int dh_ctx_counters(dh_ctx* c, uint64_t counters[DH_N_COUNTERS]);
 

@@ -77,6 +77,10 @@ extern "C" {
                             hough: *mut u16) -> c_int;
     fn dh_predict_from2dhough(c: *mut DhCtx, f: *const DhForest, depth: *const u16, w: u32, h: u32, k: *const f32,
                               out: *mut DhResult) -> c_int;
+    fn dh_predict_mask_batch(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32,
+                             depth_loc: c_int, mask: *mut u8, mask_loc: c_int) -> c_int;
+    fn dh_build_hough_image_batch(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32, k: *const f32,
+                                  depth_loc: c_int, blur: c_int, hough: *mut u16, hough_loc: c_int, from2d: *mut DhResult) -> c_int;
     // Biwi wire formats (src/db_reader/biwi.rs:27-103)
     fn dh_biwi_depth_dims(file: *const u8, len: usize, w: *mut u32, h: *mut u32) -> c_int;
     fn dh_biwi_decode_depth(c: *mut DhCtx, blob: *const u8, offsets: *const u64, n: u32, w: u32, h: u32,
@@ -259,6 +263,38 @@ impl HoughPrediction {
         self.push_fields()?;
         let mut out = vec![DhResult::default(); n as usize];
         check(unsafe { dh_predict_batch(self.context(), self.forest, frames.as_ptr(), n, w, h, k.ptr(), 0 /* DH_DEPTH_HOST */, out.as_mut_ptr()) })?;
+        Ok(out)
+    }
+    /// predict_mask of n independent frames back to back: masks [n][h][w] in frame order
+    pub fn predict_mask_batch(&self, frames: &[u16], n: u32, w: u32, h: u32) -> Result<Vec<u8>, Error> {
+        let px = (n as usize) * (w as usize) * (h as usize);
+        assert_eq!(frames.len(), px);
+        self.push_fields()?;
+        let mut out = vec![0u8; px];
+        check(unsafe { dh_predict_mask_batch(self.context(), self.forest, frames.as_ptr(), n, w, h, 0 /* DH_DEPTH_HOST */,
+                                             out.as_mut_ptr(), 0) })?;
+        Ok(out)
+    }
+    /// build_hough_image of n independent frames back to back: blurred vote images [n][h][w] in frame
+    /// order (blur = false: the vote images before the blur)
+    pub fn build_hough_image_batch(&self, frames: &[u16], n: u32, w: u32, h: u32, k: &IntrinsicMatrix, blur: bool)
+                                   -> Result<Vec<u16>, Error> {
+        let px = (n as usize) * (w as usize) * (h as usize);
+        assert_eq!(frames.len(), px);
+        self.push_fields()?;
+        let mut out = vec![0u16; px];
+        check(unsafe { dh_build_hough_image_batch(self.context(), self.forest, frames.as_ptr(), n, w, h, k.ptr(), 0 /* DH_DEPTH_HOST */,
+                                                  blur as c_int, out.as_mut_ptr(), 0, std::ptr::null_mut()) })?;
+        Ok(out)
+    }
+    /// predict_parameter_from2dhough of n independent frames back to back; results in frame order
+    pub fn predict_parameter_from2dhough_batch(&self, frames: &[u16], n: u32, w: u32, h: u32, k: &IntrinsicMatrix)
+                                               -> Result<Vec<DhResult>, Error> {
+        assert_eq!(frames.len(), (n as usize) * (w as usize) * (h as usize));
+        self.push_fields()?;
+        let mut out = vec![DhResult::default(); n as usize];
+        check(unsafe { dh_build_hough_image_batch(self.context(), self.forest, frames.as_ptr(), n, w, h, k.ptr(), 0 /* DH_DEPTH_HOST */,
+                                                  1, std::ptr::null_mut(), 0, out.as_mut_ptr()) })?;
         Ok(out)
     }
     /// n_seq independent sequences of frames_per_seq frames each (sequence-major): frame t of every
