@@ -198,6 +198,39 @@ def _as_frames(frames, device_ptr, n, w, h):
     return None, C.c_void_p(int(device_ptr)), capi.DH_DEPTH_DEVICE, int(n), int(w), int(h)
 
 
+def frame_args(n: int, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None) -> np.ndarray:
+    """capi.FRAME_ARGS_DTYPE[n] for dh_predict_frames.  intrinsics: one IntrinsicMatrix for every frame
+    or a float32 [n,3,3] array; midp_guess: float32 [n,3] mm, rot_guess: float64 [n,3] radians, or None;
+    has_midp / has_rot: bool [n] masks of the frames whose guess is used (None = every frame)."""
+    n = int(n)
+    args = np.zeros(n, capi.FRAME_ARGS_DTYPE)
+    if isinstance(intrinsics, IntrinsicMatrix):
+        args["K"] = intrinsics.mat.reshape(9)
+    else:
+        k = np.asarray(intrinsics)
+        if k.dtype != np.float32 or k.shape != (n, 3, 3):
+            raise ValueError("intrinsics must be an IntrinsicMatrix or a float32 [n,3,3] array (n = %d)" % n)
+        args["K"] = k.reshape(n, 9)
+    for bit, name, guess, dtype, has in ((1, "midp_guess", midp_guess, np.float32, has_midp),
+                                         (2, "rot_guess", rot_guess, np.float64, has_rot)):
+        if guess is None:
+            if has is not None:
+                raise ValueError("a mask for %s needs %s" % (name, name))
+            continue
+        g = np.asarray(guess)
+        if g.dtype != dtype or g.shape != (n, 3):
+            raise ValueError("%s must be a %s [n,3] array (n = %d)" % (name, np.dtype(dtype).name, n))
+        if has is None:
+            use = np.ones(n, bool)
+        else:
+            use = np.asarray(has)
+            if use.dtype != np.bool_ or use.shape != (n,):
+                raise ValueError("the mask of %s must be a bool [n] array (n = %d)" % (name, n))
+        args[name][use] = g[use]
+        args["has_guess"][use] |= bit
+    return args
+
+
 def _image_out(out_device_ptr, shape, dtype):
     """(host array or None, pointer, location) of a batch of images: a new host array, or the caller's device memory."""
     if out_device_ptr is None:
@@ -352,6 +385,21 @@ class HoughPrediction:
         out = np.zeros(int(n), capi.RESULT_DTYPE)
         capi.check(capi.load().dh_predict_batch(ctx._h, self._h, p, int(n), int(w), int(h), intrinsic._ptr(), loc,
                                                 capi.ptr(out)))
+        return out
+
+    def predict_frames(self, frames, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                       ctx: Context | None = None, device_ptr: int | None = None, n: int | None = None, w: int | None = None,
+                       h: int | None = None) -> np.ndarray:
+        """predict_parameter_parallel(img_i, K_i, midp_i, rot_i) for n independent frames in one call, equal to
+        predict_parameter_parallel frame by frame.  `frames`: [n,h,w] uint16 on the host, or device_ptr +
+        (n, w, h).  intrinsics: one IntrinsicMatrix or a float32 [n,3,3] array; midp_guess (float32 [n,3] mm)
+        and rot_guess (float64 [n,3] radians) may be None; has_midp / has_rot (bool [n]) pick the frames
+        whose guess is used (None = all).  Returns capi.RESULT_DTYPE[n]."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        args = frame_args(n, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+        ctx = ctx or default_context()
+        out = np.zeros(n, capi.RESULT_DTYPE)
+        capi.check(capi.load().dh_predict_frames(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(out)))
         return out
 
     def predict_sequences(self, frames, intrinsic: IntrinsicMatrix, min_seed_z: float = 500.0, ctx: Context | None = None,

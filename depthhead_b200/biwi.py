@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .api import Context, HoughPrediction, IntrinsicMatrix, default_context
+from .api import Context, HoughPrediction, IntrinsicMatrix, default_context, frame_args
 
 
 def encode_depth(img: np.ndarray) -> bytes:
@@ -121,14 +121,25 @@ def read_gt(data: bytes, intrinsic: IntrinsicMatrix) -> dict:
     return {"pos3d": p3, "pos2d": p2, "rot": rot}
 
 
-def predict_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w: int, h: int, intrinsic: IntrinsicMatrix,
-                  ctx: Context | None = None) -> np.ndarray:
+def predict_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w: int, h: int, intrinsic,
+                  ctx: Context | None = None, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None) -> np.ndarray:
     """read_depth + predict_parameter_parallel(img, K, None, None) per file
-    (examples/db_evaluate.rs:296), the decode on the GPU.  Returns capi.RESULT_DTYPE[n]."""
-    ctx = ctx or default_context()
+    (examples/db_evaluate.rs:296), the decode on the GPU.  Returns capi.RESULT_DTYPE[n].
+    intrinsic: one IntrinsicMatrix for every file, or a float32 [n,3,3] array with the K of every file
+    (a database of several sequence folders, each with its own depth.cal); with such an array or with
+    seeds (see HoughPrediction.predict_frames) every file is predicted with its own arguments."""
     n = len(offsets) - 1
+    per_frame = not isinstance(intrinsic, IntrinsicMatrix) or midp_guess is not None or rot_guess is not None
+    args = frame_args(n, intrinsic, midp_guess, rot_guess, has_midp, has_rot) if per_frame else None
+    if not per_frame and (has_midp is not None or has_rot is not None):
+        raise ValueError("a guess mask needs its guesses")
+    ctx = ctx or default_context()
     out = np.zeros(n, capi.RESULT_DTYPE)
     offsets = np.ascontiguousarray(offsets, np.uint64)
+    if per_frame:
+        capi.check(capi.load().dh_predict_frames_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
+                                                      capi.ptr(args), capi.ptr(out)))
+        return out
     capi.check(capi.load().dh_predict_batch_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
                                                  intrinsic._ptr(), capi.ptr(out)))
     return out

@@ -37,6 +37,12 @@ RESULT_DTYPE = np.dtype([("mid_point", np.float32, 3), ("_pad", np.uint32), ("ro
 assert RESULT_DTYPE.itemsize == C.sizeof(dh_result) == 56
 
 
+# dh_frame_args: the arguments of dh_predict for one frame of dh_predict_frames (80 bytes)
+FRAME_ARGS_DTYPE = np.dtype([("K", np.float32, 9), ("midp_guess", np.float32, 3), ("rot_guess", np.float64, 3),
+                             ("has_guess", np.uint32), ("_pad", np.uint32)], align=True)
+assert FRAME_ARGS_DTYPE.itemsize == 80
+
+
 class dh_split_stats(C.Structure):
     _fields_ = [("n", C.c_uint32 * 2), ("n_pos", C.c_uint32 * 2), ("det_off", C.c_double * 2), ("det_rot", C.c_double * 2),
                 ("impurity", C.c_double)]
@@ -108,6 +114,8 @@ SIGNATURES = {
     "dh_forest_to_json": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
     "dh_predict_mask": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp]),
     "dh_predict_sequences": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, _u32, _vp, C.c_int, _f32, _vp]),
+    "dh_predict_frames": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, C.c_int, _vp, _vp]),
+    "dh_predict_frames_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp]),
     "dh_hough_image_raw": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "dh_build_hough_image": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "dh_predict_from2dhough": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, C.POINTER(dh_result)]),

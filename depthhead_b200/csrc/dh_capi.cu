@@ -52,6 +52,18 @@ int guarded(F&& body) {
         if (!(cond)) throw dh::ModelError(DH_E_ARG, msg); \
     } while (0)
 
+static_assert(sizeof(dh_frame_args) == 80 && offsetof(dh_frame_args, K) == 0 && offsetof(dh_frame_args, midp_guess) == 36 &&
+                  offsetof(dh_frame_args, rot_guess) == 48 && offsetof(dh_frame_args, has_guess) == 72 &&
+                  offsetof(dh_frame_args, _pad) == 76,
+              "dh_frame_args layout (mirrored by capi.FRAME_ARGS_DTYPE and the Rust shim)");
+
+void check_frame_args(const char* fn, const dh_frame_args* args, uint32_t n) {
+    for (uint32_t i = 0; i < n; ++i)
+        if (args[i].has_guess & ~3u)
+            throw dh::ModelError(DH_E_ARG, std::string(fn) + ": frame " + std::to_string(i) + " has has_guess " +
+                                               std::to_string(args[i].has_guess) + " (only bits 0 and 1 are defined)");
+}
+
 }  // namespace
 
 extern "C" {
@@ -234,6 +246,23 @@ int dh_predict_batch_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, co
     return guarded([&] {
         REQUIRE(c && f && K && (n == 0 || (blob && offsets && out)), "dh_predict_batch_biwi: NULL argument");
         c->cx->predict_batch_biwi(*f->hf, blob, offsets, n, w, h, K, out);
+    });
+}
+int dh_predict_frames(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                      const dh_frame_args* args, dh_result* out) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_frames: bad depth_loc");
+        if (args) check_frame_args("dh_predict_frames", args, n);
+        REQUIRE(c && f && (n == 0 || (depth && args && out)), "dh_predict_frames: NULL argument");
+        c->cx->predict_frames(*f->hf, depth, nullptr, nullptr, n, w, h, depth_loc, args, out);
+    });
+}
+int dh_predict_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
+                           uint32_t h, const dh_frame_args* args, dh_result* out) {
+    return guarded([&] {
+        if (args) check_frame_args("dh_predict_frames_biwi", args, n);
+        REQUIRE(c && f && (n == 0 || (blob && offsets && args && out)), "dh_predict_frames_biwi: NULL argument");
+        c->cx->predict_frames(*f->hf, nullptr, blob, offsets, n, w, h, DH_DEPTH_HOST, args, out);
     });
 }
 size_t dh_biwi_encode_bound(uint32_t w, uint32_t h) { return dh::rle_frame_bound(w, h); }

@@ -132,6 +132,8 @@ Context::~Context() {
     if (h_counters_) cudaFreeHost(h_counters_);
     if (h_results_) cudaFreeHost(h_results_);
     if (h_result1_) cudaFreeHost(h_result1_);
+    if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
+    if (h_frame_k_) cudaFreeHost(h_frame_k_);
     pool_.reset();
     for (int i = 0; i < kEncSlots; ++i) {
         if (h_enc_[i]) cudaFreeHost(h_enc_[i]);
@@ -435,6 +437,7 @@ void Context::free_lane(Lane& L) {
     dev_free(L.cubes);
     dev_free(L.grids);
     dev_free(L.fs);
+    dev_free(L.frame_k);
     dev_free(L.results);
     dev_free(L.ms_trace);
     dev_free(L.img32);
@@ -481,6 +484,7 @@ void Context::alloc_lane(Lane& L) {
     L.cubes_clean = true;
     dev_alloc(L.grids, F * (size_t)(kPosGridCells + kRotGridCells));
     dev_alloc(L.fs, F);
+    dev_alloc(L.frame_k, F * 18);
     dev_alloc(L.results, F);
     if (sk_.trace_iters) dev_alloc(L.ms_trace, F * 2 * (size_t)sk_.trace_iters * 3);
     if (g.P) {
@@ -700,10 +704,31 @@ void Context::mark(int stage_begin_of) {
 // ------------------------------------------------------------------------------------------------ one pass
 // Front end shared by every entry point: SAT + traversal (+ zeroed per-frame state).
 void Context::run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameState* guess_state, const dh_result* prev_results,
-                        float min_seed_z) {
+                        float min_seed_z, const dh_frame_args* args, uint32_t f0) {
     const Geometry& g = geom_;
     cudaStream_t st = L.stream;
-    DH_CUDA(cudaMemsetAsync(L.fs, 0, sizeof(FrameState) * n, st));
+    if (args) {
+        // per-frame arguments: the pass's frame states (zero but for the seeds, as dh_predict's) and
+        // every frame's K, K^-1 (as ensure_scratch computes them for one matrix) replace the memset.
+        // Frames keep their index in the batch, so the staging of a chunk is never reused in the call.
+        FrameState* hfs = h_frame_fs_ + f0;
+        float* hk = h_frame_k_ + (size_t)f0 * 18;
+        std::memset(hfs, 0, sizeof(FrameState) * n);
+        for (uint32_t i = 0; i < n; ++i) {
+            const dh_frame_args& a = args[f0 + i];
+            hfs[i].has_guess = a.has_guess;
+            if (a.has_guess & 1u)
+                for (int k = 0; k < 3; ++k) hfs[i].midp_guess[k] = a.midp_guess[k];
+            if (a.has_guess & 2u)
+                for (int k = 0; k < 3; ++k) hfs[i].rot_guess[k] = a.rot_guess[k];
+            std::memcpy(hk + (size_t)i * 18, a.K, sizeof(float) * 9);
+            mat3_inverse_f32(a.K, hk + (size_t)i * 18 + 9);
+        }
+        DH_CUDA(cudaMemcpyAsync(L.fs, hfs, sizeof(FrameState) * n, cudaMemcpyHostToDevice, st));
+        DH_CUDA(cudaMemcpyAsync(L.frame_k, hk, sizeof(float) * 18 * n, cudaMemcpyHostToDevice, st));
+    } else {
+        DH_CUDA(cudaMemsetAsync(L.fs, 0, sizeof(FrameState) * n, st));
+    }
     DH_CUDA(cudaMemsetAsync(L.grids, 0, sizeof(uint32_t) * (size_t)(kPosGridCells + kRotGridCells) * n, st));
     if (guess_state) {
         *h_fs_ = *guess_state;
@@ -737,20 +762,20 @@ void Context::run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameS
     }
 }
 
-void Context::run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iterations) {
+void Context::run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iterations, const float* frame_k) {
     const Geometry& g = geom_;
     cudaStream_t st = L.stream;
     mark(DH_STAGE_GATE);
     // small passes (single frames, the passes of seeded sequences) are bound by the chain of launches: they keep the
     // patch gate inside the seed-grid kernel (one launch less; 0.168 instead of 0.187 ms per single frame)
-    launches_ += (uint64_t)launch_gate_coarse(b, g, fdev_, n, gate_split_ && n >= gate_split_min_, n_sms_, st);
+    launches_ += (uint64_t)launch_gate_coarse(b, g, fdev_, n, gate_split_ && n >= gate_split_min_, n_sms_, st, frame_k);
     stage_check("gate + coarse grids");
     mark(DH_STAGE_VOTE);
     // the accumulator cubes of this pass start empty: either the previous pass's mean-shift CTAs
     // cleared them behind themselves, or they are cleared here
     if (iterations && !L.cubes_clean) DH_CUDA(cudaMemsetAsync(L.cubes, 0, sizeof(uint32_t) * 2 * (size_t)vote_box_cells() * n, st));
     if (iterations) L.cubes_clean = false;
-    launches_ += (uint64_t)launch_seed_and_cubes(b, g, fdev_, n, iterations, st);
+    launches_ += (uint64_t)launch_seed_and_cubes(b, g, fdev_, n, iterations, st, frame_k);
     stage_check("seeds + accumulator cubes");
     mark(DH_STAGE_MEANSHIFT);
     launches_ += (uint64_t)launch_meanshift(b, g, fdev_, n, iterations, n_sms_, st);
@@ -890,6 +915,18 @@ void Context::predict_batch_biwi(const HostForest& hf, const uint8_t* blob, cons
     run_batch(hf, nullptr, blob, offsets, n, w, h, K, DH_DEPTH_HOST, be);
 }
 
+// dh_predict_frames / dh_predict_frames_biwi: the pose pipeline of dh_predict_batch, every frame with
+// the arguments of its own dh_predict call.  The kernels that project read the frame's K, K^-1 from
+// the lane's table (Lane::frame_k); the call's matrix in Geometry (frame 0's) is not used.
+void Context::predict_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                             uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out) {
+    static const float kIdentity[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+    BackEnd be;
+    be.results = out;
+    be.args = args;
+    run_batch(hf, depth, blob, offsets, n, w, h, n ? args[0].K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
+}
+
 // Device copies of the file offsets and room for the compressed bytes of one chunk per slot.
 void Context::ensure_biwi(const uint64_t* offsets, uint32_t n, uint32_t chunk, int slots) {
     for (uint32_t i = 0; i < n; ++i) {
@@ -1008,6 +1045,7 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
     ensure_results(n);  // pinned staging for the results
+    if (be.args) ensure_frame_args(n);
     if (depth_loc != DH_DEPTH_DEVICE) ensure_staging(2);
     if (blob) ensure_biwi(offsets, n, F, 2);
     // fork: the other lanes (and the copy stream) start after everything already queued on the caller's stream
@@ -1018,7 +1056,7 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
         const uint32_t f0 = c * F, nc = std::min<uint32_t>(F, n - f0);
         FrameBuffers b = buffers(L, d_depth);
         flush_pending(L);
-        run_front(L, b, nc, nullptr);
+        run_front(L, b, nc, nullptr, nullptr, 0.0f, be.args, f0);
         run_chunk_back(L, b, f0, nc, iterations, be);
     };
     if (depth_loc == DH_DEPTH_DEVICE) {
@@ -1084,6 +1122,19 @@ void Context::ensure_results(uint32_t n) {
         DH_CUDA(cudaHostAlloc((void**)&h_results_, sizeof(dh_result) * n, cudaHostAllocDefault));
         h_results_cap_ = n;
     }
+}
+
+// pinned staging of the per-frame arguments of a dh_predict_frames batch (run_front packs it chunk by chunk)
+void Context::ensure_frame_args(uint32_t n) {
+    if (h_frame_cap_ >= n) return;
+    if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
+    if (h_frame_k_) cudaFreeHost(h_frame_k_);
+    h_frame_fs_ = nullptr;
+    h_frame_k_ = nullptr;
+    h_frame_cap_ = 0;
+    DH_CUDA(cudaHostAlloc((void**)&h_frame_fs_, sizeof(FrameState) * n, cudaHostAllocDefault));
+    DH_CUDA(cudaHostAlloc((void**)&h_frame_k_, sizeof(float) * 18 * (size_t)n, cudaHostAllocDefault));
+    h_frame_cap_ = n;
 }
 
 // ------------------------------------------------------------------------------------------------ compressed host input
@@ -1171,6 +1222,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
     ensure_results(n);
+    if (be.args) ensure_frame_args(n);
     ensure_staging(hybrid ? 4 : 2);
     ensure_encode(n, F);
     const size_t bound = enc_frame_bound_;
@@ -1223,7 +1275,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
         const uint32_t f0 = c * F, nc = std::min<uint32_t>(F, n - f0);
         FrameBuffers b = buffers(L, d_depth_[slot]);
         flush_pending(L);
-        run_front(L, b, nc, nullptr);
+        run_front(L, b, nc, nullptr, nullptr, 0.0f, be.args, f0);
         run_chunk_back(L, b, f0, nc, iterations, be);
         DH_CUDA(cudaEventRecord(ev_consumed_[slot], L.stream));
         ++done_chunks;
@@ -1514,7 +1566,7 @@ void Context::run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
         run_image_back(L, b, f0, n, be);
         return;
     }
-    run_back(L, b, n, iterations);
+    run_back(L, b, n, iterations, be.args ? L.frame_k : nullptr);
     DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
 }
 

@@ -32,6 +32,7 @@ struct Lane {
     float4* gated = nullptr;        // [F][P]
     uint32_t* grids = nullptr;      // [F][400 + 8000]
     FrameState* fs = nullptr;       // [F]
+    float* frame_k = nullptr;       // [F][18] K, K^-1 of every frame of a dh_predict_frames pass
     dh_result* results = nullptr;   // [F]
     int32_t* ms_trace = nullptr;    // [F][2][iters][3] (debug export)
     uint32_t* cubes = nullptr;      // [F][2][kBox^3]
@@ -55,6 +56,8 @@ constexpr int kMaxLanes = 4;
 struct BackEnd {
     enum Kind { kPose, kMask, kVotes, kBlurred } kind = kPose;
     dh_result* results = nullptr;  // kPose: poses [n]; kBlurred: from2d poses [n] or nullptr (host memory)
+    const dh_frame_args* args = nullptr;  // kPose: intrinsics and seeds of every frame [n] (host memory), or nullptr:
+                                          // the call's one K and no seeds
     void* image = nullptr;         // kMask: u8 [n][h][w]; kVotes / kBlurred: u16 [n][h][w] (kBlurred: may be nullptr)
     bool image_on_device = false;  // image points to device memory on the context's GPU
 };
@@ -105,6 +108,9 @@ public:
     void biwi_decode(const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h, uint16_t* out, int out_loc);
     void predict_batch_biwi(const HostForest& hf, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h,
                             const float K[9], dh_result* out);
+    // dh_predict for every frame with its own arguments: depth at depth_loc, or Biwi files (blob != nullptr)
+    void predict_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                        uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out);
     // training: split scoring (dh_train.cu; houghforest.rs:250-295)
     TrainSet* trainset_create(const uint16_t* patches, uint64_t n, uint32_t sw, uint32_t sh, uint32_t rw, uint32_t rh,
                               const uint8_t* is_object, const float* offsets, const double* rotations);
@@ -156,6 +162,7 @@ private:
     void run_batch_encoded(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
                            const BackEnd& be);
     void ensure_results(uint32_t n);
+    void ensure_frame_args(uint32_t n);
     void ensure_image_scratch(int n_lanes);
     void ensure_blur_taps(const HostForest& hf);
     // after run_front: the chunk's back end and the copies of its results (frames f0 .. f0 + n - 1 of the batch)
@@ -165,9 +172,10 @@ private:
     void free_scratch();
     TilePlan plan_tiles(const Geometry& g) const;
     FrameBuffers buffers(const Lane& L, const uint16_t* depth) const;
+    // args: per-frame arguments of the batch (frames f0 .. f0 + n - 1 are this pass's) or nullptr
     void run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameState* guess_state, const dh_result* prev_results = nullptr,
-                   float min_seed_z = 0.0f);
-    void run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iterations);
+                   float min_seed_z = 0.0f, const dh_frame_args* args = nullptr, uint32_t f0 = 0);
+    void run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iterations, const float* frame_k = nullptr);
     void begin_call();
     void end_call();
     cudaEvent_t next_event();
@@ -259,6 +267,10 @@ private:
     dh_result* h_results_ = nullptr;      // batch results (grows with the batch; never referenced by a captured graph)
     size_t h_results_cap_ = 0;
     dh_result* h_result1_ = nullptr;      // dh_predict's own fixed slot: the D2H copy node of its CUDA graph targets it
+    // dh_predict_frames: every frame's FrameState (seeds) and K, K^-1, packed per chunk (grows with the batch)
+    FrameState* h_frame_fs_ = nullptr;
+    float* h_frame_k_ = nullptr;
+    size_t h_frame_cap_ = 0;
 
     // dh_predict as a CUDA graph: the single-frame pipeline is a dozen small launches, i.e. bound
     // by launch overhead; after one eager call with a given (model, shape, intrinsics, stream) the

@@ -1004,11 +1004,21 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
 constexpr int kGateThreads = 512;   // 3 CTAs of 59 KB per SM: 48 warps (256 threads with 48 KB: 32 warps)
 constexpr int kTouchedCap = 1024;
 
+// Per-frame intrinsics (dh_predict_frames): the kernels of the pose path take a table [F][18] of
+// every frame's K then K^-1 (kFrameK instantiations) instead of Geometry's one matrix.  A CTA
+// works on one frame: patch_gate_kernel and seed_kernel load the matrix into registers once per
+// thread, gate_coarse_kernel keeps it in shared memory (see there).
+constexpr int kFrameKFloats = 18;
+__device__ __forceinline__ void load_mat3(const float* __restrict__ src, float m[9]) {
+#pragma unroll
+    for (int k = 0; k < 9; ++k) m[k] = __ldg(src + k);
+}
+
 // 2-D projection of one centre vote onto the 20x20 seed grid (prediction.rs:661-675)
-__device__ __forceinline__ uint32_t coarse_pos_cell(const Geometry& g, float nx, float ny, float nz) {
+__device__ __forceinline__ uint32_t coarse_pos_cell(const Geometry& g, const float* K, float nx, float ny, float nz) {
     const float np[3] = {nx, ny, nz};
     float p2[2];
-    space_to_img(g.K, np, p2);  // prediction.rs:661
+    space_to_img(K, np, p2);  // prediction.rs:661
     // max!/min! macros (prediction.rs:19-25): plain comparisons, NaN -> 0.0
     const float mx = (p2[0] > 0.0f) ? p2[0] : 0.0f;
     const float x2d = (mx < (float)(g.w - 1)) ? mx : (float)(g.w - 1);
@@ -1097,7 +1107,9 @@ constexpr int kPatchGateThreads = 256;
 constexpr int kPatchGatePer = 4;  // patches per thread (one: 0.15 ms per 1024 frames of configs[1], four: 0.10 ms).  The kernel
                                   // sits at a third of the HBM rate; loading every leaf word of a patch up front,
                                   // background or not, to save dependent round trips was slower (it reads 40 % more)
-__global__ void __launch_bounds__(kPatchGateThreads) patch_gate_kernel(FrameBuffers b, Geometry g, ForestDev f) {
+template <bool kFrameK>
+__global__ void __launch_bounds__(kPatchGateThreads) patch_gate_kernel(FrameBuffers b, Geometry g, ForestDev f,
+                                                                       const float* __restrict__ frame_k) {
     const uint32_t frame = blockIdx.y, lane = threadIdx.x & 31u;
     const uint32_t T = g.n_trees;
     const int32_t* leaf_f = b.leaf + (size_t)frame * T * g.P;
@@ -1165,13 +1177,15 @@ __global__ void __launch_bounds__(kPatchGateThreads) patch_gate_kernel(FrameBuff
     uint32_t base = 0;
     if (lane == 0) base = atomicAdd(&b.fs[frame].n_gate, total);  // one reservation per warp
     base = __shfl_sync(0xffffffffu, base, 0);
+    float kinv[9];
+    if (kFrameK) load_mat3(frame_k + (size_t)frame * kFrameKFloats + 9, kinv);
 #pragma unroll
     for (int k = 0; k < kPatchGatePer; ++k) {
         if (gate[k]) {
             const uint32_t gx = p[k] % g.npx, gy = p[k] / g.npx;
             const uint32_t x = g.left_w + gx * g.stride, y = g.left_h + gy * g.stride;
             float p3[3];
-            img_to_space(g.Kinv, (float)x, (float)y, (float)z[k], p3);  // prediction.rs:554
+            img_to_space(kFrameK ? kinv : g.Kinv, (float)x, (float)y, (float)z[k], p3);  // prediction.rs:554
             b.gated[(size_t)frame * g.P + base + __popc(m[k] & ((1u << lane) - 1u))] = make_float4(p3[0], p3[1], p3[2], __uint_as_float(p[k]));
             if (b.p3) {
                 float* o = b.p3 + ((size_t)frame * g.P + p[k]) * 3;
@@ -1189,13 +1203,18 @@ __global__ void __launch_bounds__(kPatchGateThreads) patch_gate_kernel(FrameBuff
 // instead of gating the kGateThreads patches of its own index range, so that every CTA that runs
 // has a full slice behind the fixed costs of its seed grids (clearing and flushing 8400 cells);
 // CTAs beyond the end of the list leave at once.
-template <bool kFused, bool kFromList>
-__global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffers b, Geometry g, ForestDev f) {
+// kFrameK: the frame's K (and, in phase A, K^-1) come from frame_k instead of g, copied once per CTA
+// into 72 bytes of shared memory behind the other arrays: this kernel runs at the 40-register cap of
+// 3 CTAs of 512 threads per SM, and 9 more live registers spilled.
+template <bool kFused, bool kFromList, bool kFrameK>
+__global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffers b, Geometry g, ForestDev f,
+                                                                      const float* __restrict__ frame_k) {
     extern __shared__ __align__(16) uint8_t gate_smem[];
     float4* s_gated = reinterpret_cast<float4*>(gate_smem);                                   // [kGateThreads] p3 + patch index of the CTA's gated patches
     PairSlot(*s_slots)[32] = reinterpret_cast<PairSlot(*)[32]>(gate_smem + kGateThreads * 16);  // [warps][32] vote spreading, one set per warp
     uint32_t* s_grid = reinterpret_cast<uint32_t*>(gate_smem + kGateThreads * 16 + (kGateThreads / 32) * 32 * 32);  // [0,400) centre, [400,8400) rotation
     uint16_t* s_touched = reinterpret_cast<uint16_t*>(s_grid + kPosGridCells + kRotGridCells);  // rotation cells this CTA made non-zero
+    float* s_k = reinterpret_cast<float*>(gate_smem + kGateSmemBytes);  // kFrameK: the frame's K then K^-1
     __shared__ uint32_t s_ngate, s_base, s_ntouched, s_next;
     const uint32_t frame = blockIdx.y, tid = threadIdx.x, lane = tid & 31u;
     const uint32_t p = blockIdx.x * kGateThreads + tid;
@@ -1212,6 +1231,7 @@ __global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffe
         s_ntouched = 0;
         s_next = 0;
     }
+    if (kFrameK && tid < (uint32_t)kFrameKFloats) s_k[tid] = __ldg(frame_k + (size_t)frame * kFrameKFloats + tid);
     if (kFromList)
         for (int i = tid; i < kPosGridCells + kRotGridCells; i += kGateThreads) s_grid[i] = 0;
     __syncthreads();
@@ -1245,7 +1265,7 @@ __global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffe
                 const uint32_t gx = p % g.npx, gy = p / g.npx;
                 const uint32_t x = g.left_w + gx * g.stride, y = g.left_h + gy * g.stride;
                 const uint16_t z = b.depth[((size_t)frame * g.h + y) * g.w + x];  // prediction.rs:551
-                img_to_space(g.Kinv, (float)x, (float)y, (float)z, p3);           // prediction.rs:554
+                img_to_space(kFrameK ? s_k + 9 : g.Kinv, (float)x, (float)y, (float)z, p3);  // prediction.rs:554
                 if (b.p3) {
                     float* o = b.p3 + ((size_t)frame * g.P + p) * 3;
                     o[0] = p3[0]; o[1] = p3[1]; o[2] = p3[2];
@@ -1307,7 +1327,7 @@ __global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffe
             auto centre_vote = [&](uint32_t vote, uint32_t ow, const float4& c) {
                 const float4 o = __ldg(f.offsets + vote);
                 const float nx = __fsub_rn(c.x, o.x), ny = __fsub_rn(c.y, o.y), nz = __fsub_rn(c.z, o.z);
-                if (!(nz < 0.0f)) atomicAdd(&s_grid[coarse_pos_cell(g, nx, ny, nz)], ow);
+                if (!(nz < 0.0f)) atomicAdd(&s_grid[coarse_pos_cell(g, kFrameK ? s_k : g.K, nx, ny, nz)], ow);
             };
             // rotation votes -> 20^3 grid; rough = r * 20 / 120 per axis (prediction.rs:630-636), static per vote
             auto rot_vote = [&](uint32_t entry, uint32_t ow) {
@@ -1408,7 +1428,9 @@ __device__ Best block_argmax(const uint32_t* cells, int n, Best* s_red) {
     return r;
 }
 
-__global__ void __launch_bounds__(kSeedThreads) seed_kernel(FrameBuffers b, Geometry g, uint32_t iterations) {
+template <bool kFrameK>
+__global__ void __launch_bounds__(kSeedThreads) seed_kernel(FrameBuffers b, Geometry g, uint32_t iterations,
+                                                            const float* __restrict__ frame_k) {
     __shared__ Best s_red[kSeedThreads / 32];
     __shared__ unsigned long long s_sum[kSeedThreads / 32];
     __shared__ uint32_t s_cnt[kSeedThreads / 32];
@@ -1453,8 +1475,9 @@ __global__ void __launch_bounds__(kSeedThreads) seed_kernel(FrameBuffers b, Geom
         const float meanz = zc > 0 ? (float)__ddiv_rn((double)zs, (double)zc) : 0.0f;
         const float mxf = __fmul_rn(__fadd_rn((float)cgx, 0.5f), (float)gpw);  // :727-729
         const float myf = __fmul_rn(__fadd_rn((float)cgy, 0.5f), (float)gph);
-        float m3[3];
-        img_to_space(g.Kinv, mxf, myf, meanz, m3);
+        float m3[3], kinv[9];
+        if (kFrameK) load_mat3(frame_k + (size_t)frame * kFrameKFloats + 9, kinv);
+        img_to_space(kFrameK ? kinv : g.Kinv, mxf, myf, meanz, m3);
         for (int k = 0; k < 3; ++k) sm[k] = __float2int_rz(m3[k]);  // :750
         if (guessed & 1u)  // prediction.rs:437-441
             for (int k = 0; k < 3; ++k) sm[k] = __float2int_rz(fs->midp_guess[k]);
@@ -2657,14 +2680,15 @@ uint32_t vote_box_dim() { return (uint32_t)kBox; }
 
 // The back end after the traversal, in launch order.  The coarse grids, the accumulator cubes
 // and the queue header must be zero when these run.  Each returns the kernels it launched.
-int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list, int n_sms,
-                       cudaStream_t s) {
-    if (!g.P) return 0;
+template <bool kFrameK>
+static int launch_gate_coarse_t(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list,
+                                int n_sms, const float* frame_k, cudaStream_t s) {
+    constexpr int kSmem = kGateSmemBytes + (kFrameK ? kFrameKFloats * 4 : 0);
     static SmemConfig configured;
-    if (configured.raise((uint32_t)kGateSmemBytes)) {
-        cudaFuncSetAttribute(gate_coarse_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGateSmemBytes);
-        cudaFuncSetAttribute(gate_coarse_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGateSmemBytes);
-        cudaFuncSetAttribute(gate_coarse_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGateSmemBytes);
+    if (configured.raise((uint32_t)kSmem)) {
+        cudaFuncSetAttribute(gate_coarse_kernel<true, false, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+        cudaFuncSetAttribute(gate_coarse_kernel<false, false, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+        cudaFuncSetAttribute(gate_coarse_kernel<true, true, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     }
     static const bool fused = !(std::getenv("DH_GATE_FUSED") && std::atoi(std::getenv("DH_GATE_FUSED")) == 0);
     const uint32_t per_frame = (g.P + kGateThreads - 1) / kGateThreads;
@@ -2675,20 +2699,28 @@ int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev
         static const uint32_t want = std::getenv("DH_GATE_CTAS") ? (uint32_t)std::atoi(std::getenv("DH_GATE_CTAS")) : 0u;
         const uint32_t fill = (6u * (uint32_t)n_sms + n_frames - 1u) / n_frames;
         const uint32_t ctas = std::max<uint32_t>(1u, std::min<uint32_t>(per_frame, want ? want : std::max<uint32_t>(4u, fill)));
-        patch_gate_kernel<<<dim3((g.P + kPatchGateThreads * kPatchGatePer - 1) / (kPatchGateThreads * kPatchGatePer), n_frames),
-                            kPatchGateThreads, 0, s>>>(b, g, f);
-        gate_coarse_kernel<true, true><<<dim3(ctas, n_frames), kGateThreads, kGateSmemBytes, s>>>(b, g, f);
+        patch_gate_kernel<kFrameK><<<dim3((g.P + kPatchGateThreads * kPatchGatePer - 1) / (kPatchGateThreads * kPatchGatePer), n_frames),
+                                     kPatchGateThreads, 0, s>>>(b, g, f, frame_k);
+        gate_coarse_kernel<true, true, kFrameK><<<dim3(ctas, n_frames), kGateThreads, kSmem, s>>>(b, g, f, frame_k);
         return 2;
     }
     dim3 gr(per_frame, n_frames);
-    if (fused) gate_coarse_kernel<true, false><<<gr, kGateThreads, kGateSmemBytes, s>>>(b, g, f);
-    else gate_coarse_kernel<false, false><<<gr, kGateThreads, kGateSmemBytes, s>>>(b, g, f);
+    if (fused) gate_coarse_kernel<true, false, kFrameK><<<gr, kGateThreads, kSmem, s>>>(b, g, f, frame_k);
+    else gate_coarse_kernel<false, false, kFrameK><<<gr, kGateThreads, kSmem, s>>>(b, g, f, frame_k);
     return 1;
 }
 
+int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list, int n_sms,
+                       cudaStream_t s, const float* frame_k) {
+    if (!g.P) return 0;
+    return frame_k ? launch_gate_coarse_t<true>(b, g, f, n_frames, from_list, n_sms, frame_k, s)
+                   : launch_gate_coarse_t<false>(b, g, f, n_frames, from_list, n_sms, nullptr, s);
+}
+
 int launch_seed_and_cubes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames,
-                          uint32_t iterations, cudaStream_t s) {
-    seed_kernel<<<n_frames, kSeedThreads, 0, s>>>(b, g, iterations);
+                          uint32_t iterations, cudaStream_t s, const float* frame_k) {
+    if (frame_k) seed_kernel<true><<<n_frames, kSeedThreads, 0, s>>>(b, g, iterations, frame_k);
+    else seed_kernel<false><<<n_frames, kSeedThreads, 0, s>>>(b, g, iterations, nullptr);
     if (!g.P || !iterations) return 1;
     // enough blocks per frame that a thread sees a handful of hits
     const uint32_t per_frame =

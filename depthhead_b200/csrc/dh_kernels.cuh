@@ -125,11 +125,13 @@ void launch_plan_nodes(const NodeRec* nodes, HotNode* hot, UniNode* uni, size_t 
                        const double* prob_codes, cudaStream_t s);
 void launch_plan_pairs(const PairTopo* topo, const UniNode* uni, PairRec* recs, size_t n_recs, cudaStream_t s);
 // from_list: the patch gate runs as its own kernel and writes the frames' gated-patch lists; the seed-grid CTAs take
-// slices of the lists (DH_GATE_SPLIT, default) instead of gating the patches of their own index range
+// slices of the lists (DH_GATE_SPLIT, default) instead of gating the patches of their own index range.
+// frame_k: nullptr = every frame has Geometry's K / Kinv; else a device table [n_frames][18] of each
+// frame's K then K^-1 (row-major), read by the kernels that project (dh_predict_frames).
 int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list, int n_sms,
-                       cudaStream_t s);
+                       cudaStream_t s, const float* frame_k = nullptr);
 int launch_seed_and_cubes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames,
-                          uint32_t iterations, cudaStream_t s);
+                          uint32_t iterations, cudaStream_t s, const float* frame_k = nullptr);
 int launch_meanshift(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t iterations,
                      int n_sms, cudaStream_t s);
 uint32_t sat_band_rows();

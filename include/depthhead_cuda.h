@@ -14,6 +14,8 @@
  *   src/hough/prediction.rs:376-409   predict_parameter{,_parallel}            -> dh_predict, dh_predict_batch
  *   src/hough/prediction.rs:259-267   struct PredictionResult                  -> dh_result
  *   examples/live_prediction.rs:75-88 frame-to-frame seeding of a sequence     -> dh_predict_sequences
+ *   predict_parameter_parallel over n frames, each with its own K and seeds    -> dh_predict_frames,
+ *                                                                                 dh_predict_frames_biwi
  *   src/hough/prediction.rs:850-905   predict_mask                             -> dh_predict_mask
  *   src/hough/prediction.rs:760-841   build_hough_image (votes, before blur)   -> dh_hough_image_raw
  *   src/hough/prediction.rs:760-845   build_hough_image (with its blur)        -> dh_build_hough_image
@@ -155,6 +157,24 @@ int dh_predict_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint3
 int dh_predict_sequences(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n_seq, uint32_t frames_per_seq,
                          uint32_t w, uint32_t h, const float K[9], int depth_loc, float min_seed_z, dh_result* out);
 
+/* The arguments of dh_predict for one frame of dh_predict_frames: its own intrinsics and seeds. */
+typedef struct dh_frame_args {
+    float K[9];            /* row-major intrinsics of this frame */
+    float midp_guess[3];   /* mm; used iff has_guess bit 0 */
+    double rot_guess[3];   /* radians; used iff has_guess bit 1 */
+    uint32_t has_guess;    /* bit 0 midp_guess, bit 1 rot_guess; 0 = (None, None) */
+    uint32_t _pad;
+} dh_frame_args;           /* 80 bytes */
+
+/* predict_parameter_parallel(img, K_i, midp_i, rot_i) for n independent frames [n][h][w] at
+ * depth_loc, frame i with args[i] (host memory); results to out[n] (host).  Results are equal,
+ * bit for bit, to calling dh_predict frame by frame with the same arguments, through the chunked
+ * pipeline of dh_predict_batch (device-resident or host frames, the run-length host path).  K is
+ * not validated, as in dh_predict.  A has_guess with bits other than 0-1 is DH_E_ARG naming the
+ * frame.  Synchronous; n = 0 is a successful no-op. */
+int dh_predict_frames(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                      int depth_loc, const dh_frame_args* args, dh_result* out);
+
 /* predict_mask (prediction.rs:850-905): mask[h][w] u8 to host memory. */
 int dh_predict_mask(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t w, uint32_t h, uint8_t* mask);
 /* build_hough_image before its gaussian blur (prediction.rs:760-841): votes[h][w] u16 to host. */
@@ -204,6 +224,10 @@ int dh_biwi_decode_depth(dh_ctx* c, const uint8_t* blob, const uint64_t* offsets
  * examples/db_evaluate.rs:296 does per file, with the decode on the GPU. */
 int dh_predict_batch_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
                           uint32_t w, uint32_t h, const float K[9], dh_result* out);
+/* The same with the arguments of every frame (dh_predict_frames): a whole database, whose sequence
+ * folders each have their own depth.cal, in one call. */
+int dh_predict_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                           uint32_t w, uint32_t h, const dh_frame_args* args, dh_result* out);
 /* The writer for that format (the reference only reads it): n raw frames [n][h][w] u16 become n
  * files in ONE blob, file i at [offsets[i], offsets[i+1]) (offsets: n+1 entries, multiples of 16).
  * Runs are found at a granularity of 16 pixels: a group of 16 pixels with any non-zero pixel is

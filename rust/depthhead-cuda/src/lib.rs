@@ -53,6 +53,19 @@ pub struct DhTrainParams {
     pub steepness: f64, pub gaussian_sigma: f32, pub _pad: u32, pub seed: u64,
 }
 
+/// include/depthhead_cuda.h: dh_frame_args, the arguments of dh_predict for one frame of
+/// dh_predict_frames (80 bytes)
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct DhFrameArgs {
+    pub k: [f32; 9],
+    pub midp_guess: [f32; 3],
+    pub rot_guess: [f64; 3],
+    pub has_guess: u32,
+    pub _pad: u32,
+}
+const _: () = assert!(std::mem::size_of::<DhFrameArgs>() == 80);
+
 extern "C" {
     fn dh_last_error() -> *const c_char;
     fn dh_forest_from_json(json: *const c_char, len: usize, out: *mut *mut DhForest) -> c_int;
@@ -70,6 +83,8 @@ extern "C" {
                   midp_guess: *const f32, rot_guess: *const f64, out: *mut DhResult) -> c_int;
     fn dh_predict_batch(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32,
                         k: *const f32, depth_loc: c_int, out: *mut DhResult) -> c_int;
+    fn dh_predict_frames(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32, depth_loc: c_int,
+                         args: *const DhFrameArgs, out: *mut DhResult) -> c_int;
     fn dh_predict_sequences(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n_seq: u32, frames_per_seq: u32,
                             w: u32, h: u32, k: *const f32, depth_loc: c_int, min_seed_z: f32, out: *mut DhResult) -> c_int;
     fn dh_predict_mask(c: *mut DhCtx, f: *const DhForest, depth: *const u16, w: u32, h: u32, mask: *mut u8) -> c_int;
@@ -87,6 +102,8 @@ extern "C" {
                             out: *mut u16, out_loc: c_int) -> c_int;
     fn dh_predict_batch_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32,
                              w: u32, h: u32, k: *const f32, out: *mut DhResult) -> c_int;
+    fn dh_predict_frames_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32,
+                              w: u32, h: u32, args: *const DhFrameArgs, out: *mut DhResult) -> c_int;
     fn dh_biwi_parse_cal(text: *const c_char, len: usize, k: *mut f32) -> c_int;
     fn dh_biwi_parse_pose(file: *const u8, len: usize, k: *const f32, pos3d: *mut f32, pos2d: *mut f32,
                           rot: *mut f32) -> c_int;
@@ -265,6 +282,20 @@ impl HoughPrediction {
         check(unsafe { dh_predict_batch(self.context(), self.forest, frames.as_ptr(), n, w, h, k.ptr(), 0 /* DH_DEPTH_HOST */, out.as_mut_ptr()) })?;
         Ok(out)
     }
+    /// predict_parameter_parallel(img_i, &intrinsics[i], midp_guess[i], rot_guess[i]) for n independent
+    /// frames back to back in one call (a camera and seeds per frame: trackers, multi-camera rigs,
+    /// seeds from a detector); equal to calling predict_parameter_parallel frame by frame
+    pub fn predict_frames(&self, frames: &[u16], n: u32, w: u32, h: u32, intrinsics: &[IntrinsicMatrix],
+                          midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>]) -> Vec<PredictionResult> {
+        assert_eq!(frames.len(), (n as usize) * (w as usize) * (h as usize));
+        let args = frame_args(n, intrinsics, midp_guess, rot_guess);
+        self.push_fields().expect("depthhead-cuda: invalid stepwidth / meanshift_iterations");
+        let mut out = vec![DhResult::default(); n as usize];
+        check(unsafe { dh_predict_frames(self.context(), self.forest, frames.as_ptr(), n, w, h, 0 /* DH_DEPTH_HOST */,
+                                         args.as_ptr(), out.as_mut_ptr()) })
+            .expect("depthhead-cuda: prediction failed");
+        out.iter().map(PredictionResult::from_c).collect()
+    }
     /// predict_mask of n independent frames back to back: masks [n][h][w] in frame order
     pub fn predict_mask_batch(&self, frames: &[u16], n: u32, w: u32, h: u32) -> Result<Vec<u8>, Error> {
         let px = (n as usize) * (w as usize) * (h as usize);
@@ -334,6 +365,20 @@ impl Drop for HoughPrediction {
             dh_forest_free(self.forest);
         }
     }
+}
+
+/// one DhFrameArgs per frame; every slice has n entries
+fn frame_args(n: u32, intrinsics: &[IntrinsicMatrix], midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>])
+              -> Vec<DhFrameArgs> {
+    let n = n as usize;
+    assert!(intrinsics.len() == n && midp_guess.len() == n && rot_guess.len() == n, "one matrix and one pair of seeds per frame");
+    (0..n).map(|i| {
+        let mut a = DhFrameArgs::default();
+        for r in 0..3 { a.k[3 * r..3 * r + 3].copy_from_slice(&intrinsics[i].0[r]); }
+        if let Some(m) = midp_guess[i] { a.midp_guess = m; a.has_guess |= 1; }
+        if let Some(r) = rot_guess[i] { a.rot_guess = r; a.has_guess |= 2; }
+        a
+    }).collect()
 }
 
 /// `#[derive(Deserialize)]` of the reference (prediction.rs:238): any serde deserializer works; the
@@ -408,6 +453,18 @@ pub mod biwi {
             let mut out = vec![DhResult::default(); n as usize];
             check(unsafe { dh_predict_batch_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
                                                  files.width, files.height, k.0.as_ptr() as *const f32, out.as_mut_ptr()) })?;
+            Ok(out)
+        }
+        /// predict_files with the arguments of every file: a whole database, whose sequence folders
+        /// each have their own depth.cal, in one call
+        pub fn predict_files_frames(&self, files: &PackedFiles, intrinsics: &[IntrinsicMatrix], midp_guess: &[Option<[f32; 3]>],
+                                    rot_guess: &[Option<[f64; 3]>]) -> Result<Vec<DhResult>, Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            let args = frame_args(n, intrinsics, midp_guess, rot_guess);
+            self.push_fields()?;
+            let mut out = vec![DhResult::default(); n as usize];
+            check(unsafe { dh_predict_frames_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
+                                                  files.width, files.height, args.as_ptr(), out.as_mut_ptr()) })?;
             Ok(out)
         }
     }
