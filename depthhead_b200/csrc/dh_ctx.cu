@@ -108,8 +108,6 @@ Context::Context(int device) : device_(device) {
     DH_CUDA(cudaEventCreateWithFlags(&ev_copy_tail_, cudaEventDisableTiming));
     if (const char* v = std::getenv("DH_HOST_ENCODE")) host_encode_ = *v ? (int)std::strtol(v, nullptr, 10) : -1;
     use_graphs_ = env_flag("DH_GRAPH", true);
-    cube_clear_fused_ = env_flag("DH_CUBE_CLEAR_FUSED", true);
-    gate_split_ = env_flag("DH_GATE_SPLIT", true);
     gate_split_min_ = env_u32("DH_GATE_SPLIT_MIN", 64);
     chunk_frames_ = env_u32("DH_CHUNK_FRAMES", 0);  // 0 = adaptive (128 for host input, 512 for device input)
     debug_sync_ = env_u32("DH_DEBUG_SYNC", 0) != 0;
@@ -178,11 +176,6 @@ void Context::free_forest() {
     hot_tex_ = 0;
     hot_tw_ = 0;
     dev_free(df_roots_);
-    dev_free(df_pair_recs_);
-    dev_free(df_pair_topo_);
-    dev_free(df_pair_roots_);
-    dev_free(df_pair_perm_);
-    df_n_pairs_ = 0;
     dev_free(df_leaf_prob_);
     dev_free(df_leaf_info_);
     dev_free(df_offsets_);
@@ -196,78 +189,6 @@ void Context::free_forest() {
     blur_serial_ = 0;
 }
 
-// PairRec topology (dh_types.hpp): every internal node at an even depth below its root becomes a
-// record together with its two children; records in breadth-first order, so the (up to four)
-// grandchild records of a record are consecutive; the leaves under a record get consecutive
-// device leaf numbers, mapped back to global leaf ids by the permutation table.
-void Context::build_pair_tables(const HostForest& hf, const std::vector<int32_t>& dev_index) {
-    if (hf.n_leaves() >= (1u << 26) || hf.max_depth >= 63) return;  // the permutation entry packs leaf id (26 bits) and depth (6 bits)
-    std::vector<PairTopo> topo;
-    std::vector<uint32_t> depth;  // of the record's node X below its root
-    std::vector<int32_t> perm, roots((size_t)hf.n_trees);
-    topo.reserve(hf.n_nodes());
-    perm.reserve(hf.n_leaves() + hf.n_leaves() / 2);
-    for (int32_t t = 0; t < hf.n_trees; ++t) {
-        const int32_t root = hf.roots[(size_t)t];
-        if (root < 0) {  // a tree that is its single leaf
-            roots[(size_t)t] = ~(int32_t)perm.size();
-            perm.push_back(~root);  // depth 0: no node visit
-            continue;
-        }
-        roots[(size_t)t] = (int32_t)topo.size();
-        topo.push_back(PairTopo{root, -1, -1, 0u, 0u});
-        depth.push_back(0u);
-        for (size_t r = (size_t)roots[(size_t)t]; r < topo.size(); ++r) {
-            const NodeRec& X = hf.nodes[(size_t)topo[r].x];
-            int32_t c[2], slot[4];
-            for (int b = 0; b < 2; ++b) {
-                const int32_t C = X.child[b];
-                if (C >= 0) {
-                    c[b] = C;
-                    slot[2 * b] = hf.nodes[(size_t)C].child[0];
-                    slot[2 * b + 1] = hf.nodes[(size_t)C].child[1];
-                } else {
-                    c[b] = -1;
-                    slot[2 * b] = slot[2 * b + 1] = C;  // the dummy test always answers 0; slot 2b+1 is never taken
-                }
-            }
-            const uint32_t first = (uint32_t)topo.size(), first_leaf = (uint32_t)perm.size();
-            uint32_t mask = 0;
-            for (int k = 0; k < 4; ++k) {
-                if (slot[k] < 0) {
-                    // node visits of a walk that ends here: X and, unless the child itself is the leaf, the child
-                    const uint32_t visits = depth[r] + (c[k >> 1] < 0 ? 1u : 2u);
-                    mask |= 1u << k;
-                    perm.push_back((int32_t)((uint32_t)~slot[k] | (visits << 26)));
-                } else {
-                    topo.push_back(PairTopo{slot[k], -1, -1, 0u, 0u});
-                    depth.push_back(depth[r] + 2u);
-                }
-            }
-            if (first_leaf >= (1u << 26) || topo.size() >= (1ull << 31)) return;  // too large for the packed fields: the plain tables serve
-            topo[r].c0 = c[0];
-            topo[r].c1 = c[1];
-            topo[r].first = first;
-            topo[r].tail = (first_leaf << 6) | ((c[1] < 0 ? 1u : 0u) << 5) | ((c[0] < 0 ? 1u : 0u) << 4) | mask;
-        }
-    }
-    if (!dev_index.empty())  // the device node table is laid out differently from the host's (ensure_forest)
-        for (PairTopo& pt : topo) {
-            pt.x = dev_index[(size_t)pt.x];
-            if (pt.c0 >= 0) pt.c0 = dev_index[(size_t)pt.c0];
-            if (pt.c1 >= 0) pt.c1 = dev_index[(size_t)pt.c1];
-        }
-    df_n_pairs_ = topo.size();
-    dev_alloc(df_pair_recs_, topo.size());
-    dev_alloc(df_pair_topo_, topo.size());
-    dev_alloc(df_pair_roots_, roots.size());
-    dev_alloc(df_pair_perm_, perm.size());
-    if (!topo.empty()) DH_CUDA(cudaMemcpyAsync(df_pair_topo_, topo.data(), topo.size() * sizeof(PairTopo), cudaMemcpyHostToDevice, stream_));
-    DH_CUDA(cudaMemcpyAsync(df_pair_roots_, roots.data(), roots.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream_));
-    if (!perm.empty()) DH_CUDA(cudaMemcpyAsync(df_pair_perm_, perm.data(), perm.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream_));
-    DH_CUDA(cudaStreamSynchronize(stream_));  // the host vectors go away
-}
-
 void Context::ensure_forest(const HostForest& hf) {
     if (df_serial_ != hf.serial) {
         DH_CUDA(cudaStreamSynchronize(stream_));
@@ -278,18 +199,16 @@ void Context::ensure_forest(const HostForest& hf) {
         // texels); forests whose rectangles all have one size get the 16-byte box-sum nodes.
         uni_rw_ = uni_rh_ = 0;
         const bool use_tex = env_flag("DH_TEX", true);
-        const bool uni_ldg = env_flag("DH_UNI_LDG", false);
-        const bool want_uni = NN && env_flag("DH_UNIFORM", true) && hf.uniform_rw && (uni_ldg || (use_tex && NN < (1ull << 26)));
-        // Device order of the node table.  The host keeps every tree in breadth-first order, so the
-        // internal children of a node are neighbours; with 16-byte nodes a 32-byte sector holds two
-        // of them, and a pad record in front of a pair that would straddle two sectors makes the
-        // lanes of a warp that part ways at a node fetch ONE sector for both sides (DH_NODE_ALIGN=0:
-        // host order; pads are never visited).
-        std::vector<int32_t> dev_index;
+        const bool want_uni = NN && env_flag("DH_UNIFORM", true) && hf.uniform_rw && use_tex && NN < (1ull << 26);
+        // Device order of the box-sum node table.  The host keeps every tree in breadth-first order
+        // (dh_forest.cpp), so the internal children of a node are neighbours; with 16-byte nodes a
+        // 32-byte sector holds two of them, and a pad record in front of a pair that would straddle
+        // two sectors makes the lanes of a warp that part ways at a node fetch ONE sector for both
+        // sides (pads are never visited).  Other forests keep the host order.
         std::vector<NodeRec> dev_nodes;
         std::vector<int32_t> dev_roots(hf.roots);
-        if (want_uni && env_flag("DH_NODE_ALIGN", true)) {
-            dev_index.assign(NN, -1);
+        if (want_uni) {
+            std::vector<int32_t> dev_index(NN, -1);
             int32_t d = 0;
             bool ok = true;
             for (int32_t t = 0; t < hf.n_trees && ok; ++t) {
@@ -309,23 +228,22 @@ void Context::ensure_forest(const HostForest& hf) {
                 }
                 if (next != n1) ok = false;
             }
-            if (ok && (size_t)d < (1ull << 27)) {
-                NodeRec pad;
-                std::memset(&pad, 0, sizeof(pad));
-                pad.child[0] = pad.child[1] = -1;
-                dev_nodes.assign((size_t)d, pad);
-                for (size_t h = 0; h < NN; ++h) {
-                    NodeRec r = hf.nodes[h];
-                    for (int b = 0; b < 2; ++b)
-                        if (r.child[b] >= 0) r.child[b] = dev_index[(size_t)r.child[b]];
-                    dev_nodes[(size_t)dev_index[h]] = r;
-                }
-                for (int32_t& r : dev_roots)
-                    if (r >= 0) r = dev_index[(size_t)r];
-                NN = (size_t)d;
-            } else {
-                dev_index.clear();
+            // NN < 2^26 (want_uni) bounds d, pads included, below 2 * NN
+            if (!ok || (size_t)d >= (1ull << 27))
+                throw ModelError(DH_E_STATE, "internal error: the host node table is not in breadth-first order");
+            NodeRec pad;
+            std::memset(&pad, 0, sizeof(pad));
+            pad.child[0] = pad.child[1] = -1;
+            dev_nodes.assign((size_t)d, pad);
+            for (size_t h = 0; h < NN; ++h) {
+                NodeRec r = hf.nodes[h];
+                for (int b = 0; b < 2; ++b)
+                    if (r.child[b] >= 0) r.child[b] = dev_index[(size_t)r.child[b]];
+                dev_nodes[(size_t)dev_index[h]] = r;
             }
+            for (int32_t& r : dev_roots)
+                if (r >= 0) r = dev_index[(size_t)r];
+            NN = (size_t)d;
         }
         dev_alloc(df_nodes_, NN);
         dev_alloc(df_hot_, NN);
@@ -335,7 +253,7 @@ void Context::ensure_forest(const HostForest& hf) {
             uni_rw_ = hf.uniform_rw;
             uni_rh_ = hf.uniform_rh;
         }
-        if (use_tex && NN && !(df_uni_ && uni_ldg) && (df_uni_ || NN * 2 < (1ull << 27))) {
+        if (use_tex && NN && (df_uni_ || NN * 2 < (1ull << 27))) {
             cudaResourceDesc rd{};
             rd.resType = cudaResourceTypeLinear;
             rd.res.linear.devPtr = df_uni_ ? (void*)df_uni_ : (void*)df_hot_;
@@ -345,7 +263,6 @@ void Context::ensure_forest(const HostForest& hf) {
             td.readMode = cudaReadModeElementType;
             DH_CUDA(cudaCreateTextureObject(&hot_tex_, &rd, &td, nullptr));
         }
-        if (df_uni_ && hot_tex_ && env_flag("DH_TRAV_PAIR", false)) build_pair_tables(hf, dev_index);
         dev_alloc(df_roots_, (size_t)hf.n_trees);
         dev_alloc(df_leaf_prob_, NL);
         dev_alloc(df_leaf_info_, NL);
@@ -390,7 +307,7 @@ void Context::ensure_forest(const HostForest& hf) {
             if (!(hf.leaf_prob[l] >= 0.0 && hf.leaf_prob[l] <= 1.0)) prob_codes_ok_ = false;
         if (!env_flag("DH_PROB_CODES", true)) prob_codes_ok_ = false;
         // the walks store the packed words only from the uniform (box-sum) node table, one level per fetch
-        leaf_codes_ = prob_codes_ok_ && gate_split_ && df_uni_ && !df_pair_recs_;
+        leaf_codes_ = prob_codes_ok_ && df_uni_;
         df_serial_ = hf.serial;
         df_sigma_version_ = 0;
         df_n_leaves_ = NL;
@@ -411,10 +328,6 @@ void Context::ensure_forest(const HostForest& hf) {
     fdev_.uni_rw = uni_rw_;
     fdev_.uni_rh = uni_rh_;
     fdev_.roots = df_roots_;
-    fdev_.pair_recs = df_pair_recs_;
-    fdev_.pair_topo = df_pair_topo_;
-    fdev_.pair_roots = df_pair_roots_;
-    fdev_.pair_leaf_perm = df_pair_perm_;
     fdev_.leaf_prob = df_leaf_prob_;
     fdev_.leaf_info = df_leaf_info_;
     fdev_.offsets = df_offsets_;
@@ -507,11 +420,11 @@ void Context::alloc_lane(Lane& L) {
 TilePlan Context::plan_tiles(const Geometry& g) const {
     // Choose the patch tile that minimises total shared-memory fill traffic per frame, subject to
     // the tile (plus bookkeeping) fitting `limit` bytes so that several CTAs share an SM.
-    const uint32_t want_threads = env_u32("DH_TRAV_THREADS", 1024);
-    const uint32_t trav_threads = want_threads >= 1024 ? 1024u : (want_threads >= 768 ? 768u : 512u);
-    const uint32_t big = trav_threads >= 768 ? 1u : 0u;  // two CTAs per SM; 512 threads: three
-    const uint32_t two = env_u32("DH_TRAV_SMEM", 113000u);  // bytes per CTA that still let two CTAs share an SM
-    const uint32_t limits[3] = {big ? two : 75000u, 113000u, smem_optin_ > 2048u ? smem_optin_ - 1024u : smem_optin_};
+    // 1024-thread CTAs, two per SM, when the tile fits kTwoPerSm bytes; 512-thread CTAs, three per SM,
+    // for larger tiles (DH_TRAV_THREADS below 1024 forces them)
+    constexpr uint32_t kTwoPerSm = 113000u;  // bytes per CTA that still let two CTAs share an SM
+    const bool big = env_u32("DH_TRAV_THREADS", 1024) >= 1024;
+    const uint32_t limits[3] = {big ? kTwoPerSm : 75000u, kTwoPerSm, smem_optin_ > 2048u ? smem_optin_ - 1024u : smem_optin_};
     for (uint32_t limit : limits) {
         TilePlan best{};
         double best_cost = 1e300;
@@ -531,28 +444,21 @@ TilePlan Context::plan_tiles(const Geometry& g) const {
                 const double cost = (double)tiles_x * tiles_y * ((double)tw * th * 4.0 + 8192.0);
                 if (cost < best_cost) {
                     best_cost = cost;
-                    best = TilePlan{tpx, tpy, tiles_x, tiles_y, tw, th, bytes, (big && limit <= 113000u) ? trav_threads : 512u};
+                    best = TilePlan{tpx, tpy, tiles_x, tiles_y, tw, th, bytes, (big && limit <= kTwoPerSm) ? 1024u : 512u};
                 }
             }
         if (best.tpx) {
-            best.tma_first = env_flag("DH_TRAV_TMA_FIRST", true) ? 1u : 0u;  // measured: 1.110 -> 1.052 ms per 1024 frames
-            best.ldg_levels = env_u32("DH_TRAV_LDG_LEVELS", 7);  // measured: 1.071 -> 1.048 ms (3: 1.057, 5: 1.051, 7-11: 1.048, 13: 1.057)
-            if (env_flag("DH_TRAV_BLOCK", true)) {  // measured with the early load: 1.052 -> 1.037 ms
-                // a warp walks a block of 8 x 4 neighbouring patches: its lanes stay on the same nodes for
-                // longer.  On one node lane (c, r) reads word stride * (c + r * tw) + const: with
-                // stride * tw = 8 (mod 32) and an odd stride the 32 lanes hit 32 different banks.
-                best.blocked = 1u;
-                for (uint32_t tw2 = best.tw; tw2 < best.tw + 32u && tw2 <= 256u; tw2 += 4u) {
-                    const uint32_t bytes = traverse_smem_bytes(tw2, best.th, best.tpx * best.tpy);
-                    if (((g.stride * tw2) & 31u) == 8u && bytes <= limit) {
-                        best.tw = tw2;
-                        best.smem_bytes = bytes;
-                        break;
-                    }
+            // a warp walks a block of 8 x 4 neighbouring patches (traverse_kernel).  On one node lane (c, r)
+            // reads word stride * (c + r * tw) + const: with stride * tw = 8 (mod 32) and an odd stride the
+            // 32 lanes hit 32 different banks.
+            for (uint32_t tw2 = best.tw; tw2 < best.tw + 32u && tw2 <= 256u; tw2 += 4u) {
+                const uint32_t bytes = traverse_smem_bytes(tw2, best.th, best.tpx * best.tpy);
+                if (((g.stride * tw2) & 31u) == 8u && bytes <= limit) {
+                    best.tw = tw2;
+                    best.smem_bytes = bytes;
+                    break;
                 }
             }
-            // experiment: extra dynamic shared memory per CTA lowers the CTAs per SM without changing the tile
-            best.smem_bytes += std::min<uint32_t>(env_u32("DH_TRAV_PAD_SMEM", 0), smem_optin_ > best.smem_bytes ? smem_optin_ - best.smem_bytes : 0u);
             return best;
         }
     }
@@ -675,7 +581,7 @@ FrameBuffers Context::buffers(const Lane& L, const uint16_t* depth) const {
     b.ms_trace_cap = sk_.trace_iters;
     b.leaf_mask = leaf_codes_ ? kLeafIdMask : 0x7fffffffu;
     b.debug = debug_ ? 1u : 0u;
-    b.clear_cubes = (!debug_ && cube_clear_fused_) ? 1u : 0u;  // debug passes export the cubes after the call
+    b.clear_cubes = debug_ ? 0u : 1u;  // debug passes export the cubes after the call
     return b;
 }
 
@@ -740,7 +646,6 @@ void Context::run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameS
     }
     if (g.P && hot_tw_ != tiles_.tw) {  // node table for this tile plan (once per forest x plan)
         launch_plan_nodes(df_nodes_, df_hot_, df_uni_, df_n_nodes_, tiles_.tw, leaf_codes_ ? df_leaf_prob_ : nullptr, stream_);
-        if (df_pair_recs_) launch_plan_pairs(df_pair_topo_, df_uni_, df_pair_recs_, df_n_pairs_, stream_);
         DH_CUDA(cudaStreamSynchronize(stream_));
         hot_tw_ = tiles_.tw;
     }
@@ -768,7 +673,7 @@ void Context::run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iter
     mark(DH_STAGE_GATE);
     // small passes (single frames, the passes of seeded sequences) are bound by the chain of launches: they keep the
     // patch gate inside the seed-grid kernel (one launch less; 0.168 instead of 0.187 ms per single frame)
-    launches_ += (uint64_t)launch_gate_coarse(b, g, fdev_, n, gate_split_ && n >= gate_split_min_, n_sms_, st, frame_k);
+    launches_ += (uint64_t)launch_gate_coarse(b, g, fdev_, n, n >= gate_split_min_, n_sms_, st, frame_k);
     stage_check("gate + coarse grids");
     mark(DH_STAGE_VOTE);
     // the accumulator cubes of this pass start empty: either the previous pass's mean-shift CTAs

@@ -147,7 +147,6 @@ public:
 private:
     void ensure_forest(const HostForest& hf);
     void free_forest();
-    void build_pair_tables(const HostForest& hf, const std::vector<int32_t>& dev_index);
     void ensure_scratch(const HostForest& hf, uint32_t w, uint32_t h, uint32_t n_frames_hint, const float K[9], int n_lanes = 1);
     void alloc_lane(Lane& L);
     void free_lane(Lane& L);
@@ -201,12 +200,6 @@ private:
     UniNode* df_uni_ = nullptr;            // uniform-rectangle forests: box-sum nodes for tile width hot_tw_
     uint32_t uni_rw_ = 0, uni_rh_ = 0;
     size_t df_n_nodes_ = 0;
-    // two-levels-per-record tables for the box-sum traversal (PairRec, dh_types.hpp; DH_TRAV_PAIR)
-    PairRec* df_pair_recs_ = nullptr;
-    PairTopo* df_pair_topo_ = nullptr;
-    int32_t* df_pair_roots_ = nullptr;
-    int32_t* df_pair_perm_ = nullptr;
-    size_t df_n_pairs_ = 0;
     int32_t* df_roots_ = nullptr;
     double* df_leaf_prob_ = nullptr;
     LeafInfo* df_leaf_info_ = nullptr;
@@ -299,8 +292,6 @@ private:
     bool prob_codes_ok_ = false;     // the uploaded forest's leaf probabilities can ride in the node table as 8-bit codes
     bool leaf_codes_ = false;        // ... and do: leaf words carry them (FrameBuffers::leaf_mask, patch_gate_kernel)
     uint32_t gate_split_min_ = 64;   // frames per pass from which the patch gate runs as its own kernel (DH_GATE_SPLIT_MIN)
-    bool gate_split_ = true;         // DH_GATE_SPLIT=0: the patch gate inside the seed-grid kernel instead of its own kernel + list
-    bool cube_clear_fused_ = true;   // DH_CUBE_CLEAR_FUSED=0: one memset of all cubes per pass instead
 
     // measurement
     bool timing_ = false, debug_ = false, have_debug_ = false, debug_sync_ = false;

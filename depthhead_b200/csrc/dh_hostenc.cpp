@@ -34,32 +34,10 @@ inline bool group_is_zero(const uint16_t* p) {
 inline void put_u32(uint8_t* o, uint32_t v) {  // little endian, any alignment
     o[0] = (uint8_t)v; o[1] = (uint8_t)(v >> 8); o[2] = (uint8_t)(v >> 16); o[3] = (uint8_t)(v >> 24);
 }
-// DH_ENCODE_NT=1 turns streaming stores on (off by default: the copy engine's reads of the pinned slot
-// are served from the last-level cache when ordinary stores left the bytes there; measured, see DESIGN.md)
-const bool g_stream_stores = [] {
-    const char* v = std::getenv("DH_ENCODE_NT");
-    return v && *v && std::strtol(v, nullptr, 10) != 0;
-}();
-
+// Ordinary stores: the copy engine's reads of the pinned slot are then served from the last-level
+// cache (streaming stores did not help, DESIGN.md section 5)
 inline void put_pixels(uint8_t* o, const uint16_t* src, size_t n) {
 #if defined(__BYTE_ORDER__) && __BYTE_ORDER__ == __ORDER_LITTLE_ENDIAN__
-#if defined(__SSE2__)
-    // The rewritten bytes are read next by the copy engine, never again by this core: streaming
-    // (non-temporal) stores keep them out of the cache and spare the read-for-ownership of every
-    // destination line.  16-byte aligned body, ordinary stores for the ragged ends.
-    size_t bytes = n * 2;
-    if (g_stream_stores && bytes >= 256) {
-        const uint8_t* s = reinterpret_cast<const uint8_t*>(src);
-        const size_t head = (16 - (reinterpret_cast<uintptr_t>(o) & 15)) & 15;
-        std::memcpy(o, s, head);
-        o += head; s += head; bytes -= head;
-        const size_t body = bytes & ~(size_t)15;
-        for (size_t i = 0; i < body; i += 16)
-            _mm_stream_si128(reinterpret_cast<__m128i*>(o + i), _mm_loadu_si128(reinterpret_cast<const __m128i*>(s + i)));
-        std::memcpy(o + body, s + body, bytes - body);
-        return;
-    }
-#endif
     std::memcpy(o, src, n * 2);
 #else
     for (size_t i = 0; i < n; ++i) { o[2 * i] = (uint8_t)src[i]; o[2 * i + 1] = (uint8_t)(src[i] >> 8); }
@@ -102,9 +80,6 @@ size_t rle_encode_frame(const uint16_t* src, uint32_t w, uint32_t h, uint8_t* ds
         covered += n_empty + n_full;
     }
     while ((o - dst) & 3) *o++ = 0;  // files start at multiples of 4 bytes inside a blob
-#if defined(__SSE2__)
-    if (g_stream_stores) _mm_sfence();  // the streaming stores are globally visible before the frame is handed on
-#endif
     return (size_t)(o - dst);
 }
 

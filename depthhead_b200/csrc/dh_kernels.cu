@@ -11,7 +11,7 @@
 //                                (ordered f64 prob sum only where the codes cannot decide), back-projection,
 //                                gated-patch list (prediction.rs:551-554,582-584)
 //   K3b gate_coarse_kernel       the two coarse seed grids from slices of the gated-patch list
-//                                (prediction.rs:590-595,630-636,661-675); <., false>: gate and grids in one kernel
+//                                (prediction.rs:590-595,630-636,661-675); <false, .>: gate and grids in one kernel
 //   K4a seed_kernel              arg-max seeds (prediction.rs:694-752, 437-460)
 //   K4b box_build_kernel         dense local cubes of the SparseArray3D<u32> accumulators
 //                                (meanshift.rs:14-68, prediction.rs:635,667)
@@ -299,60 +299,52 @@ __global__ void __launch_bounds__(kSatBandRows * 32) sat_band_kernel(const uint1
 // nine shuffles (rectangle width a multiple of the lane's pixel count) or through exclusive
 // prefix sums along x staged in a warp-private row of shared memory, B[y][x] = P[x + rw] - P[x];
 // 16-byte stores.  No block-level barrier; all arithmetic in u32 (rw*rh*65535 < 2^31 is checked
-// at load; prefix sums may wrap, differences are exact).  DH_BOX_PX=4 selects 4 pixels per lane
-// (twice the warps, half the ring each): measured slower (0.47 vs 0.43 ms), kept as a variant.
+// at load; prefix sums may wrap, differences are exact).  4 pixels per lane (twice the warps, half
+// the ring each) measured slower: 0.47 vs 0.43 ms.
 constexpr int kBoxMaxWarps = 8;                 // warps per CTA = strips of one (frame, band), when there are at most 8
 constexpr int kBoxAhead = 8;                    // rows fetched ahead
+constexpr int kBoxPx = 8;                       // pixels per lane: one 16-byte load, strips of 256 columns
 
-// kPx pixels per lane: 8 (16-byte loads, strips of 256 columns) or 4 (8-byte loads, strips of 128
-// columns: twice the warps for the same frame, half the ring per warp)
-template <int kPx>
 struct BoxRow {
-    uint32_t q[kPx / 2];  // kPx u16 pixels
+    uint32_t q[kBoxPx / 2];  // kBoxPx u16 pixels
 };
-template <int kPx>
-__device__ __forceinline__ BoxRow<kPx> box_fetch(const uint16_t* __restrict__ row, uint32_t w, uint32_t x, bool vec_ok, bool on) {
-    BoxRow<kPx> r;
+__device__ __forceinline__ BoxRow box_fetch(const uint16_t* __restrict__ row, uint32_t w, uint32_t x, bool vec_ok, bool on) {
+    BoxRow r;
 #pragma unroll
-    for (int j = 0; j < kPx / 2; ++j) r.q[j] = 0u;
+    for (int j = 0; j < kBoxPx / 2; ++j) r.q[j] = 0u;
     if (!on) return r;
     if (vec_ok) {
-        if (kPx == 8) {
-            const uint4 t = __ldg(reinterpret_cast<const uint4*>(row + x));
-            r.q[0] = t.x; r.q[1] = t.y; r.q[kPx / 2 - 2] = t.z; r.q[kPx / 2 - 1] = t.w;
-        } else {
-            const uint2 t = __ldg(reinterpret_cast<const uint2*>(row + x));
-            r.q[0] = t.x; r.q[1] = t.y;
-        }
+        const uint4 t = __ldg(reinterpret_cast<const uint4*>(row + x));
+        r.q[0] = t.x; r.q[1] = t.y; r.q[2] = t.z; r.q[3] = t.w;
         return r;
     }
 #pragma unroll
-    for (int j = 0; j < kPx / 2; ++j) {
+    for (int j = 0; j < kBoxPx / 2; ++j) {
         const uint32_t lo = (x + 2 * j < w) ? (uint32_t)__ldg(row + x + 2 * j) : 0u;
         const uint32_t hi = (x + 2 * j + 1 < w) ? (uint32_t)__ldg(row + x + 2 * j + 1) : 0u;
         r.q[j] = lo | (hi << 16);
     }
     return r;
 }
-template <int kPx, bool kAdd>
-__device__ __forceinline__ void box_apply(uint32_t acc[kPx], const BoxRow<kPx>& r) {
+template <bool kAdd>
+__device__ __forceinline__ void box_apply(uint32_t acc[kBoxPx], const BoxRow& r) {
 #pragma unroll
-    for (int j = 0; j < kPx / 2; ++j) {
+    for (int j = 0; j < kBoxPx / 2; ++j) {
         const uint32_t lo = r.q[j] & 0xffffu, hi = r.q[j] >> 16;
         acc[2 * j] = kAdd ? acc[2 * j] + lo : acc[2 * j] - lo;
         acc[2 * j + 1] = kAdd ? acc[2 * j + 1] + hi : acc[2 * j + 1] - hi;
     }
 }
 
-// kWhole: rw is a multiple of kPx, i.e. a rectangle row is a suffix of one lane's columns,
-// rw/kPx - 1 whole lanes and a prefix of one more lane: B comes straight out of shuffles, without
+// kWhole: rw is a multiple of kBoxPx, i.e. a rectangle row is a suffix of one lane's columns,
+// rw/kBoxPx - 1 whole lanes and a prefix of one more lane: B comes straight out of shuffles, without
 // the prefix sums over the whole warp and their trip through shared memory.
-template <int kPx, bool kWhole>
+template <bool kWhole>
 __global__ void __launch_bounds__(kBoxMaxWarps * 32) box_image_kernel(const uint16_t* __restrict__ depth, uint32_t* __restrict__ box,
                                                                 uint32_t w, uint32_t h, uint32_t rw, uint32_t rh, uint32_t bw,
                                                                 uint32_t bh, uint32_t bpitch, uint32_t strip_out, uint32_t n_strips,
                                                                 uint32_t band_rows, uint32_t n_bands, uint32_t n_units) {
-    constexpr uint32_t kRowPitch = 32 * kPx + 16;      // P[0 .. 32*kPx] + the slack the last active lane may read
+    constexpr uint32_t kRowPitch = 32 * kBoxPx + 16;      // P[0 .. 32*kBoxPx] + the slack the last active lane may read
     extern __shared__ __align__(16) uint32_t s_box[];  // [warps][2][kRowPitch] prefix rows (general widths only), then [warps][rh][32] pixel rings
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     const uint32_t n_warps = blockDim.x >> 5;  // the strips of one (frame, band) sit in one CTA: their reads and writes
@@ -362,29 +354,29 @@ __global__ void __launch_bounds__(kBoxMaxWarps * 32) box_image_kernel(const uint
     const uint32_t strip = unit % n_strips;
     unit /= n_strips;
     const uint32_t band = unit % n_bands, frame = unit / n_bands;
-    const uint32_t c0 = strip * strip_out, c1 = min(bw, c0 + strip_out);  // output columns (c0 is a multiple of kPx)
+    const uint32_t c0 = strip * strip_out, c1 = min(bw, c0 + strip_out);  // output columns (c0 is a multiple of kBoxPx)
     const uint32_t y0 = band * band_rows, y1 = min(bh, y0 + band_rows);   // output rows
     if (c0 >= c1 || y0 >= y1) return;
     const uint32_t x_end = c1 + rw - 1u;          // one past the last input column (<= w)
     const uint32_t r_end = y1 + rh - 1u;          // one past the last input row (<= h)
     const uint16_t* img = depth + (size_t)frame * h * w;
-    const bool vec_ok = ((w & (kPx - 1u)) == 0u) && ((reinterpret_cast<uintptr_t>(img) & (2u * kPx - 1u)) == 0u);
-    const uint32_t my_x = c0 + lane * kPx;
+    const bool vec_ok = ((w & (kBoxPx - 1u)) == 0u) && ((reinterpret_cast<uintptr_t>(img) & (2u * kBoxPx - 1u)) == 0u);
+    const uint32_t my_x = c0 + lane * kBoxPx;
     const bool lane_in = my_x < x_end;            // the lane holds input pixels
     const bool lane_out = my_x < c1;              // the lane holds output columns
     const bool q_vec = (rw & 3u) == 0u;
     const uint32_t p_words = kWhole ? 0u : n_warps * 2u * kRowPitch;
-    uint32_t* sp0 = s_box + warp * 2u * kRowPitch + lane * kPx;
-    BoxRow<kPx>* ring = reinterpret_cast<BoxRow<kPx>*>(s_box + p_words) + (size_t)warp * rh * 32u + lane;
+    uint32_t* sp0 = s_box + warp * 2u * kRowPitch + lane * kBoxPx;
+    BoxRow* ring = reinterpret_cast<BoxRow*>(s_box + p_words) + (size_t)warp * rh * 32u + lane;
     uint32_t* out = box + ((size_t)frame * bh + y0) * bpitch + my_x;
     const uint16_t* row_nxt = img + (size_t)y0 * w;   // next input row to fetch
-    uint32_t acc[kPx];
+    uint32_t acc[kBoxPx];
 #pragma unroll
-    for (int j = 0; j < kPx; ++j) acc[j] = 0u;
-    BoxRow<kPx> q[kBoxAhead];
+    for (int j = 0; j < kBoxPx; ++j) acc[j] = 0u;
+    BoxRow q[kBoxAhead];
 #pragma unroll
     for (int k = 0; k < kBoxAhead; ++k) {
-        q[k] = box_fetch<kPx>(row_nxt, w, my_x, vec_ok, lane_in && y0 + (uint32_t)k < r_end);
+        q[k] = box_fetch(row_nxt, w, my_x, vec_ok, lane_in && y0 + (uint32_t)k < r_end);
         row_nxt += w;
     }
     uint32_t buf = 0, slot = 0;                   // slot = (r - y0) mod rh
@@ -393,30 +385,30 @@ __global__ void __launch_bounds__(kBoxMaxWarps * 32) box_image_kernel(const uint
         for (int k = 0; k < kBoxAhead; ++k) {
             const uint32_t r = r0 + (uint32_t)k;
             if (r >= r_end) break;
-            const BoxRow<kPx> cur = q[k];
-            q[k] = box_fetch<kPx>(row_nxt, w, my_x, vec_ok, lane_in && r + kBoxAhead < r_end);
+            const BoxRow cur = q[k];
+            q[k] = box_fetch(row_nxt, w, my_x, vec_ok, lane_in && r + kBoxAhead < r_end);
             row_nxt += w;
             ring[slot * 32u] = cur;               // row r takes the place of row r - rh (left the window last round)
             if (++slot == rh) slot = 0;
-            box_apply<kPx, true>(acc, cur);
+            box_apply<true>(acc, cur);
             if (r + 1u >= y0 + rh) {              // the window [r - rh + 1, r] is complete
-                const BoxRow<kPx> old = ring[slot * 32u];  // row r - rh + 1 leaves the window
+                const BoxRow old = ring[slot * 32u];  // row r - rh + 1 leaves the window
                 // exclusive prefix sums of the lane's window sums
-                uint32_t e[kPx], tot = 0;
+                uint32_t e[kBoxPx], tot = 0;
 #pragma unroll
-                for (int j = 0; j < kPx; ++j) {
+                for (int j = 0; j < kBoxPx; ++j) {
                     e[j] = tot;
                     tot += acc[j];
                 }
-                uint32_t t[kPx];
+                uint32_t t[kBoxPx];
                 if (kWhole) {
-                    // B[kPx*l + j] = (T_l - e_l[j]) + T_{l+1} + .. + T_{l+k-1} + e_{l+k}[j],  k = rw / kPx
-                    const uint32_t k2 = rw / kPx;
+                    // B[kBoxPx*l + j] = (T_l - e_l[j]) + T_{l+1} + .. + T_{l+k-1} + e_{l+k}[j],  k = rw / kBoxPx
+                    const uint32_t k2 = rw / kBoxPx;
                     uint32_t whole = tot;
                     for (uint32_t i = 1; i < k2; ++i) whole += __shfl_down_sync(0xffffffffu, tot, i);
                     t[0] = whole;
 #pragma unroll
-                    for (int j = 1; j < kPx; ++j) t[j] = whole - e[j] + __shfl_down_sync(0xffffffffu, e[j], k2);
+                    for (int j = 1; j < kBoxPx; ++j) t[j] = whole - e[j] + __shfl_down_sync(0xffffffffu, e[j], k2);
                 } else {
                     // general width: prefix sums over the whole warp, staged in shared memory
                     uint32_t incl = tot;
@@ -427,22 +419,22 @@ __global__ void __launch_bounds__(kBoxMaxWarps * 32) box_image_kernel(const uint
                     }
                     const uint32_t base = incl - tot;
 #pragma unroll
-                    for (int j = 0; j < kPx; ++j) e[j] += base;
+                    for (int j = 0; j < kBoxPx; ++j) e[j] += base;
                     uint32_t* sp = sp0 + buf * kRowPitch;
 #pragma unroll
-                    for (int j = 0; j < kPx; j += 4) *reinterpret_cast<uint4*>(sp + j) = make_uint4(e[j], e[j + 1], e[j + 2], e[j + 3]);
-                    if (lane == 31u) sp[kPx] = incl;  // P[32 * kPx]
+                    for (int j = 0; j < kBoxPx; j += 4) *reinterpret_cast<uint4*>(sp + j) = make_uint4(e[j], e[j + 1], e[j + 2], e[j + 3]);
+                    if (lane == 31u) sp[kBoxPx] = incl;  // P[32 * kBoxPx]
                     __syncwarp();
                     if (lane_out) {
                         if (q_vec) {
 #pragma unroll
-                            for (int j = 0; j < kPx; j += 4) {
+                            for (int j = 0; j < kBoxPx; j += 4) {
                                 const uint4 a = *reinterpret_cast<const uint4*>(sp + rw + j);
                                 t[j] = a.x - e[j]; t[j + 1] = a.y - e[j + 1]; t[j + 2] = a.z - e[j + 2]; t[j + 3] = a.w - e[j + 3];
                             }
                         } else {
 #pragma unroll
-                            for (int j = 0; j < kPx; ++j) t[j] = sp[rw + j] - e[j];
+                            for (int j = 0; j < kBoxPx; ++j) t[j] = sp[rw + j] - e[j];
                         }
                     }
                     buf ^= 1u;
@@ -450,11 +442,11 @@ __global__ void __launch_bounds__(kBoxMaxWarps * 32) box_image_kernel(const uint
                 if (lane_out) {
                     // columns at or beyond bw are row padding (never read); beyond the pitch nothing is stored
 #pragma unroll
-                    for (int j = 0; j < kPx; j += 4)
+                    for (int j = 0; j < kBoxPx; j += 4)
                         if (my_x + (uint32_t)j < bpitch) *reinterpret_cast<uint4*>(out + j) = make_uint4(t[j], t[j + 1], t[j + 2], t[j + 3]);
                 }
                 out += bpitch;
-                box_apply<kPx, false>(acc, old);
+                box_apply<false>(acc, old);
             }
         }
     }
@@ -524,35 +516,6 @@ __global__ void __launch_bounds__(256) plan_nodes_kernel(const NodeRec* __restri
     }
 }
 
-// PairRec (two tree levels per 32-byte record) for the current tile plan: tests copied from the
-// UniNode table plan_nodes_kernel has just written, topology from the host.
-__global__ void __launch_bounds__(256) plan_pairs_kernel(const PairTopo* __restrict__ topo, const UniNode* __restrict__ uni,
-                                                         PairRec* __restrict__ recs, size_t n) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const PairTopo t = topo[i];
-    PairRec r;
-    const UniNode x = uni[t.x];
-    r.taps_x = x.taps;
-    r.e2_x = x.e2;
-    // a child that is a leaf: a test that is never greater and never equal (2*(s1 - s2) is even)
-    r.taps_c0 = 0u; r.e2_c0 = 0x7fffffff;
-    r.taps_c1 = 0u; r.e2_c1 = 0x7fffffff;
-    if (t.c0 >= 0) { const UniNode c = uni[t.c0]; r.taps_c0 = c.taps; r.e2_c0 = c.e2; }
-    if (t.c1 >= 0) { const UniNode c = uni[t.c1]; r.taps_c1 = c.taps; r.e2_c1 = c.e2; }
-    r.first = t.first;
-    r.tail = t.tail;
-    recs[i] = r;
-}
-
-__device__ __forceinline__ PairRec ldg_pair(const PairRec* p) {
-    PairRec r;
-    asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(r.taps_x), "=r"(r.e2_x), "=r"(r.taps_c0), "=r"(r.e2_c0), "=r"(r.taps_c1), "=r"(r.e2_c1), "=r"(r.first), "=r"(r.tail)
-                 : "l"(p));
-    return r;
-}
-
 __device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
     uint32_t v;
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
@@ -584,18 +547,18 @@ __device__ __noinline__ bool binarize_ieee(const NodeRec* __restrict__ nodes, in
 // One CTA per (tile of patches, frame).  The tile's SAT window (tw x th u32) is brought into
 // shared memory by ONE TMA bulk-tensor load; all 8 taps of every node test are then shared-memory
 // loads (32-bit shared addresses, ld.shared).  Tiles whose whole window is background (window sum
-// 0, four taps of the global SAT) skip the load.  Non-background patches of the tile are
+// 0, four taps of the global SAT) do no further work.  Non-background patches of the tile are
 // compacted (ballot) so that every lane of the traversal loop owns a live patch x tree pair; lanes
 // of a warp are neighbouring patches of the same tree, so the upper levels read the same node
 // record (broadcast) and nearby taps.
 // kMode 0: general rectangles, nodes through the LSU path; 1: general, nodes through the texture
-// path; 2: uniform rectangles (box-sum tile, UniNode through the texture path); 3: the same with
-// UniNode through the LSU path; 4 and 5: as 2 and 3, but the TMA load brings a window of the
-// box-sum image (box_image_kernel) instead of the summed-area table, so the tile needs no
-// conversion and is (sw - rw + 1)-ish wide instead of (sw + 1)-ish; 6: as 4 with TWO walks per
-// thread in flight (two independent fetch -> tap -> compare chains hide each other's latency).
+// path; 2: uniform rectangles (box-sum tile, UniNode through the texture path); 4: as 2, but the
+// TMA load brings a window of the box-sum image (box_image_kernel) instead of the summed-area
+// table, so the tile needs no conversion and is (sw - rw + 1)-ish wide instead of (sw + 1)-ish.
+// Mode 4 fetches the nodes of its first kLdgLevels levels through the LSU path.
+constexpr uint32_t kLdgLevels = 7;  // measured: 1.071 -> 1.048 ms (3: 1.057, 5: 1.051, 7-11: 1.048, 13: 1.057)
 template <int kThreads, int kMode>
-__global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_kernel(const __grid_constant__ CUtensorMap sat_map,
+__global__ void __launch_bounds__(kThreads, kThreads == 1024 ? 2 : 3) traverse_kernel(const __grid_constant__ CUtensorMap sat_map,
                                                             cudaTextureObject_t hot_tex,
                                                             const HotNode* __restrict__ hot,
                                                             const UniNode* __restrict__ uni,
@@ -603,8 +566,7 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
                                                             const int32_t* __restrict__ roots, int32_t* __restrict__ leaf,
                                                             const uint32_t* __restrict__ sat,
                                                             FrameState* __restrict__ fs, Geometry g, TilePlan tp,
-                                                            uint32_t uni_rw, uint32_t uni_rh, const PairRec* __restrict__ pair_recs,
-                                                            const int32_t* __restrict__ pair_roots, const int32_t* __restrict__ pair_perm) {
+                                                            uint32_t uni_rw, uint32_t uni_rh) {
     extern __shared__ uint8_t smem_raw[];
     // 128-byte aligned tile (TMA destination), then the barrier, then the compacted patch list;
     // everything is addressed through 32-bit shared-window addresses
@@ -618,7 +580,6 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
     const uint32_t tile_x = blockIdx.x % tp.tiles_x, tile_y = blockIdx.x / tp.tiles_x;
     const uint32_t px0 = tile_x * tp.tpx, py0 = tile_y * tp.tpy;  // first patch of the tile
     const uint32_t tid = threadIdx.x;
-    const uint32_t npt = tp.tpx * tp.tpy;
     const int T = (int)g.n_trees;
     int32_t* leaf_f = leaf + (size_t)frame * T * g.P;
 
@@ -630,15 +591,13 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
         asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar_a), "r"(1u) : "memory");
         fence_mbar_init();
         s_nlive = 0;
-        if (tp.tma_first) {
-            // the load is issued before the tile's background check and lands while warp 0 tests
-            // the window (one global round trip less in front of every non-empty tile)
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(tile_bytes) : "memory");
-            asm volatile(
-                "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(tile_a),
-                "l"(&sat_map), "r"((int)ax0), "r"((int)y0), "r"((int)frame), "r"(bar_a)
-                : "memory");
-        }
+        // the load is issued before the tile's background check and lands while warp 0 tests the
+        // window (one global round trip less in front of every non-empty tile; measured 1.110 -> 1.052 ms)
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(tile_bytes) : "memory");
+        asm volatile(
+            "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(tile_a),
+            "l"(&sat_map), "r"((int)ax0), "r"((int)y0), "r"((int)frame), "r"(bar_a)
+            : "memory");
     }
     if (tid < 32u) {
         // window of the tile's patches: [x0, x1) x [y0, y1); every patch of the tile is background
@@ -646,7 +605,7 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
         const uint32_t lastx = min(px0 + tp.tpx, g.npx) - 1u, lasty = min(py0 + tp.tpy, g.npy) - 1u;
         const uint32_t x1 = lastx * g.stride + g.sw, y1 = lasty * g.stride + g.sh;
         bool any;
-        if (kMode >= 4) {
+        if (kMode == 4) {
             // covered by rw x rh rectangles of the box-sum image (the last one of a row / column
             // is pulled back inside the window; sums are non-negative, so overlap is harmless)
             const uint32_t nkx = (x1 - x0 + uni_rw - 1u) / uni_rw, nky = (y1 - y0 + uni_rh - 1u) / uni_rh;
@@ -666,21 +625,11 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
                                  __ldg(S + (size_t)y1 * g.sat_pitch + x0) + __ldg(S + (size_t)y0 * g.sat_pitch + x0);
             any = sum != 0u;
         }
-        if (tid == 0) {
-            s_empty = !any;
-            if (any && !tp.tma_first) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(tile_bytes) : "memory");
-                asm volatile(
-                    "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(tile_a),
-                    "l"(&sat_map), "r"((int)ax0), "r"((int)y0), "r"((int)frame), "r"(bar_a)
-                    : "memory");
-            }
-        }
+        if (tid == 0) s_empty = !any;
     }
     __syncthreads();
-    // an empty tile whose load is already in flight (tma_first) still waits for it: the CTA must not
-    // leave while the async proxy writes its shared memory
-    if (s_empty && !tp.tma_first) return;  // prediction.rs:567-571 fails for every patch of the tile: their leaf ids stay -1
+    // an empty tile still waits for its load: the CTA must not leave while the async proxy writes its
+    // shared memory
     {
         asm volatile(
             "{\n"
@@ -694,32 +643,26 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
             "r"(0u)
             : "memory");
     }
-    if (s_empty) return;
+    if (s_empty) return;  // prediction.rs:567-571 fails for every patch of the tile: their leaf ids stay -1
 
     // ---- background test (prediction.rs:567-571: mean over the whole patch > 0  <=>  sum != 0)
     const uint32_t tw4 = tp.tw * 4u;
     const uint32_t org_a = tile_a + dx * 4u;  // patch (0,0) of the tile
-    // patches in row order, 32 per warp, or (tp.blocked) in blocks of 8 x 4 patches, one per warp
+    // patches in blocks of 8 x 4, one per warp: the lanes of a warp stay on the same nodes for longer
+    // (measured 1.052 -> 1.037 ms against rows of 32 patches)
     const uint32_t nbx = (tp.tpx + 7u) >> 3;
-    const uint32_t n_lp = tp.blocked ? nbx * ((tp.tpy + 3u) >> 2) * 32u : ((npt + 31u) & ~31u);
+    const uint32_t n_lp = nbx * ((tp.tpy + 3u) >> 2) * 32u;
     for (uint32_t lp = tid; lp < n_lp; lp += kThreads) {
         bool ok = false;
         uint32_t packed = 0;
-        uint32_t lx, ly;
-        if (tp.blocked) {
-            const uint32_t blk = lp >> 5;
-            lx = (blk % nbx) * 8u + (lp & 7u);
-            ly = (blk / nbx) * 4u + ((lp >> 3) & 3u);
-        } else {
-            lx = lp % tp.tpx;
-            ly = lp / tp.tpx;
-        }
+        const uint32_t blk = lp >> 5;
+        const uint32_t lx = (blk % nbx) * 8u + (lp & 7u), ly = (blk / nbx) * 4u + ((lp >> 3) & 3u);
         if (lx < tp.tpx && ly < tp.tpy) {
             const uint32_t gx = px0 + lx, gy = py0 + ly;
             if (gx < g.npx && gy < g.npy) {
                 const uint32_t o = org_a + ly * g.stride * tw4 + lx * g.stride * 4u;
                 uint32_t sum;
-                if (kMode >= 4) {  // the patch covered by rw x rh rectangles, the last ones pulled back inside
+                if (kMode == 4) {  // the patch covered by rw x rh rectangles, the last ones pulled back inside
                     sum = 0;
                     for (uint32_t vy = 0; vy < g.sh; vy += uni_rh) {
                         const uint32_t ra = o + min(vy, g.sh - uni_rh) * tw4;
@@ -744,7 +687,7 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
     const uint32_t nlive = s_nlive;
     if (tid == 0 && nlive) atomicAdd(&fs[frame].n_valid, nlive);
 
-    if ((kMode == 2 || kMode == 3) && nlive) {
+    if (kMode == 2 && nlive) {
         // ---- uniform rectangles: turn the SAT tile into box sums in place,
         //      B[y][x] = S[y+rh][x+rw] - S[y][x+rw] - S[y+rh][x] + S[y][x]  (types.rs:317-339 for the
         //      rw x rh rectangle at (x, y)), so that a rectangle is ONE tap.  Rows go in waves of one
@@ -780,43 +723,7 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
     const uint4* hot4 = reinterpret_cast<const uint4*>(hot);
     // it / nlive by multiply-high (exact while it * nlive < 2^32)
     const uint32_t nl_magic = (nlive >= 2u && (unsigned long long)items * nlive < (1ull << 32)) ? (uint32_t)((1ull << 32) / nlive) + 1u : 0u;
-    if (kMode == 6) {
-        // two walks per thread: items it and it + kThreads
-        for (uint32_t it = tid; it < items; it += 2u * kThreads) {
-            const uint32_t itB = it + kThreads;
-            const bool hasB = itB < items;
-            const uint32_t tA = nl_magic ? __umulhi(it, nl_magic) : it / nlive;
-            const uint32_t tB = hasB ? (nl_magic ? __umulhi(itB, nl_magic) : itB / nlive) : 0u;
-            const uint32_t lpA = lds_u32(live_a + 4u * (it - tA * nlive));
-            const uint32_t lpB = hasB ? lds_u32(live_a + 4u * (itB - tB * nlive)) : 0u;
-            const uint32_t oA = org_a + ((lpA & 0xffffu) << 2), oB = org_a + ((lpB & 0xffffu) << 2);
-            int32_t nA = __ldg(roots + tA), nB = hasB ? __ldg(roots + tB) : -1;
-            while ((nA & nB) >= 0) {  // at least one of the two is still inside its tree
-                const bool a = nA >= 0, b2 = nB >= 0;
-                uint4 UA = make_uint4(0u, 0u, 0u, 0u), UB = UA;
-                if (a) UA = tex1Dfetch<uint4>(hot_tex, nA);
-                if (b2) UB = tex1Dfetch<uint4>(hot_tex, nB);
-                if (a) {
-                    const uint32_t s1 = lds_u32(oA + ((UA.x & 0xffffu) << 2)), s2 = lds_u32(oA + ((UA.x >> 16) << 2));
-                    const int32_t d2 = (int32_t)(s1 - s2) << 1, E = (int32_t)UA.w;
-                    int32_t next = d2 > E ? (int)UA.z : (int)UA.y;
-                    if (d2 == E) next = binarize_ieee(nodes, nA, s1, s2) ? (int)UA.z : (int)UA.y;
-                    nA = next;
-                    ++visits;
-                }
-                if (b2) {
-                    const uint32_t s1 = lds_u32(oB + ((UB.x & 0xffffu) << 2)), s2 = lds_u32(oB + ((UB.x >> 16) << 2));
-                    const int32_t d2 = (int32_t)(s1 - s2) << 1, E = (int32_t)UB.w;
-                    int32_t next = d2 > E ? (int)UB.z : (int)UB.y;
-                    if (d2 == E) next = binarize_ieee(nodes, nB, s1, s2) ? (int)UB.z : (int)UB.y;
-                    nB = next;
-                    ++visits;
-                }
-            }
-            leaf_f[(size_t)tA * g.P + (py0 + (lpA >> 24)) * g.npx + (px0 + ((lpA >> 16) & 0xffu))] = ~nA;
-            if (hasB) leaf_f[(size_t)tB * g.P + (py0 + (lpB >> 24)) * g.npx + (px0 + ((lpB >> 16) & 0xffu))] = ~nB;
-        }
-    } else if (kMode == 4) {
+    if (kMode == 4) {
         // the default walk (uniform rectangles, box-sum tile, nodes through the texture path), in two
         // passes.  The fast pass contains no call: an exact tie (2*(s1 - s2) == E, possible for even E
         // only) abandons the walk and marks the evaluation's leaf slot; the second pass, entered only
@@ -833,8 +740,8 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
             bool tie = false;
             // the first levels below the root, where the lanes of a warp still sit on a handful of nodes, through
             // the LSU path (a warp-wide load of one address is one wavefront; a texture fetch costs eight or more
-            // whatever the addresses): DH_TRAV_LDG_LEVELS
-            for (uint32_t lv = 0; lv < tp.ldg_levels && node >= 0; ++lv) {
+            // whatever the addresses)
+            for (uint32_t lv = 0; lv < kLdgLevels && node >= 0; ++lv) {
                 const uint4 U = __ldg(reinterpret_cast<const uint4*>(uni) + node);
                 const uint32_t s1 = lds_u32(o + ((U.x & 0xffffu) << 2)), s2 = lds_u32(o + ((U.x >> 16) << 2));
                 const int32_t d2 = (int32_t)(s1 - s2) << 1, E = (int32_t)U.w;
@@ -882,55 +789,6 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
                 *slot = ~node;
             }
         }
-    } else if (kMode == 7) {
-        // two levels per fetch: PairRec (dh_types.hpp).  The loop carries only the record index and
-        // the patch origin; the leaf's depth (= node visits of the walk) rides in the top bits of
-        // the leaf permutation entry.  An exact tie (possible for even e2 only) abandons the fast
-        // walk: that evaluation is redone by the one-level walk below, which owns the IEEE path.
-        for (uint32_t it = tid; it < items; it += kThreads) {
-            const uint32_t t = nl_magic ? __umulhi(it, nl_magic) : it / nlive;
-            const uint32_t o = org_a + ((lds_u32(live_a + 4u * (it - t * nlive)) & 0xffffu) << 2);
-            int32_t rec = __ldg(pair_roots + t);
-            bool tie = false;
-            while (rec >= 0) {
-                const PairRec R = ldg_pair(pair_recs + rec);
-                const uint32_t s1 = lds_u32(o + ((R.taps_x & 0xffffu) << 2)), s2 = lds_u32(o + ((R.taps_x >> 16) << 2));
-                const int32_t d1 = (int32_t)(s1 - s2) << 1;
-                const bool b1 = d1 > R.e2_x;
-                const uint32_t taps2 = b1 ? R.taps_c1 : R.taps_c0;
-                const int32_t e2 = b1 ? R.e2_c1 : R.e2_c0;
-                const uint32_t s3 = lds_u32(o + ((taps2 & 0xffffu) << 2)), s4 = lds_u32(o + ((taps2 >> 16) << 2));
-                const int32_t d2 = (int32_t)(s3 - s4) << 1;
-                if (d1 == R.e2_x || d2 == e2) {
-                    tie = true;
-                    break;
-                }
-                const uint32_t slot = (b1 ? 2u : 0u) + (d2 > e2 ? 1u : 0u);
-                const uint32_t mask = R.tail & 15u, below = (uint32_t)__popc(mask & ((1u << slot) - 1u));
-                rec = ((mask >> slot) & 1u) ? ~(int32_t)((R.tail >> 6) + below) : (int32_t)(R.first + slot - below);
-            }
-            int32_t leaf_id;
-            if (!tie) {
-                const uint32_t v = (uint32_t)__ldg(pair_perm + ~rec);  // global leaf id | depth << 26
-                leaf_id = (int32_t)(v & 0x3ffffffu);
-                visits += v >> 26;
-            } else {
-                int32_t node = __ldg(roots + t);
-                while (node >= 0) {
-                    const uint4 U = tex1Dfetch<uint4>(hot_tex, node);
-                    const uint32_t s1 = lds_u32(o + ((U.x & 0xffffu) << 2)), s2 = lds_u32(o + ((U.x >> 16) << 2));
-                    const int32_t d2 = (int32_t)(s1 - s2) << 1, E = (int32_t)U.w;
-                    int32_t next = d2 > E ? (int)U.z : (int)U.y;
-                    if (d2 == E) next = binarize_ieee(nodes, node, s1, s2) ? (int)U.z : (int)U.y;
-                    node = next;
-                    ++visits;
-                }
-                leaf_id = ~node;
-            }
-            const uint32_t lp = lds_u32(live_a + 4u * (it - t * nlive));
-            const uint32_t gp = (py0 + (lp >> 24)) * g.npx + (px0 + ((lp >> 16) & 0xffu));
-            leaf_f[(size_t)t * g.P + gp] = leaf_id;
-        }
     } else
     for (uint32_t it = tid; it < items; it += kThreads) {
         const uint32_t t = nl_magic ? __umulhi(it, nl_magic) : it / nlive;
@@ -938,10 +796,10 @@ __global__ void __launch_bounds__(kThreads, kThreads >= 768 ? 2 : 3) traverse_ke
         const uint32_t lx = (lp >> 16) & 0xffu, ly = lp >> 24;
         const uint32_t o = org_a + ((lp & 0xffffu) << 2);
         int32_t node = __ldg(roots + t);
-        if (kMode >= 2) {
+        if (kMode == 2) {
             while (node >= 0) {
                 // taps, child[0], child[1], threshold * count
-                const uint4 U = (kMode == 2 || kMode == 4) ? tex1Dfetch<uint4>(hot_tex, node) : __ldg(reinterpret_cast<const uint4*>(uni) + node);
+                const uint4 U = tex1Dfetch<uint4>(hot_tex, node);
                 const uint32_t s1 = lds_u32(o + ((U.x & 0xffffu) << 2)), s2 = lds_u32(o + ((U.x >> 16) << 2));
                 // binarize (houghforest.rs:185-193) for equal pixel counts c: avg1 - avg2 > thr, decided
                 // on integers.  U.w = E (plan_nodes_kernel): the answer is 2*(s1 - s2) > E, and only
@@ -1196,8 +1054,8 @@ __global__ void __launch_bounds__(kPatchGateThreads) patch_gate_kernel(FrameBuff
     }
 }
 
-// kFused: one pass over the votes of every pair feeds both grids (a vote is an offset and a rotation;
-// the pair's tag says which of the two spread gates is open) instead of one pass per grid.
+// One pass over the votes of every pair feeds both grids (a vote is an offset and a rotation; the
+// pair's tag says which of the two spread gates is open).
 // kFromList: the patch gate has already been applied by patch_gate_kernel: the CTA
 // takes slices of kGateThreads entries of the frame's gated-patch list (blockIdx.x, + gridDim.x, ...)
 // instead of gating the kGateThreads patches of its own index range, so that every CTA that runs
@@ -1206,7 +1064,7 @@ __global__ void __launch_bounds__(kPatchGateThreads) patch_gate_kernel(FrameBuff
 // kFrameK: the frame's K (and, in phase A, K^-1) come from frame_k instead of g, copied once per CTA
 // into 72 bytes of shared memory behind the other arrays: this kernel runs at the 40-register cap of
 // 3 CTAs of 512 threads per SM, and 9 more live registers spilled.
-template <bool kFused, bool kFromList, bool kFrameK>
+template <bool kFromList, bool kFrameK>
 __global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffers b, Geometry g, ForestDev f,
                                                                       const float* __restrict__ frame_k) {
     extern __shared__ __align__(16) uint8_t gate_smem[];
@@ -1337,17 +1195,14 @@ __global__ void __launch_bounds__(kGateThreads, 3) gate_coarse_kernel(FrameBuffe
                     if (slot < (uint32_t)kTouchedCap) s_touched[slot] = (uint16_t)cell;
                 }
             };
-            if (kFused) {
-                // one pass: item j of a pair is its centre vote j (j < n_c) and its rotation cell j (j < n_r <= n_votes)
+            {
+                // item j of a pair is its centre vote j (j < n_c) and its rotation cell j (j < n_r <= n_votes)
                 const uint32_t tag = (n_c ? 1u : 0u) | (n_r << 1);
                 for_each_vote(max(n_c, n_r), v0, wgt, tag, h, s_slots[tid >> 5], lane,
                               [&](uint32_t vote, uint32_t ow, uint32_t tg, const float4& c, uint32_t j) {
                                   if (tg & 1u) centre_vote(vote, ow, c);
                                   if (j < (tg >> 1)) rot_vote(vote, ow);
                               });
-            } else {
-                for_each_vote(n_c, v0, wgt, 0u, h, s_slots[tid >> 5], lane, [&](uint32_t vote, uint32_t ow, uint32_t, const float4& c, uint32_t) { centre_vote(vote, ow, c); });
-                for_each_vote(n_r, v0, wgt, 0u, h, s_slots[tid >> 5], lane, [&](uint32_t vote, uint32_t ow, uint32_t, const float4&, uint32_t) { rot_vote(vote, ow); });
             }
         }
         if (!kFromList) break;
@@ -1638,8 +1493,7 @@ constexpr int kMsWarps = kMsThreads / 32;
 constexpr int kMsSegment = 1024;  // non-zero window cells summed per pass
 constexpr uint32_t kMsChunks = kKernelCells / 32;  // 250 steps of 32 cells
 constexpr int kMsLoads = (kKernelCells + kMsThreads - 1) / kMsThreads;  // 16 window cells per thread
-constexpr int kMsSmemBytes = kKernelCells * 4 + 4 * kMsSegment * 4;   // window + summands
-constexpr int kMsSmemBytesCompact = kMsSegment * 8 + 4 * kMsSegment * 4 + (kMsLoads / 2) * kMsThreads * 4;  // list of non-zero cells + summands + cell offsets
+constexpr int kMsSmemBytes = kMsSegment * 8 + 4 * kMsSegment * 4 + (kMsLoads / 2) * kMsThreads * 4;  // list of non-zero cells + summands + cell offsets
 constexpr uint32_t kMsNoCell = 0xffffu;  // packed cell offset of a thread's load slot beyond the window
 
 __device__ __forceinline__ void store_result(dh_result* r, uint32_t which, const int32_t* pos) {
@@ -1677,19 +1531,17 @@ __device__ __noinline__ void rebuild_cube(const float4* __restrict__ gated, uint
     __syncthreads();
 }
 
-// kCompact: the window never goes to shared memory.  A thread keeps its 16 cells in registers from the
-// gather to the ranking, the non-zero ones are written as (cell, value) at their rank, and the summands
-// are then computed densely, one thread per non-zero cell (the kCompact = false form walks all 250
-// chunks of 32 cells with only the non-zero lanes working: 53 % of the kernel's instructions, measured).
-template <bool kCompact>
+// The window never goes to shared memory.  A thread keeps its 16 cells in registers from the gather to
+// the ranking, the non-zero ones are written as (cell, value) at their rank, and the summands are then
+// computed densely, one thread per non-zero cell (walking all 250 chunks of 32 cells with only the
+// non-zero lanes working took 53 % of the kernel's instructions, measured).
 __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b, Geometry g, ForestDev f, uint32_t iterations,
                                                                   uint32_t n_items) {
     extern __shared__ __align__(16) uint8_t ms_smem[];
-    uint32_t* s_win = reinterpret_cast<uint32_t*>(ms_smem);  // [8000] window cells in reference order (!kCompact)
-    uint2* s_list = reinterpret_cast<uint2*>(ms_smem);       // [kMsSegment] (ord, value) of the non-zero cells by rank (kCompact)
-    float(*s_terms)[kMsSegment] = reinterpret_cast<float(*)[kMsSegment]>(ms_smem + (kCompact ? kMsSegment * 8 : kKernelCells * 4));  // [4][kMsSegment]
+    uint2* s_list = reinterpret_cast<uint2*>(ms_smem);       // [kMsSegment] (ord, value) of the non-zero cells by rank
+    float(*s_terms)[kMsSegment] = reinterpret_cast<float(*)[kMsSegment]>(ms_smem + kMsSegment * 8);  // [4][kMsSegment]
                                                        // summands (num x,y,z, den) in reference order
-    uint32_t* s_offp = reinterpret_cast<uint32_t*>(ms_smem + kMsSegment * 8 + 4 * kMsSegment * 4);  // [kMsLoads / 2][kMsThreads] (kCompact)
+    uint32_t* s_offp = reinterpret_cast<uint32_t*>(ms_smem + kMsSegment * 8 + 4 * kMsSegment * 4);  // [kMsLoads / 2][kMsThreads]
     __shared__ uint32_t s_mask[kMsChunks];             // non-zero window cells, bit j of word c = ord c*32+j
     __shared__ uint32_t s_off[kMsChunks + 1];          // rank of the first non-zero cell of every chunk
     __shared__ int32_t s_hist[kMsHistory + 1][3];      // positions P_0 (seed), P_1, ... for cycle detection
@@ -1697,20 +1549,18 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
     __shared__ uint32_t s_flags, s_done;
     __shared__ uint32_t s_item;
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    // kCompact: cube offsets of this thread's window cells ord = j * kMsThreads + tid, two per word,
-    // computed once and parked in shared memory (eight registers less across the rounds)
-    if (kCompact) {
+    // cube offsets of this thread's window cells ord = j * kMsThreads + tid, two per word, computed
+    // once and parked in shared memory (eight registers less across the rounds)
 #pragma unroll
-        for (int j = 0; j < kMsLoads; j += 2) {
-            uint32_t pk = 0;
+    for (int j = 0; j < kMsLoads; j += 2) {
+        uint32_t pk = 0;
 #pragma unroll
-            for (int u = 0; u < 2; ++u) {
-                const uint32_t ord = (uint32_t)(j + u) * kMsThreads + tid;
-                const uint32_t xo = ord / 400u, yo = (ord / 20u) % 20u, zo = ord % 20u;
-                pk |= (ord < (uint32_t)kKernelCells ? (xo * kBox + yo) * kBox + zo : kMsNoCell) << (16 * u);
-            }
-            s_offp[(j >> 1) * kMsThreads + tid] = pk;
+        for (int u = 0; u < 2; ++u) {
+            const uint32_t ord = (uint32_t)(j + u) * kMsThreads + tid;
+            const uint32_t xo = ord / 400u, yo = (ord / 20u) % 20u, zo = ord % 20u;
+            pk |= (ord < (uint32_t)kKernelCells ? (xo * kBox + yo) * kBox + zo : kMsNoCell) << (16 * u);
         }
+        s_offp[(j >> 1) * kMsThreads + tid] = pk;
     }
     // The CTAs of the launch (as many as fit the GPU at once) take accumulators from a counter: the first
     // one by their index, the following ones as they become free (a launch of one CTA per accumulator ran
@@ -1754,42 +1604,19 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
         // gather the 20^3 window, all loads of a thread in flight at once.  ord enumerates the cells in
         // the reference loop order (x outermost, z innermost); a warp's load j is chunk j * kMsWarps + warp.
         uint32_t v[kMsLoads];
-        if (kCompact) {
 #pragma unroll
-            for (int j = 0; j < kMsLoads; j += 2) {
-                const uint32_t pk = s_offp[(j >> 1) * kMsThreads + tid];
-                const uint32_t o0 = pk & 0xffffu, o1 = pk >> 16;
-                v[j] = o0 != kMsNoCell ? __ldcg(box + base + o0) : 0u;
-                v[j + 1] = o1 != kMsNoCell ? __ldcg(box + base + o1) : 0u;
-            }
-            // non-zero mask of every 32-cell chunk straight from the registers
+        for (int j = 0; j < kMsLoads; j += 2) {
+            const uint32_t pk = s_offp[(j >> 1) * kMsThreads + tid];
+            const uint32_t o0 = pk & 0xffffu, o1 = pk >> 16;
+            v[j] = o0 != kMsNoCell ? __ldcg(box + base + o0) : 0u;
+            v[j + 1] = o1 != kMsNoCell ? __ldcg(box + base + o1) : 0u;
+        }
+        // non-zero mask of every 32-cell chunk straight from the registers
 #pragma unroll
-            for (int j = 0; j < kMsLoads; ++j) {
-                const uint32_t m = __ballot_sync(0xffffffffu, v[j] != 0u);
-                const uint32_t c = (uint32_t)j * kMsWarps + warp;
-                if (lane == 0 && c < kMsChunks) s_mask[c] = m;
-            }
-        } else {
-#pragma unroll
-            for (int j = 0; j < kMsLoads; ++j) {
-                const uint32_t ord = (uint32_t)j * kMsThreads + tid;
-                v[j] = 0u;
-                if (ord < (uint32_t)kKernelCells) {
-                    const uint32_t xo = ord / 400u, yo = (ord / 20u) % 20u, zo = ord % 20u;
-                    v[j] = __ldcg(box + base + (xo * kBox + yo) * kBox + zo);
-                }
-            }
-#pragma unroll
-            for (int j = 0; j < kMsLoads; ++j) {
-                const uint32_t ord = (uint32_t)j * kMsThreads + tid;
-                if (ord < (uint32_t)kKernelCells) s_win[ord] = v[j];
-            }
-            __syncthreads();
-            // non-zero mask of every 32-cell chunk
-            for (uint32_t c = warp; c < kMsChunks; c += kMsWarps) {
-                const uint32_t m = __ballot_sync(0xffffffffu, s_win[c * 32u + lane] != 0u);
-                if (lane == 0) s_mask[c] = m;
-            }
+        for (int j = 0; j < kMsLoads; ++j) {
+            const uint32_t m = __ballot_sync(0xffffffffu, v[j] != 0u);
+            const uint32_t c = (uint32_t)j * kMsWarps + warp;
+            if (lane == 0 && c < kMsChunks) s_mask[c] = m;
         }
         __syncthreads();
         // (warp 0) the exclusive prefix of the chunks' populations = rank of their first non-zero cell
@@ -1813,46 +1640,28 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
         const uint32_t nnz = s_off[kMsChunks];
         float acc = 0.0f;
         for (uint32_t seg = 0; seg < nnz; seg += kMsSegment) {
-            if (kCompact) {
-                // every non-zero cell goes to the list at its rank in reference order ...
+            // every non-zero cell goes to the list at its rank in reference order ...
 #pragma unroll
-                for (int j = 0; j < kMsLoads; ++j) {
-                    if (v[j] != 0u) {
-                        const uint32_t c = (uint32_t)j * kMsWarps + warp;
-                        const uint32_t r = s_off[c] + (uint32_t)__popc(s_mask[c] & ((1u << lane) - 1u)) - seg;
-                        if (r < (uint32_t)kMsSegment) s_list[r] = make_uint2((uint32_t)j * kMsThreads + tid, v[j]);
-                    }
+            for (int j = 0; j < kMsLoads; ++j) {
+                if (v[j] != 0u) {
+                    const uint32_t c = (uint32_t)j * kMsWarps + warp;
+                    const uint32_t r = s_off[c] + (uint32_t)__popc(s_mask[c] & ((1u << lane) - 1u)) - seg;
+                    if (r < (uint32_t)kMsSegment) s_list[r] = make_uint2((uint32_t)j * kMsThreads + tid, v[j]);
                 }
-                __syncthreads();
-                // ... and its four summands are computed by the thread of that rank
-                const uint32_t cnt = min((uint32_t)kMsSegment, nnz - seg);
-                for (uint32_t r = tid; r < cnt; r += kMsThreads) {
-                    const uint2 e = s_list[r];
-                    const uint32_t xo = e.x / 400u, yo = (e.x / 20u) % 20u, zo = e.x % 20u;
-                    // influence * factor with kernel[(x+10, y+10, z+10)], dense index z*400 + y*20 + x
-                    // (meanshift.rs:370-377, 78-88); then abs_pos * that
-                    const float wgt = __fmul_rn(__ldg(f.ms_kernel + zo * 400u + yo * 20u + xo), (float)e.y);
-                    s_terms[0][r] = __fmul_rn((float)(int)((uint32_t)pos[0] + xo - 10u), wgt);
-                    s_terms[1][r] = __fmul_rn((float)(int)((uint32_t)pos[1] + yo - 10u), wgt);
-                    s_terms[2][r] = __fmul_rn((float)(int)((uint32_t)pos[2] + zo - 10u), wgt);
-                    s_terms[3][r] = wgt;
-                }
-            } else {
-                // every non-zero cell stages its four summands at its rank in reference order
-                for (uint32_t c = warp; c < kMsChunks; c += kMsWarps) {
-                    if (s_off[c + 1] <= seg || s_off[c] >= seg + kMsSegment) continue;  // warp-uniform
-                    const uint32_t m = s_mask[c];
-                    if (!((m >> lane) & 1u)) continue;
-                    const uint32_t r = s_off[c] + (uint32_t)__popc(m & ((1u << lane) - 1u));
-                    if (r < seg || r >= seg + kMsSegment) continue;
-                    const uint32_t ord = c * 32u + lane;
-                    const uint32_t xo = ord / 400u, yo = (ord / 20u) % 20u, zo = ord % 20u;
-                    const float wgt = __fmul_rn(__ldg(f.ms_kernel + zo * 400u + yo * 20u + xo), (float)s_win[ord]);
-                    s_terms[0][r - seg] = __fmul_rn((float)(int)((uint32_t)pos[0] + xo - 10u), wgt);
-                    s_terms[1][r - seg] = __fmul_rn((float)(int)((uint32_t)pos[1] + yo - 10u), wgt);
-                    s_terms[2][r - seg] = __fmul_rn((float)(int)((uint32_t)pos[2] + zo - 10u), wgt);
-                    s_terms[3][r - seg] = wgt;
-                }
+            }
+            __syncthreads();
+            // ... and its four summands are computed by the thread of that rank
+            const uint32_t cnt = min((uint32_t)kMsSegment, nnz - seg);
+            for (uint32_t r = tid; r < cnt; r += kMsThreads) {
+                const uint2 e = s_list[r];
+                const uint32_t xo = e.x / 400u, yo = (e.x / 20u) % 20u, zo = e.x % 20u;
+                // influence * factor with kernel[(x+10, y+10, z+10)], dense index z*400 + y*20 + x
+                // (meanshift.rs:370-377, 78-88); then abs_pos * that
+                const float wgt = __fmul_rn(__ldg(f.ms_kernel + zo * 400u + yo * 20u + xo), (float)e.y);
+                s_terms[0][r] = __fmul_rn((float)(int)((uint32_t)pos[0] + xo - 10u), wgt);
+                s_terms[1][r] = __fmul_rn((float)(int)((uint32_t)pos[1] + yo - 10u), wgt);
+                s_terms[2][r] = __fmul_rn((float)(int)((uint32_t)pos[2] + zo - 10u), wgt);
+                s_terms[3][r] = wgt;
             }
             __syncthreads();
             if (warp == 0 && lane < 4) {  // sequential f32 accumulation in reference order (meanshift.rs:337-380)
@@ -2554,20 +2363,21 @@ bool box_image_supported(uint32_t w, uint32_t h, uint32_t sw, uint32_t sh, uint3
     return ((sw + rw - 1u) / rw) * ((sh + rh - 1u) / rh) <= 64u;
 }
 
-template <int kPx>
-static int launch_box_image_t(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, bool whole, cudaStream_t s) {
-    // strips: a multiple of kPx output columns each, at most 32*kPx + 1 - rw (column c reads P[c + rw] <= P[32*kPx])
-    const uint32_t max_out = (32u * kPx + 1u - g.rw) & ~(uint32_t)(kPx - 1);
+int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, cudaStream_t s) {
+    static const bool allow_whole = !(std::getenv("DH_BOX_WHOLE") && std::atoi(std::getenv("DH_BOX_WHOLE")) == 0);
+    const bool whole = allow_whole && (g.rw & 7u) == 0u;
+    // strips: a multiple of kBoxPx output columns each, at most 32*kBoxPx + 1 - rw (column c reads P[c + rw] <= P[32*kBoxPx])
+    const uint32_t max_out = (32u * kBoxPx + 1u - g.rw) & ~(uint32_t)(kBoxPx - 1);
     const uint32_t n_strips = (g.box_w + max_out - 1u) / max_out;
-    const uint32_t strip_out = (((g.box_w + n_strips - 1u) / n_strips) + kPx - 1u) & ~(uint32_t)(kPx - 1);
-    const uint32_t per_warp = (whole ? 0u : 2u * (32u * kPx + 16u) * 4u) + g.rh * 64u * kPx;
+    const uint32_t strip_out = (((g.box_w + n_strips - 1u) / n_strips) + kBoxPx - 1u) & ~(uint32_t)(kBoxPx - 1);
+    const uint32_t per_warp = (whole ? 0u : 2u * (32u * kBoxPx + 16u) * 4u) + g.rh * 64u * kBoxPx;
     uint32_t wpc = n_strips <= (uint32_t)kBoxMaxWarps ? n_strips : 2u;  // warps per CTA
     while (wpc > 1u && wpc * per_warp > 100u * 1024u) --wpc;           // tall rectangles: long pixel rings
     const uint32_t smem = wpc * per_warp;
     static SmemConfig configured;
     if (configured.raise(smem)) {
-        cudaFuncSetAttribute(box_image_kernel<kPx, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(box_image_kernel<kPx, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(box_image_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(box_image_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     }
     // bands: a band re-reads the rh - 1 rows above it, so few of them, but enough that the launch has
     // about two rounds of CTAs (the CTAs of a single round do not divide evenly over the SMs and the
@@ -2584,20 +2394,12 @@ static int launch_box_image_t(const FrameBuffers& b, const Geometry& g, uint32_t
     const uint32_t n_units = n_strips * n_bands * n_frames;
     const uint32_t blocks = (n_units + wpc - 1u) / wpc;
     if (whole)
-        box_image_kernel<kPx, true><<<blocks, wpc * 32u, smem, s>>>(b.depth, b.box, g.w, g.h, g.rw, g.rh, g.box_w, g.box_h, g.box_pitch,
-                                                                   strip_out, n_strips, band_rows, n_bands, n_units);
+        box_image_kernel<true><<<blocks, wpc * 32u, smem, s>>>(b.depth, b.box, g.w, g.h, g.rw, g.rh, g.box_w, g.box_h, g.box_pitch,
+                                                              strip_out, n_strips, band_rows, n_bands, n_units);
     else
-        box_image_kernel<kPx, false><<<blocks, wpc * 32u, smem, s>>>(b.depth, b.box, g.w, g.h, g.rw, g.rh, g.box_w, g.box_h, g.box_pitch,
-                                                                    strip_out, n_strips, band_rows, n_bands, n_units);
+        box_image_kernel<false><<<blocks, wpc * 32u, smem, s>>>(b.depth, b.box, g.w, g.h, g.rw, g.rh, g.box_w, g.box_h, g.box_pitch,
+                                                               strip_out, n_strips, band_rows, n_bands, n_units);
     return 1;
-}
-
-int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, cudaStream_t s) {
-    static const bool allow_whole = !(std::getenv("DH_BOX_WHOLE") && std::atoi(std::getenv("DH_BOX_WHOLE")) == 0);
-    static const int px = std::getenv("DH_BOX_PX") ? std::atoi(std::getenv("DH_BOX_PX")) : 8;
-    // 4 pixels per lane: only through the shuffle path (rw a multiple of 4, at most 124)
-    if (px == 4 && allow_whole && (g.rw & 3u) == 0u && g.rw <= 124u) return launch_box_image_t<4>(b, g, n_frames, n_sms, true, s);
-    return launch_box_image_t<8>(b, g, n_frames, n_sms, allow_whole && (g.rw & 7u) == 0u, s);
 }
 
 uint32_t traverse_smem_bytes(uint32_t tw, uint32_t th, uint32_t patches_per_tile) {
@@ -2622,44 +2424,26 @@ static void launch_traverse_t(const CUtensorMap& sat_map, const FrameBuffers& b,
         cudaFuncSetAttribute(traverse_kernel<kThreads, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
         cudaFuncSetAttribute(traverse_kernel<kThreads, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
         cudaFuncSetAttribute(traverse_kernel<kThreads, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
-        cudaFuncSetAttribute(traverse_kernel<kThreads, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
         cudaFuncSetAttribute(traverse_kernel<kThreads, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
-        cudaFuncSetAttribute(traverse_kernel<kThreads, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
-        cudaFuncSetAttribute(traverse_kernel<kThreads, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
-        cudaFuncSetAttribute(traverse_kernel<kThreads, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_bytes);
     }
-    static const bool two_walks = std::getenv("DH_TRAV_ILP") && std::atoi(std::getenv("DH_TRAV_ILP")) == 2;
     dim3 gr(tp.tiles_x * tp.tiles_y, n_frames);
-    if (f.uni && g.rw && f.pair_recs)
-        traverse_kernel<kThreads, 7><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, f.hot_tex, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.box,
-                                                                       b.fs, g, tp, f.uni_rw, f.uni_rh, f.pair_recs, f.pair_roots, f.pair_leaf_perm);
-    else if (f.uni && g.rw && f.hot_tex && two_walks)
-        traverse_kernel<kThreads, 6><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, f.hot_tex, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.box,
-                                                                       b.fs, g, tp, f.uni_rw, f.uni_rh, f.pair_recs, f.pair_roots, f.pair_leaf_perm);
-    else if (f.uni && g.rw && f.hot_tex)
+    if (f.uni && g.rw)
         traverse_kernel<kThreads, 4><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, f.hot_tex, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.box,
-                                                                       b.fs, g, tp, f.uni_rw, f.uni_rh, f.pair_recs, f.pair_roots, f.pair_leaf_perm);
-    else if (f.uni && g.rw)
-        traverse_kernel<kThreads, 5><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, 0, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.box, b.fs, g,
-                                                                       tp, f.uni_rw, f.uni_rh, f.pair_recs, f.pair_roots, f.pair_leaf_perm);
-    else if (f.uni && f.hot_tex)
-        traverse_kernel<kThreads, 2><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, f.hot_tex, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.sat,
-                                                                       b.fs, g, tp, f.uni_rw, f.uni_rh, f.pair_recs, f.pair_roots, f.pair_leaf_perm);
+                                                                       b.fs, g, tp, f.uni_rw, f.uni_rh);
     else if (f.uni)
-        traverse_kernel<kThreads, 3><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, 0, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.sat, b.fs, g,
-                                                                       tp, f.uni_rw, f.uni_rh, f.pair_recs, f.pair_roots, f.pair_leaf_perm);
+        traverse_kernel<kThreads, 2><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, f.hot_tex, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.sat,
+                                                                       b.fs, g, tp, f.uni_rw, f.uni_rh);
     else if (f.hot_tex)
         traverse_kernel<kThreads, 1><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, f.hot_tex, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.sat,
-                                                                       b.fs, g, tp, 0u, 0u, nullptr, nullptr, nullptr);
+                                                                       b.fs, g, tp, 0u, 0u);
     else
         traverse_kernel<kThreads, 0><<<gr, kThreads, tp.smem_bytes, s>>>(sat_map, 0, f.hot, f.uni, f.nodes, f.roots, b.leaf, b.sat, b.fs, g,
-                                                                       tp, 0u, 0u, nullptr, nullptr, nullptr);
+                                                                       tp, 0u, 0u);
 }
 
 void launch_traverse(const CUtensorMap& sat_map, const FrameBuffers& b, const Geometry& g, const TilePlan& tp,
                      const ForestDev& f, uint32_t n_frames, cudaStream_t s) {
     if (tp.threads >= 1024) launch_traverse_t<1024>(sat_map, b, g, tp, f, n_frames, s);
-    else if (tp.threads >= 768) launch_traverse_t<768>(sat_map, b, g, tp, f, n_frames, s);
     else launch_traverse_t<512>(sat_map, b, g, tp, f, n_frames, s);
 }
 
@@ -2667,11 +2451,6 @@ void launch_plan_nodes(const NodeRec* nodes, HotNode* hot, UniNode* uni, size_t 
                        const double* prob_codes, cudaStream_t s) {
     if (n_nodes == 0) return;
     plan_nodes_kernel<<<(unsigned)((n_nodes + 255) / 256), 256, 0, s>>>(nodes, hot, uni, n_nodes, tile_width, prob_codes);
-}
-
-void launch_plan_pairs(const PairTopo* topo, const UniNode* uni, PairRec* recs, size_t n_recs, cudaStream_t s) {
-    if (n_recs == 0) return;
-    plan_pairs_kernel<<<(unsigned)((n_recs + 255) / 256), 256, 0, s>>>(topo, uni, recs, n_recs);
 }
 
 uint32_t sat_band_rows() { return (uint32_t)kSatBandRows; }
@@ -2686,11 +2465,9 @@ static int launch_gate_coarse_t(const FrameBuffers& b, const Geometry& g, const 
     constexpr int kSmem = kGateSmemBytes + (kFrameK ? kFrameKFloats * 4 : 0);
     static SmemConfig configured;
     if (configured.raise((uint32_t)kSmem)) {
-        cudaFuncSetAttribute(gate_coarse_kernel<true, false, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-        cudaFuncSetAttribute(gate_coarse_kernel<false, false, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-        cudaFuncSetAttribute(gate_coarse_kernel<true, true, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+        cudaFuncSetAttribute(gate_coarse_kernel<false, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+        cudaFuncSetAttribute(gate_coarse_kernel<true, kFrameK>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     }
-    static const bool fused = !(std::getenv("DH_GATE_FUSED") && std::atoi(std::getenv("DH_GATE_FUSED")) == 0);
     const uint32_t per_frame = (g.P + kGateThreads - 1) / kGateThreads;
     if (from_list) {
         // the patch gate writes the frames' gated-patch lists, the seed-grid CTAs take slices of them.  Few CTAs per
@@ -2701,12 +2478,10 @@ static int launch_gate_coarse_t(const FrameBuffers& b, const Geometry& g, const 
         const uint32_t ctas = std::max<uint32_t>(1u, std::min<uint32_t>(per_frame, want ? want : std::max<uint32_t>(4u, fill)));
         patch_gate_kernel<kFrameK><<<dim3((g.P + kPatchGateThreads * kPatchGatePer - 1) / (kPatchGateThreads * kPatchGatePer), n_frames),
                                      kPatchGateThreads, 0, s>>>(b, g, f, frame_k);
-        gate_coarse_kernel<true, true, kFrameK><<<dim3(ctas, n_frames), kGateThreads, kSmem, s>>>(b, g, f, frame_k);
+        gate_coarse_kernel<true, kFrameK><<<dim3(ctas, n_frames), kGateThreads, kSmem, s>>>(b, g, f, frame_k);
         return 2;
     }
-    dim3 gr(per_frame, n_frames);
-    if (fused) gate_coarse_kernel<true, false, kFrameK><<<gr, kGateThreads, kSmem, s>>>(b, g, f, frame_k);
-    else gate_coarse_kernel<false, false, kFrameK><<<gr, kGateThreads, kSmem, s>>>(b, g, f, frame_k);
+    gate_coarse_kernel<false, kFrameK><<<dim3(per_frame, n_frames), kGateThreads, kSmem, s>>>(b, g, f, frame_k);
     return 1;
 }
 
@@ -2733,17 +2508,12 @@ int launch_seed_and_cubes(const FrameBuffers& b, const Geometry& g, const Forest
 int launch_meanshift(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t iterations,
                      int n_sms, cudaStream_t s) {
     static SmemConfig configured;
-    if (configured.raise((uint32_t)kMsSmemBytes)) {
-        cudaFuncSetAttribute(meanshift_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMsSmemBytes);
-        cudaFuncSetAttribute(meanshift_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMsSmemBytesCompact);
-    }
-    static const bool compact = !(std::getenv("DH_MS_COMPACT") && std::atoi(std::getenv("DH_MS_COMPACT")) == 0);
-    // persistent CTAs: three per SM (registers), DH_MS_PERSIST=0: one CTA per accumulator
-    static const bool persist = !(std::getenv("DH_MS_PERSIST") && std::atoi(std::getenv("DH_MS_PERSIST")) == 0);
+    if (configured.raise((uint32_t)kMsSmemBytes))
+        cudaFuncSetAttribute(meanshift_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMsSmemBytes);
+    // persistent CTAs: three per SM (registers; measured 0.247 -> 0.239 ms against one CTA per accumulator)
     const uint32_t n_items = 2u * n_frames;
-    const uint32_t grid = persist ? std::min<uint32_t>(n_items, 3u * (uint32_t)std::max(n_sms, 1)) : n_items;
-    if (compact) meanshift_kernel<true><<<grid, kMsThreads, kMsSmemBytesCompact, s>>>(b, g, f, iterations, n_items);
-    else meanshift_kernel<false><<<grid, kMsThreads, kMsSmemBytes, s>>>(b, g, f, iterations, n_items);
+    const uint32_t grid = std::min<uint32_t>(n_items, 3u * (uint32_t)std::max(n_sms, 1));
+    meanshift_kernel<<<grid, kMsThreads, kMsSmemBytes, s>>>(b, g, f, iterations, n_items);
     return 1;
 }
 

@@ -62,10 +62,6 @@ struct TilePlan {
                               // table window, or box-sum image window in box-image mode
     uint32_t smem_bytes;
     uint32_t threads;
-    uint32_t blocked;         // 1: the patches of a tile are enumerated in blocks of 8 x 4 (a warp = a compact block)
-                              // instead of row by row (experimental, DH_TRAV_BLOCK=1)
-    uint32_t tma_first;       // 1: the tile's TMA load is issued before its background check (DH_TRAV_TMA_FIRST)
-    uint32_t ldg_levels;      // levels below the root whose nodes the default walk fetches through the LSU path (DH_TRAV_LDG_LEVELS)
 };
 
 struct ForestDev {
@@ -75,11 +71,9 @@ struct ForestDev {
     const UniNode* uni;        // uniform-rectangle forests: 16-byte nodes for the box-sum traversal (or nullptr)
     uint32_t uni_rw, uni_rh;   // the common rectangle size
     const int32_t* roots;
-    // two-levels-per-record tables (PairRec, dh_types.hpp) for the box-sum traversal, or nullptr
-    const PairRec* pair_recs;
-    const PairTopo* pair_topo;
-    const int32_t* pair_roots;      // per tree: >= 0 record index, < 0 ~(device leaf number)
-    const int32_t* pair_leaf_perm;  // device leaf number -> global leaf id
+    // Unused: holds the offsets of the fields below, which the kernels that take ForestDev by value
+    // read (ptxas schedules patch_gate_kernel and gate_coarse_kernel differently when they move)
+    const void* unused_[4];
     const double* leaf_prob;
     const LeafInfo* leaf_info;
     const float4* offsets;     // per vote: x, y, z (mm), w unused — one 16-byte load
@@ -123,9 +117,8 @@ void launch_traverse(const CUtensorMap& sat_map, const FrameBuffers& b, const Ge
                      const ForestDev& f, uint32_t n_frames, cudaStream_t s);
 void launch_plan_nodes(const NodeRec* nodes, HotNode* hot, UniNode* uni, size_t n_nodes, uint32_t tile_width,
                        const double* prob_codes, cudaStream_t s);
-void launch_plan_pairs(const PairTopo* topo, const UniNode* uni, PairRec* recs, size_t n_recs, cudaStream_t s);
 // from_list: the patch gate runs as its own kernel and writes the frames' gated-patch lists; the seed-grid CTAs take
-// slices of the lists (DH_GATE_SPLIT, default) instead of gating the patches of their own index range.
+// slices of the lists instead of gating the patches of their own index range.
 // frame_k: nullptr = every frame has Geometry's K / Kinv; else a device table [n_frames][18] of each
 // frame's K then K^-1 (row-major), read by the kernels that project (dh_predict_frames).
 int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list, int n_sms,

@@ -66,34 +66,6 @@ struct alignas(16) UniNode {
 };
 static_assert(sizeof(UniNode) == 16, "UniNode must be 16 bytes");
 
-// Two tree levels in one 32-byte record (one LDG.E.256): an internal node X at an even depth
-// below its root together with its two children C0, C1.  A walk fetches ONE record per two levels;
-// the number of distinct cache lines a warp's divergent fetches touch (what bounds the traversal,
-// see DESIGN.md) drops accordingly.  The four grandchild slots s = 2*b1 + b2 (b1: X's decision,
-// b2: the child's) are either records or leaves: the slots that are records are consecutive
-// records starting at `first`, the slots that are leaves are consecutive DEVICE leaf numbers
-// starting at first_leaf (PairTables::leaf_perm maps them back to global leaf ids).  A child that
-// is itself a leaf carries a dummy test (taps 0, e2 INT_MAX: never greater, never equal) and both
-// of its slots name that leaf.
-struct alignas(32) PairRec {
-    uint32_t taps_x;   // as UniNode::taps
-    int32_t e2_x;
-    uint32_t taps_c0;
-    int32_t e2_c0;
-    uint32_t taps_c1;
-    int32_t e2_c1;
-    uint32_t first;    // record index of the first grandchild slot that is a record
-    uint32_t tail;     // first_leaf << 6 | child 1 is a leaf << 5 | child 0 is a leaf << 4 | mask of the slots that are leaves
-};
-static_assert(sizeof(PairRec) == 32, "PairRec must be one 32-byte sector");
-// Topology of a record, written on the host once per forest; plan_pairs_kernel turns it into
-// PairRec for the current tile plan, the walk reads it again only at exact ties (node indices
-// for the IEEE-division path).
-struct PairTopo {
-    int32_t x, c0, c1;  // global node indices (c < 0: that child is a leaf)
-    uint32_t first, tail;
-};
-
 // Everything the accumulator-cube kernel needs to know about a leaf before it touches its votes, in ONE
 // 32-byte sector (the kernel gathers one record per gated patch x tree pair, 13.7 M per 1024 frames of
 // configs[1], and the L1 miss path delivers about half a sector per cycle per SM: with LeafInfo and a

@@ -4,9 +4,10 @@ configs[2] (Biwi-shaped sequence sharded by frame), configs[3] (large forest: 50
 dense stride-1 sampling) and configs[4] (vote-heavy: a million votes per frame) are run against
 the oracle at sizes it finishes in seconds, and at (or near) full size through size-independent
 properties: batch == single frame, chunking / sharding independence, permutation equivariance,
-work-counter identities.  The variant test forces each fallback kernel (LSU node fetch, general
-rectangles instead of box sums, two-pass summed-area table, 512-thread traversal, one lane) and
-repeats the stage-by-stage comparison.
+work-counter identities.  The variant test forces each path the library selects for some input
+(LSU node fetch, general rectangles instead of box sums, box sums made in the tile, two-pass
+summed-area table, box-image launch shapes, 512-thread traversal, the patch gate with and without
+probability codes, lanes and chunks) and repeats the stage-by-stage comparison.
 """
 import numpy as np
 import pytest
@@ -38,40 +39,18 @@ VARIANTS = [
     {"DH_TEX": "0"},                                # general rectangles need the LSU path when the texture is off
     {"DH_UNIFORM": "0"},                            # general 8-tap traversal on a uniform forest
     {"DH_UNIFORM": "0", "DH_TEX": "0"},
-    {"DH_UNI_LDG": "1"},                            # box sums, nodes through the LSU path
     {"DH_SAT_BANDS": "0", "DH_BOX_IMAGE": "0"},     # two-pass summed-area table
     {"DH_BOX_IMAGE": "0"},                          # uniform forest on the summed-area table (box sums made in the tile)
-    {"DH_BOX_IMAGE": "0", "DH_UNI_LDG": "1"},
-    {"DH_BOX_PX": "4"},                             # box image with 4 pixels per lane
     {"DH_BOX_BANDS": "1"},                          # box image: one band per frame / five bands instead of the launch heuristic
     {"DH_BOX_BANDS": "5"},
     {"DH_BOX_WHOLE": "0"},                          # box image through warp-wide prefix sums (the path of widths not divisible by 8)
     {"DH_TRAV_THREADS": "512"},                     # 512-thread traversal tiles
-    {"DH_TRAV_ILP": "2", "DH_TRAV_THREADS": "768"}, # two walks in flight per thread, 768-thread tiles
-    {"DH_GATE_FUSED": "0"},                         # seed grids: one pass over the votes per grid instead of one for both
-    {"DH_TRAV_BLOCK": "0"},                         # a warp walks a row of 32 patches instead of a block of 8 x 4
-    {"DH_TRAV_BLOCK": "0", "DH_BOX_IMAGE": "0"},
-    {"DH_TRAV_TMA_FIRST": "0"},                     # the tile's TMA load is issued after its background check
-    {"DH_TRAV_TMA_FIRST": "0", "DH_BOX_IMAGE": "0"},
-    {"DH_TRAV_TMA_FIRST": "0", "DH_TRAV_BLOCK": "0"},
-    {"DH_TRAV_PAIR": "1"},                          # two tree levels per 32-byte record
-    {"DH_TRAV_PAIR": "1", "DH_TRAV_THREADS": "768", "DH_TRAV_TMA_FIRST": "0"},
-    {"DH_CUBE_CLEAR_FUSED": "0"},                   # one memset of all accumulator cubes per pass instead of the clear behind mean-shift
     {"DH_LANES": "1"},
     {"DH_LANES": "4", "DH_CHUNK_FRAMES": "2"},
-    {"DH_TRAV_LDG_LEVELS": "0"},                    # every node of the default walk through the texture path
-    {"DH_TRAV_LDG_LEVELS": "3", "DH_TRAV_SMEM": "98000"},
-    {"DH_TRAV_LDG_LEVELS": "40"},                   # ... through the LSU path
-    {"DH_NODE_ALIGN": "0"},                         # device node table in host order (no pad records in front of sibling pairs)
-    {"DH_NODE_ALIGN": "0", "DH_TRAV_PAIR": "1"},
-    {"DH_MS_PERSIST": "0"},                         # mean-shift: one CTA per accumulator instead of persistent CTAs
-    {"DH_MS_PERSIST": "0", "DH_MS_COMPACT": "0"},
-    {"DH_MS_COMPACT": "0"},                         # mean-shift: window staged in shared memory, summands per 32-cell chunk
     {"DH_GATE_SPLIT_MIN": "64"},                    # the library's default: small passes gate inside the seed-grid kernel
     {"DH_PROB_CODES": "0"},                         # no probability codes in the node table: the patch gate runs as its own kernel
     {"DH_PROB_CODES": "0", "DH_GATE_CTAS": "2"},
-    {"DH_GATE_SPLIT": "0"},                         # patch gate inside the seed-grid kernel instead of the traversal's tail
-    {"DH_GATE_SPLIT": "0", "DH_GATE_FUSED": "0"},
+    {"DH_PROB_CODES": "0", "DH_GATE_SPLIT_MIN": "64"},  # patch gate inside the seed-grid kernel, leaf words without codes
     {"DH_GATE_CTAS": "1"},                          # one seed-grid CTA per frame walks every slice of the gated-patch list
     {"DH_GATE_CTAS": "2", "DH_TRAV_THREADS": "512"},
     {"DH_BOX_IMAGE": "0", "DH_UNIFORM": "0", "DH_GATE_CTAS": "3"},
@@ -389,14 +368,17 @@ def test_graph_replay_survives_a_growing_batch_between_single_calls(monkeypatch)
         assert np.array_equal(a[5 + k][0], a[4]["mid_point"][3 + k]) and np.array_equal(a[5 + k][1], a[4]["rotation"][3 + k])
 
 
-@pytest.mark.parametrize("threads", ["1024", "768"])
-def test_two_levels_per_record_traversal(monkeypatch, threads):
-    """PairRec walk (DH_TRAV_PAIR=1): full trees of odd and even depth, sparse trees (leaves at every
-    depth, children that are leaves), trees that are a single leaf, shuffled node order, exact ties
-    (the fast walk hands them to the one-level walk), and the work counter node_visits, which the
-    fast walk reads off the leaf's depth."""
-    monkeypatch.setenv("DH_TRAV_PAIR", "1")
-    monkeypatch.setenv("DH_TRAV_THREADS", threads)
+@pytest.mark.parametrize("threads", [None, "512"], ids=["default", "512"])
+def test_default_walk_tree_shapes(monkeypatch, threads):
+    """The default walk (box-sum tile, the first levels through the LSU path, the rest through the
+    texture path) with the library's tiles and with 512-thread tiles: full trees of odd and even depth,
+    sparse trees (leaves at every depth, children that are leaves), trees that are a single leaf,
+    shuffled node order, exact ties (the fast pass hands them to the IEEE-division pass), and the work
+    counter node_visits, which must count every node of a walk once, ties included."""
+    if threads is None:
+        monkeypatch.delenv("DH_TRAV_THREADS", raising=False)
+    else:
+        monkeypatch.setenv("DH_TRAV_THREADS", threads)
     c = Context(0)
     try:
         frames = synth.make_frames(3, seed=61)

@@ -2,7 +2,7 @@
 # A/B runs of the default bench command under different environment switches (run under gpurun,
 # one GPU).  Every argument is one configuration: a space-separated list of VAR=value pairs
 # ("A=1" = the defaults).  Prints frames/s and the CUDA-event stage times of each.
-#   bash tools/ab_bench.sh "A=1" "DH_BOX_BANDS=1" "DH_TRAV_BLOCK=1 DH_TRAV_THREADS=768" "A=1"
+#   bash tools/ab_bench.sh "A=1" "DH_BOX_BANDS=1" "DH_TRAV_THREADS=512 DH_GATE_CTAS=2" "A=1"
 cd "$(dirname "$0")/.." || exit 1
 mkdir -p gpurun_out
 for cfg in "$@"; do
