@@ -111,6 +111,9 @@ Context::Context(int device) : device_(device) {
     gate_split_min_ = env_u32("DH_GATE_SPLIT_MIN", 64);
     chunk_frames_ = env_u32("DH_CHUNK_FRAMES", 0);  // 0 = adaptive (128 for host input, 512 for device input)
     debug_sync_ = env_u32("DH_DEBUG_SYNC", 0) != 0;
+    box_whole_ = env_flag("DH_BOX_WHOLE", true);
+    box_bands_ = env_u32("DH_BOX_BANDS", 0);
+    gate_ctas_ = env_u32("DH_GATE_CTAS", 0);
     std::memset(stage_ms_, 0, sizeof(stage_ms_));
     std::memset(counters_, 0, sizeof(counters_));
 }
@@ -650,7 +653,7 @@ void Context::run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameS
         hot_tw_ = tiles_.tw;
     }
     mark(DH_STAGE_SAT);
-    launches_ += (uint64_t)(g.rw ? launch_box_image(b, g, n, n_sms_, st) : launch_sat(b, g, n, st));
+    launches_ += (uint64_t)(g.rw ? launch_box_image(b, g, n, n_sms_, box_whole_, box_bands_, st) : launch_sat(b, g, n, st));
     stage_check("sat");
     mark(DH_STAGE_TRAVERSE);
     if (g.P) {
@@ -673,7 +676,7 @@ void Context::run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iter
     mark(DH_STAGE_GATE);
     // small passes (single frames, the passes of seeded sequences) are bound by the chain of launches: they keep the
     // patch gate inside the seed-grid kernel (one launch less; 0.168 instead of 0.187 ms per single frame)
-    launches_ += (uint64_t)launch_gate_coarse(b, g, fdev_, n, n >= gate_split_min_, n_sms_, st, frame_k);
+    launches_ += (uint64_t)launch_gate_coarse(b, g, fdev_, n, n >= gate_split_min_, n_sms_, gate_ctas_, st, frame_k);
     stage_check("gate + coarse grids");
     mark(DH_STAGE_VOTE);
     // the accumulator cubes of this pass start empty: either the previous pass's mean-shift CTAs

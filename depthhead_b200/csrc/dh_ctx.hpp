@@ -292,6 +292,9 @@ private:
     bool prob_codes_ok_ = false;     // the uploaded forest's leaf probabilities can ride in the node table as 8-bit codes
     bool leaf_codes_ = false;        // ... and do: leaf words carry them (FrameBuffers::leaf_mask, patch_gate_kernel)
     uint32_t gate_split_min_ = 64;   // frames per pass from which the patch gate runs as its own kernel (DH_GATE_SPLIT_MIN)
+    bool box_whole_ = true;          // DH_BOX_WHOLE=0: every box image through the warp-wide prefix sums
+    uint32_t box_bands_ = 0;         // DH_BOX_BANDS: box-image bands per frame (0 = the launch heuristic)
+    uint32_t gate_ctas_ = 0;         // DH_GATE_CTAS: seed-grid CTAs per frame on the gated-patch lists (0 = the launch heuristic)
 
     // measurement
     bool timing_ = false, debug_ = false, have_debug_ = false, debug_sync_ = false;

@@ -2363,8 +2363,8 @@ bool box_image_supported(uint32_t w, uint32_t h, uint32_t sw, uint32_t sh, uint3
     return ((sw + rw - 1u) / rw) * ((sh + rh - 1u) / rh) <= 64u;
 }
 
-int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, cudaStream_t s) {
-    static const bool allow_whole = !(std::getenv("DH_BOX_WHOLE") && std::atoi(std::getenv("DH_BOX_WHOLE")) == 0);
+int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, bool allow_whole, uint32_t bands,
+                     cudaStream_t s) {
     const bool whole = allow_whole && (g.rw & 7u) == 0u;
     // strips: a multiple of kBoxPx output columns each, at most 32*kBoxPx + 1 - rw (column c reads P[c + rw] <= P[32*kBoxPx])
     const uint32_t max_out = (32u * kBoxPx + 1u - g.rw) & ~(uint32_t)(kBoxPx - 1);
@@ -2382,13 +2382,12 @@ int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames
     // bands: a band re-reads the rh - 1 rows above it, so few of them, but enough that the launch has
     // about two rounds of CTAs (the CTAs of a single round do not divide evenly over the SMs and the
     // fullest SM sets the time: 512 frames x 1 band = 3.46 CTAs per SM ran 0.428 ms, 4 bands 0.376 ms);
-    // never shorter than rh rows.  DH_BOX_BANDS=n forces the count.
+    // never shorter than rh rows.  bands > 0 forces the count.
     const uint32_t ctas_per_sm = std::max<uint32_t>(1u, std::min<uint32_t>(16u, (227u * 1024u) / (smem + 1024u)));
     const uint32_t slots = (uint32_t)n_sms * ctas_per_sm * wpc;
     const uint32_t units = n_strips * n_frames;
     uint32_t n_bands = std::max<uint32_t>(1u, std::min<uint32_t>((2u * slots + units - 1u) / units, std::max<uint32_t>(1u, g.box_h / g.rh)));
-    static const uint32_t bands_env = std::getenv("DH_BOX_BANDS") ? (uint32_t)std::atoi(std::getenv("DH_BOX_BANDS")) : 0u;
-    if (bands_env) n_bands = std::max<uint32_t>(1u, std::min<uint32_t>(bands_env, std::max<uint32_t>(1u, g.box_h / g.rh)));
+    if (bands) n_bands = std::max<uint32_t>(1u, std::min<uint32_t>(bands, std::max<uint32_t>(1u, g.box_h / g.rh)));
     const uint32_t band_rows = (g.box_h + n_bands - 1u) / n_bands;
     n_bands = (g.box_h + band_rows - 1u) / band_rows;
     const uint32_t n_units = n_strips * n_bands * n_frames;
@@ -2461,7 +2460,7 @@ uint32_t vote_box_dim() { return (uint32_t)kBox; }
 // and the queue header must be zero when these run.  Each returns the kernels it launched.
 template <bool kFrameK>
 static int launch_gate_coarse_t(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list,
-                                int n_sms, const float* frame_k, cudaStream_t s) {
+                                int n_sms, uint32_t want_ctas, const float* frame_k, cudaStream_t s) {
     constexpr int kSmem = kGateSmemBytes + (kFrameK ? kFrameKFloats * 4 : 0);
     static SmemConfig configured;
     if (configured.raise((uint32_t)kSmem)) {
@@ -2473,9 +2472,8 @@ static int launch_gate_coarse_t(const FrameBuffers& b, const Geometry& g, const 
         // the patch gate writes the frames' gated-patch lists, the seed-grid CTAs take slices of them.  Few CTAs per
         // frame when there are many frames (a slice is a full CTA of work), every possible slice its own
         // CTA when there are few frames (a single frame must still spread over the GPU).
-        static const uint32_t want = std::getenv("DH_GATE_CTAS") ? (uint32_t)std::atoi(std::getenv("DH_GATE_CTAS")) : 0u;
         const uint32_t fill = (6u * (uint32_t)n_sms + n_frames - 1u) / n_frames;
-        const uint32_t ctas = std::max<uint32_t>(1u, std::min<uint32_t>(per_frame, want ? want : std::max<uint32_t>(4u, fill)));
+        const uint32_t ctas = std::max<uint32_t>(1u, std::min<uint32_t>(per_frame, want_ctas ? want_ctas : std::max<uint32_t>(4u, fill)));
         patch_gate_kernel<kFrameK><<<dim3((g.P + kPatchGateThreads * kPatchGatePer - 1) / (kPatchGateThreads * kPatchGatePer), n_frames),
                                      kPatchGateThreads, 0, s>>>(b, g, f, frame_k);
         gate_coarse_kernel<true, kFrameK><<<dim3(ctas, n_frames), kGateThreads, kSmem, s>>>(b, g, f, frame_k);
@@ -2486,10 +2484,10 @@ static int launch_gate_coarse_t(const FrameBuffers& b, const Geometry& g, const 
 }
 
 int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list, int n_sms,
-                       cudaStream_t s, const float* frame_k) {
+                       uint32_t want_ctas, cudaStream_t s, const float* frame_k) {
     if (!g.P) return 0;
-    return frame_k ? launch_gate_coarse_t<true>(b, g, f, n_frames, from_list, n_sms, frame_k, s)
-                   : launch_gate_coarse_t<false>(b, g, f, n_frames, from_list, n_sms, nullptr, s);
+    return frame_k ? launch_gate_coarse_t<true>(b, g, f, n_frames, from_list, n_sms, want_ctas, frame_k, s)
+                   : launch_gate_coarse_t<false>(b, g, f, n_frames, from_list, n_sms, want_ctas, nullptr, s);
 }
 
 int launch_seed_and_cubes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames,

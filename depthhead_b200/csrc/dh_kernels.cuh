@@ -111,7 +111,10 @@ constexpr uint32_t kProbCodeShift = 23u;
 constexpr uint32_t kLeafIdMask = (1u << kProbCodeShift) - 1u;
 
 int launch_sat(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, cudaStream_t s);
-int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, cudaStream_t s);
+// allow_whole: rectangles whose width is a multiple of 8 may take the whole-group box sums (false: every
+// width goes through the warp-wide prefix sums); bands: bands per frame, 0 = the launch heuristic
+int launch_box_image(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, int n_sms, bool allow_whole, uint32_t bands,
+                     cudaStream_t s);
 bool box_image_supported(uint32_t w, uint32_t h, uint32_t sw, uint32_t sh, uint32_t rw, uint32_t rh);
 void launch_traverse(const CUtensorMap& sat_map, const FrameBuffers& b, const Geometry& g, const TilePlan& tp,
                      const ForestDev& f, uint32_t n_frames, cudaStream_t s);
@@ -119,10 +122,11 @@ void launch_plan_nodes(const NodeRec* nodes, HotNode* hot, UniNode* uni, size_t 
                        const double* prob_codes, cudaStream_t s);
 // from_list: the patch gate runs as its own kernel and writes the frames' gated-patch lists; the seed-grid CTAs take
 // slices of the lists instead of gating the patches of their own index range.
+// want_ctas: seed-grid CTAs per frame of a from_list launch, 0 = the launch heuristic.
 // frame_k: nullptr = every frame has Geometry's K / Kinv; else a device table [n_frames][18] of each
 // frame's K then K^-1 (row-major), read by the kernels that project (dh_predict_frames).
 int launch_gate_coarse(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, bool from_list, int n_sms,
-                       cudaStream_t s, const float* frame_k = nullptr);
+                       uint32_t want_ctas, cudaStream_t s, const float* frame_k = nullptr);
 int launch_seed_and_cubes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames,
                           uint32_t iterations, cudaStream_t s, const float* frame_k = nullptr);
 int launch_meanshift(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t iterations,

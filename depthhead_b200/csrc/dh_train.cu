@@ -246,7 +246,7 @@ TrainSet* Context::trainset_create(const uint16_t* patches, uint64_t n, uint32_t
         FrameBuffers b{};
         b.depth = d_px.p;
         b.box = ts->box + f0 * (size_t)ts->bh * ts->bpitch;
-        launch_box_image(b, g, (uint32_t)nc, n_sms_, stream_);
+        launch_box_image(b, g, (uint32_t)nc, n_sms_, box_whole_, box_bands_, stream_);
         DH_CUDA_T(cudaGetLastError());
         DH_CUDA_T(cudaStreamSynchronize(stream_));
     }

@@ -57,23 +57,55 @@ VARIANTS = [
 ]
 
 
+GATE_SLICE = 512  # entries of a frame's gated-patch list per seed-grid slice (kGateThreads)
+
+
+def _noise_frame(seed):
+    """random u16 depth with half of the pixels zeroed: a few thousand gated patches per VGA frame"""
+    rng = np.random.default_rng(seed)
+    d = rng.integers(0, 65536, (480, 640)).astype(np.uint16)
+    d[rng.random((480, 640)) < 0.5] = 0
+    return d
+
+
 @pytest.mark.parametrize("env", VARIANTS, ids=lambda e: ",".join("%s=%s" % kv for kv in e.items()))
 def test_kernel_variants(monkeypatch, env):
+    gate_ctas = int(env.get("DH_GATE_CTAS", 0))
+    if gate_ctas:
+        # DH_GATE_CTAS shapes the seed-grid launch over the gated-patch lists, which passes of at least
+        # DH_GATE_SPLIT_MIN frames use: every pass here does
+        monkeypatch.setenv("DH_GATE_SPLIT_MIN", "1")
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    c = Context(0)  # the switches are read when a context uploads a model / sizes its scratch
+    c = Context(0)  # the switches are read when a context is created, uploads a model or sizes its scratch
     try:
         for kw in (dict(seed=3, n_trees=4, max_depth=7), dict(seed=5, n_trees=3, max_depth=8, stop_prob=0.2, ragged_rects=True)):
             arr = synth.make_forest(**kw)
             js = synth.forest_to_json(arr, stepwidth=6)
             hp = HoughPrediction.from_json(js)
             of = oracle.OracleForest.from_json(js)
-            frames = synth.make_frames(5, seed=21)
+            frames = np.concatenate([synth.make_frames(5, seed=21), _noise_frame(21)[None]])
             _compare_frame(c, hp, of, frames[0])
+            _compare_frame(c, hp, of, frames[5])
+            if gate_ctas:
+                # the noise frame's list has more slices than the frame has seed-grid CTAs: a CTA walks several
+                assert c.counters()["gate_patches"] > gate_ctas * GATE_SLICE, c.counters()
             out = hp.predict_batch(frames, K, ctx=c)
             for i, d in enumerate(frames):
                 tr = of.predict(d, synth.KINECT_K, mode=oracle.MODE_SAT, keep=False)
                 assert np.array_equal(out["mid_point"][i], tr.mid_point) and np.array_equal(out["rotation"][i], tr.rotation)
+            if gate_ctas:
+                # the pass took the list path: one launch more (patch_gate_kernel) than with the gate inside the
+                # seed-grid kernel
+                launches = c.counters()["launches"]
+                monkeypatch.setenv("DH_GATE_SPLIT_MIN", "64")
+                ref = Context(0)
+                try:
+                    assert hp.predict_batch(frames, K, ctx=ref).tobytes() == out.tobytes()
+                    assert launches == ref.counters()["launches"] + 1
+                finally:
+                    ref.close()
+                    monkeypatch.setenv("DH_GATE_SPLIT_MIN", "1")
     finally:
         c.close()
 

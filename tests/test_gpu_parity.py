@@ -31,10 +31,13 @@ def _filter_acc(keys, vals, origin, dim):
     return keys[m], vals[m]
 
 
-def _compare_frame(ctx, hp, of, depth, midp_guess=None, rot_guess=None, check_patches=True):
+def _compare_frame(ctx, hp, of, depth, midp_guess=None, rot_guess=None, check_patches=True, intrinsic=None):
+    """every stage of one frame against the oracle; intrinsic: a float32 3x3 matrix for both sides
+    (None = the Kinect default)"""
+    k = synth.KINECT_K if intrinsic is None else np.asarray(intrinsic, np.float32)
     ctx.enable_debug(True)
-    res = hp.predict_parameter_parallel(depth, K, midp_guess, rot_guess, ctx=ctx)
-    tr = of.predict(depth, synth.KINECT_K, midp_guess, rot_guess, mode=oracle.MODE_SAT, keep=True)
+    res = hp.predict_parameter_parallel(depth, K if intrinsic is None else IntrinsicMatrix(k), midp_guess, rot_guess, ctx=ctx)
+    tr = of.predict(depth, k, midp_guess, rot_guess, mode=oracle.MODE_SAT, keep=True)
     npx, npy, T = ctx.debug_dims()
     assert (npx, npy, T) == (tr.npx, tr.npy, of.n_trees)
     # --- leaf index per patch x tree: bit-exact
