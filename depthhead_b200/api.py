@@ -231,6 +231,18 @@ def frame_args(n: int, intrinsics, midp_guess=None, rot_guess=None, has_midp=Non
     return args
 
 
+def _track_offsets(lengths):
+    """(uint64 [n_seq+1] offsets from 0, n_seq, total) of the track lengths of dh_predict_tracks"""
+    ln = np.asarray(lengths)
+    if ln.ndim != 1 or not (np.issubdtype(ln.dtype, np.integer) or ln.size == 0) or (ln.size and ln.min() < 0):
+        raise ValueError("lengths must be a 1-D array of non-negative integers")
+    seq_off = np.zeros(len(ln) + 1, np.uint64)
+    np.cumsum(ln.astype(np.uint64), out=seq_off[1:])
+    if seq_off[-1] > 0x7FFFFFFF:
+        raise ValueError("more than 2^31 - 1 frames")
+    return seq_off, len(ln), int(seq_off[-1])
+
+
 def _image_out(out_device_ptr, shape, dtype):
     """(host array or None, pointer, location) of a batch of images: a new host array, or the caller's device memory."""
     if out_device_ptr is None:
@@ -400,6 +412,26 @@ class HoughPrediction:
         ctx = ctx or default_context()
         out = np.zeros(n, capi.RESULT_DTYPE)
         capi.check(capi.load().dh_predict_frames(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(out)))
+        return out
+
+    def predict_tracks(self, frames, lengths, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                       min_seed_z: float = 500.0, ctx: Context | None = None, device_ptr: int | None = None, w: int | None = None,
+                       h: int | None = None) -> np.ndarray:
+        """Tracks of any length in one call: track s is the next lengths[s] frames of `frames` (in time
+        order), from a camera of its own, intrinsics[s], with optional seeds of its first frame; every later
+        frame is seeded with the pose of the frame before it as in predict_sequences (centre seed only if
+        the previous z > min_seed_z).  `frames`: [total,h,w] uint16 on the host, or device_ptr + (w, h),
+        with total = sum(lengths).  intrinsics: one IntrinsicMatrix or a float32 [n_seq,3,3] array; the
+        seeds are per track as in predict_frames.  Returns capi.RESULT_DTYPE[total] in input order."""
+        seq_off, n_seq, total = _track_offsets(lengths)
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, total, w, h)
+        if n != total:
+            raise ValueError("sum(lengths) = %d but there are %d frames" % (total, n))
+        args = frame_args(n_seq, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+        ctx = ctx or default_context()
+        out = np.zeros(total, capi.RESULT_DTYPE)
+        capi.check(capi.load().dh_predict_tracks(ctx._h, self._h, p, n_seq, capi.ptr(seq_off), w, h, loc, capi.ptr(args),
+                                                 float(min_seed_z), capi.ptr(out)))
         return out
 
     def predict_sequences(self, frames, intrinsic: IntrinsicMatrix, min_seed_z: float = 500.0, ctx: Context | None = None,

@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .api import Context, HoughPrediction, IntrinsicMatrix, default_context, frame_args
+from .api import Context, HoughPrediction, IntrinsicMatrix, _track_offsets, default_context, frame_args
 
 
 def encode_depth(img: np.ndarray) -> bytes:
@@ -142,4 +142,24 @@ def predict_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w:
         return out
     capi.check(capi.load().dh_predict_batch_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
                                                  intrinsic._ptr(), capi.ptr(out)))
+    return out
+
+
+def predict_track_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, lengths, w: int, h: int, intrinsics,
+                        midp_guess=None, rot_guess=None, has_midp=None, has_rot=None, min_seed_z: float = 500.0,
+                        ctx: Context | None = None) -> np.ndarray:
+    """HoughPrediction.predict_tracks over Biwi files: track s is the next lengths[s] files (in time order),
+    with intrinsics[s] (one IntrinsicMatrix or a float32 [n_seq,3,3] array, e.g. the depth.cal of every
+    sequence folder) and optional seeds of its first frame.  The decode runs on the GPU.  Returns
+    capi.RESULT_DTYPE[n] in file order; a damaged file is DH_E_ARG naming the lowest bad file."""
+    seq_off, n_seq, total = _track_offsets(lengths)
+    n = len(offsets) - 1
+    if n != total:
+        raise ValueError("sum(lengths) = %d but there are %d files" % (total, n))
+    args = frame_args(n_seq, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+    ctx = ctx or default_context()
+    out = np.zeros(n, capi.RESULT_DTYPE)
+    offsets = np.ascontiguousarray(offsets, np.uint64)
+    capi.check(capi.load().dh_predict_tracks_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n_seq, capi.ptr(seq_off),
+                                                  int(w), int(h), capi.ptr(args), float(min_seed_z), capi.ptr(out)))
     return out

@@ -57,11 +57,20 @@ static_assert(sizeof(dh_frame_args) == 80 && offsetof(dh_frame_args, K) == 0 && 
                   offsetof(dh_frame_args, _pad) == 76,
               "dh_frame_args layout (mirrored by capi.FRAME_ARGS_DTYPE and the Rust shim)");
 
-void check_frame_args(const char* fn, const dh_frame_args* args, uint32_t n) {
+void check_frame_args(const char* fn, const dh_frame_args* args, uint32_t n, const char* what = "frame") {
     for (uint32_t i = 0; i < n; ++i)
         if (args[i].has_guess & ~3u)
-            throw dh::ModelError(DH_E_ARG, std::string(fn) + ": frame " + std::to_string(i) + " has has_guess " +
+            throw dh::ModelError(DH_E_ARG, std::string(fn) + ": " + what + " " + std::to_string(i) + " has has_guess " +
                                                std::to_string(args[i].has_guess) + " (only bits 0 and 1 are defined)");
+}
+
+// seq_off of dh_predict_tracks: n_seq + 1 offsets from 0, monotone, at most 2^31 - 1 frames
+void check_seq_off(const char* fn, const uint64_t* seq_off, uint32_t n_seq) {
+    if (seq_off[0] != 0) throw dh::ModelError(DH_E_ARG, std::string(fn) + ": seq_off[0] is not 0");
+    for (uint32_t s = 0; s < n_seq; ++s)
+        if (seq_off[s + 1] < seq_off[s])
+            throw dh::ModelError(DH_E_ARG, std::string(fn) + ": seq_off is not monotone at track " + std::to_string(s));
+    if (seq_off[n_seq] > 0x7fffffffull) throw dh::ModelError(DH_E_ARG, std::string(fn) + ": more than 2^31 - 1 frames");
 }
 
 }  // namespace
@@ -263,6 +272,30 @@ int dh_predict_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, c
         if (args) check_frame_args("dh_predict_frames_biwi", args, n);
         REQUIRE(c && f && (n == 0 || (blob && offsets && args && out)), "dh_predict_frames_biwi: NULL argument");
         c->cx->predict_frames(*f->hf, nullptr, blob, offsets, n, w, h, DH_DEPTH_HOST, args, out);
+    });
+}
+
+int dh_predict_tracks(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n_seq, const uint64_t* seq_off, uint32_t w,
+                      uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z, dh_result* out) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_tracks: bad depth_loc");
+        if (seq_off) check_seq_off("dh_predict_tracks", seq_off, n_seq);
+        if (seq_args) check_frame_args("dh_predict_tracks", seq_args, n_seq, "track");
+        REQUIRE(c && f && seq_off && (n_seq == 0 || seq_args) && (seq_off[n_seq] == 0 || (depth && out)), "dh_predict_tracks: NULL argument");
+        c->cx->predict_tracks(*f->hf, depth, nullptr, nullptr, n_seq, seq_off, w, h, depth_loc, seq_args, min_seed_z, out);
+    });
+}
+
+int dh_predict_tracks_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
+                           const uint64_t* seq_off, uint32_t w, uint32_t h, const dh_frame_args* seq_args, float min_seed_z,
+                           dh_result* out) {
+    return guarded([&] {
+        if (seq_off) check_seq_off("dh_predict_tracks_biwi", seq_off, n_seq);
+        if (seq_args) check_frame_args("dh_predict_tracks_biwi", seq_args, n_seq, "track");
+        if (seq_off && offsets) dh::check_biwi_offsets(offsets, (uint32_t)seq_off[n_seq]);
+        REQUIRE(c && f && seq_off && (n_seq == 0 || seq_args) && (seq_off[n_seq] == 0 || (blob && offsets && out)),
+                "dh_predict_tracks_biwi: NULL argument");
+        c->cx->predict_tracks(*f->hf, nullptr, blob, offsets, n_seq, seq_off, w, h, DH_DEPTH_HOST, seq_args, min_seed_z, out);
     });
 }
 size_t dh_biwi_encode_bound(uint32_t w, uint32_t h) { return dh::rle_frame_bound(w, h); }

@@ -105,6 +105,7 @@ Context::Context(int device) : device_(device) {
     DH_CUDA(cudaHostAlloc((void**)&h_counters_, sizeof(unsigned long long) * DH_N_COUNTERS, cudaHostAllocDefault));
     DH_CUDA(cudaHostAlloc((void**)&h_result1_, sizeof(dh_result), cudaHostAllocDefault));
     for (int i = 0; i < kEncSlots; ++i) DH_CUDA(cudaEventCreateWithFlags(&ev_enc_copied_[i], cudaEventDisableTiming));
+    for (int i = 0; i < 2; ++i) DH_CUDA(cudaEventCreateWithFlags(&tb_.ev_win[i], cudaEventDisableTiming));
     DH_CUDA(cudaEventCreateWithFlags(&ev_copy_tail_, cudaEventDisableTiming));
     if (const char* v = std::getenv("DH_HOST_ENCODE")) host_encode_ = *v ? (int)std::strtol(v, nullptr, 10) : -1;
     use_graphs_ = env_flag("DH_GRAPH", true);
@@ -135,6 +136,9 @@ Context::~Context() {
     if (h_result1_) cudaFreeHost(h_result1_);
     if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
     if (h_frame_k_) cudaFreeHost(h_frame_k_);
+    free_track_buffers();
+    for (int i = 0; i < 2; ++i)
+        if (tb_.ev_win[i]) cudaEventDestroy(tb_.ev_win[i]);
     pool_.reset();
     for (int i = 0; i < kEncSlots; ++i) {
         if (h_enc_[i]) cudaFreeHost(h_enc_[i]);
@@ -613,7 +617,7 @@ void Context::mark(int stage_begin_of) {
 // ------------------------------------------------------------------------------------------------ one pass
 // Front end shared by every entry point: SAT + traversal (+ zeroed per-frame state).
 void Context::run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameState* guess_state, const dh_result* prev_results,
-                        float min_seed_z, const dh_frame_args* args, uint32_t f0) {
+                        float min_seed_z, const dh_frame_args* args, uint32_t f0, bool fs_written) {
     const Geometry& g = geom_;
     cudaStream_t st = L.stream;
     if (args) {
@@ -635,7 +639,7 @@ void Context::run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameS
         }
         DH_CUDA(cudaMemcpyAsync(L.fs, hfs, sizeof(FrameState) * n, cudaMemcpyHostToDevice, st));
         DH_CUDA(cudaMemcpyAsync(L.frame_k, hk, sizeof(float) * 18 * n, cudaMemcpyHostToDevice, st));
-    } else {
+    } else if (!fs_written) {
         DH_CUDA(cudaMemsetAsync(L.fs, 0, sizeof(FrameState) * n, st));
     }
     DH_CUDA(cudaMemsetAsync(L.grids, 0, sizeof(uint32_t) * (size_t)(kPosGridCells + kRotGridCells) * n, st));
@@ -835,13 +839,27 @@ void Context::predict_frames(const HostForest& hf, const uint16_t* depth, const 
     run_batch(hf, depth, blob, offsets, n, w, h, n ? args[0].K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
 }
 
-// Device copies of the file offsets and room for the compressed bytes of one chunk per slot.
-void Context::ensure_biwi(const uint64_t* offsets, uint32_t n, uint32_t chunk, int slots) {
+void check_biwi_offsets(const uint64_t* offsets, uint32_t n) {
     for (uint32_t i = 0; i < n; ++i) {
         if (offsets[i + 1] < offsets[i]) throw ModelError(DH_E_ARG, "Biwi offsets are not monotone at frame " + std::to_string(i));
         if (offsets[i] & 3u) throw ModelError(DH_E_ARG, "Biwi frame " + std::to_string(i) + " does not start at a multiple of 4 bytes");
         if (offsets[i + 1] - offsets[i] > 0xfffffff0ull) throw ModelError(DH_E_ARG, "Biwi frame " + std::to_string(i) + " is larger than 4 GB");
     }
+}
+
+namespace {
+// DH_E_ARG for Biwi frame i, whose decode status is `status` (biwi_decode_kernel)
+[[noreturn]] void throw_biwi_status(size_t i, uint32_t status) {
+    static const char* what[] = {"", "is truncated (the reference fails with UnexpectedEof, biwi.rs:90-96)",
+                                 "has a run past the last pixel (the reference panics, biwi.rs:92,97)",
+                                 "has a header that differs from the requested width x height"};
+    throw ModelError(DH_E_ARG, "Biwi frame " + std::to_string(i) + " " + what[std::min<uint32_t>(status, 3u)]);
+}
+}  // namespace
+
+// Device copies of the file offsets and room for the compressed bytes of one chunk per slot.
+void Context::ensure_biwi(const uint64_t* offsets, uint32_t n, uint32_t chunk, int slots) {
+    check_biwi_offsets(offsets, n);
     size_t need = 0;
     for (uint32_t f0 = 0; f0 < n; f0 += chunk) need = std::max<size_t>(need, (size_t)(offsets[std::min(n, f0 + chunk)] - offsets[f0]));
     need += 64;  // the decode kernel reads whole 4-byte words
@@ -872,12 +890,7 @@ void Context::check_biwi_status(uint32_t n) {
     DH_CUDA(cudaMemcpyAsync(h_status_, d_status_, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, stream_));
     DH_CUDA(cudaStreamSynchronize(stream_));
     for (uint32_t i = 0; i < n; ++i)
-        if (h_status_[i]) {
-            static const char* what[] = {"", "is truncated (the reference fails with UnexpectedEof, biwi.rs:90-96)",
-                                         "has a run past the last pixel (the reference panics, biwi.rs:92,97)",
-                                         "has a header that differs from the requested width x height"};
-            throw ModelError(DH_E_ARG, "Biwi frame " + std::to_string(i) + " " + what[std::min<uint32_t>(h_status_[i], 3u)]);
-        }
+        if (h_status_[i]) throw_biwi_status(i, h_status_[i]);
 }
 
 void Context::biwi_decode(const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h, uint16_t* out,
@@ -1322,71 +1335,325 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
 }
 
-// ------------------------------------------------------------------------------------------------ seeded sequences
+// ------------------------------------------------------------------------------------------------ tracks and seeded sequences
 // The reference's real use (examples/live_prediction.rs:75-88) predicts a SEQUENCE: every frame is
 // seeded with the pose of the frame before it, which makes a sequence sequential — but separate
-// sequences stay independent.  Frame t of all n_seq sequences goes through the pipeline as one
-// pass of n_seq frames (gathered out of the sequence-major input by one strided copy), the seeds
-// of pass t are written on the device from the results of pass t - 1, and nothing returns to the
-// host before the last pass.  Results in the input's order: out[s * frames_per_seq + t].
-void Context::predict_sequences(const HostForest& hf, const uint16_t* depth, uint32_t n_seq, uint32_t frames_per_seq, uint32_t w, uint32_t h,
-                                const float K[9], int depth_loc, float min_seed_z, dh_result* out) {
+// sequences stay independent.  A track is one such sequence from one camera: its own K, optional
+// seeds for its first frame, frames t > 0 seeded from frame t - 1 of the same track (centre iff its
+// z > min_seed_z, rotation always).  A pass holds up to F frames (the chunk size), one per slot;
+// each slot holds the next frame of one track.  The seeds of a pass are written on the device from
+// the results of the previous one, and nothing returns to the host between passes but finished
+// windows of results.
+namespace {
+// Where every frame runs: tracks longest first (ties by index), one per slot; when a track ends its
+// slot takes the next waiting track in the next pass, so passes stay full while tracks wait, and with
+// n_seq <= F there are as many passes as the longest track has frames.  The entries of a pass are
+// its occupied slots in slot order; the plan decides only where a frame runs, never what it computes.
+struct TrackPlan {
+    std::vector<TrackSlot> slots;    // the entries of every pass, pass after pass
+    std::vector<uint32_t> pass_off;  // pass p: slots[pass_off[p], pass_off[p + 1])
+};
+TrackPlan plan_tracks(uint32_t n_seq, const uint64_t* seq_off, uint32_t F) {
+    TrackPlan pl;
+    std::vector<uint32_t> order;
+    for (uint32_t s = 0; s < n_seq; ++s)
+        if (seq_off[s + 1] > seq_off[s]) order.push_back(s);
+    std::stable_sort(order.begin(), order.end(),
+                     [&](uint32_t a, uint32_t b) { return seq_off[a + 1] - seq_off[a] > seq_off[b + 1] - seq_off[b]; });
+    struct Slot {
+        int32_t track = -1;
+        uint64_t t = 0;    // the track's next frame
+        int32_t pos = -1;  // the slot's position in the last pass
+    };
+    std::vector<Slot> sl(std::min<size_t>(F, order.size()));
+    size_t next = 0;
+    for (Slot& s : sl) s.track = (int32_t)order[next++];
+    pl.slots.reserve((size_t)seq_off[n_seq]);
+    pl.pass_off.push_back(0);
+    for (;;) {
+        int32_t pos = 0;
+        for (Slot& s : sl) {
+            if (s.track < 0) continue;
+            pl.slots.push_back(TrackSlot{(int32_t)(seq_off[s.track] + s.t), s.track, s.t ? s.pos : -1});
+            s.pos = pos++;
+        }
+        if (pos == 0) break;
+        pl.pass_off.push_back((uint32_t)pl.slots.size());
+        for (Slot& s : sl) {
+            if (s.track < 0 || ++s.t < seq_off[s.track + 1] - seq_off[s.track]) continue;
+            s.t = 0;
+            s.track = next < order.size() ? (int32_t)order[next++] : -1;
+        }
+    }
+    return pl;
+}
+
+constexpr size_t kTrackWindowResults = 1u << 16;  // results per window of passes (3.7 MB)
+
+template <typename T>
+void host_alloc(T*& p, size_t n) {
+    p = nullptr;
+    DH_CUDA(cudaHostAlloc((void**)&p, sizeof(T) * std::max<size_t>(n, 1), cudaHostAllocDefault));
+}
+template <typename T>
+void host_free(T*& p) {
+    if (p) cudaFreeHost(p);
+    p = nullptr;
+}
+}  // namespace
+
+void Context::free_track_buffers() {
+    for (int i = 0; i < 2; ++i) {
+        dev_free(tb_.d_plan[i]);
+        host_free(tb_.h_plan[i]);
+        host_free(tb_.h_win[i]);
+        host_free(tb_.h_blob[i]);
+    }
+    dev_free(tb_.d_win);
+    dev_free(tb_.d_tracks);
+    host_free(tb_.h_tracks);
+    dev_free(tb_.d_status);
+    dev_free(tb_.d_bad);
+    host_free(tb_.h_bad);
+    tb_.win_cap = tb_.tracks_cap = tb_.blob_cap = tb_.status_cap = 0;
+}
+
+void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
+                             const uint64_t* seq_off, uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z,
+                             dh_result* out) {
     begin_call();
     have_debug_ = false;
     last_encoded_chunks_ = 0;
     last_h2d_bytes_ = 0;
-    const size_t total = (size_t)n_seq * frames_per_seq;
+    const uint64_t total = n_seq ? seq_off[n_seq] : 0;
+    if (total > 0x7fffffffull) throw ModelError(DH_E_ARG, "more than 2^31 - 1 frames in one call");
     if (total == 0) {
         end_call();
         return;
     }
-    if (total > 0x7fffffffull) throw ModelError(DH_E_ARG, "dh_predict_sequences: more than 2^31 frames");
+    if (blob) check_biwi_offsets(offsets, (uint32_t)total);
     ensure_forest(hf);
-    const uint32_t want = chunk_frames_ ? std::min(chunk_frames_, n_seq) : std::min<uint32_t>(n_seq, 512u);
-    ensure_scratch(hf, w, h, want, K, 1);
+    // One K, equal lengths, no starting seeds and frames in memory: the operations dh_predict_sequences
+    // has always issued (one strided copy per pass, seq_guess_kernel, the one-K kernels).
+    bool uniform = !blob;
+    uint32_t live = 0;
+    for (uint32_t s = 0; s < n_seq; ++s) {
+        live += seq_off[s + 1] > seq_off[s] ? 1u : 0u;
+        uniform = uniform && seq_off[s + 1] - seq_off[s] == seq_off[1] && seq_args[s].has_guess == 0 &&
+                  std::memcmp(seq_args[s].K, seq_args[0].K, sizeof(seq_args[0].K)) == 0;
+    }
+    const uint32_t want = chunk_frames_ ? std::min(chunk_frames_, live) : std::min<uint32_t>(live, 512u);
+    ensure_scratch(hf, w, h, want, seq_args[0].K, 1);
     ensure_staging(2);
     const uint32_t iterations = hf.meanshift_iterations.load();
-    const uint32_t F = call_chunk_;  // sequences per group
+    const uint32_t F = call_chunk_;
+    const TrackPlan pl = plan_tracks(n_seq, seq_off, F);
+    const uint32_t n_pass = (uint32_t)pl.pass_off.size() - 1;
+    const uint32_t W = (uint32_t)std::max<size_t>(1, kTrackWindowResults / F);  // passes per window
+    const size_t win = (size_t)W * F;
     const size_t px = (size_t)w * h;
+
+    // buffers (each grows alone; a free waits for the work that may still use it)
+    auto drain = [&] {
+        DH_CUDA(cudaStreamSynchronize(stream_));
+        DH_CUDA(cudaStreamSynchronize(copy_stream_));
+    };
+    if (win > tb_.win_cap) {
+        drain();
+        for (int i = 0; i < 2; ++i) {
+            dev_free(tb_.d_plan[i]);
+            host_free(tb_.h_plan[i]);
+            host_free(tb_.h_win[i]);
+        }
+        dev_free(tb_.d_win);
+        for (int i = 0; i < 2; ++i) {
+            dev_alloc(tb_.d_plan[i], win);
+            host_alloc(tb_.h_plan[i], win);
+            host_alloc(tb_.h_win[i], win);
+        }
+        dev_alloc(tb_.d_win, win);
+        tb_.win_cap = win;
+    }
+    if (!tb_.d_bad) {
+        dev_alloc(tb_.d_bad, 1);
+        host_alloc(tb_.h_bad, 1);
+    }
+    if (!uniform) {
+        if (n_seq > tb_.tracks_cap) {
+            drain();
+            dev_free(tb_.d_tracks);
+            host_free(tb_.h_tracks);
+            dev_alloc(tb_.d_tracks, n_seq);
+            host_alloc(tb_.h_tracks, n_seq);
+            tb_.tracks_cap = n_seq;
+        }
+        // the per-track table, once per call: K, K^-1 (as ensure_scratch computes them for one matrix), first seeds
+        for (uint32_t s = 0; s < n_seq; ++s) {
+            const dh_frame_args& a = seq_args[s];
+            TrackArgs& t = tb_.h_tracks[s];
+            std::memset(&t, 0, sizeof(t));
+            std::memcpy(t.K, a.K, sizeof(float) * 9);
+            mat3_inverse_f32(a.K, t.K + 9);
+            t.has_guess = a.has_guess;
+            if (a.has_guess & 1u)
+                for (int k = 0; k < 3; ++k) t.midp_guess[k] = a.midp_guess[k];
+            if (a.has_guess & 2u)
+                for (int k = 0; k < 3; ++k) t.rot_guess[k] = a.rot_guess[k];
+        }
+        DH_CUDA(cudaMemcpyAsync(tb_.d_tracks, tb_.h_tracks, sizeof(TrackArgs) * n_seq, cudaMemcpyHostToDevice, stream_));
+    }
+    auto file_bytes = [&](int32_t f) { return (size_t)((offsets[f + 1] - offsets[f] + 3) & ~3ull); };
+    if (blob) {
+        // a pass's (start, end) pairs, then its files at multiples of 4 bytes, then the decode's read-ahead
+        size_t need = 0;
+        for (uint32_t p = 0; p < n_pass; ++p) {
+            size_t b = 16ull * (pl.pass_off[p + 1] - pl.pass_off[p]) + 64;
+            for (uint32_t j = pl.pass_off[p]; j < pl.pass_off[p + 1]; ++j) b += file_bytes(pl.slots[j].frame);
+            need = std::max(need, b);
+        }
+        if (need > blob_cap_) {
+            drain();
+            for (int i = 0; i < 2; ++i) dev_free(d_blob_[i]);
+            blob_cap_ = need;
+        }
+        for (int i = 0; i < 2; ++i)
+            if (!d_blob_[i]) dev_alloc(d_blob_[i], blob_cap_);
+        if (need > tb_.blob_cap) {
+            drain();
+            for (int i = 0; i < 2; ++i) host_free(tb_.h_blob[i]);
+            for (int i = 0; i < 2; ++i) host_alloc(tb_.h_blob[i], need);
+            tb_.blob_cap = need;
+        }
+        if (F > tb_.status_cap) {
+            drain();
+            dev_free(tb_.d_status);
+            dev_alloc(tb_.d_status, F);
+            tb_.status_cap = F;
+        }
+        DH_CUDA(cudaMemsetAsync(tb_.d_bad, 0xFF, sizeof(unsigned long long), stream_));
+    }
+
+    // window wi's results, from pinned memory to `out` in input order
+    auto scatter = [&](uint32_t wi) {
+        const dh_result* r = tb_.h_win[wi & 1u];
+        for (uint32_t p = wi * W; p < std::min(n_pass, (wi + 1) * W); ++p)
+            for (uint32_t j = pl.pass_off[p]; j < pl.pass_off[p + 1]; ++j)
+                out[pl.slots[j].frame] = r[(size_t)(p - wi * W) * F + (j - pl.pass_off[p])];
+    };
     const cudaMemcpyKind kind = depth_loc == DH_DEPTH_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    dh_result* d_all = nullptr;  // [frames_per_seq][group] poses of the current group, pass-major
-    dev_alloc(d_all, (size_t)frames_per_seq * F);
-    std::vector<dh_result> host_all((size_t)frames_per_seq * F);
     Lane& L = lanes_[0];
     try {
         DH_CUDA(cudaEventRecord(ev_fork_, stream_));
         DH_CUDA(cudaStreamWaitEvent(copy_stream_, ev_fork_, 0));
-        for (uint32_t g0 = 0; g0 < n_seq; g0 += F) {
-            const uint32_t ns = std::min<uint32_t>(F, n_seq - g0);
-            for (uint32_t t = 0; t < frames_per_seq; ++t) {
-                const int slot = (int)(t & 1u);
-                // frame t of sequences g0 .. g0 + ns - 1: rows of one strided copy (row = a frame, pitch = a sequence)
-                if (t >= 2 || g0) DH_CUDA(cudaStreamWaitEvent(copy_stream_, ev_consumed_[slot], 0));
-                DH_CUDA(cudaMemcpy2DAsync(d_depth_[slot], px * sizeof(uint16_t), depth + ((size_t)g0 * frames_per_seq + t) * px,
-                                          (size_t)frames_per_seq * px * sizeof(uint16_t), px * sizeof(uint16_t), ns, kind, copy_stream_));
-                if (depth_loc != DH_DEPTH_DEVICE) last_h2d_bytes_ += (uint64_t)ns * px * sizeof(uint16_t);
-                DH_CUDA(cudaEventRecord(ev_copied_[slot], copy_stream_));
-                DH_CUDA(cudaStreamWaitEvent(L.stream, ev_copied_[slot], 0));
-                FrameBuffers b = buffers(L, d_depth_[slot]);
-                run_front(L, b, ns, nullptr, t ? L.results : nullptr, min_seed_z);
-                run_back(L, b, ns, iterations);
-                DH_CUDA(cudaMemcpyAsync(d_all + (size_t)t * F, L.results, sizeof(dh_result) * ns, cudaMemcpyDeviceToDevice, L.stream));
-                DH_CUDA(cudaEventRecord(ev_consumed_[slot], L.stream));
+        for (uint32_t p = 0; p < n_pass; ++p) {
+            const uint32_t wi = p / W, pw = p % W, n = pl.pass_off[p + 1] - pl.pass_off[p];
+            const TrackSlot* e = pl.slots.data() + pl.pass_off[p];
+            const TrackSlot* d_e = tb_.d_plan[wi & 1u] + (pl.pass_off[p] - pl.pass_off[wi * W]);
+            const int slot = (int)(p & 1u);
+            if (pw == 0 && wi >= 2) {  // the pinned buffers of this window's parity are free once window wi - 2 is out
+                DH_CUDA(cudaEventSynchronize(tb_.ev_win[wi & 1u]));
+                scatter(wi - 2);
             }
-            DH_CUDA(cudaMemcpyAsync(host_all.data(), d_all, sizeof(dh_result) * (size_t)frames_per_seq * F, cudaMemcpyDeviceToHost, L.stream));
-            DH_CUDA(cudaStreamSynchronize(L.stream));
-            for (uint32_t s2 = 0; s2 < ns; ++s2)
-                for (uint32_t t = 0; t < frames_per_seq; ++t) out[((size_t)g0 + s2) * frames_per_seq + t] = host_all[(size_t)t * F + s2];
+            if (p >= 2) DH_CUDA(cudaStreamWaitEvent(copy_stream_, ev_consumed_[slot], 0));
+            if (pw == 0 && !uniform) {  // the window's slot tables (pass p - 2 consumed: window wi - 2 is done with them)
+                const uint32_t e1 = pl.pass_off[std::min(n_pass, p + W)];
+                std::memcpy(tb_.h_plan[wi & 1u], e, sizeof(TrackSlot) * (e1 - pl.pass_off[p]));
+                DH_CUDA(cudaMemcpyAsync(tb_.d_plan[wi & 1u], tb_.h_plan[wi & 1u], sizeof(TrackSlot) * (e1 - pl.pass_off[p]),
+                                        cudaMemcpyHostToDevice, copy_stream_));
+            }
+            if (uniform) {
+                // the same frame of consecutive tracks: rows of one strided copy (row = a frame, pitch = a track)
+                const size_t fps = (size_t)seq_off[1];
+                DH_CUDA(cudaMemcpy2DAsync(d_depth_[slot], px * sizeof(uint16_t), depth + (size_t)e[0].frame * px,
+                                          fps * px * sizeof(uint16_t), px * sizeof(uint16_t), n, kind, copy_stream_));
+                if (depth_loc != DH_DEPTH_DEVICE) last_h2d_bytes_ += (uint64_t)n * px * sizeof(uint16_t);
+            } else if (blob) {
+                DH_CUDA(cudaEventSynchronize(ev_copied_[slot]));  // pass p - 2 has left this pinned slot
+                unsigned long long* pairs = reinterpret_cast<unsigned long long*>(tb_.h_blob[slot]);
+                uint8_t* files = tb_.h_blob[slot] + 16ull * n;
+                size_t o = 0;
+                for (uint32_t j = 0; j < n; ++j) {
+                    const int32_t f = e[j].frame;
+                    const size_t len = (size_t)(offsets[f + 1] - offsets[f]);
+                    pairs[j] = o;
+                    pairs[n + j] = o + len;
+                    std::memcpy(files + o, blob + offsets[f], len);
+                    o += file_bytes(f);
+                }
+                DH_CUDA(cudaMemcpyAsync(d_blob_[slot], tb_.h_blob[slot], 16ull * n + o, cudaMemcpyHostToDevice, copy_stream_));
+                last_h2d_bytes_ += 16ull * n + o;
+            } else if (depth_loc == DH_DEPTH_DEVICE) {
+                launch_track_gather(depth, d_depth_[slot], d_e, n, px, copy_stream_);
+                launches_ += 1;
+            } else {
+                for (uint32_t j = 0; j < n; ++j)
+                    DH_CUDA(cudaMemcpyAsync(d_depth_[slot] + (size_t)j * px, depth + (size_t)e[j].frame * px, px * sizeof(uint16_t),
+                                            cudaMemcpyHostToDevice, copy_stream_));
+                last_h2d_bytes_ += (uint64_t)n * px * sizeof(uint16_t);
+            }
+            DH_CUDA(cudaEventRecord(ev_copied_[slot], copy_stream_));
+            DH_CUDA(cudaStreamWaitEvent(L.stream, ev_copied_[slot], 0));
+            FrameBuffers b = buffers(L, d_depth_[slot]);
+            if (blob) {
+                mark(DH_STAGE_H2D);  // the expansion counts as input transfer
+                DH_CUDA(cudaMemsetAsync(d_depth_[slot], 0, (size_t)n * px * sizeof(uint16_t), L.stream));
+                const unsigned long long* d_pairs = reinterpret_cast<const unsigned long long*>(d_blob_[slot]);
+                launch_biwi_decode(d_blob_[slot] + 16ull * n, d_pairs, d_pairs + n, 0ull, n, w, h, d_depth_[slot], tb_.d_status, L.stream);
+                launches_ += 1;
+            }
+            if (uniform) {
+                run_front(L, b, n, nullptr, e[0].prev >= 0 ? L.results : nullptr, min_seed_z);
+                run_back(L, b, n, iterations);
+            } else {
+                launch_track_guess(L.fs, L.frame_k, d_e, tb_.d_tracks, L.results, n, min_seed_z, blob ? tb_.d_status : nullptr,
+                                   tb_.d_bad, L.stream);
+                launches_ += 1;
+                run_front(L, b, n, nullptr, nullptr, 0.0f, nullptr, 0, true);
+                run_back(L, b, n, iterations, L.frame_k);
+            }
+            DH_CUDA(cudaMemcpyAsync(tb_.d_win + (size_t)pw * F, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToDevice, L.stream));
+            DH_CUDA(cudaEventRecord(ev_consumed_[slot], L.stream));
+            if (pw + 1 == W || p + 1 == n_pass) {
+                DH_CUDA(cudaMemcpyAsync(tb_.h_win[wi & 1u], tb_.d_win, sizeof(dh_result) * (size_t)(pw + 1) * F, cudaMemcpyDeviceToHost,
+                                        L.stream));
+                DH_CUDA(cudaEventRecord(tb_.ev_win[wi & 1u], L.stream));
+            }
         }
+        if (blob) DH_CUDA(cudaMemcpyAsync(tb_.h_bad, tb_.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream_));
     } catch (...) {
         cudaStreamSynchronize(copy_stream_);
         cudaStreamSynchronize(stream_);
-        dev_free(d_all);
         throw;
     }
-    dev_free(d_all);
     mark(-1);
     end_call();
+    const uint32_t last = (n_pass - 1) / W;
+    for (uint32_t wi = last >= 1 ? last - 1 : 0; wi <= last; ++wi) scatter(wi);
+    if (blob && *tb_.h_bad != ~0ull) throw_biwi_status((size_t)(*tb_.h_bad >> 2), (uint32_t)(*tb_.h_bad & 3u));
+}
+
+// n_seq tracks of frames_per_seq frames with one K and no starting seeds (sequence-major input):
+// the pass loop of predict_tracks takes the operations this call has always issued.
+void Context::predict_sequences(const HostForest& hf, const uint16_t* depth, uint32_t n_seq, uint32_t frames_per_seq, uint32_t w, uint32_t h,
+                                const float K[9], int depth_loc, float min_seed_z, dh_result* out) {
+    const uint64_t total = (uint64_t)n_seq * frames_per_seq;
+    if (total == 0 || total > 0x7fffffffull) {  // (no per-track tables for a call that does nothing)
+        if (total) throw ModelError(DH_E_ARG, "dh_predict_sequences: more than 2^31 frames");
+        begin_call();
+        have_debug_ = false;
+        last_encoded_chunks_ = 0;
+        last_h2d_bytes_ = 0;
+        end_call();
+        return;
+    }
+    std::vector<uint64_t> seq_off((size_t)n_seq + 1);
+    for (uint32_t s = 0; s <= n_seq; ++s) seq_off[s] = (uint64_t)s * frames_per_seq;
+    std::vector<dh_frame_args> args(n_seq);
+    for (dh_frame_args& a : args) {
+        std::memset(&a, 0, sizeof(a));
+        std::memcpy(a.K, K, sizeof(a.K));
+    }
+    predict_tracks(hf, depth, nullptr, nullptr, n_seq, seq_off.data(), w, h, depth_loc, args.data(), min_seed_z, out);
 }
 
 // ------------------------------------------------------------------------------------------------ 2-D back ends

@@ -52,6 +52,10 @@ struct Lane {
 };
 constexpr int kMaxLanes = 4;
 
+// The checks dh_predict_batch_biwi makes of n + 1 Biwi file offsets (monotone, 4-byte aligned starts,
+// files below 4 GB); DH_E_ARG naming the frame
+void check_biwi_offsets(const uint64_t* offsets, uint32_t n);
+
 // What a batch computes after the front end (SAT + traversal) of every chunk.
 struct BackEnd {
     enum Kind { kPose, kMask, kVotes, kBlurred } kind = kPose;
@@ -104,6 +108,11 @@ public:
     // seeded with the pose of frame t - 1 (examples/live_prediction.rs:75-88)
     void predict_sequences(const HostForest& hf, const uint16_t* depth, uint32_t n_seq, uint32_t frames_per_seq, uint32_t w, uint32_t h,
                            const float K[9], int depth_loc, float min_seed_z, dh_result* out);
+    // n_seq tracks: track s owns frames [seq_off[s], seq_off[s+1]) of depth at depth_loc, or of the Biwi
+    // files of blob / offsets (blob != nullptr); seq_args[s]: its K and the seeds of its first frame
+    void predict_tracks(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
+                        const uint64_t* seq_off, uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z,
+                        dh_result* out);
     // Biwi run-length coded frames (biwi.rs:81-103): blob/offsets in host memory, see depthhead_cuda.h
     void biwi_decode(const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h, uint16_t* out, int out_loc);
     void predict_batch_biwi(const HostForest& hf, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h,
@@ -172,8 +181,9 @@ private:
     TilePlan plan_tiles(const Geometry& g) const;
     FrameBuffers buffers(const Lane& L, const uint16_t* depth) const;
     // args: per-frame arguments of the batch (frames f0 .. f0 + n - 1 are this pass's) or nullptr
+    // fs_written: a kernel of the caller has already written the pass's frame states (track_guess_kernel)
     void run_front(Lane& L, const FrameBuffers& b, uint32_t n, const FrameState* guess_state, const dh_result* prev_results = nullptr,
-                   float min_seed_z = 0.0f, const dh_frame_args* args = nullptr, uint32_t f0 = 0);
+                   float min_seed_z = 0.0f, const dh_frame_args* args = nullptr, uint32_t f0 = 0, bool fs_written = false);
     void run_back(Lane& L, const FrameBuffers& b, uint32_t n, uint32_t iterations, const float* frame_k = nullptr);
     void begin_call();
     void end_call();
@@ -264,6 +274,27 @@ private:
     FrameState* h_frame_fs_ = nullptr;
     float* h_frame_k_ = nullptr;
     size_t h_frame_cap_ = 0;
+
+    // dh_predict_tracks / dh_predict_sequences (predict_tracks): buffers of the pass loop, grown and kept.
+    // Results and slot tables move in windows of passes; none of these depends on the call's frame count.
+    struct TrackBuffers {
+        TrackSlot* d_plan[2] = {nullptr, nullptr};   // a window's slot tables, by window parity
+        TrackSlot* h_plan[2] = {nullptr, nullptr};   // (pinned)
+        dh_result* d_win = nullptr;                  // results of the window's passes, [passes][F]
+        dh_result* h_win[2] = {nullptr, nullptr};    // (pinned, by window parity)
+        size_t win_cap = 0;                          // entries of each of the six above
+        TrackArgs* d_tracks = nullptr;               // [n_seq]
+        TrackArgs* h_tracks = nullptr;               // (pinned)
+        size_t tracks_cap = 0;
+        uint8_t* h_blob[2] = {nullptr, nullptr};     // Biwi passes: (start, end) pairs then the files (pinned, by staging slot)
+        size_t blob_cap = 0;
+        uint32_t* d_status = nullptr;                // [F] decode status of a Biwi pass
+        size_t status_cap = 0;
+        unsigned long long* d_bad = nullptr;         // lowest bad Biwi frame << 2 | its status
+        unsigned long long* h_bad = nullptr;
+        cudaEvent_t ev_win[2] = {nullptr, nullptr};  // the window's results are in h_win
+    } tb_;
+    void free_track_buffers();
 
     // dh_predict as a CUDA graph: the single-frame pipeline is a dozen small launches, i.e. bound
     // by launch overhead; after one eager call with a given (model, shape, intrinsics, stream) the

@@ -2278,6 +2278,57 @@ __global__ void __launch_bounds__(128) seq_guess_kernel(FrameState* __restrict__
     fs[i].has_guess = g;
 }
 
+// ================================================================ tracks (dh_predict_tracks)
+// One thread per slot of a pass: the slot's frame state (zero but for the seeds, as dh_predict's) and
+// its row of the K / K^-1 table.  A track's first frame takes the caller's seeds; every later frame
+// the previous pass's result at the planned position, by the rule of seq_guess_kernel.  Biwi passes
+// also fold the decode status of the slot into the lowest bad global frame index (index << 2 | code).
+__global__ void __launch_bounds__(128) track_guess_kernel(FrameState* __restrict__ fs, float* __restrict__ frame_k,
+                                                          const TrackSlot* __restrict__ slots, const TrackArgs* __restrict__ tracks,
+                                                          const dh_result* __restrict__ prev, uint32_t n, float min_seed_z,
+                                                          const uint32_t* __restrict__ status, unsigned long long* __restrict__ bad) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const TrackSlot s = slots[i];
+    const TrackArgs& a = tracks[s.track];
+    FrameState st = {};
+    if (s.prev < 0) {
+        st.has_guess = a.has_guess;
+        if (a.has_guess & 1u)
+            for (int k = 0; k < 3; ++k) st.midp_guess[k] = a.midp_guess[k];
+        if (a.has_guess & 2u)
+            for (int k = 0; k < 3; ++k) st.rot_guess[k] = a.rot_guess[k];
+    } else {
+        const dh_result r = prev[s.prev];
+        st.has_guess = 2u;
+        if (r.mid_point[2] > min_seed_z) {
+            st.has_guess |= 1u;
+            for (int k = 0; k < 3; ++k) st.midp_guess[k] = r.mid_point[k];
+        }
+        for (int k = 0; k < 3; ++k) st.rot_guess[k] = r.rotation[k];
+    }
+    fs[i] = st;
+    for (int k = 0; k < 18; ++k) frame_k[(size_t)i * 18 + k] = a.K[k];
+    if (status && status[i]) atomicMin(bad, ((unsigned long long)(uint32_t)s.frame << 2) | (status[i] & 3u));
+}
+
+// Device-resident frames of a pass: frame slots[f].frame of src into slot f of dst, 16 bytes per load
+// when every frame starts 16-byte aligned (else 2).  blockIdx.y = slot.
+__global__ void __launch_bounds__(256) track_gather_kernel(const uint16_t* __restrict__ src, uint16_t* __restrict__ dst,
+                                                           const TrackSlot* __restrict__ slots, size_t frame_px, uint32_t vec) {
+    const uint32_t f = blockIdx.y;
+    const uint16_t* s = src + (size_t)(uint32_t)slots[f].frame * frame_px;
+    uint16_t* d = dst + (size_t)f * frame_px;
+    const size_t step = (size_t)gridDim.x * blockDim.x, i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (vec) {
+        const uint4* s4 = reinterpret_cast<const uint4*>(s);
+        uint4* d4 = reinterpret_cast<uint4*>(d);
+        for (size_t i = i0; i < frame_px / 8; i += step) d4[i] = __ldg(s4 + i);
+    } else {
+        for (size_t i = i0; i < frame_px; i += step) d[i] = __ldg(s + i);
+    }
+}
+
 // ================================================================ work counters of a pass
 __global__ void __launch_bounds__(256) counters_kernel(const FrameState* __restrict__ fs, uint32_t n_frames,
                                                        unsigned long long* __restrict__ out, uint32_t P, uint32_t T) {
@@ -2554,6 +2605,19 @@ void launch_hough2d_pose(const unsigned long long* keys, const uint16_t* depth, 
 
 void launch_seq_guess(FrameState* fs, const dh_result* prev, uint32_t n, float min_seed_z, cudaStream_t s) {
     if (n) seq_guess_kernel<<<(n + 127) / 128, 128, 0, s>>>(fs, prev, n, min_seed_z);
+}
+
+void launch_track_guess(FrameState* fs, float* frame_k, const TrackSlot* slots, const TrackArgs* tracks, const dh_result* prev,
+                        uint32_t n, float min_seed_z, const uint32_t* status, unsigned long long* bad, cudaStream_t s) {
+    if (n) track_guess_kernel<<<(n + 127) / 128, 128, 0, s>>>(fs, frame_k, slots, tracks, prev, n, min_seed_z, status, bad);
+}
+
+void launch_track_gather(const uint16_t* src, uint16_t* dst, const TrackSlot* slots, uint32_t n, size_t frame_px, cudaStream_t s) {
+    if (!n) return;
+    const uint32_t vec = ((reinterpret_cast<uintptr_t>(src) & 15u) == 0 && frame_px % 8 == 0) ? 1u : 0u;
+    const size_t words = vec ? frame_px / 8 : frame_px;
+    const uint32_t blocks = (uint32_t)std::min<size_t>(64, std::max<size_t>(1, (words + 1023) / 1024));
+    track_gather_kernel<<<dim3(blocks, n), 256, 0, s>>>(src, dst, slots, frame_px, vec);
 }
 
 void launch_counters(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, unsigned long long* out,

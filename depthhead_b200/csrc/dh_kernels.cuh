@@ -148,6 +148,23 @@ int launch_gaussian_blur(const uint32_t* in, uint16_t* tmp, uint16_t* out, unsig
 void launch_hough2d_pose(const unsigned long long* keys, const uint16_t* depth, const Geometry& g, uint32_t n_frames, dh_result* out,
                          cudaStream_t s);
 void launch_seq_guess(FrameState* fs, const dh_result* prev, uint32_t n, float min_seed_z, cudaStream_t s);
+
+// dh_predict_tracks: one slot of a pass (frame = global frame index, track = its track, prev = the
+// track's position in the previous pass or -1 for its first frame) and the arguments of one track
+struct TrackSlot {
+    int32_t frame, track, prev;
+};
+struct TrackArgs {
+    float K[18];          // K then K^-1 (row-major, K^-1 by mat3_inverse_f32 on the host)
+    float midp_guess[3];  // seeds of the track's first frame
+    uint32_t has_guess;
+    double rot_guess[3];
+};
+// slot i: frame state and K / K^-1 row (frame_k [n][18]); status (pass-local Biwi decode status) may be nullptr
+void launch_track_guess(FrameState* fs, float* frame_k, const TrackSlot* slots, const TrackArgs* tracks, const dh_result* prev,
+                        uint32_t n, float min_seed_z, const uint32_t* status, unsigned long long* bad, cudaStream_t s);
+// dst[i] = frame slots[i].frame of src (device memory, [..][frame_px] u16)
+void launch_track_gather(const uint16_t* src, uint16_t* dst, const TrackSlot* slots, uint32_t n, size_t frame_px, cudaStream_t s);
 void launch_counters(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, unsigned long long* out,
                      cudaStream_t s);
 // Biwi run-length decode: frame i = blob[offsets[i] - blob_base, offsets[i+1] - blob_base), or up to ends[i] - blob_base

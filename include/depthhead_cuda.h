@@ -16,6 +16,8 @@
  *   examples/live_prediction.rs:75-88 frame-to-frame seeding of a sequence     -> dh_predict_sequences
  *   predict_parameter_parallel over n frames, each with its own K and seeds    -> dh_predict_frames,
  *                                                                                 dh_predict_frames_biwi
+ *   the same seeding over tracks of any length, each with its own K and first seeds -> dh_predict_tracks,
+ *                                                                                 dh_predict_tracks_biwi
  *   src/hough/prediction.rs:850-905   predict_mask                             -> dh_predict_mask
  *   src/hough/prediction.rs:760-841   build_hough_image (votes, before blur)   -> dh_hough_image_raw
  *   src/hough/prediction.rs:760-845   build_hough_image (with its blur)        -> dh_build_hough_image
@@ -228,6 +230,26 @@ int dh_predict_batch_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, co
  * folders each have their own depth.cal, in one call. */
 int dh_predict_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
                            uint32_t w, uint32_t h, const dh_frame_args* args, dh_result* out);
+
+/* Tracks: the seeding of dh_predict_sequences over sequences of any length, each from its own camera
+ * and with an optional starting pose (multi-camera rigs, a detector that starts tracks, the Biwi
+ * database's sequence folders with their own depth.cal).  n_seq tracks; track s owns frames
+ * [seq_off[s], seq_off[s+1]) of depth ([total][h][w], frames of one track consecutive and in time
+ * order; seq_off: n_seq + 1 entries, seq_off[0] = 0, monotone, total = seq_off[n_seq] < 2^31).
+ * seq_args[s]: K of the track, and seeds of its FIRST frame (has_guess bits as in dh_frame_args).
+ * Frame t > 0 of a track is seeded from frame t-1 of the same track by the rule of
+ * dh_predict_sequences (centre iff z > min_seed_z, rotation always).  out[total] in input order.
+ * Equal, bit for bit on mid_point and rotation, to dh_predict frame by frame with those seeds, for
+ * any chunk size.  Zero-length tracks are allowed; n_seq = 0 or total = 0 is a no-op.  K is not
+ * validated, as in dh_predict; a has_guess with bits other than 0-1 is DH_E_ARG naming the track.
+ * Synchronous. */
+int dh_predict_tracks(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n_seq, const uint64_t* seq_off,
+                      uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z, dh_result* out);
+/* The same from Biwi files: frame i at blob[offsets[i], offsets[i+1]) (as dh_predict_frames_biwi);
+ * a damaged file is DH_E_ARG naming the lowest bad frame index, whatever order the passes ran in. */
+int dh_predict_tracks_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
+                           const uint64_t* seq_off, uint32_t w, uint32_t h, const dh_frame_args* seq_args, float min_seed_z,
+                           dh_result* out);
 /* The writer for that format (the reference only reads it): n raw frames [n][h][w] u16 become n
  * files in ONE blob, file i at [offsets[i], offsets[i+1]) (offsets: n+1 entries, multiples of 16).
  * Runs are found at a granularity of 16 pixels: a group of 16 pixels with any non-zero pixel is

@@ -104,6 +104,11 @@ extern "C" {
                              w: u32, h: u32, k: *const f32, out: *mut DhResult) -> c_int;
     fn dh_predict_frames_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32,
                               w: u32, h: u32, args: *const DhFrameArgs, out: *mut DhResult) -> c_int;
+    fn dh_predict_tracks(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n_seq: u32, seq_off: *const u64, w: u32, h: u32,
+                         depth_loc: c_int, seq_args: *const DhFrameArgs, min_seed_z: f32, out: *mut DhResult) -> c_int;
+    fn dh_predict_tracks_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n_seq: u32,
+                              seq_off: *const u64, w: u32, h: u32, seq_args: *const DhFrameArgs, min_seed_z: f32,
+                              out: *mut DhResult) -> c_int;
     fn dh_biwi_parse_cal(text: *const c_char, len: usize, k: *mut f32) -> c_int;
     fn dh_biwi_parse_pose(file: *const u8, len: usize, k: *const f32, pos3d: *mut f32, pos2d: *mut f32,
                           rot: *mut f32) -> c_int;
@@ -341,6 +346,23 @@ impl HoughPrediction {
                                             out.as_mut_ptr()) })?;
         Ok(out)
     }
+    /// Tracks of any length in one call: track s is the next lengths[s] frames of `frames` (in time order),
+    /// from its own camera intrinsics[s], with optional seeds of its first frame; every later frame is
+    /// seeded from the frame before it as in predict_sequences.  Results in input order, equal to
+    /// predict_parameter_parallel frame by frame with those seeds.
+    pub fn predict_tracks(&self, frames: &[u16], lengths: &[u32], w: u32, h: u32, intrinsics: &[IntrinsicMatrix],
+                          midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>], min_seed_z: f32)
+                          -> Result<Vec<DhResult>, Error> {
+        let seq_off = track_offsets(lengths);
+        let n = *seq_off.last().unwrap() as usize;
+        assert_eq!(frames.len(), n * (w as usize) * (h as usize));
+        let args = frame_args(lengths.len() as u32, intrinsics, midp_guess, rot_guess);
+        self.push_fields()?;
+        let mut out = vec![DhResult::default(); n];
+        check(unsafe { dh_predict_tracks(self.context(), self.forest, frames.as_ptr(), lengths.len() as u32, seq_off.as_ptr(), w, h,
+                                         0 /* DH_DEPTH_HOST */, args.as_ptr(), min_seed_z, out.as_mut_ptr()) })?;
+        Ok(out)
+    }
     /// HoughLearning::learn (prediction.rs:145-234) on the GPU: `depth`/`mask` are n frames back to
     /// back, `k` one row-major 3x3 matrix per frame, `pos3d`/`rot` the annotated head pose per frame.
     pub fn learn(params: &DhTrainParams, n: u32, w: u32, h: u32, depth: &[u16], mask: &[u8], k: &[f32],
@@ -365,6 +387,14 @@ impl Drop for HoughPrediction {
             dh_forest_free(self.forest);
         }
     }
+}
+
+/// n_seq + 1 frame offsets of tracks of the given lengths
+fn track_offsets(lengths: &[u32]) -> Vec<u64> {
+    let mut off = Vec::with_capacity(lengths.len() + 1);
+    off.push(0u64);
+    for &l in lengths { off.push(off.last().unwrap() + l as u64); }
+    off
 }
 
 /// one DhFrameArgs per frame; every slice has n entries
@@ -465,6 +495,22 @@ pub mod biwi {
             let mut out = vec![DhResult::default(); n as usize];
             check(unsafe { dh_predict_frames_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
                                                   files.width, files.height, args.as_ptr(), out.as_mut_ptr()) })?;
+            Ok(out)
+        }
+        /// predict_tracks over the files: track s is the next lengths[s] files (a sequence folder, in time
+        /// order) with its own depth.cal and optional seeds of its first frame; results in file order
+        pub fn predict_tracks_biwi(&self, files: &PackedFiles, lengths: &[u32], intrinsics: &[IntrinsicMatrix],
+                                   midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>], min_seed_z: f32)
+                                   -> Result<Vec<DhResult>, Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            let seq_off = track_offsets(lengths);
+            assert_eq!(*seq_off.last().unwrap(), n as u64, "the track lengths must add up to the number of files");
+            let args = frame_args(lengths.len() as u32, intrinsics, midp_guess, rot_guess);
+            self.push_fields()?;
+            let mut out = vec![DhResult::default(); n as usize];
+            check(unsafe { dh_predict_tracks_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(),
+                                                  lengths.len() as u32, seq_off.as_ptr(), files.width, files.height, args.as_ptr(),
+                                                  min_seed_z, out.as_mut_ptr()) })?;
             Ok(out)
         }
     }
