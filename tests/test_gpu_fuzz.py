@@ -4,25 +4,22 @@ configurations drawn at random from the whole parameter space of the prediction 
 tree count / depth / sparsity, node order in the file, stride, image size,
 gaussian sigma, mean-shift iterations, caller seeds, frame content.  Every stage is compared as
 in test_gpu_parity (leaf ids and accumulators bit-exact, trajectories and the pose identical).
+Every frame and the batch run on both gate paths: patch_gate_kernel (probability codes where the
+forest has box-sum rectangles) with the seed grids from gated-patch lists, and the fold inside
+gate_coarse_kernel (test_gpu_parity.list_ctx / fold_ctx).  The random shapes give patch counts that
+are rarely multiples of patch_gate_kernel's 1024 patches per CTA.
 The draws depend only on the case number, so a failure reproduces with `-k "case17"`.
 """
 import numpy as np
 import pytest
 
 import oracle
-from depthhead_b200 import Context, HoughPrediction, IntrinsicMatrix, synth
-from test_gpu_parity import _compare_frame
+from depthhead_b200 import HoughPrediction, IntrinsicMatrix, synth
+from test_gpu_parity import _compare_frame, fold_ctx, list_ctx  # noqa: F401 (module fixtures)
 
 pytestmark = pytest.mark.gpu
 
 N_CASES = 96
-
-
-@pytest.fixture(scope="module")
-def ctx():
-    c = Context(0)
-    yield c
-    c.close()
 
 
 def _draw(case):
@@ -70,7 +67,7 @@ def _frames(rng, h, w, case):
 
 
 @pytest.mark.parametrize("case", range(N_CASES), ids=lambda c: "case%d" % c)
-def test_random_configuration(ctx, case):
+def test_random_configuration(list_ctx, fold_ctx, case):
     rng, forest, model, h, w = _draw(case)
     arr = synth.make_forest(**forest)
     js = synth.forest_to_json(arr, **model)
@@ -83,10 +80,13 @@ def test_random_configuration(ctx, case):
             mid = [float(v) for v in rng.uniform([-200, -150, 500], [200, 150, 1400])]
         if rng.random() < 0.3:
             rot = [float(v) for v in rng.uniform(-1.0, 1.0, 3)]  # radians (prediction.rs:437-460)
-        _compare_frame(ctx, hp, of, d, mid, rot)
+        tr = of.predict(d, synth.KINECT_K, mid, rot, mode=oracle.MODE_SAT, keep=True)
+        for c in (list_ctx, fold_ctx):
+            _compare_frame(c, hp, of, d, mid, rot, trace=tr)
     # the batch entry point on the same frames (no caller seeds)
-    out = hp.predict_batch(np.stack(frames), IntrinsicMatrix.default_kinect_intrinsic(), ctx=ctx)
+    outs = [hp.predict_batch(np.stack(frames), IntrinsicMatrix.default_kinect_intrinsic(), ctx=c) for c in (list_ctx, fold_ctx)]
     for i, d in enumerate(frames):
         tr = of.predict(d, synth.KINECT_K, mode=oracle.MODE_SAT, keep=False)
-        assert np.array_equal(out["mid_point"][i], tr.mid_point)
-        assert np.array_equal(out["rotation"][i].view(np.uint64), tr.rotation.view(np.uint64))
+        for out in outs:
+            assert np.array_equal(out["mid_point"][i], tr.mid_point)
+            assert np.array_equal(out["rotation"][i].view(np.uint64), tr.rotation.view(np.uint64))

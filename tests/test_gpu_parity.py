@@ -4,11 +4,14 @@ Bars (BASELINE.json north_star): leaf index per patch x tree bit-exact; votes ex
 and u32 sums — tighter than the 1e-5 relative the north star allows); seeds identical; final head
 centre / rotation identical (the bar is 1 mm / 0.1 degree, i.e. the same 3-degree bin).
 """
+import os
+
 import numpy as np
 import pytest
 
 import oracle
 from depthhead_b200 import Context, HoughPrediction, IntrinsicMatrix, capi, synth
+from test_prob_codes_cpu import codes_of, thresholds
 
 pytestmark = pytest.mark.gpu
 
@@ -22,6 +25,42 @@ def ctx():
     c.close()
 
 
+def context_with(**env):
+    """a Context created with the given DH_* switches set, or unset where the value is None (the
+    constructor reads them; the process environment is restored afterwards)"""
+    old = {k: os.environ.get(k) for k in env}
+    for k, v in env.items():
+        if v is None:
+            os.environ.pop(k, None)
+        else:
+            os.environ[k] = str(v)
+    try:
+        return Context(0)
+    finally:
+        for k, v in old.items():
+            if v is None:
+                del os.environ[k]
+            else:
+                os.environ[k] = v
+
+
+# Passes of DH_GATE_SPLIT_MIN frames or more gate their patches in patch_gate_kernel (probability codes
+# in the leaf words decide most patches, the gated-patch lists feed gate_coarse_kernel<true, .>); smaller
+# passes fold every patch's probabilities in phase A of gate_coarse_kernel<false, .>, one launch less.
+@pytest.fixture(scope="module")
+def list_ctx():
+    c = context_with(DH_GATE_SPLIT_MIN=1)
+    yield c
+    c.close()
+
+
+@pytest.fixture(scope="module")
+def fold_ctx():
+    c = context_with(DH_GATE_SPLIT_MIN=1 << 30)
+    yield c
+    c.close()
+
+
 def _filter_acc(keys, vals, origin, dim):
     """non-zero cells inside the cube [origin, origin + dim)^3"""
     if len(vals) == 0 or dim == 0:
@@ -31,13 +70,14 @@ def _filter_acc(keys, vals, origin, dim):
     return keys[m], vals[m]
 
 
-def _compare_frame(ctx, hp, of, depth, midp_guess=None, rot_guess=None, check_patches=True, intrinsic=None):
+def _compare_frame(ctx, hp, of, depth, midp_guess=None, rot_guess=None, check_patches=True, intrinsic=None, trace=None):
     """every stage of one frame against the oracle; intrinsic: a float32 3x3 matrix for both sides
-    (None = the Kinect default)"""
+    (None = the Kinect default); trace: the oracle's trace of this frame with these arguments
+    (keep=True), when the caller already has it"""
     k = synth.KINECT_K if intrinsic is None else np.asarray(intrinsic, np.float32)
     ctx.enable_debug(True)
     res = hp.predict_parameter_parallel(depth, K if intrinsic is None else IntrinsicMatrix(k), midp_guess, rot_guess, ctx=ctx)
-    tr = of.predict(depth, k, midp_guess, rot_guess, mode=oracle.MODE_SAT, keep=True)
+    tr = of.predict(depth, k, midp_guess, rot_guess, mode=oracle.MODE_SAT, keep=True) if trace is None else trace
     npx, npy, T = ctx.debug_dims()
     assert (npx, npy, T) == (tr.npx, tr.npy, of.n_trees)
     # --- leaf index per patch x tree: bit-exact
@@ -133,35 +173,83 @@ def test_exact_ties_in_the_node_test(ctx):
         _compare_frame(ctx, hp, of, d)
 
 
-@pytest.mark.parametrize("n_trees", [1, 3, 10])
-def test_patch_gate_at_the_threshold(ctx, n_trees):
-    """prob > 0.7 (prediction.rs:582-584) with leaf probabilities whose sums sit on, one ulp around and
-    within 1/256 of 0.7 * T: the traversal's gate tail decides from 8-bit probability codes and must send
-    every such patch through the exact f64 fold; probabilities of exactly 0.0 and 1.0 sit at the ends of
-    the code range."""
-    rng = np.random.default_rng(n_trees)
-    arr = synth.make_forest(seed=40 + n_trees, n_trees=n_trees, max_depth=6)
-    NL = len(arr["prob"])
-    base = np.full(NL, 0.7)
-    kind = rng.integers(0, 8, NL)
-    prob = np.where(kind == 0, np.nextafter(base, 1.0), base)
-    prob = np.where(kind == 1, np.nextafter(base, 0.0), prob)
-    prob = np.where(kind == 2, 0.7 + 1.0 / 300, prob)
-    prob = np.where(kind == 3, 0.7 - 1.0 / 300, prob)
-    prob = np.where(kind == 4, 1.0, prob)
-    prob = np.where(kind == 5, 0.0, prob)
-    prob = np.where(kind == 6, 0.4, prob)
+def _threshold_menus(T):
+    """leaf probability sub-menus ((value, weight) lists), one forest each, whose sums of T leaves
+    concentrate on the code thresholds of T trees (test_prob_codes_cpu.thresholds)"""
+    up, dn = 1.0, -1.0
+    _, pass_codes, fail_codes = thresholds(T)
+    nx = np.nextafter
+    code178 = [0.7 - 1.0 / 300, nx(179 / 256, dn)]
+    code179 = [179 / 256, nx(179 / 256, up), 0.7, nx(0.7, up), nx(0.7, dn), nx(180 / 256, dn)]
+    code180 = [180 / 256, nx(180 / 256, up), 0.7 + 1.0 / 300]
+    q_pass = min(max((pass_codes - 0.5 - 179 * T) / T, 0.0), 1.0)           # mean S = pass_codes - 1/2
+    q_fail = min(max((fail_codes + 0.5 - T - 178 * T) / T, 0.0), 1.0)       # mean S + T = fail_codes + 1/2
+    return [
+        [(v, 1.0) for v in (0.7, nx(0.7, up), nx(0.7, dn))],                 # every code 179: ulp decisions
+        [(v, (1 - q_pass) / 6) for v in code179] + [(v, q_pass / 3) for v in code180],
+        [(v, (1 - q_fail) / 2) for v in code178] + [(v, q_fail / 6) for v in code179],
+        [(179 / 256, 0.8), (180 / 256, 0.2)],                                # exact folds: S / 256 is the sum
+    ]
+
+
+def _threshold_forest(T, k, menu):
+    """depth-6 trees whose leaves draw from `menu`, plus 0.0 and 1.0 (the ends of the code range) at 1 % each"""
+    arr = synth.make_forest(seed=40 + 7 * T + k, n_trees=T, max_depth=6)
+    rng = np.random.default_rng([T, k])
+    vals = np.array([v for v, _ in menu] + [0.0, 1.0])
+    w = np.array([p for _, p in menu])
+    w = np.concatenate([0.98 * w / w.sum(), [0.01, 0.01]])
+    prob = vals[rng.choice(len(vals), len(arr["prob"]), p=w)]
     nv = np.diff(arr["vote_off"])
-    prob = np.where((nv == 0) & (prob > 0), 0.0, prob)  # prob > 0 needs votes (prediction.rs:594)
-    arr["prob"] = prob.astype(np.float64)
-    js = synth.forest_to_json(arr, stepwidth=6)
-    hp = HoughPrediction.from_json(js)
-    of = oracle.OracleForest.from_json(js)
-    gates = 0
-    for d in synth.make_frames(2, seed=61):
-        _, tr = _compare_frame(ctx, hp, of, d)
-        gates += int(tr.gate.sum())
-    assert gates > 0
+    arr["prob"] = np.where((nv == 0) & (prob > 0), 0.0, prob).astype(np.float64)  # prob > 0 needs votes (prediction.rs:594)
+    return arr
+
+
+@pytest.mark.parametrize("n_trees", [1, 3, 5, 10, 20])
+def test_patch_gate_at_the_threshold(list_ctx, fold_ctx, n_trees):
+    """prob > 0.7 (prediction.rs:582-584) with leaf probabilities on, one ulp around and 1/300 around 0.7,
+    on the code boundaries 179/256 and 180/256 and one ulp around them, and 0.0 and 1.0, drawn so that
+    the sums of T leaves sit on the code thresholds.  Every frame runs on both gate paths: on list_ctx,
+    patch_gate_kernel<false> decides a patch from its code sum S when S >= gate_pass_codes or
+    S + T <= gate_fail_codes and folds the rest; on fold_ctx, phase A of gate_coarse_kernel<false, false>
+    folds every patch.  Both must give the reference's gate flags, p3 bits and everything after them."""
+    T = n_trees
+    smin, pass_codes, fail_codes = thresholds(T)
+    frames = synth.make_frames(2, seed=61)
+    cls = dict.fromkeys(("S = pass", "S = pass - 1, folds below", "S + T = fail", "S + T = fail + 1",
+                         "undecided, passes", "undecided, fails", "fold = gate_min_sum"), 0)
+    for k, menu in enumerate(_threshold_menus(T)):
+        arr = _threshold_forest(T, k, menu)
+        js = synth.forest_to_json(arr, stepwidth=6)
+        hp = HoughPrediction.from_json(js)
+        of = oracle.OracleForest.from_json(js)
+        for d in frames:
+            tr = of.predict(d, synth.KINECT_K, mode=oracle.MODE_SAT, keep=True)
+            _compare_frame(fold_ctx, hp, of, d, trace=tr)
+            launches = fold_ctx.counters()["launches"]
+            _compare_frame(list_ctx, hp, of, d, trace=tr)
+            # the list path ran: patch_gate_kernel is the one extra launch
+            assert list_ctx.counters()["launches"] == launches + 1
+            # what the code decision saw (the leaf words' codes have no accessor: restated from the oracle's leaf ids)
+            leaf = tr.leaf[tr.leaf[:, 0] >= 0]
+            prob = arr["prob"][leaf]
+            S = codes_of(prob).sum(axis=1)
+            fold = np.zeros(len(leaf))
+            for t in range(T):
+                fold = fold + prob[:, t]
+            ref = fold / T > 0.7
+            assert np.array_equal(ref, tr.gate[tr.leaf[:, 0] >= 0] == 1)
+            undecided = (S < pass_codes) & (S + T > fail_codes)
+            cls["S = pass"] += int(np.sum(S == pass_codes))
+            cls["S = pass - 1, folds below"] += int(np.sum((S == pass_codes - 1) & undecided & ~ref))
+            cls["S + T = fail"] += int(np.sum(S + T == fail_codes))
+            cls["S + T = fail + 1"] += int(np.sum(S + T == fail_codes + 1))
+            cls["undecided, passes"] += int(np.sum(undecided & ref))
+            cls["undecided, fails"] += int(np.sum(undecided & ~ref))
+            cls["fold = gate_min_sum"] += int(np.sum(fold == smin))
+    if T == 20:
+        cls.pop("fold = gate_min_sum")  # no sum of these values lands on 14.000000000000002
+    assert all(cls.values()), cls
 
 
 def test_caller_seeds(ctx, small_case):

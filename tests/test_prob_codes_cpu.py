@@ -1,8 +1,10 @@
 """The patch gate from 8-bit probability codes (patch_gate_kernel, DESIGN.md section 5), restated in numpy
 with the thresholds the context computes (dh_ctx.cu: Geometry::gate_pass_codes / gate_fail_codes): a
 decision taken from the code sum alone must never contradict the reference's gate, the ordered f64 fold
-`sum(prob) / T > 0.7` (prediction.rs:582-584).  CPU only: this pins the arithmetic, the GPU tests pin the
-kernel (tests/test_gpu_parity.py::test_patch_gate_at_the_threshold)."""
+`sum(prob) / T > 0.7` (prediction.rs:582-584).  CPU only: this pins the arithmetic.  The kernel is pinned
+on the GPU by tests/test_gpu_parity.py::test_patch_gate_at_the_threshold, which runs patch_gate_kernel<false>
+with codes (passes of at least DH_GATE_SPLIT_MIN frames) on leaf sums at these thresholds, and by
+tests/test_gpu_gate_list.py (the kFrameK instantiations, gated-list slices, probabilities outside [0, 1])."""
 import math
 
 import numpy as np
