@@ -231,6 +231,12 @@ def frame_args(n: int, intrinsics, midp_guess=None, rot_guess=None, has_midp=Non
     return args
 
 
+def intrinsic_array(n: int, intrinsics) -> np.ndarray:
+    """float32 [n,9] row-major matrices of dh_build_hough_image_frames from one IntrinsicMatrix or a
+    float32 [n,3,3] array (checked as in frame_args)."""
+    return np.ascontiguousarray(frame_args(n, intrinsics)["K"])
+
+
 def _track_offsets(lengths):
     """(uint64 [n_seq+1] offsets from 0, n_seq, total) of the track lengths of dh_predict_tracks"""
     ln = np.asarray(lengths)
@@ -539,6 +545,37 @@ class HoughPrediction:
         capi.check(capi.load().dh_build_hough_image_batch(ctx._h, self._h, p, n, w, h, intrinsic._ptr(), loc, 1, None,
                                                           capi.DH_DEPTH_HOST, capi.ptr(res)))
         return res
+
+    # ---- the same three with a K per frame (frames of several cameras in one call): intrinsics is one
+    # IntrinsicMatrix or a float32 [n,3,3] array; results equal the single-frame calls with each frame's K.
+    def _hough_frames(self, frames, intrinsics, ctx, device_ptr, n, w, h, out_device_ptr, blur, image, from2d):
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        Ks = intrinsic_array(n, intrinsics)
+        ctx = ctx or default_context()
+        out, op, oloc = _image_out(out_device_ptr, (n, h, w), np.uint16) if image else (None, None, capi.DH_DEPTH_HOST)
+        res = np.zeros(n, capi.RESULT_DTYPE) if from2d else None
+        capi.check(capi.load().dh_build_hough_image_frames(ctx._h, self._h, p, n, w, h, loc, capi.ptr(Ks), int(blur), op, oloc,
+                                                           capi.ptr(res)))
+        return out, res
+
+    def hough_image_raw_frames(self, frames, intrinsics, ctx: Context | None = None, device_ptr: int | None = None,
+                               n: int | None = None, w: int | None = None, h: int | None = None,
+                               out_device_ptr: int | None = None) -> np.ndarray | None:
+        """hough_image_raw_batch with a K per frame: uint16 [n,h,w]."""
+        return self._hough_frames(frames, intrinsics, ctx, device_ptr, n, w, h, out_device_ptr, False, True, False)[0]
+
+    def build_hough_image_frames(self, frames, intrinsics, ctx: Context | None = None, device_ptr: int | None = None,
+                                 n: int | None = None, w: int | None = None, h: int | None = None, out_device_ptr: int | None = None,
+                                 from2d: bool = False):
+        """build_hough_image_batch with a K per frame: uint16 [n,h,w] (None with out_device_ptr);
+        from2d=True: (images, capi.RESULT_DTYPE[n] of predict_parameter_from2dhough)."""
+        out, res = self._hough_frames(frames, intrinsics, ctx, device_ptr, n, w, h, out_device_ptr, True, True, from2d)
+        return (out, res) if from2d else out
+
+    def predict_parameter_from2dhough_frames(self, frames, intrinsics, ctx: Context | None = None, device_ptr: int | None = None,
+                                             n: int | None = None, w: int | None = None, h: int | None = None) -> np.ndarray:
+        """predict_parameter_from2dhough_batch with a K per frame: capi.RESULT_DTYPE[n]."""
+        return self._hough_frames(frames, intrinsics, ctx, device_ptr, n, w, h, None, True, False, True)[1]
 
     def debug_leaf_static(self, ctx: Context | None = None):
         ctx = ctx or default_context()

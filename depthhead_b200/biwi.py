@@ -12,7 +12,8 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .api import Context, HoughPrediction, IntrinsicMatrix, _track_offsets, default_context, frame_args
+from .api import (Context, HoughPrediction, IntrinsicMatrix, _image_out, _track_offsets, default_context, frame_args,
+                  intrinsic_array)
 
 
 def encode_depth(img: np.ndarray) -> bytes:
@@ -142,6 +143,35 @@ def predict_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w:
         return out
     capi.check(capi.load().dh_predict_batch_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
                                                  intrinsic._ptr(), capi.ptr(out)))
+    return out
+
+
+def build_hough_image_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w: int, h: int, intrinsics, blur: bool = True,
+                            from2d: bool = False, images: bool = True, ctx: Context | None = None, out_device_ptr: int | None = None):
+    """read_depth + build_hough_image (blur=True; blur=False: the vote image before its blur) per file,
+    every file with its own K (examples/db_prediction.rs:154 over a database of several sequence folders),
+    the decode on the GPU.  intrinsics: one IntrinsicMatrix or a float32 [n,3,3] array.  Returns uint16
+    [n,h,w] (None with out_device_ptr or images=False); from2d=True (needs blur): (images,
+    capi.RESULT_DTYPE[n] of predict_parameter_from2dhough)."""
+    n = len(offsets) - 1
+    Ks = intrinsic_array(n, intrinsics)
+    ctx = ctx or default_context()
+    out, op, oloc = _image_out(out_device_ptr, (n, int(h), int(w)), np.uint16) if images else (None, None, capi.DH_DEPTH_HOST)
+    res = np.zeros(n, capi.RESULT_DTYPE) if from2d else None
+    offsets = np.ascontiguousarray(offsets, np.uint64)
+    capi.check(capi.load().dh_build_hough_image_frames_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
+                                                            capi.ptr(Ks), int(bool(blur)), op, oloc, capi.ptr(res)))
+    return (out, res) if from2d else out
+
+
+def predict_mask_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w: int, h: int, ctx: Context | None = None,
+                       out_device_ptr: int | None = None) -> np.ndarray | None:
+    """read_depth + predict_mask per file, the decode on the GPU: uint8 [n,h,w] (None with out_device_ptr)."""
+    n = len(offsets) - 1
+    ctx = ctx or default_context()
+    out, op, oloc = _image_out(out_device_ptr, (n, int(h), int(w)), np.uint8)
+    offsets = np.ascontiguousarray(offsets, np.uint64)
+    capi.check(capi.load().dh_predict_mask_batch_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h), op, oloc))
     return out
 
 

@@ -73,6 +73,15 @@ void check_seq_off(const char* fn, const uint64_t* seq_off, uint32_t n_seq) {
     if (seq_off[n_seq] > 0x7fffffffull) throw dh::ModelError(DH_E_ARG, std::string(fn) + ": more than 2^31 - 1 frames");
 }
 
+// check_biwi_offsets with the entry point named in the message
+void check_offsets(const char* fn, const uint64_t* offsets, uint32_t n) {
+    try {
+        dh::check_biwi_offsets(offsets, n);
+    } catch (const dh::ModelError& e) {
+        throw dh::ModelError(e.code, std::string(fn) + ": " + e.what());
+    }
+}
+
 }  // namespace
 
 extern "C" {
@@ -462,6 +471,40 @@ int dh_build_hough_image_batch(dh_ctx* c, const dh_forest* f, const uint16_t* de
         REQUIRE(blur || !from2d, "dh_build_hough_image_batch: from2d needs blur = 1 (the arg-max of the blurred image)");
         REQUIRE(c && f && K && (n == 0 || depth), "dh_build_hough_image_batch: NULL argument");
         c->cx->hough_image_batch(*f->hf, depth, n, w, h, K, depth_loc, blur != 0, hough, hough_loc, from2d);
+    });
+}
+int dh_build_hough_image_frames(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                                int depth_loc, const float* K, int blur, uint16_t* hough, int hough_loc, dh_result* from2d) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_build_hough_image_frames: bad depth_loc");
+        REQUIRE(hough_loc == DH_DEPTH_HOST || hough_loc == DH_DEPTH_DEVICE, "dh_build_hough_image_frames: bad hough_loc");
+        REQUIRE(blur == 0 || blur == 1, "dh_build_hough_image_frames: blur must be 0 or 1");
+        REQUIRE(hough || from2d, "dh_build_hough_image_frames: hough and from2d are both NULL");
+        REQUIRE(blur || !from2d, "dh_build_hough_image_frames: from2d needs blur = 1 (the arg-max of the blurred image)");
+        REQUIRE(c && f && (n == 0 || (depth && K)), "dh_build_hough_image_frames: NULL argument");
+        c->cx->hough_image_frames(*f->hf, depth, nullptr, nullptr, n, w, h, depth_loc, K, blur != 0, hough, hough_loc, from2d);
+    });
+}
+int dh_build_hough_image_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                                     uint32_t w, uint32_t h, const float* K, int blur, uint16_t* hough, int hough_loc,
+                                     dh_result* from2d) {
+    return guarded([&] {
+        REQUIRE(hough_loc == DH_DEPTH_HOST || hough_loc == DH_DEPTH_DEVICE, "dh_build_hough_image_frames_biwi: bad hough_loc");
+        REQUIRE(blur == 0 || blur == 1, "dh_build_hough_image_frames_biwi: blur must be 0 or 1");
+        REQUIRE(hough || from2d, "dh_build_hough_image_frames_biwi: hough and from2d are both NULL");
+        REQUIRE(blur || !from2d, "dh_build_hough_image_frames_biwi: from2d needs blur = 1 (the arg-max of the blurred image)");
+        if (offsets) check_offsets("dh_build_hough_image_frames_biwi", offsets, n);
+        REQUIRE(c && f && (n == 0 || (blob && offsets && K)), "dh_build_hough_image_frames_biwi: NULL argument");
+        c->cx->hough_image_frames(*f->hf, nullptr, blob, offsets, n, w, h, DH_DEPTH_HOST, K, blur != 0, hough, hough_loc, from2d);
+    });
+}
+int dh_predict_mask_batch_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
+                               uint32_t h, uint8_t* mask, int mask_loc) {
+    return guarded([&] {
+        REQUIRE(mask_loc == DH_DEPTH_HOST || mask_loc == DH_DEPTH_DEVICE, "dh_predict_mask_batch_biwi: bad mask_loc");
+        if (offsets) check_offsets("dh_predict_mask_batch_biwi", offsets, n);
+        REQUIRE(c && f && (n == 0 || (blob && offsets && mask)), "dh_predict_mask_batch_biwi: NULL argument");
+        c->cx->predict_mask_batch_biwi(*f->hf, blob, offsets, n, w, h, mask, mask_loc);
     });
 }
 

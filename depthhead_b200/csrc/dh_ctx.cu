@@ -1045,7 +1045,7 @@ void Context::ensure_results(uint32_t n) {
     }
 }
 
-// pinned staging of the per-frame arguments of a dh_predict_frames batch (run_front packs it chunk by chunk)
+// pinned staging of the per-frame arguments of a batch (BackEnd::args; run_front packs it chunk by chunk)
 void Context::ensure_frame_args(uint32_t n) {
     if (h_frame_cap_ >= n) return;
     if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
@@ -1686,8 +1686,18 @@ void Context::predict_mask_batch(const HostForest& hf, const uint16_t* depth, ui
     run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, be);
 }
 
-void Context::hough_image_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
-                                int depth_loc, bool blur, uint16_t* votes, int votes_loc, dh_result* from2d) {
+void Context::predict_mask_batch_biwi(const HostForest& hf, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
+                                      uint32_t h, uint8_t* mask, int mask_loc) {
+    const float K[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+    BackEnd be;
+    be.kind = BackEnd::kMask;
+    be.image = mask;
+    be.image_on_device = mask_loc == DH_DEPTH_DEVICE;
+    run_batch(hf, nullptr, blob, offsets, n, w, h, K, DH_DEPTH_HOST, be);
+}
+
+namespace {
+BackEnd hough_back_end(bool blur, uint16_t* votes, int votes_loc, dh_result* from2d) {
     if (from2d && !blur) throw ModelError(DH_E_ARG, "predict_parameter_from2dhough takes the arg-max of the BLURRED vote image");
     if (!votes && !from2d) throw ModelError(DH_E_ARG, "neither a vote image nor from2d results are asked for");
     BackEnd be;
@@ -1695,7 +1705,27 @@ void Context::hough_image_batch(const HostForest& hf, const uint16_t* depth, uin
     be.results = from2d;
     be.image = votes;
     be.image_on_device = votes_loc == DH_DEPTH_DEVICE;
-    run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, be);
+    return be;
+}
+}  // namespace
+
+void Context::hough_image_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
+                                int depth_loc, bool blur, uint16_t* votes, int votes_loc, dh_result* from2d) {
+    run_batch(hf, depth, nullptr, nullptr, n, w, h, K, depth_loc, hough_back_end(blur, votes, votes_loc, from2d));
+}
+
+// dh_build_hough_image_frames / _biwi: every frame's K reaches the kernels that project through the
+// per-frame path of dh_predict_frames (arguments without seeds; run_front packs K and K^-1 per chunk
+// into Lane::frame_k).  Geometry holds frame 0's K, which the kFrameK kernels do not read.
+void Context::hough_image_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                                 uint32_t w, uint32_t h, int depth_loc, const float* K, bool blur, uint16_t* votes, int votes_loc,
+                                 dh_result* from2d) {
+    BackEnd be = hough_back_end(blur, votes, votes_loc, from2d);
+    std::vector<dh_frame_args> args(n);
+    for (uint32_t i = 0; i < n; ++i) std::memcpy(args[i].K, K + (size_t)9 * i, sizeof(float) * 9);
+    be.args = args.data();
+    static const float kIdentity[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+    run_batch(hf, depth, blob, offsets, n, w, h, n ? K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
 }
 
 // u32 sums + two u16 planes per frame of a chunk, and the arg-max keys, on every lane of the call
@@ -1752,6 +1782,7 @@ void Context::run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
     const Geometry& g = geom_;
     cudaStream_t st = L.stream;
     const size_t frame_px = (size_t)g.w * g.h, px = frame_px * n;
+    const float* frame_k = be.args ? L.frame_k : nullptr;  // masks project nothing
     uint16_t* plane0 = L.img16;
     uint16_t* plane1 = L.img16 + L.img_px;
     mark(DH_STAGE_VOTE);  // the whole 2-D back end is booked here
@@ -1769,7 +1800,7 @@ void Context::run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
     } else {
         DH_CUDA(cudaMemsetAsync(L.img32, 0, px * sizeof(uint32_t), st));
         if (g.P) {
-            launch_hough_votes(b, g, fdev_, n, L.img32, st);
+            launch_hough_votes(b, g, fdev_, n, L.img32, st, frame_k);
             launches_ += 1;
         }
         if (be.image) image = be.image_on_device ? static_cast<uint16_t*>(be.image) + (size_t)f0 * frame_px : plane1;
@@ -1781,7 +1812,7 @@ void Context::run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
             launches_ += (uint64_t)launch_gaussian_blur(L.img32, plane0, static_cast<uint16_t*>(image), be.results ? L.img_keys : nullptr,
                                                         g.w, g.h, n, d_blur_taps_, blur_radius_, st);
             if (be.results) {
-                launch_hough2d_pose(L.img_keys, b.depth, g, n, L.results, st);
+                launch_hough2d_pose(L.img_keys, b.depth, g, n, L.results, st, frame_k);
                 launches_ += 1;
             }
         }

@@ -32,7 +32,7 @@ struct Lane {
     float4* gated = nullptr;        // [F][P]
     uint32_t* grids = nullptr;      // [F][400 + 8000]
     FrameState* fs = nullptr;       // [F]
-    float* frame_k = nullptr;       // [F][18] K, K^-1 of every frame of a dh_predict_frames pass
+    float* frame_k = nullptr;       // [F][18] K, K^-1 of every frame of a pass with per-frame arguments (BackEnd::args)
     dh_result* results = nullptr;   // [F]
     int32_t* ms_trace = nullptr;    // [F][2][iters][3] (debug export)
     uint32_t* cubes = nullptr;      // [F][2][kBox^3]
@@ -60,8 +60,8 @@ void check_biwi_offsets(const uint64_t* offsets, uint32_t n);
 struct BackEnd {
     enum Kind { kPose, kMask, kVotes, kBlurred } kind = kPose;
     dh_result* results = nullptr;  // kPose: poses [n]; kBlurred: from2d poses [n] or nullptr (host memory)
-    const dh_frame_args* args = nullptr;  // kPose: intrinsics and seeds of every frame [n] (host memory), or nullptr:
-                                          // the call's one K and no seeds
+    const dh_frame_args* args = nullptr;  // intrinsics and seeds of every frame [n] (host memory), or nullptr: the call's
+                                          // one K and no seeds (kVotes / kBlurred: intrinsics only; kMask: unused)
     void* image = nullptr;         // kMask: u8 [n][h][w]; kVotes / kBlurred: u16 [n][h][w] (kBlurred: may be nullptr)
     bool image_on_device = false;  // image points to device memory on the context's GPU
 };
@@ -138,6 +138,12 @@ public:
                             uint8_t* mask, int mask_loc);
     void hough_image_batch(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
                            int depth_loc, bool blur, uint16_t* votes, int votes_loc, dh_result* from2d);
+    // the same with frame i's intrinsics at K[9 * i .. 9 * i + 9): depth at depth_loc, or Biwi files (blob != nullptr)
+    void hough_image_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                            uint32_t w, uint32_t h, int depth_loc, const float* K, bool blur, uint16_t* votes, int votes_loc,
+                            dh_result* from2d);
+    void predict_mask_batch_biwi(const HostForest& hf, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h,
+                                 uint8_t* mask, int mask_loc);
     void hough_image_raw(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9],
                          uint16_t* votes);
     void hough_image(const HostForest& hf, const uint16_t* depth, uint32_t w, uint32_t h, const float K[9], uint16_t* votes,

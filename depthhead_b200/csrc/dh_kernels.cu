@@ -1914,8 +1914,11 @@ __global__ void __launch_bounds__(256) mask_kernel(FrameBuffers b, Geometry g, c
 
 // build_hough_image before the blur (prediction.rs:760-841).  u16 wrap-around adds are done as
 // u32 atomics into the frame's accumulator and truncated by the reader (sum mod 2^16 is the same
-// either way).  One thread per (frame, tree, patch).
-__global__ void __launch_bounds__(256) hough_image_kernel(FrameBuffers b, Geometry g, ForestDev f, uint32_t* __restrict__ acc) {
+// either way).  One thread per (frame, tree, patch).  kFrameK: the frame's K and K^-1 come from
+// frame_k, loaded into registers by the threads that pass the leaf tests (most return before).
+template <bool kFrameK>
+__global__ void __launch_bounds__(256) hough_image_kernel(FrameBuffers b, Geometry g, ForestDev f, uint32_t* __restrict__ acc,
+                                                         const float* __restrict__ frame_k) {
     const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x, frame = blockIdx.y;
     const uint32_t T = g.n_trees;
     if (idx >= g.P * T) return;
@@ -1932,15 +1935,19 @@ __global__ void __launch_bounds__(256) hough_image_kernel(FrameBuffers b, Geomet
     const uint32_t x = g.left_w + gx * g.stride, y = g.left_h + gy * g.stride;
     const size_t frame_px = (size_t)g.w * g.h;
     acc += (size_t)frame * frame_px;
-    float p3[3];
-    img_to_space(g.Kinv, (float)x, (float)y, (float)b.depth[(size_t)frame * frame_px + (size_t)y * g.w + x], p3);
+    float p3[3], fk[9], fkinv[9];
+    if (kFrameK) {
+        load_mat3(frame_k + (size_t)frame * kFrameKFloats, fk);
+        load_mat3(frame_k + (size_t)frame * kFrameKFloats + 9, fkinv);
+    }
+    img_to_space(kFrameK ? fkinv : g.Kinv, (float)x, (float)y, (float)b.depth[(size_t)frame * frame_px + (size_t)y * g.w + x], p3);
     for (uint32_t k = 0; k < n; ++k) {
         float np[3], p2[2];
         const float4 o = f.offsets[v0 + k];
         np[0] = __fsub_rn(p3[0], o.x);
         np[1] = __fsub_rn(p3[1], o.y);
         np[2] = __fsub_rn(p3[2], o.z);
-        space_to_img(g.K, np, p2);
+        space_to_img(kFrameK ? fk : g.K, np, p2);
         const int nx = __float2int_rz(p2[0]), ny = __float2int_rz(p2[1]);  // :816
         if (nx < 0 || (uint32_t)nx >= g.w || ny < 0 || (uint32_t)ny >= g.h) continue;
         atomicAdd(&acc[(size_t)ny * g.w + nx], valtoadd);
@@ -2039,14 +2046,17 @@ __global__ void __launch_bounds__(kBlurVx * kBlurVy) blur_v_kernel(const uint16_
 }
 // predict_parameter_from2dhough (prediction.rs:343-367) from the frames' arg-max keys: z = the
 // depth at that pixel and the back-projection of (x, y, z); rotation 0, bounding box 0.  One thread per frame.
+// kFrameK: the back-projection uses the frame's K^-1 from frame_k.
+template <bool kFrameK>
 __global__ void hough2d_pose_kernel(const unsigned long long* __restrict__ keys, const uint16_t* __restrict__ depth, Geometry g,
-                                    uint32_t n_frames, dh_result* __restrict__ out) {
+                                    uint32_t n_frames, dh_result* __restrict__ out, const float* __restrict__ frame_k) {
     const uint32_t frame = blockIdx.x * blockDim.x + threadIdx.x;
     if (frame >= n_frames) return;
     const uint32_t w = g.w, bi = (uint32_t)(keys[frame] & 0xffffffffull);
     const uint32_t x = bi % w, y = bi / w;
-    float p[3];
-    img_to_space(g.Kinv, (float)x, (float)y, (float)depth[(size_t)frame * w * g.h + (size_t)y * w + x], p);
+    float p[3], kinv[9];
+    if (kFrameK) load_mat3(frame_k + (size_t)frame * kFrameKFloats + 9, kinv);
+    img_to_space(kFrameK ? kinv : g.Kinv, (float)x, (float)y, (float)depth[(size_t)frame * w * g.h + (size_t)y * w + x], p);
     dh_result& r = out[frame];
     r.mid_point[0] = p[0]; r.mid_point[1] = p[1]; r.mid_point[2] = p[2];
     r._pad = 0;
@@ -2577,9 +2587,12 @@ void launch_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, u
     mask_kernel<<<dim3((g.P + 255) / 256, n_frames), 256, 0, s>>>(b, g, f.leaf_prob, mask);
 }
 
-void launch_hough_votes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t* acc32, cudaStream_t s) {
+void launch_hough_votes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t* acc32, cudaStream_t s,
+                        const float* frame_k) {
     const uint32_t n = g.P * g.n_trees;
-    hough_image_kernel<<<dim3((n + 255) / 256, n_frames), 256, 0, s>>>(b, g, f, acc32);
+    const dim3 grid((n + 255) / 256, n_frames);
+    if (frame_k) hough_image_kernel<true><<<grid, 256, 0, s>>>(b, g, f, acc32, frame_k);
+    else hough_image_kernel<false><<<grid, 256, 0, s>>>(b, g, f, acc32, nullptr);
 }
 
 void launch_narrow_u16(const uint32_t* acc32, uint16_t* out16, size_t n, cudaStream_t s) {
@@ -2599,8 +2612,9 @@ int launch_gaussian_blur(const uint32_t* in, uint16_t* tmp, uint16_t* out, unsig
     return 2;
 }
 void launch_hough2d_pose(const unsigned long long* keys, const uint16_t* depth, const Geometry& g, uint32_t n_frames, dh_result* out,
-                         cudaStream_t s) {
-    hough2d_pose_kernel<<<(n_frames + 127) / 128, 128, 0, s>>>(keys, depth, g, n_frames, out);
+                         cudaStream_t s, const float* frame_k) {
+    if (frame_k) hough2d_pose_kernel<true><<<(n_frames + 127) / 128, 128, 0, s>>>(keys, depth, g, n_frames, out, frame_k);
+    else hough2d_pose_kernel<false><<<(n_frames + 127) / 128, 128, 0, s>>>(keys, depth, g, n_frames, out, nullptr);
 }
 
 void launch_seq_guess(FrameState* fs, const dh_result* prev, uint32_t n, float min_seed_z, cudaStream_t s) {

@@ -24,8 +24,11 @@
  *   src/hough/prediction.rs:343-367   predict_parameter_from2dhough            -> dh_predict_from2dhough
  *   the three above over n frames                                              -> dh_predict_mask_batch,
  *                                                                                 dh_build_hough_image_batch
+ *   the last three over n frames, each with its own K (examples/db_prediction.rs) -> dh_build_hough_image_frames
  *   src/db_reader/biwi.rs:81-103      read_depth (run-length coded depth file)  -> dh_biwi_depth_dims,
- *                                                                                 dh_biwi_decode_depth, dh_predict_batch_biwi
+ *                                                                                 dh_biwi_decode_depth, dh_predict_batch_biwi,
+ *                                                                                 dh_predict_mask_batch_biwi,
+ *                                                                                 dh_build_hough_image_frames_biwi
  *   src/db_reader/biwi.rs:27-60       read_cal (depth.cal -> IntrinsicMatrix)   -> dh_biwi_parse_cal
  *   src/db_reader/biwi.rs:63-77       read_gt (ground-truth pose file)          -> dh_biwi_parse_pose
  *   src/hough/houghforest.rs:250-295  HoughTreeFunctions::impurity (training)   -> dh_train_score_level
@@ -206,6 +209,15 @@ int dh_predict_mask_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, 
  * per frame.  from2d needs blur = 1; hough and from2d both NULL is DH_E_ARG. */
 int dh_build_hough_image_batch(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
                                const float K[9], int depth_loc, int blur, uint16_t* hough, int hough_loc, dh_result* from2d);
+/* dh_build_hough_image_batch with frame i's intrinsics at K[9*i .. 9*i+9) (row-major, host memory):
+ * frames of several cameras, e.g. the sequence folders of a database, each with its own depth.cal,
+ * in one call.  Equal, bit for bit, to dh_hough_image_raw / dh_build_hough_image /
+ * dh_predict_from2dhough frame by frame with that frame's K.  K is not validated, as in
+ * dh_build_hough_image.  Argument rules as dh_build_hough_image_batch; NULL K with n > 0 is
+ * DH_E_ARG.  Synchronous; n = 0 is a successful no-op. */
+int dh_build_hough_image_frames(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                                int depth_loc, const float* K /*[n][9]*/, int blur, uint16_t* hough, int hough_loc,
+                                dh_result* from2d);
 
 /* ------------------------------------------------------------------ Biwi Kinect Head Pose wire formats */
 /* read_depth (biwi.rs:81-103): u32 width, u32 height, then until width*height pixels are covered
@@ -230,6 +242,13 @@ int dh_predict_batch_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, co
  * folders each have their own depth.cal, in one call. */
 int dh_predict_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
                            uint32_t w, uint32_t h, const dh_frame_args* args, dh_result* out);
+/* read_depth + dh_build_hough_image_frames (a K per file; a caller with one K repeats it), and
+ * read_depth + dh_predict_mask_batch.  The offsets are checked before any device work. */
+int dh_build_hough_image_frames_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                                     uint32_t w, uint32_t h, const float* K /*[n][9]*/, int blur, uint16_t* hough,
+                                     int hough_loc, dh_result* from2d);
+int dh_predict_mask_batch_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                               uint32_t w, uint32_t h, uint8_t* mask, int mask_loc);
 
 /* Tracks: the seeding of dh_predict_sequences over sequences of any length, each from its own camera
  * and with an optional starting pose (multi-camera rigs, a detector that starts tracks, the Biwi

@@ -96,6 +96,8 @@ extern "C" {
                              depth_loc: c_int, mask: *mut u8, mask_loc: c_int) -> c_int;
     fn dh_build_hough_image_batch(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32, k: *const f32,
                                   depth_loc: c_int, blur: c_int, hough: *mut u16, hough_loc: c_int, from2d: *mut DhResult) -> c_int;
+    fn dh_build_hough_image_frames(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32, depth_loc: c_int,
+                                   k: *const f32, blur: c_int, hough: *mut u16, hough_loc: c_int, from2d: *mut DhResult) -> c_int;
     // Biwi wire formats (src/db_reader/biwi.rs:27-103)
     fn dh_biwi_depth_dims(file: *const u8, len: usize, w: *mut u32, h: *mut u32) -> c_int;
     fn dh_biwi_decode_depth(c: *mut DhCtx, blob: *const u8, offsets: *const u64, n: u32, w: u32, h: u32,
@@ -104,6 +106,11 @@ extern "C" {
                              w: u32, h: u32, k: *const f32, out: *mut DhResult) -> c_int;
     fn dh_predict_frames_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32,
                               w: u32, h: u32, args: *const DhFrameArgs, out: *mut DhResult) -> c_int;
+    fn dh_build_hough_image_frames_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32,
+                                        w: u32, h: u32, k: *const f32, blur: c_int, hough: *mut u16, hough_loc: c_int,
+                                        from2d: *mut DhResult) -> c_int;
+    fn dh_predict_mask_batch_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32,
+                                  w: u32, h: u32, mask: *mut u8, mask_loc: c_int) -> c_int;
     fn dh_predict_tracks(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n_seq: u32, seq_off: *const u64, w: u32, h: u32,
                          depth_loc: c_int, seq_args: *const DhFrameArgs, min_seed_z: f32, out: *mut DhResult) -> c_int;
     fn dh_predict_tracks_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n_seq: u32,
@@ -333,6 +340,30 @@ impl HoughPrediction {
                                                   1, std::ptr::null_mut(), 0, out.as_mut_ptr()) })?;
         Ok(out)
     }
+    /// build_hough_image_batch with intrinsics[i] for frame i (frames of several cameras, e.g. a
+    /// database's sequence folders, in one call); equal to build_hough_image frame by frame
+    pub fn build_hough_image_frames(&self, frames: &[u16], n: u32, w: u32, h: u32, intrinsics: &[IntrinsicMatrix], blur: bool)
+                                    -> Result<Vec<u16>, Error> {
+        let px = (n as usize) * (w as usize) * (h as usize);
+        assert_eq!(frames.len(), px);
+        let k = matrices(n, intrinsics);
+        self.push_fields()?;
+        let mut out = vec![0u16; px];
+        check(unsafe { dh_build_hough_image_frames(self.context(), self.forest, frames.as_ptr(), n, w, h, 0 /* DH_DEPTH_HOST */,
+                                                   k.as_ptr(), blur as c_int, out.as_mut_ptr(), 0, std::ptr::null_mut()) })?;
+        Ok(out)
+    }
+    /// predict_parameter_from2dhough_batch with intrinsics[i] for frame i
+    pub fn predict_parameter_from2dhough_frames(&self, frames: &[u16], n: u32, w: u32, h: u32, intrinsics: &[IntrinsicMatrix])
+                                                -> Result<Vec<DhResult>, Error> {
+        assert_eq!(frames.len(), (n as usize) * (w as usize) * (h as usize));
+        let k = matrices(n, intrinsics);
+        self.push_fields()?;
+        let mut out = vec![DhResult::default(); n as usize];
+        check(unsafe { dh_build_hough_image_frames(self.context(), self.forest, frames.as_ptr(), n, w, h, 0 /* DH_DEPTH_HOST */,
+                                                   k.as_ptr(), 1, std::ptr::null_mut(), 0, out.as_mut_ptr()) })?;
+        Ok(out)
+    }
     /// n_seq independent sequences of frames_per_seq frames each (sequence-major): frame t of every
     /// sequence is seeded with the pose of frame t - 1 exactly as examples/live_prediction.rs:75-88
     /// does (a centre seed only if its z exceeds min_seed_z, 500.0 there)
@@ -409,6 +440,12 @@ fn frame_args(n: u32, intrinsics: &[IntrinsicMatrix], midp_guess: &[Option<[f32;
         if let Some(r) = rot_guess[i] { a.rot_guess = r; a.has_guess |= 2; }
         a
     }).collect()
+}
+
+/// n row-major matrices back to back, [n][9]
+fn matrices(n: u32, intrinsics: &[IntrinsicMatrix]) -> Vec<f32> {
+    assert_eq!(intrinsics.len(), n as usize, "one matrix per frame");
+    intrinsics.iter().flat_map(|k| k.0.iter().flatten().copied()).collect()
 }
 
 /// `#[derive(Deserialize)]` of the reference (prediction.rs:238): any serde deserializer works; the
@@ -495,6 +532,38 @@ pub mod biwi {
             let mut out = vec![DhResult::default(); n as usize];
             check(unsafe { dh_predict_frames_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
                                                   files.width, files.height, args.as_ptr(), out.as_mut_ptr()) })?;
+            Ok(out)
+        }
+        /// read_depth + build_hough_image (blur = false: the vote images before the blur) per file, file i
+        /// with intrinsics[i] (examples/db_prediction.rs over a database whose folders each have a depth.cal)
+        pub fn build_hough_image_files(&self, files: &PackedFiles, intrinsics: &[IntrinsicMatrix], blur: bool) -> Result<Vec<u16>, Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            let k = matrices(n, intrinsics);
+            self.push_fields()?;
+            let mut out = vec![0u16; n as usize * files.width as usize * files.height as usize];
+            check(unsafe { dh_build_hough_image_frames_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
+                                                            files.width, files.height, k.as_ptr(), blur as c_int, out.as_mut_ptr(), 0,
+                                                            std::ptr::null_mut()) })?;
+            Ok(out)
+        }
+        /// read_depth + predict_parameter_from2dhough per file, file i with intrinsics[i]
+        pub fn predict_from2dhough_files(&self, files: &PackedFiles, intrinsics: &[IntrinsicMatrix]) -> Result<Vec<DhResult>, Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            let k = matrices(n, intrinsics);
+            self.push_fields()?;
+            let mut out = vec![DhResult::default(); n as usize];
+            check(unsafe { dh_build_hough_image_frames_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
+                                                            files.width, files.height, k.as_ptr(), 1, std::ptr::null_mut(), 0,
+                                                            out.as_mut_ptr()) })?;
+            Ok(out)
+        }
+        /// read_depth + predict_mask per file: masks [n][h][w] in file order
+        pub fn predict_mask_files(&self, files: &PackedFiles) -> Result<Vec<u8>, Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            self.push_fields()?;
+            let mut out = vec![0u8; n as usize * files.width as usize * files.height as usize];
+            check(unsafe { dh_predict_mask_batch_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
+                                                      files.width, files.height, out.as_mut_ptr(), 0 /* DH_DEPTH_HOST */) })?;
             Ok(out)
         }
         /// predict_tracks over the files: track s is the next lengths[s] files (a sequence folder, in time
