@@ -218,8 +218,12 @@ TrainSet* Context::trainset_create(const uint16_t* patches, uint64_t n, uint32_t
                                    const uint8_t* is_object, const float* offsets, const double* rotations) {
     DH_CUDA_T(cudaSetDevice(device_));
     if (n == 0 || n > 0x7fffffffull) throw ModelError(DH_E_ARG, "training set must hold 1 .. 2^31-1 samples");
-    if (!box_image_supported(sw, sh, sw, sh, rw, rh) || (uint64_t)rw * rh > 16383u)
-        throw ModelError(DH_E_SHAPE, "feature rectangle size not supported by the box-sum tables (see DESIGN.md)");
+    // What box_image_kernel needs of a training table: sides of 1..128 inside the sub-image and
+    // rw * rh <= 16383.  The prediction path's further limit on how many rectangles cover a patch
+    // (box_image_supported) belongs to its background test, which training does not run.
+    if (!rw || !rh || rw > sw || rh > sh || rw > 128u || rh > 128u || (uint64_t)rw * rh > 16383u)
+        throw ModelError(DH_E_SHAPE, "feature rectangle size not supported by the box-sum tables: sides of 1 .. 128 inside the "
+                                     "sub-image, rw * rh <= 16383 (see DESIGN.md)");
     std::unique_ptr<TrainSet> ts(new TrainSet());
     ts->device = device_;
     ts->n = n; ts->sw = sw; ts->sh = sh; ts->rw = rw; ts->rh = rh;
@@ -261,7 +265,7 @@ void Context::train_score_level(const TrainSet& ts, const uint32_t* sample_idx, 
     if (n_nodes == 0 || m == 0) return;
     const uint64_t total = node_off[n_nodes];
     for (uint32_t k = 0; k < n_nodes; ++k)
-        if (node_off[k + 1] < node_off[k]) throw ModelError(DH_E_ARG, "node_off is not monotone");
+        if (node_off[k + 1] < node_off[k]) throw ModelError(DH_E_ARG, "dh_train_score_level: node_off is not monotone");
     for (uint64_t s = 0; s < total; ++s)
         if (sample_idx[s] >= ts.n) throw ModelError(DH_E_ARG, "sample index out of range");
     std::vector<dev::Cand> cands;
@@ -273,10 +277,17 @@ void Context::train_score_level(const TrainSet& ts, const uint32_t* sample_idx, 
     DH_CUDA_T(cudaMemcpyAsync(d_idx.p, sample_idx, total * sizeof(uint32_t), cudaMemcpyHostToDevice, stream_));
     DH_CUDA_T(cudaMemcpyAsync(d_off.p, node_off, (n_nodes + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, stream_));
     DH_CUDA_T(cudaMemcpyAsync(d_c.p, cands.data(), cands.size() * sizeof(dev::Cand), cudaMemcpyHostToDevice, stream_));
-    dim3 gr((m + 127) / 128, n_nodes);
-    dev::train_score_kernel<<<gr, 128, 0, stream_>>>(ts.box, ts.bh * ts.bpitch, ts.is_obj, ts.off, ts.rot, d_idx.p, d_off.p, d_c.p, m,
-                                                     (double)((uint64_t)ts.rw * ts.rh), d_out.p);
-    DH_CUDA_T(cudaGetLastError());
+    // the node is blockIdx.y, at most 65535 per launch: wider levels go in slices of nodes (node_off
+    // holds offsets into the whole sample_idx, so a slice only moves the node_off, cands and out bases)
+    constexpr uint32_t kMaxNodesPerLaunch = 65535u;
+    for (uint32_t k0 = 0; k0 < n_nodes; k0 += kMaxNodesPerLaunch) {
+        const uint32_t nk = std::min(kMaxNodesPerLaunch, n_nodes - k0);
+        dim3 gr((m + 127) / 128, nk);
+        dev::train_score_kernel<<<gr, 128, 0, stream_>>>(ts.box, ts.bh * ts.bpitch, ts.is_obj, ts.off, ts.rot, d_idx.p, d_off.p + k0,
+                                                         d_c.p + (size_t)k0 * m, m, (double)((uint64_t)ts.rw * ts.rh),
+                                                         d_out.p + (size_t)k0 * m);
+        DH_CUDA_T(cudaGetLastError());
+    }
     DH_CUDA_T(cudaMemcpyAsync(out, d_out.p, cands.size() * sizeof(dh_split_stats), cudaMemcpyDeviceToHost, stream_));
     DH_CUDA_T(cudaStreamSynchronize(stream_));
     for (size_t i = 0; i < cands.size(); ++i) {
@@ -292,6 +303,8 @@ void Context::train_split_level(const TrainSet& ts, const uint32_t* sample_idx, 
     if (ts.device != device_) throw ModelError(DH_E_ARG, "the training set lives on another GPU than this context");
     if (n_nodes == 0) return;
     const uint64_t total = node_off[n_nodes];
+    for (uint32_t k = 0; k < n_nodes; ++k)
+        if (node_off[k + 1] < node_off[k]) throw ModelError(DH_E_ARG, "dh_train_split_level: node_off is not monotone");
     if (total == 0) return;
     for (uint64_t s = 0; s < total; ++s)
         if (sample_idx[s] >= ts.n) throw ModelError(DH_E_ARG, "sample index out of range");

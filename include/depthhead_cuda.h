@@ -297,7 +297,8 @@ typedef struct dh_trainset dh_trainset;  /* training samples resident on one GPU
 /* n samples: patches[n][sh][sw] u16 (the cropped sub-images of prediction.rs:223-226),
  * is_object[n] (Truth::Object or NoObject), offsets[n][3] f32 mm and rotations[n][3] f64 of the
  * Object samples (ignored for the others).  rw x rh: the one rectangle size every candidate
- * feature will have (subrect_feature_scale of hough_tree_trainer.rs:165 applied to the sub-image). */
+ * feature will have (subrect_feature_scale of hough_tree_trainer.rs:165 applied to the sub-image):
+ * sides of 1 .. 128 inside the sub-image and rw * rh <= 16383, else DH_E_SHAPE. */
 int dh_trainset_create(dh_ctx* c, const uint16_t* patches, uint64_t n, uint32_t sw, uint32_t sh, uint32_t rw, uint32_t rh,
                        const uint8_t* is_object, const float* offsets, const double* rotations, dh_trainset** out);
 void dh_trainset_free(dh_trainset* t);
@@ -312,7 +313,9 @@ typedef struct dh_split_stats {
 } dh_split_stats;
 /* One tree level: node k owns sample_idx[node_off[k] .. node_off[k+1]) (indices into the training
  * set, in set order); cand_rects[n_nodes][m][8] (r1 x0,y0,x1,y1, r2 ..; bottomright exclusive) and
- * cand_thr[n_nodes][m] are its m candidates; out[n_nodes][m]. */
+ * cand_thr[n_nodes][m] are its m candidates; out[n_nodes][m].  Any number of nodes per level, empty
+ * nodes included; a decreasing node_off or a rectangle of another size or outside the sub-image is
+ * DH_E_ARG, here and in dh_train_split_level. */
 int dh_train_score_level(dh_ctx* c, const dh_trainset* t, const uint32_t* sample_idx, const uint64_t* node_off, uint32_t n_nodes,
                          const int32_t* cand_rects, const double* cand_thr, uint32_t m, uint64_t depth, double steepness,
                          dh_split_stats* out);

@@ -458,3 +458,77 @@ def train_early_stop(is_object, idx, depth: int, max_depth: int, min_subset_size
     o = np.ascontiguousarray(is_object, np.uint8)
     i = np.ascontiguousarray(idx, np.uint32)
     return bool(lib().orc_train_early_stop(_p(o), _p(i), len(i), int(depth), int(max_depth), int(min_subset_size)))
+
+
+def train_feature(patch: np.ndarray, rects8) -> float:
+    """avg1 - avg2 of binarize (houghforest.rs:185-193) on one patch [sh, sw]: the value a threshold
+    ties with."""
+    p = np.ascontiguousarray(patch, np.uint16)
+    sh, sw = p.shape
+    sub = np.array([0, 0, sw, sh], np.uint32)
+    r = np.asarray(rects8, np.int64).reshape(8)
+    a = [lib().orc_rect_average(_p(p), sw, sh, _p(sub), _p(np.ascontiguousarray(r[k:k + 4], np.uint32)), MODE_NAIVE) for k in (0, 4)]
+    return a[0] - a[1]
+
+
+# the layout of dh_split_stats (include/depthhead_cuda.h), restated so that the oracle does not import the product
+TRAIN_STATS_DTYPE = np.dtype([("n", np.uint32, 2), ("n_pos", np.uint32, 2), ("det_off", np.float64, 2), ("det_rot", np.float64, 2),
+                              ("impurity", np.float64)], align=True)
+
+
+class OracleTrainSet:
+    """A training set scored on the CPU, with the attributes `depthhead_b200.train.HoughLearning.train_tree`
+    uses (`n`, `is_object`, `offsets`, `rotations`, `score_level`, `split_level`): every candidate is
+    scored with `train_binarize` and `train_impurity`, and its impurity is NaN where a side is empty
+    or the reference hits unreachable!() — the candidates the trainer skips (DESIGN.md §9).  So
+    `HoughLearning(...).train_forest(OracleTrainSet(...), CounterRng(seed))` grows a forest without
+    the GPU, with the same driver and random stream as the product.
+
+    After each `score_level`, `last_bad` [n_nodes, m] flags the unreachable!() candidates and
+    `last_value` holds the impurity the reference computes before its checks."""
+
+    def __init__(self, patches, is_object, offsets, rotations):
+        self.patches = np.ascontiguousarray(patches, np.uint16)
+        if self.patches.ndim != 3:
+            raise ValueError("patches must be [n, sub_h, sub_w] uint16")
+        self.n = len(self.patches)
+        self.is_object = np.ascontiguousarray(is_object, np.uint8).reshape(self.n)
+        self.offsets = np.ascontiguousarray(offsets, np.float32).reshape(self.n, 3)
+        self.rotations = np.ascontiguousarray(rotations, np.float64).reshape(self.n, 3)
+        self.last_bad = self.last_value = None
+
+    def close(self):
+        pass
+
+    def score_level(self, sample_idx, node_off, cand_rects, cand_thr, depth: int, steepness: float) -> np.ndarray:
+        idx = np.asarray(sample_idx, np.uint32)
+        off = np.asarray(node_off, np.int64)
+        k = len(off) - 1
+        thr = np.asarray(cand_thr, np.float64).reshape(k, -1)
+        m = thr.shape[1]
+        rects = np.asarray(cand_rects, np.int32).reshape(k, m, 8)
+        out = np.zeros((k, m), TRAIN_STATS_DTYPE)
+        self.last_bad = np.zeros((k, m), bool)
+        self.last_value = np.zeros((k, m), np.float64)
+        for a in range(k):
+            s = idx[off[a]:off[a + 1]]
+            for j in range(m):
+                bits = train_binarize(self.patches, s, rects[a, j], thr[a, j])
+                left, right = s[bits == 0], s[bits != 0]
+                v, st, bad = train_impurity(self.is_object, self.offsets, self.rotations, left, right, depth, steepness)
+                o = out[a, j]
+                o["n"], o["n_pos"] = st["n"], st["n_pos"]
+                o["det_off"], o["det_rot"] = st["det_off"], st["det_rot"]
+                o["impurity"] = np.nan if (len(left) == 0 or len(right) == 0 or bad) else v
+                self.last_bad[a, j], self.last_value[a, j] = bad, v
+        return out
+
+    def split_level(self, sample_idx, node_off, rects, thr) -> np.ndarray:
+        idx = np.asarray(sample_idx, np.uint32)
+        off = np.asarray(node_off, np.int64)
+        r = np.asarray(rects, np.int32).reshape(-1, 8)
+        t = np.asarray(thr, np.float64).reshape(-1)
+        bits = np.zeros(int(off[-1]), np.uint8)
+        for a in range(len(off) - 1):
+            bits[off[a]:off[a + 1]] = train_binarize(self.patches, idx[off[a]:off[a + 1]], r[a], t[a])
+        return bits

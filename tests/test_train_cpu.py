@@ -113,3 +113,94 @@ def test_extract_samples_against_oracle_backprojection():
         assert np.array_equal((p3 - centres[0]).view(np.uint32), offs[i].view(np.uint32))
         assert masks[0][y, x] != 0
     assert np.array_equal(rr[0], rots[0].astype(np.float64))
+
+
+def _avg(patch, x0, y0, x1, y1):
+    # average_value_in_rect (types.rs:317-339): integer sum, then sum as f64 / count as f64
+    return float(int(patch[y0:y1, x0:x1].astype(np.int64).sum())) / float((x1 - x0) * (y1 - y0))
+
+
+def _cov_det(pts):
+    # estimate_mean_cov (meancov_estimation.rs:359-378) and Mat3::det (:339-343) in plain Python floats
+    m = [0.0, 0.0, 0.0]
+    for p in pts:
+        m = [m[k] + float(p[k]) for k in range(3)]
+    m = [v / len(pts) for v in m]
+    c = [[0.0] * 3 for _ in range(3)]
+    for p in pts:
+        d = [float(p[k]) - m[k] for k in range(3)]
+        c = [[c[a][b] + d[a] * d[b] for b in range(3)] for a in range(3)]
+    c = [[v / (len(pts) - 1) for v in row] for row in c]
+    return (c[0][0] * (c[1][1] * c[2][2] - c[1][2] * c[2][1]) - c[1][0] * (c[0][1] * c[2][2] - c[0][2] * c[2][1])
+            + c[2][0] * (c[0][1] * c[1][2] - c[0][2] * c[1][1]))
+
+
+def _impurity_by_hand(is_obj, off, rot, left, right, depth, steepness):
+    def entropy(side):
+        p = sum(int(is_obj[i]) for i in side) / len(side)
+        return p * _ln(p) + (1 - p) * _ln(1 - p)
+
+    def reglog(side):
+        pos = [i for i in side if is_obj[i]]
+        if len(pos) < 2:   # none, or one: 0/0 covariance, NaN determinant, neither match arm
+            return 0.0
+        x = _cov_det(off[pos]) + _cov_det(rot[pos])
+        return math.log(x) if x > 0 else 0.0
+    n = len(left) + len(right)
+    lf, rf = len(left) / n, len(right) / n
+    return -(lf * entropy(left) + rf * entropy(right)) + (1 - math.exp(-(depth / steepness))) * (lf * reglog(left) + rf * reglog(right))
+
+
+def test_oracle_trainer_grows_a_tree_by_hand():
+    """HoughLearning.train_forest on oracle.OracleTrainSet: the root's candidates scored by hand, the
+    root takes the smallest of them, and the grown tree partitions its samples as the driver states
+    (DESIGN.md section 9): children[bit] gets binarize == bit, in set order; leaf prob = objects / samples."""
+    rng = np.random.default_rng(17)
+    n = 40
+    patches = rng.integers(0, 2000, (n, 12, 10)).astype(np.uint16)
+    patches[: n // 2, :6, :] += 1500                       # something for the features to find
+    is_obj = (np.arange(n) < n // 2).astype(np.uint8)
+    rng.shuffle(is_obj)
+    off = rng.normal(0.0, 40.0, (n, 3)).astype(np.float32)
+    rot = rng.normal(0.0, 20.0, (n, 3))
+    hl = train.HoughLearning(1, 10, 12, 4, 1, 32, 0.5, 12, 4, 5.0)
+    ts = oracle.OracleTrainSet(patches, is_obj, off, rot)
+    arr = hl.train_forest(ts, train.CounterRng(9))
+    # the driver's first draws: the subset, then the root's candidates
+    r = train.CounterRng(9)
+    subset = r.permutation(n)[:32]
+    rects, thr = hl.param_set(r, 12)
+    assert np.all(rects[:, 2] - rects[:, 0] == 5) and np.all(rects[:, 3] - rects[:, 1] == 6)
+    hand = []
+    for j in range(12):
+        bits = np.array([_avg(patches[i], *rects[j, :4]) - _avg(patches[i], *rects[j, 4:]) > thr[j] for i in subset])
+        assert np.array_equal(bits.astype(np.uint8), oracle.train_binarize(patches, subset, rects[j], thr[j]))
+        left, right = subset[~bits], subset[bits]
+        hand.append(np.nan if len(left) == 0 or len(right) == 0 else _impurity_by_hand(is_obj, off, rot, left, right, 0, 5.0))
+    st = ts.score_level(subset, [0, 32], rects[None], thr[None], 0, 5.0)[0]
+    assert np.array_equal(np.isnan(st["impurity"]), np.isnan(hand)) and np.count_nonzero(~np.isnan(hand)) >= 6
+    ok = ~np.isnan(hand)
+    assert np.allclose(st["impurity"][ok], np.asarray(hand)[ok], rtol=1e-12, atol=1e-12)
+    best = int(np.flatnonzero(ok)[np.argmin(np.asarray(hand)[ok])])
+    assert arr["tree_node_off"][1] > 0, "the root did not split"
+    assert np.array_equal(arr["rects"][0], rects[best]) and arr["threshold"][0] == thr[best]
+    # route the subset down the tree: every leaf holds the objects that reach it, in set order
+    reach = {}
+
+    def walk(node, idx):
+        if node < 0:
+            reach[~node] = idx
+            return
+        rr, t = arr["rects"][node], arr["threshold"][node]
+        b = np.array([_avg(patches[i], *rr[:4]) - _avg(patches[i], *rr[4:]) > t for i in idx], bool)
+        kids = arr["child"][node]
+        walk(int(kids[0]), idx[~b])
+        walk(int(kids[1]), idx[b])
+    walk(0, subset)
+    assert sorted(reach) == list(range(len(arr["prob"])))
+    assert sum(len(v) for v in reach.values()) == 32
+    for leaf, idx in reach.items():
+        pos = idx[is_obj[idx] != 0]
+        assert arr["prob"][leaf] == len(pos) / len(idx)
+        v0, v1 = arr["vote_off"][leaf], arr["vote_off"][leaf + 1]
+        assert np.array_equal(arr["offsets"][v0:v1], off[pos]) and np.array_equal(arr["rotations"][v0:v1], rot[pos])
