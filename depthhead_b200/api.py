@@ -440,6 +440,39 @@ class HoughPrediction:
                                                  float(min_seed_z), capi.ptr(out)))
         return out
 
+    # ---- pose and head mask of the same frames from one traversal (examples/live_prediction.rs asks both of
+    # every frame).  Masks: returned as a host uint8 array, or written to the caller's device memory at
+    # mask_device_ptr (nothing returned on the host).
+    def predict_frames_with_mask(self, frames, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                                 ctx: Context | None = None, device_ptr: int | None = None, n: int | None = None,
+                                 w: int | None = None, h: int | None = None, mask_device_ptr: int | None = None):
+        """predict_frames and predict_mask_batch of the same frames in one pass: (capi.RESULT_DTYPE[n], uint8
+        [n,h,w] or None), each equal to what its own call returns."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        args = frame_args(n, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+        ctx = ctx or default_context()
+        out = np.zeros(n, capi.RESULT_DTYPE)
+        masks, mp, mloc = _image_out(mask_device_ptr, (n, h, w), np.uint8)
+        capi.check(capi.load().dh_predict_frames_mask(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(out), mp, mloc))
+        return out, masks
+
+    def predict_tracks_with_mask(self, frames, lengths, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                                 min_seed_z: float = 500.0, ctx: Context | None = None, device_ptr: int | None = None,
+                                 w: int | None = None, h: int | None = None, mask_device_ptr: int | None = None):
+        """predict_tracks and the head mask of every frame in one pass: (capi.RESULT_DTYPE[total], uint8
+        [total,h,w] or None), both in input order."""
+        seq_off, n_seq, total = _track_offsets(lengths)
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, total, w, h)
+        if n != total:
+            raise ValueError("sum(lengths) = %d but there are %d frames" % (total, n))
+        args = frame_args(n_seq, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+        ctx = ctx or default_context()
+        out = np.zeros(total, capi.RESULT_DTYPE)
+        masks, mp, mloc = _image_out(mask_device_ptr, (total, h, w), np.uint8)
+        capi.check(capi.load().dh_predict_tracks_mask(ctx._h, self._h, p, n_seq, capi.ptr(seq_off), w, h, loc, capi.ptr(args),
+                                                      float(min_seed_z), capi.ptr(out), mp, mloc))
+        return out, masks
+
     def predict_sequences(self, frames, intrinsic: IntrinsicMatrix, min_seed_z: float = 500.0, ctx: Context | None = None,
                           device_ptr: int | None = None, n_seq: int | None = None, frames_per_seq: int | None = None,
                           w: int | None = None, h: int | None = None) -> np.ndarray:

@@ -193,3 +193,39 @@ def predict_track_files(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarr
     capi.check(capi.load().dh_predict_tracks_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n_seq, capi.ptr(seq_off),
                                                   int(w), int(h), capi.ptr(args), float(min_seed_z), capi.ptr(out)))
     return out
+
+
+def predict_files_with_mask(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w: int, h: int, intrinsic,
+                            ctx: Context | None = None, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                            mask_device_ptr: int | None = None):
+    """read_depth + pose and head mask per file from one traversal, the decode on the GPU: (capi.RESULT_DTYPE[n],
+    uint8 [n,h,w] or None with mask_device_ptr), equal to predict_files and predict_mask_files.  intrinsic: one
+    IntrinsicMatrix (repeated for every file) or a float32 [n,3,3] array; seeds as in predict_files."""
+    n = len(offsets) - 1
+    args = frame_args(n, intrinsic, midp_guess, rot_guess, has_midp, has_rot)
+    ctx = ctx or default_context()
+    out = np.zeros(n, capi.RESULT_DTYPE)
+    masks, mp, mloc = _image_out(mask_device_ptr, (n, int(h), int(w)), np.uint8)
+    offsets = np.ascontiguousarray(offsets, np.uint64)
+    capi.check(capi.load().dh_predict_frames_mask_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
+                                                       capi.ptr(args), capi.ptr(out), mp, mloc))
+    return out, masks
+
+
+def predict_track_files_with_mask(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, lengths, w: int, h: int, intrinsics,
+                                  midp_guess=None, rot_guess=None, has_midp=None, has_rot=None, min_seed_z: float = 500.0,
+                                  ctx: Context | None = None, mask_device_ptr: int | None = None):
+    """predict_track_files plus the head mask of every file from the same traversal: (capi.RESULT_DTYPE[n],
+    uint8 [n,h,w] or None with mask_device_ptr), both in file order."""
+    seq_off, n_seq, total = _track_offsets(lengths)
+    n = len(offsets) - 1
+    if n != total:
+        raise ValueError("sum(lengths) = %d but there are %d files" % (total, n))
+    args = frame_args(n_seq, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+    ctx = ctx or default_context()
+    out = np.zeros(n, capi.RESULT_DTYPE)
+    masks, mp, mloc = _image_out(mask_device_ptr, (n, int(h), int(w)), np.uint8)
+    offsets = np.ascontiguousarray(offsets, np.uint64)
+    capi.check(capi.load().dh_predict_tracks_mask_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n_seq, capi.ptr(seq_off),
+                                                       int(w), int(h), capi.ptr(args), float(min_seed_z), capi.ptr(out), mp, mloc))
+    return out, masks

@@ -307,6 +307,63 @@ int dh_predict_tracks_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, c
         c->cx->predict_tracks(*f->hf, nullptr, blob, offsets, n_seq, seq_off, w, h, DH_DEPTH_HOST, seq_args, min_seed_z, out);
     });
 }
+
+// Pose and head mask from one traversal: the pose call's argument rules, then the two outputs named
+int dh_predict_frames_mask(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                           const dh_frame_args* args, dh_result* out, uint8_t* mask, int mask_loc) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_frames_mask: bad depth_loc");
+        REQUIRE(mask_loc == DH_DEPTH_HOST || mask_loc == DH_DEPTH_DEVICE, "dh_predict_frames_mask: bad mask_loc");
+        if (args) check_frame_args("dh_predict_frames_mask", args, n);
+        REQUIRE(n == 0 || out, "dh_predict_frames_mask: NULL out");
+        REQUIRE(n == 0 || mask, "dh_predict_frames_mask: NULL mask");
+        REQUIRE(c && f && (n == 0 || (depth && args)), "dh_predict_frames_mask: NULL argument");
+        c->cx->predict_frames(*f->hf, depth, nullptr, nullptr, n, w, h, depth_loc, args, out, mask, mask_loc);
+    });
+}
+int dh_predict_frames_mask_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
+                                uint32_t h, const dh_frame_args* args, dh_result* out, uint8_t* mask, int mask_loc) {
+    return guarded([&] {
+        REQUIRE(mask_loc == DH_DEPTH_HOST || mask_loc == DH_DEPTH_DEVICE, "dh_predict_frames_mask_biwi: bad mask_loc");
+        if (args) check_frame_args("dh_predict_frames_mask_biwi", args, n);
+        if (offsets) check_offsets("dh_predict_frames_mask_biwi", offsets, n);
+        REQUIRE(n == 0 || out, "dh_predict_frames_mask_biwi: NULL out");
+        REQUIRE(n == 0 || mask, "dh_predict_frames_mask_biwi: NULL mask");
+        REQUIRE(c && f && (n == 0 || (blob && offsets && args)), "dh_predict_frames_mask_biwi: NULL argument");
+        c->cx->predict_frames(*f->hf, nullptr, blob, offsets, n, w, h, DH_DEPTH_HOST, args, out, mask, mask_loc);
+    });
+}
+int dh_predict_tracks_mask(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n_seq, const uint64_t* seq_off, uint32_t w,
+                           uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z, dh_result* out, uint8_t* mask,
+                           int mask_loc) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_tracks_mask: bad depth_loc");
+        REQUIRE(mask_loc == DH_DEPTH_HOST || mask_loc == DH_DEPTH_DEVICE, "dh_predict_tracks_mask: bad mask_loc");
+        if (seq_off) check_seq_off("dh_predict_tracks_mask", seq_off, n_seq);
+        if (seq_args) check_frame_args("dh_predict_tracks_mask", seq_args, n_seq, "track");
+        const bool work = seq_off && seq_off[n_seq] > 0;
+        REQUIRE(!work || out, "dh_predict_tracks_mask: NULL out");
+        REQUIRE(!work || mask, "dh_predict_tracks_mask: NULL mask");
+        REQUIRE(c && f && seq_off && (n_seq == 0 || seq_args) && (!work || depth), "dh_predict_tracks_mask: NULL argument");
+        c->cx->predict_tracks(*f->hf, depth, nullptr, nullptr, n_seq, seq_off, w, h, depth_loc, seq_args, min_seed_z, out, mask, mask_loc);
+    });
+}
+int dh_predict_tracks_mask_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
+                                const uint64_t* seq_off, uint32_t w, uint32_t h, const dh_frame_args* seq_args, float min_seed_z,
+                                dh_result* out, uint8_t* mask, int mask_loc) {
+    return guarded([&] {
+        REQUIRE(mask_loc == DH_DEPTH_HOST || mask_loc == DH_DEPTH_DEVICE, "dh_predict_tracks_mask_biwi: bad mask_loc");
+        if (seq_off) check_seq_off("dh_predict_tracks_mask_biwi", seq_off, n_seq);
+        if (seq_args) check_frame_args("dh_predict_tracks_mask_biwi", seq_args, n_seq, "track");
+        if (seq_off && offsets) check_offsets("dh_predict_tracks_mask_biwi", offsets, (uint32_t)seq_off[n_seq]);
+        const bool work = seq_off && seq_off[n_seq] > 0;
+        REQUIRE(!work || out, "dh_predict_tracks_mask_biwi: NULL out");
+        REQUIRE(!work || mask, "dh_predict_tracks_mask_biwi: NULL mask");
+        REQUIRE(c && f && seq_off && (n_seq == 0 || seq_args) && (!work || (blob && offsets)), "dh_predict_tracks_mask_biwi: NULL argument");
+        c->cx->predict_tracks(*f->hf, nullptr, blob, offsets, n_seq, seq_off, w, h, DH_DEPTH_HOST, seq_args, min_seed_z, out, mask,
+                              mask_loc);
+    });
+}
 size_t dh_biwi_encode_bound(uint32_t w, uint32_t h) { return dh::rle_frame_bound(w, h); }
 int dh_biwi_encode_depth(const uint16_t* frames, uint32_t n, uint32_t w, uint32_t h, uint32_t threads, uint8_t* blob, size_t cap,
                          uint64_t* offsets, size_t* needed) {

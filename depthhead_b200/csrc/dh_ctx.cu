@@ -105,7 +105,11 @@ Context::Context(int device) : device_(device) {
     DH_CUDA(cudaHostAlloc((void**)&h_counters_, sizeof(unsigned long long) * DH_N_COUNTERS, cudaHostAllocDefault));
     DH_CUDA(cudaHostAlloc((void**)&h_result1_, sizeof(dh_result), cudaHostAllocDefault));
     for (int i = 0; i < kEncSlots; ++i) DH_CUDA(cudaEventCreateWithFlags(&ev_enc_copied_[i], cudaEventDisableTiming));
-    for (int i = 0; i < 2; ++i) DH_CUDA(cudaEventCreateWithFlags(&tb_.ev_win[i], cudaEventDisableTiming));
+    for (int i = 0; i < 2; ++i) {
+        DH_CUDA(cudaEventCreateWithFlags(&tb_.ev_win[i], cudaEventDisableTiming));
+        DH_CUDA(cudaEventCreateWithFlags(&tb_.ev_mwin_ready[i], cudaEventDisableTiming));
+        DH_CUDA(cudaEventCreateWithFlags(&tb_.ev_mwin_copied[i], cudaEventDisableTiming));
+    }
     DH_CUDA(cudaEventCreateWithFlags(&ev_copy_tail_, cudaEventDisableTiming));
     if (const char* v = std::getenv("DH_HOST_ENCODE")) host_encode_ = *v ? (int)std::strtol(v, nullptr, 10) : -1;
     use_graphs_ = env_flag("DH_GRAPH", true);
@@ -137,8 +141,11 @@ Context::~Context() {
     if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
     if (h_frame_k_) cudaFreeHost(h_frame_k_);
     free_track_buffers();
-    for (int i = 0; i < 2; ++i)
+    for (int i = 0; i < 2; ++i) {
         if (tb_.ev_win[i]) cudaEventDestroy(tb_.ev_win[i]);
+        if (tb_.ev_mwin_ready[i]) cudaEventDestroy(tb_.ev_mwin_ready[i]);
+        if (tb_.ev_mwin_copied[i]) cudaEventDestroy(tb_.ev_mwin_copied[i]);
+    }
     pool_.reset();
     for (int i = 0; i < kEncSlots; ++i) {
         if (h_enc_[i]) cudaFreeHost(h_enc_[i]);
@@ -364,6 +371,8 @@ void Context::free_lane(Lane& L) {
     dev_free(L.img16);
     dev_free(L.img_keys);
     L.img_px = 0;
+    dev_free(L.mask_plane);
+    L.mask_px = 0;
     L.pending_bytes = 0;
     L.allocated = false;
     L.cubes_clean = false;
@@ -830,12 +839,18 @@ void Context::predict_batch_biwi(const HostForest& hf, const uint8_t* blob, cons
 // dh_predict_frames / dh_predict_frames_biwi: the pose pipeline of dh_predict_batch, every frame with
 // the arguments of its own dh_predict call.  The kernels that project read the frame's K, K^-1 from
 // the lane's table (Lane::frame_k); the call's matrix in Geometry (frame 0's) is not used.
+// With a mask destination (dh_predict_frames_mask) the back end also writes predict_mask of every
+// frame from the leaf words of the same traversal (run_pose_mask): chunks, lanes and staging stay
+// those of the pose call.
 void Context::predict_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
-                             uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out) {
+                             uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out, uint8_t* mask,
+                             int mask_loc) {
     static const float kIdentity[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
     BackEnd be;
     be.results = out;
     be.args = args;
+    be.image = mask;
+    be.image_on_device = mask_loc == DH_DEPTH_DEVICE;
     run_batch(hf, depth, blob, offsets, n, w, h, n ? args[0].K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
 }
 
@@ -960,6 +975,7 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     const int n_lanes = timing_ ? 1 : (int)std::max<uint32_t>(1u, std::min<uint32_t>((uint32_t)max_lanes_, (n + want_chunk - 1) / want_chunk));
     ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
     if (be.kind != BackEnd::kPose) ensure_image_scratch(n_lanes);
+    if (be.kind == BackEnd::kPose && be.image && !be.image_on_device) ensure_mask_plane(n_lanes);
     if (be.kind == BackEnd::kBlurred) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
@@ -1137,6 +1153,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     const int n_lanes = hybrid ? 2 : 1;
     ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
     if (be.kind != BackEnd::kPose) ensure_image_scratch(n_lanes);
+    if (be.kind == BackEnd::kPose && be.image && !be.image_on_device) ensure_mask_plane(n_lanes);
     if (be.kind == BackEnd::kBlurred) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
@@ -1389,6 +1406,8 @@ TrackPlan plan_tracks(uint32_t n_seq, const uint64_t* seq_off, uint32_t F) {
 }
 
 constexpr size_t kTrackWindowResults = 1u << 16;  // results per window of passes (3.7 MB)
+// host-bound masks of dh_predict_tracks_mask: a window holds at most this many bytes of masks, or one pass
+constexpr size_t kTrackWindowMaskBytes = 64ull << 20;
 
 template <typename T>
 void host_alloc(T*& p, size_t n) {
@@ -1408,6 +1427,8 @@ void Context::free_track_buffers() {
         host_free(tb_.h_plan[i]);
         host_free(tb_.h_win[i]);
         host_free(tb_.h_blob[i]);
+        dev_free(tb_.d_mwin[i]);
+        host_free(tb_.h_mwin[i]);
     }
     dev_free(tb_.d_win);
     dev_free(tb_.d_tracks);
@@ -1415,12 +1436,12 @@ void Context::free_track_buffers() {
     dev_free(tb_.d_status);
     dev_free(tb_.d_bad);
     host_free(tb_.h_bad);
-    tb_.win_cap = tb_.tracks_cap = tb_.blob_cap = tb_.status_cap = 0;
+    tb_.win_cap = tb_.tracks_cap = tb_.blob_cap = tb_.status_cap = tb_.mwin_cap = 0;
 }
 
 void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
                              const uint64_t* seq_off, uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z,
-                             dh_result* out) {
+                             dh_result* out, uint8_t* mask, int mask_loc) {
     begin_call();
     have_debug_ = false;
     last_encoded_chunks_ = 0;
@@ -1449,9 +1470,14 @@ void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const 
     const uint32_t F = call_chunk_;
     const TrackPlan pl = plan_tracks(n_seq, seq_off, F);
     const uint32_t n_pass = (uint32_t)pl.pass_off.size() - 1;
-    const uint32_t W = (uint32_t)std::max<size_t>(1, kTrackWindowResults / F);  // passes per window
-    const size_t win = (size_t)W * F;
     const size_t px = (size_t)w * h;
+    // Host-bound masks travel in the windows of the results: a window's passes write their masks to
+    // d_mwin in pass order, one copy brings them to h_mwin, and the host scatters them where it scatters
+    // the window's results.  Their windows hold at most kTrackWindowMaskBytes of masks, or one pass.
+    const bool mask_host = mask && mask_loc != DH_DEPTH_DEVICE;
+    const uint32_t W = (uint32_t)std::max<size_t>(
+        1, std::min(kTrackWindowResults / F, mask_host ? kTrackWindowMaskBytes / ((size_t)F * px) : kTrackWindowResults));  // passes per window
+    const size_t win = (size_t)W * F;
 
     // buffers (each grows alone; a free waits for the work that may still use it)
     auto drain = [&] {
@@ -1477,6 +1503,18 @@ void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const 
     if (!tb_.d_bad) {
         dev_alloc(tb_.d_bad, 1);
         host_alloc(tb_.h_bad, 1);
+    }
+    if (mask_host && win * px > tb_.mwin_cap) {
+        drain();
+        for (int i = 0; i < 2; ++i) {
+            dev_free(tb_.d_mwin[i]);
+            host_free(tb_.h_mwin[i]);
+        }
+        for (int i = 0; i < 2; ++i) {
+            dev_alloc(tb_.d_mwin[i], win * px);
+            host_alloc(tb_.h_mwin[i], win * px);
+        }
+        tb_.mwin_cap = win * px;
     }
     if (!uniform) {
         if (n_seq > tb_.tracks_cap) {
@@ -1540,6 +1578,13 @@ void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const 
             for (uint32_t j = pl.pass_off[p]; j < pl.pass_off[p + 1]; ++j)
                 out[pl.slots[j].frame] = r[(size_t)(p - wi * W) * F + (j - pl.pass_off[p])];
     };
+    // ... and its masks (host-bound), once tb_.ev_mwin_copied of its parity has passed
+    auto scatter_masks = [&](uint32_t wi) {
+        const uint8_t* m = tb_.h_mwin[wi & 1u];
+        for (uint32_t p = wi * W; p < std::min(n_pass, (wi + 1) * W); ++p)
+            for (uint32_t j = pl.pass_off[p]; j < pl.pass_off[p + 1]; ++j)
+                std::memcpy(mask + (size_t)pl.slots[j].frame * px, m + ((size_t)(p - wi * W) * F + (j - pl.pass_off[p])) * px, px);
+    };
     const cudaMemcpyKind kind = depth_loc == DH_DEPTH_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     Lane& L = lanes_[0];
     try {
@@ -1553,6 +1598,10 @@ void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const 
             if (pw == 0 && wi >= 2) {  // the pinned buffers of this window's parity are free once window wi - 2 is out
                 DH_CUDA(cudaEventSynchronize(tb_.ev_win[wi & 1u]));
                 scatter(wi - 2);
+                if (mask_host) {  // (and d_mwin of this parity: the lane writes it again only after this point)
+                    DH_CUDA(cudaEventSynchronize(tb_.ev_mwin_copied[wi & 1u]));
+                    scatter_masks(wi - 2);
+                }
             }
             if (p >= 2) DH_CUDA(cudaStreamWaitEvent(copy_stream_, ev_consumed_[slot], 0));
             if (pw == 0 && !uniform) {  // the window's slot tables (pass p - 2 consumed: window wi - 2 is done with them)
@@ -1601,14 +1650,30 @@ void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const 
                 launch_biwi_decode(d_blob_[slot] + 16ull * n, d_pairs, d_pairs + n, 0ull, n, w, h, d_depth_[slot], tb_.d_status, L.stream);
                 launches_ += 1;
             }
+            // the pass's masks, from the leaf words of its traversal: to their frames of `mask` (the slot table, or on the
+            // uniform path, which uploads none, the stride of its strided copy), or to the window's plane in pass order
+            auto pass_masks = [&] {
+                if (!mask) return;
+                mark(DH_STAGE_VOTE);  // booked as the 2-D calls book their back end
+                if (mask_host)
+                    launch_track_mask(b, geom_, fdev_, n, nullptr, 0u, 1u, tb_.d_mwin[wi & 1u] + (size_t)pw * F * px, L.stream);
+                else if (uniform)
+                    launch_track_mask(b, geom_, fdev_, n, nullptr, (uint32_t)e[0].frame, (uint32_t)seq_off[1], mask, L.stream);
+                else
+                    launch_track_mask(b, geom_, fdev_, n, d_e, 0u, 0u, mask, L.stream);
+                launches_ += 1;
+                stage_check("mask");
+            };
             if (uniform) {
                 run_front(L, b, n, nullptr, e[0].prev >= 0 ? L.results : nullptr, min_seed_z);
+                pass_masks();
                 run_back(L, b, n, iterations);
             } else {
                 launch_track_guess(L.fs, L.frame_k, d_e, tb_.d_tracks, L.results, n, min_seed_z, blob ? tb_.d_status : nullptr,
                                    tb_.d_bad, L.stream);
                 launches_ += 1;
                 run_front(L, b, n, nullptr, nullptr, 0.0f, nullptr, 0, true);
+                pass_masks();
                 run_back(L, b, n, iterations, L.frame_k);
             }
             DH_CUDA(cudaMemcpyAsync(tb_.d_win + (size_t)pw * F, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToDevice, L.stream));
@@ -1617,18 +1682,30 @@ void Context::predict_tracks(const HostForest& hf, const uint16_t* depth, const 
                 DH_CUDA(cudaMemcpyAsync(tb_.h_win[wi & 1u], tb_.d_win, sizeof(dh_result) * (size_t)(pw + 1) * F, cudaMemcpyDeviceToHost,
                                         L.stream));
                 DH_CUDA(cudaEventRecord(tb_.ev_win[wi & 1u], L.stream));
+                if (mask_host) {  // the window's masks leave on the second copy stream while the lane goes on
+                    DH_CUDA(cudaEventRecord(tb_.ev_mwin_ready[wi & 1u], L.stream));
+                    DH_CUDA(cudaStreamWaitEvent(copy_stream2_, tb_.ev_mwin_ready[wi & 1u], 0));
+                    DH_CUDA(cudaMemcpyAsync(tb_.h_mwin[wi & 1u], tb_.d_mwin[wi & 1u], (size_t)(pw + 1) * F * px, cudaMemcpyDeviceToHost,
+                                            copy_stream2_));
+                    DH_CUDA(cudaEventRecord(tb_.ev_mwin_copied[wi & 1u], copy_stream2_));
+                }
             }
         }
         if (blob) DH_CUDA(cudaMemcpyAsync(tb_.h_bad, tb_.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream_));
     } catch (...) {
         cudaStreamSynchronize(copy_stream_);
+        cudaStreamSynchronize(copy_stream2_);
         cudaStreamSynchronize(stream_);
         throw;
     }
     mark(-1);
     end_call();
     const uint32_t last = (n_pass - 1) / W;
-    for (uint32_t wi = last >= 1 ? last - 1 : 0; wi <= last; ++wi) scatter(wi);
+    if (mask_host) DH_CUDA(cudaStreamSynchronize(copy_stream2_));
+    for (uint32_t wi = last >= 1 ? last - 1 : 0; wi <= last; ++wi) {
+        scatter(wi);
+        if (mask_host) scatter_masks(wi);
+    }
     if (blob && *tb_.h_bad != ~0ull) throw_biwi_status((size_t)(*tb_.h_bad >> 2), (uint32_t)(*tb_.h_bad & 3u));
 }
 
@@ -1771,8 +1848,46 @@ void Context::run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
         run_image_back(L, b, f0, n, be);
         return;
     }
+    if (be.image) run_pose_mask(L, b, f0, n, be);
     run_back(L, b, n, iterations, be.args ? L.frame_k : nullptr);
     DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
+}
+
+// The masks of a pose chunk, between its traversal and its patch gate (nothing after the traversal
+// writes the leaf words, and the lane's next chunk rewrites them only after this launch in stream
+// order).  mask_kernel as in run_image_back: it reads ids through b.leaf_mask whether or not the words
+// carry probability codes, and decides background on the tree-0 slice.  Device-bound masks are
+// written in place; host-bound ones go to the lane's plane and out through the deferred copy.
+void Context::run_pose_mask(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be) {
+    const Geometry& g = geom_;
+    const size_t frame_px = (size_t)g.w * g.h, px = frame_px * n;
+    mark(DH_STAGE_VOTE);  // booked as the 2-D calls book their back end
+    uint8_t* mask = be.image_on_device ? static_cast<uint8_t*>(be.image) + (size_t)f0 * frame_px : L.mask_plane;
+    DH_CUDA(cudaMemsetAsync(mask, 0, px, L.stream));
+    if (g.P) {
+        launch_mask(b, g, fdev_, n, mask, L.stream);
+        launches_ += 1;
+    }
+    stage_check("mask");
+    if (!be.image_on_device) {
+        L.pending_dst = static_cast<uint8_t*>(be.image) + (size_t)f0 * frame_px;
+        L.pending_src = mask;
+        L.pending_bytes = px;
+    }
+}
+
+// one u8 plane per frame of a chunk, on every lane of the call (host-bound masks of the pose back end)
+void Context::ensure_mask_plane(int n_lanes) {
+    const size_t need = (size_t)call_chunk_ * sk_.w * sk_.h;
+    for (int i = 0; i < std::max(1, std::min(n_lanes, kMaxLanes)); ++i) {
+        Lane& L = lanes_[i];
+        if (L.mask_px >= need) continue;
+        DH_CUDA(cudaStreamSynchronize(stream_));
+        dev_free(L.mask_plane);
+        L.mask_px = 0;
+        dev_alloc(L.mask_plane, need);
+        L.mask_px = need;
+    }
 }
 
 // The 2-D back end of one chunk; the launches do not depend on the number of frames.  Images the

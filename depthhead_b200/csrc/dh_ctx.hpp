@@ -41,6 +41,9 @@ struct Lane {
     uint16_t* img16 = nullptr;      // [2][F][h][w] horizontal blur, then the image handed out (mask: u8 in the second plane)
     unsigned long long* img_keys = nullptr;  // [F] arg-max keys of the from2d pass
     size_t img_px = 0;              // F * h * w the image scratch holds
+    // pose back end with host-bound masks (dh_predict_frames_mask): the u8 masks of a chunk, allocated by the first such call
+    uint8_t* mask_plane = nullptr;  // [F][h][w]
+    size_t mask_px = 0;             // F * h * w it holds
     // a host-bound image copy of this lane's last chunk, issued before the lane's next chunk (a copy
     // to pageable memory blocks the host: deferred, it overlaps the other lane's kernels)
     void* pending_dst = nullptr;
@@ -62,7 +65,8 @@ struct BackEnd {
     dh_result* results = nullptr;  // kPose: poses [n]; kBlurred: from2d poses [n] or nullptr (host memory)
     const dh_frame_args* args = nullptr;  // intrinsics and seeds of every frame [n] (host memory), or nullptr: the call's
                                           // one K and no seeds (kVotes / kBlurred: intrinsics only; kMask: unused)
-    void* image = nullptr;         // kMask: u8 [n][h][w]; kVotes / kBlurred: u16 [n][h][w] (kBlurred: may be nullptr)
+    void* image = nullptr;         // kMask: u8 [n][h][w]; kVotes / kBlurred: u16 [n][h][w] (kBlurred: may be nullptr);
+                                   // kPose: u8 head masks [n][h][w] from the pose pass's own leaf words, or nullptr
     bool image_on_device = false;  // image points to device memory on the context's GPU
 };
 // Image back ends keep a u32 accumulator and two u16 planes per frame of a chunk (8 bytes per
@@ -110,16 +114,19 @@ public:
                            const float K[9], int depth_loc, float min_seed_z, dh_result* out);
     // n_seq tracks: track s owns frames [seq_off[s], seq_off[s+1]) of depth at depth_loc, or of the Biwi
     // files of blob / offsets (blob != nullptr); seq_args[s]: its K and the seeds of its first frame
+    // mask != nullptr (dh_predict_tracks_mask): also every frame's predict_mask to [total][h][w] u8 at mask_loc, in input order
     void predict_tracks(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
                         const uint64_t* seq_off, uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z,
-                        dh_result* out);
+                        dh_result* out, uint8_t* mask = nullptr, int mask_loc = DH_DEPTH_HOST);
     // Biwi run-length coded frames (biwi.rs:81-103): blob/offsets in host memory, see depthhead_cuda.h
     void biwi_decode(const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h, uint16_t* out, int out_loc);
     void predict_batch_biwi(const HostForest& hf, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w, uint32_t h,
                             const float K[9], dh_result* out);
     // dh_predict for every frame with its own arguments: depth at depth_loc, or Biwi files (blob != nullptr)
+    // mask != nullptr (dh_predict_frames_mask): also every frame's predict_mask to [n][h][w] u8 at mask_loc
     void predict_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
-                        uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out);
+                        uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out, uint8_t* mask = nullptr,
+                        int mask_loc = DH_DEPTH_HOST);
     // training: split scoring (dh_train.cu; houghforest.rs:250-295)
     TrainSet* trainset_create(const uint16_t* patches, uint64_t n, uint32_t sw, uint32_t sh, uint32_t rw, uint32_t rh,
                               const uint8_t* is_object, const float* offsets, const double* rotations);
@@ -178,10 +185,13 @@ private:
     void ensure_results(uint32_t n);
     void ensure_frame_args(uint32_t n);
     void ensure_image_scratch(int n_lanes);
+    void ensure_mask_plane(int n_lanes);
     void ensure_blur_taps(const HostForest& hf);
     // after run_front: the chunk's back end and the copies of its results (frames f0 .. f0 + n - 1 of the batch)
     void run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be);
     void run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be);
+    // kPose with a mask destination: the chunk's masks from the leaf words its traversal left
+    void run_pose_mask(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be);
     void flush_pending(Lane& L);
     void free_scratch();
     TilePlan plan_tiles(const Geometry& g) const;
@@ -299,6 +309,12 @@ private:
         unsigned long long* d_bad = nullptr;         // lowest bad Biwi frame << 2 | its status
         unsigned long long* h_bad = nullptr;
         cudaEvent_t ev_win[2] = {nullptr, nullptr};  // the window's results are in h_win
+        // host-bound masks of dh_predict_tracks_mask: a window's masks in pass order, [passes][F][h][w] u8
+        uint8_t* d_mwin[2] = {nullptr, nullptr};     // (device, by window parity; written by track_mask_kernel)
+        uint8_t* h_mwin[2] = {nullptr, nullptr};     // (pinned, by window parity)
+        size_t mwin_cap = 0;                         // bytes of each of the four above
+        cudaEvent_t ev_mwin_ready[2] = {nullptr, nullptr};   // the window's masks are in d_mwin
+        cudaEvent_t ev_mwin_copied[2] = {nullptr, nullptr};  // ... and in h_mwin
     } tb_;
     void free_track_buffers();
 

@@ -19,7 +19,8 @@
 //                                per accumulator; rebuilds its cube around positions that drift out of it
 //   K5  leaf_gate_kernel         estimate_mean_cov traces + valtoadd per leaf, once per model
 //                                (meancov_estimation.rs:359-378, prediction.rs:594-600,643)
-//   +   mask_kernel, hough_image_kernel (prediction.rs:850-905, 760-841), biwi_decode_kernel
+//   +   mask_kernel (and track_mask_kernel, its writer for scattered frames), hough_image_kernel
+//       (prediction.rs:850-905, 760-841), biwi_decode_kernel
 //       (db_reader/biwi.rs:81-103); training's split scoring lives in dh_train.cu
 //
 // Exactness rules (SURVEY Appendix A): float->int is truncation (cvt.rzi, saturating, NaN->0 ==
@@ -1912,6 +1913,58 @@ __global__ void __launch_bounds__(256) mask_kernel(FrameBuffers b, Geometry g, c
         }
 }
 
+// predict_mask for the passes of dh_predict_tracks_mask, whose frames are scattered over the output:
+// slot j of a pass is output frame slots[j].frame (slots != nullptr) or frame0 + j * frame_step.  A
+// memset of the chunk cannot clear scattered frames, so this writer stores EVERY pixel: a CTA owns a
+// tile of kTrackMaskTileW x kTrackMaskTileH pixels of one frame, settles the u8 of every patch whose
+// block meets the tile in shared memory (the arithmetic of mask_kernel; 0 for background), then
+// gives each pixel the value of the block that holds it, or 0 outside every block.  Pixel X lies in
+// the block of patch column gx = (X + s/2 - left_w) / s iff X + s/2 >= left_w and gx < npx (blocks
+// are s wide, s apart, and start at the patch centre - s/2), the same for rows.
+constexpr uint32_t kTrackMaskTileW = 128, kTrackMaskTileH = 8;
+__global__ void __launch_bounds__(256) track_mask_kernel(FrameBuffers b, Geometry g, const double* __restrict__ leaf_prob,
+                                                         const TrackSlot* __restrict__ slots, uint32_t frame0, uint32_t frame_step,
+                                                         uint8_t* __restrict__ mask) {
+    // at most (tile - 1) / s + 2 block columns / rows meet a tile
+    __shared__ uint8_t pv_s[(kTrackMaskTileW + 1) * (kTrackMaskTileH + 1)];
+    const uint32_t j = blockIdx.z, x0 = blockIdx.x * kTrackMaskTileW, y0 = blockIdx.y * kTrackMaskTileH;
+    const uint32_t s = g.stride, half = s / 2;
+    const uint32_t x1 = min(x0 + kTrackMaskTileW, g.w) - 1u, y1 = min(y0 + kTrackMaskTileH, g.h) - 1u;  // last pixel of the tile
+    // block columns [cx0, cx1) and rows [cy0, cy1) that meet the tile
+    const uint32_t cx0 = x0 + half >= g.left_w ? (x0 + half - g.left_w) / s : 0u;
+    const uint32_t cx1 = x1 + half >= g.left_w ? min((x1 + half - g.left_w) / s + 1u, g.npx) : 0u;
+    const uint32_t cy0 = y0 + half >= g.left_h ? (y0 + half - g.left_h) / s : 0u;
+    const uint32_t cy1 = y1 + half >= g.left_h ? min((y1 + half - g.left_h) / s + 1u, g.npy) : 0u;
+    const uint32_t ncx = cx1 > cx0 ? cx1 - cx0 : 0u, ncy = cy1 > cy0 ? cy1 - cy0 : 0u;
+    const int T = (int)g.n_trees;
+    const int32_t* leaf = b.leaf + (size_t)j * g.n_trees * g.P;
+    for (uint32_t k = threadIdx.x; k < ncx * ncy; k += blockDim.x) {
+        const uint32_t p = (cy0 + k / ncx) * g.npx + cx0 + k % ncx;
+        uint8_t pv = 0;
+        if (leaf[p] >= 0) {
+            double sum = 0.0;
+            for (int t = 0; t < T; ++t) sum = __dadd_rn(sum, __ldg(leaf_prob + ((uint32_t)leaf[(size_t)t * g.P + p] & b.leaf_mask)));
+            const double scaled = __dmul_rn(__ddiv_rn(sum, (double)T), 255.0);
+            pv = !(scaled > 0.0) ? 0 : (scaled >= 255.0 ? 255 : (uint8_t)__double2uint_rz(scaled));
+        }
+        pv_s[k] = pv;
+    }
+    __syncthreads();
+    const uint32_t frame = slots ? (uint32_t)slots[j].frame : frame0 + j * frame_step;
+    uint8_t* out = mask + (size_t)frame * g.w * g.h;
+    const uint32_t lane = threadIdx.x & 31u, row = threadIdx.x >> 5;  // a warp stores 32 adjacent bytes of one row
+    const uint32_t y = y0 + row;
+    if (y > y1) return;
+    const uint32_t gy = (y + half - g.left_h) / s;
+    const bool in_y = y + half >= g.left_h && gy < g.npy;
+    for (uint32_t x = x0 + lane; x <= x1; x += 32u) {
+        const uint32_t gx = (x + half - g.left_w) / s;
+        uint8_t v = 0;
+        if (in_y && x + half >= g.left_w && gx < g.npx) v = pv_s[(gy - cy0) * ncx + (gx - cx0)];
+        out[(size_t)y * g.w + x] = v;
+    }
+}
+
 // build_hough_image before the blur (prediction.rs:760-841).  u16 wrap-around adds are done as
 // u32 atomics into the frame's accumulator and truncated by the reader (sum mod 2^16 is the same
 // either way).  One thread per (frame, tree, patch).  kFrameK: the frame's K and K^-1 come from
@@ -2585,6 +2638,13 @@ void launch_leaf_gates(const double* leaf_prob, const uint32_t* vote_start, cons
 
 void launch_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint8_t* mask, cudaStream_t s) {
     mask_kernel<<<dim3((g.P + 255) / 256, n_frames), 256, 0, s>>>(b, g, f.leaf_prob, mask);
+}
+
+void launch_track_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, const TrackSlot* slots,
+                       uint32_t frame0, uint32_t frame_step, uint8_t* mask, cudaStream_t s) {
+    if (!n_frames) return;
+    const dim3 grid((g.w + kTrackMaskTileW - 1) / kTrackMaskTileW, (g.h + kTrackMaskTileH - 1) / kTrackMaskTileH, n_frames);
+    track_mask_kernel<<<grid, kTrackMaskTileW * kTrackMaskTileH / 4, 0, s>>>(b, g, f.leaf_prob, slots, frame0, frame_step, mask);
 }
 
 void launch_hough_votes(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, uint32_t* acc32, cudaStream_t s,

@@ -165,6 +165,11 @@ struct TrackArgs {
 // slot i: frame state and K / K^-1 row (frame_k [n][18]); status (pass-local Biwi decode status) may be nullptr
 void launch_track_guess(FrameState* fs, float* frame_k, const TrackSlot* slots, const TrackArgs* tracks, const dh_result* prev,
                         uint32_t n, float min_seed_z, const uint32_t* status, unsigned long long* bad, cudaStream_t s);
+// predict_mask of a pass whose frames are scattered over the output: slot i goes to frame slots[i].frame of
+// mask ([..][h][w] u8), or to frame frame0 + i * frame_step when slots is nullptr.  Every pixel of those
+// frames is written (no memset before it).
+void launch_track_mask(const FrameBuffers& b, const Geometry& g, const ForestDev& f, uint32_t n_frames, const TrackSlot* slots,
+                       uint32_t frame0, uint32_t frame_step, uint8_t* mask, cudaStream_t s);
 // dst[i] = frame slots[i].frame of src (device memory, [..][frame_px] u16)
 void launch_track_gather(const uint16_t* src, uint16_t* dst, const TrackSlot* slots, uint32_t n, size_t frame_px, cudaStream_t s);
 void launch_counters(const FrameBuffers& b, const Geometry& g, uint32_t n_frames, unsigned long long* out,

@@ -29,6 +29,10 @@
  *                                                                                 dh_biwi_decode_depth, dh_predict_batch_biwi,
  *                                                                                 dh_predict_mask_batch_biwi,
  *                                                                                 dh_build_hough_image_frames_biwi
+ *   examples/live_prediction.rs:76,86,108: pose and mask of one frame          -> dh_predict_frames_mask,
+ *                                                                                 dh_predict_frames_mask_biwi,
+ *                                                                                 dh_predict_tracks_mask,
+ *                                                                                 dh_predict_tracks_mask_biwi
  *   src/db_reader/biwi.rs:27-60       read_cal (depth.cal -> IntrinsicMatrix)   -> dh_biwi_parse_cal
  *   src/db_reader/biwi.rs:63-77       read_gt (ground-truth pose file)          -> dh_biwi_parse_pose
  *   src/hough/houghforest.rs:250-295  HoughTreeFunctions::impurity (training)   -> dh_train_score_level
@@ -269,6 +273,38 @@ int dh_predict_tracks(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint
 int dh_predict_tracks_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
                            const uint64_t* seq_off, uint32_t w, uint32_t h, const dh_frame_args* seq_args, float min_seed_z,
                            dh_result* out);
+
+/* Pose AND head mask of the same frames from one traversal: what examples/live_prediction.rs asks of
+ * every frame (predict_parameter_parallel seeded from the previous frame, then predict_mask).  The
+ * box-sum image and the forest walk of a frame run once; the mask is written from the leaf words the
+ * pose pass found.  Arguments as the pose call named in each line, plus
+ *   mask:     [n][h][w] u8 ([total][h][w] for tracks, in input order) at mask_loc (DH_DEPTH_HOST or
+ *             DH_DEPTH_DEVICE).  Every pixel is written, whatever the buffer held before.
+ * Contract:
+ *   - out equals, byte for byte over the whole dh_result array, the pose call with the same arguments
+ *     (dh_predict_frames, _frames_biwi, _tracks, _tracks_biwi), at every chunk size;
+ *   - mask equals dh_predict_mask_batch over the same frames, byte for byte;
+ *   - argument rules are the pose call's; in addition, with any frame to process a NULL mask or a NULL
+ *     out is DH_E_ARG naming it, and so is a mask_loc that is neither DH_DEPTH_HOST nor
+ *     DH_DEPTH_DEVICE.  Like the pose call's own, these checks happen before any device work.  A
+ *     caller who wants only one of the two outputs has the existing calls;
+ *   - a damaged Biwi file gives the pose call's error: DH_E_ARG naming the lowest bad frame;
+ *   - n = 0 (total = 0 for tracks) is a successful no-op;
+ *   - counters [0]-[8], [10], [11] and dh_ctx_transfer_info equal the pose call's; [9] (launches) is the
+ *     pose call's plus one per pass, the mask launch (on the frames form, none for a frame that holds
+ *     no patch); with stage timing on, the mask is booked under DH_STAGE_VOTE.
+ * Synchronous. */
+int dh_predict_frames_mask(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                           int depth_loc, const dh_frame_args* args, dh_result* out, uint8_t* mask, int mask_loc);
+int dh_predict_frames_mask_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                                uint32_t w, uint32_t h, const dh_frame_args* args, dh_result* out, uint8_t* mask, int mask_loc);
+int dh_predict_tracks_mask(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n_seq, const uint64_t* seq_off,
+                           uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* seq_args, float min_seed_z,
+                           dh_result* out, uint8_t* mask, int mask_loc);
+int dh_predict_tracks_mask_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n_seq,
+                                const uint64_t* seq_off, uint32_t w, uint32_t h, const dh_frame_args* seq_args, float min_seed_z,
+                                dh_result* out, uint8_t* mask, int mask_loc);
+
 /* The writer for that format (the reference only reads it): n raw frames [n][h][w] u16 become n
  * files in ONE blob, file i at [offsets[i], offsets[i+1]) (offsets: n+1 entries, multiples of 16).
  * Runs are found at a granularity of 16 pixels: a group of 16 pixels with any non-zero pixel is
@@ -359,7 +395,9 @@ int dh_forest_to_json(const dh_forest* f, char* buf, size_t cap, size_t* needed)
  * summed over its chunks, in milliseconds.  Order of stages: see DH_STAGE_*.  After the 2-D calls
  * (dh_predict_mask*, dh_hough_image_raw, dh_build_hough_image*, dh_predict_from2dhough) H2D, SAT,
  * TRAVERSE and D2H mean the same, and their whole back end (mask or vote image, blur, arg-max) is
- * booked under DH_STAGE_VOTE; GATE and MEANSHIFT stay 0. */
+ * booked under DH_STAGE_VOTE; GATE and MEANSHIFT stay 0.  The pose-and-mask calls
+ * (dh_predict_frames_mask*, dh_predict_tracks_mask*) book their mask launch under DH_STAGE_VOTE too,
+ * beside the seeds and cubes of the pose. */
 #define DH_STAGE_H2D 0
 #define DH_STAGE_SAT 1
 #define DH_STAGE_TRAVERSE 2

@@ -116,6 +116,17 @@ extern "C" {
     fn dh_predict_tracks_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n_seq: u32,
                               seq_off: *const u64, w: u32, h: u32, seq_args: *const DhFrameArgs, min_seed_z: f32,
                               out: *mut DhResult) -> c_int;
+    // pose and head mask of the same frames from one traversal
+    fn dh_predict_frames_mask(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n: u32, w: u32, h: u32, depth_loc: c_int,
+                              args: *const DhFrameArgs, out: *mut DhResult, mask: *mut u8, mask_loc: c_int) -> c_int;
+    fn dh_predict_frames_mask_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n: u32, w: u32, h: u32,
+                                   args: *const DhFrameArgs, out: *mut DhResult, mask: *mut u8, mask_loc: c_int) -> c_int;
+    fn dh_predict_tracks_mask(c: *mut DhCtx, f: *const DhForest, depth: *const u16, n_seq: u32, seq_off: *const u64, w: u32, h: u32,
+                              depth_loc: c_int, seq_args: *const DhFrameArgs, min_seed_z: f32, out: *mut DhResult, mask: *mut u8,
+                              mask_loc: c_int) -> c_int;
+    fn dh_predict_tracks_mask_biwi(c: *mut DhCtx, f: *const DhForest, blob: *const u8, offsets: *const u64, n_seq: u32,
+                                   seq_off: *const u64, w: u32, h: u32, seq_args: *const DhFrameArgs, min_seed_z: f32,
+                                   out: *mut DhResult, mask: *mut u8, mask_loc: c_int) -> c_int;
     fn dh_biwi_parse_cal(text: *const c_char, len: usize, k: *mut f32) -> c_int;
     fn dh_biwi_parse_pose(file: *const u8, len: usize, k: *const f32, pos3d: *mut f32, pos2d: *mut f32,
                           rot: *mut f32) -> c_int;
@@ -394,6 +405,37 @@ impl HoughPrediction {
                                          0 /* DH_DEPTH_HOST */, args.as_ptr(), min_seed_z, out.as_mut_ptr()) })?;
         Ok(out)
     }
+    /// predict_frames and predict_mask_batch of the same frames from one traversal (what
+    /// examples/live_prediction.rs:76,86,108 asks of every frame): poses in frame order, masks [n][h][w]
+    pub fn predict_frames_with_mask(&self, frames: &[u16], n: u32, w: u32, h: u32, intrinsics: &[IntrinsicMatrix],
+                                    midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>])
+                                    -> Result<(Vec<DhResult>, Vec<u8>), Error> {
+        let px = (n as usize) * (w as usize) * (h as usize);
+        assert_eq!(frames.len(), px);
+        let args = frame_args(n, intrinsics, midp_guess, rot_guess);
+        self.push_fields()?;
+        let mut out = vec![DhResult::default(); n as usize];
+        let mut mask = vec![0u8; px];
+        check(unsafe { dh_predict_frames_mask(self.context(), self.forest, frames.as_ptr(), n, w, h, 0 /* DH_DEPTH_HOST */,
+                                              args.as_ptr(), out.as_mut_ptr(), mask.as_mut_ptr(), 0) })?;
+        Ok((out, mask))
+    }
+    /// predict_tracks plus the head mask of every frame from the same traversal; both in input order
+    pub fn predict_tracks_with_mask(&self, frames: &[u16], lengths: &[u32], w: u32, h: u32, intrinsics: &[IntrinsicMatrix],
+                                    midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>], min_seed_z: f32)
+                                    -> Result<(Vec<DhResult>, Vec<u8>), Error> {
+        let seq_off = track_offsets(lengths);
+        let n = *seq_off.last().unwrap() as usize;
+        assert_eq!(frames.len(), n * (w as usize) * (h as usize));
+        let args = frame_args(lengths.len() as u32, intrinsics, midp_guess, rot_guess);
+        self.push_fields()?;
+        let mut out = vec![DhResult::default(); n];
+        let mut mask = vec![0u8; frames.len()];
+        check(unsafe { dh_predict_tracks_mask(self.context(), self.forest, frames.as_ptr(), lengths.len() as u32, seq_off.as_ptr(), w, h,
+                                              0 /* DH_DEPTH_HOST */, args.as_ptr(), min_seed_z, out.as_mut_ptr(), mask.as_mut_ptr(),
+                                              0) })?;
+        Ok((out, mask))
+    }
     /// HoughLearning::learn (prediction.rs:145-234) on the GPU: `depth`/`mask` are n frames back to
     /// back, `k` one row-major 3x3 matrix per frame, `pos3d`/`rot` the annotated head pose per frame.
     pub fn learn(params: &DhTrainParams, n: u32, w: u32, h: u32, depth: &[u16], mask: &[u8], k: &[f32],
@@ -581,6 +623,35 @@ pub mod biwi {
                                                   lengths.len() as u32, seq_off.as_ptr(), files.width, files.height, args.as_ptr(),
                                                   min_seed_z, out.as_mut_ptr()) })?;
             Ok(out)
+        }
+        /// predict_files_frames and predict_mask_files of the same files from one traversal: (poses, masks [n][h][w])
+        pub fn predict_files_with_mask(&self, files: &PackedFiles, intrinsics: &[IntrinsicMatrix], midp_guess: &[Option<[f32; 3]>],
+                                       rot_guess: &[Option<[f64; 3]>]) -> Result<(Vec<DhResult>, Vec<u8>), Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            let args = frame_args(n, intrinsics, midp_guess, rot_guess);
+            self.push_fields()?;
+            let mut out = vec![DhResult::default(); n as usize];
+            let mut mask = vec![0u8; n as usize * files.width as usize * files.height as usize];
+            check(unsafe { dh_predict_frames_mask_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(), n,
+                                                       files.width, files.height, args.as_ptr(), out.as_mut_ptr(), mask.as_mut_ptr(),
+                                                       0 /* DH_DEPTH_HOST */) })?;
+            Ok((out, mask))
+        }
+        /// predict_tracks_biwi plus the head mask of every file from the same traversal; both in file order
+        pub fn predict_tracks_biwi_with_mask(&self, files: &PackedFiles, lengths: &[u32], intrinsics: &[IntrinsicMatrix],
+                                             midp_guess: &[Option<[f32; 3]>], rot_guess: &[Option<[f64; 3]>], min_seed_z: f32)
+                                             -> Result<(Vec<DhResult>, Vec<u8>), Error> {
+            let n = (files.offsets.len() - 1) as u32;
+            let seq_off = track_offsets(lengths);
+            assert_eq!(*seq_off.last().unwrap(), n as u64, "the track lengths must add up to the number of files");
+            let args = frame_args(lengths.len() as u32, intrinsics, midp_guess, rot_guess);
+            self.push_fields()?;
+            let mut out = vec![DhResult::default(); n as usize];
+            let mut mask = vec![0u8; n as usize * files.width as usize * files.height as usize];
+            check(unsafe { dh_predict_tracks_mask_biwi(self.context(), self.forest, files.blob.as_ptr(), files.offsets.as_ptr(),
+                                                       lengths.len() as u32, seq_off.as_ptr(), files.width, files.height, args.as_ptr(),
+                                                       min_seed_z, out.as_mut_ptr(), mask.as_mut_ptr(), 0 /* DH_DEPTH_HOST */) })?;
+            Ok((out, mask))
         }
     }
 }
