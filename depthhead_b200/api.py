@@ -456,6 +456,29 @@ class HoughPrediction:
         capi.check(capi.load().dh_predict_frames_mask(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(out), mp, mloc))
         return out, masks
 
+    # ---- pose and 2-D Hough result of the same frames from one traversal (examples/db_prediction.rs:140,154
+    # asks both of every Biwi frame).  Images: returned as a host uint16 array, or written to the caller's
+    # device memory at hough_device_ptr (nothing returned on the host).
+    def predict_frames_with_hough(self, frames, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                                  blur: bool = True, image: bool = True, from2d: bool = True, ctx: Context | None = None,
+                                  device_ptr: int | None = None, n: int | None = None, w: int | None = None, h: int | None = None,
+                                  hough_device_ptr: int | None = None):
+        """predict_frames and build_hough_image_frames (blur=False: hough_image_raw_frames) of the same frames in
+        one pass, the 2-D outputs with every frame's own K: (capi.RESULT_DTYPE[n], uint16 [n,h,w] or None,
+        capi.RESULT_DTYPE[n] of predict_parameter_from2dhough or None), each equal to what its own call returns.
+        image=False asks for no image, from2d=False for no from2d results (from2d needs blur)."""
+        if hough_device_ptr is not None and not image:
+            raise ValueError("hough_device_ptr needs image=True")
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        args = frame_args(n, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+        ctx = ctx or default_context()
+        out = np.zeros(n, capi.RESULT_DTYPE)
+        images, ip, iloc = _image_out(hough_device_ptr, (n, h, w), np.uint16) if image else (None, None, capi.DH_DEPTH_HOST)
+        res = np.zeros(n, capi.RESULT_DTYPE) if from2d else None
+        capi.check(capi.load().dh_predict_frames_hough(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(out), int(bool(blur)),
+                                                       ip, iloc, capi.ptr(res)))
+        return out, images, res
+
     def predict_tracks_with_mask(self, frames, lengths, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
                                  min_seed_z: float = 500.0, ctx: Context | None = None, device_ptr: int | None = None,
                                  w: int | None = None, h: int | None = None, mask_device_ptr: int | None = None):

@@ -229,3 +229,25 @@ def predict_track_files_with_mask(hp: HoughPrediction, blob: np.ndarray, offsets
     capi.check(capi.load().dh_predict_tracks_mask_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n_seq, capi.ptr(seq_off),
                                                        int(w), int(h), capi.ptr(args), float(min_seed_z), capi.ptr(out), mp, mloc))
     return out, masks
+
+
+def predict_files_with_hough(hp: HoughPrediction, blob: np.ndarray, offsets: np.ndarray, w: int, h: int, intrinsic,
+                             ctx: Context | None = None, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                             blur: bool = True, image: bool = True, from2d: bool = True, hough_device_ptr: int | None = None):
+    """read_depth + pose and 2-D Hough result per file from one traversal, the decode on the GPU
+    (examples/db_prediction.rs:140,154): (capi.RESULT_DTYPE[n], uint16 [n,h,w] or None, capi.RESULT_DTYPE[n]
+    or None), equal to predict_files and build_hough_image_files with every file's K.  intrinsic: one
+    IntrinsicMatrix (repeated for every file) or a float32 [n,3,3] array; seeds as in predict_files (they act
+    on the poses only); blur, image and from2d as in HoughPrediction.predict_frames_with_hough."""
+    if hough_device_ptr is not None and not image:
+        raise ValueError("hough_device_ptr needs image=True")
+    n = len(offsets) - 1
+    args = frame_args(n, intrinsic, midp_guess, rot_guess, has_midp, has_rot)
+    ctx = ctx or default_context()
+    out = np.zeros(n, capi.RESULT_DTYPE)
+    images, ip, iloc = _image_out(hough_device_ptr, (n, int(h), int(w)), np.uint16) if image else (None, None, capi.DH_DEPTH_HOST)
+    res = np.zeros(n, capi.RESULT_DTYPE) if from2d else None
+    offsets = np.ascontiguousarray(offsets, np.uint64)
+    capi.check(capi.load().dh_predict_frames_hough_biwi(ctx._h, hp._h, capi.ptr(blob), capi.ptr(offsets), n, int(w), int(h),
+                                                        capi.ptr(args), capi.ptr(out), int(bool(blur)), ip, iloc, capi.ptr(res)))
+    return out, images, res

@@ -122,6 +122,8 @@ SIGNATURES = {
     "dh_predict_frames_mask_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp, _vp, C.c_int]),
     "dh_predict_tracks_mask": (C.c_int, [_vp, _vp, _vp, _u32, _vp, _u32, _u32, C.c_int, _vp, _f32, _vp, _vp, C.c_int]),
     "dh_predict_tracks_mask_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _vp, _u32, _u32, _vp, _f32, _vp, _vp, C.c_int]),
+    "dh_predict_frames_hough": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, C.c_int, _vp, _vp, C.c_int, _vp, C.c_int, _vp]),
+    "dh_predict_frames_hough_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp, C.c_int, _vp, C.c_int, _vp]),
     "dh_hough_image_raw": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "dh_build_hough_image": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),
     "dh_predict_from2dhough": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, C.POINTER(dh_result)]),

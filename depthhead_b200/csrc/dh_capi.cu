@@ -364,6 +364,37 @@ int dh_predict_tracks_mask_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* bl
                               mask_loc);
     });
 }
+
+// Pose and Hough image from one traversal: the argument rules of the pose call and of the 2-D call
+int dh_predict_frames_hough(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                            const dh_frame_args* args, dh_result* out, int blur, uint16_t* hough, int hough_loc, dh_result* from2d) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_frames_hough: bad depth_loc");
+        REQUIRE(hough_loc == DH_DEPTH_HOST || hough_loc == DH_DEPTH_DEVICE, "dh_predict_frames_hough: bad hough_loc");
+        REQUIRE(blur == 0 || blur == 1, "dh_predict_frames_hough: blur must be 0 or 1");
+        REQUIRE(hough || from2d, "dh_predict_frames_hough: hough and from2d are both NULL");
+        REQUIRE(blur || !from2d, "dh_predict_frames_hough: from2d needs blur = 1 (the arg-max of the blurred image)");
+        if (args) check_frame_args("dh_predict_frames_hough", args, n);
+        REQUIRE(n == 0 || out, "dh_predict_frames_hough: NULL out");
+        REQUIRE(c && f && (n == 0 || (depth && args)), "dh_predict_frames_hough: NULL argument");
+        c->cx->predict_frames_hough(*f->hf, depth, nullptr, nullptr, n, w, h, depth_loc, args, out, blur != 0, hough, hough_loc, from2d);
+    });
+}
+int dh_predict_frames_hough_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n, uint32_t w,
+                                 uint32_t h, const dh_frame_args* args, dh_result* out, int blur, uint16_t* hough, int hough_loc,
+                                 dh_result* from2d) {
+    return guarded([&] {
+        REQUIRE(hough_loc == DH_DEPTH_HOST || hough_loc == DH_DEPTH_DEVICE, "dh_predict_frames_hough_biwi: bad hough_loc");
+        REQUIRE(blur == 0 || blur == 1, "dh_predict_frames_hough_biwi: blur must be 0 or 1");
+        REQUIRE(hough || from2d, "dh_predict_frames_hough_biwi: hough and from2d are both NULL");
+        REQUIRE(blur || !from2d, "dh_predict_frames_hough_biwi: from2d needs blur = 1 (the arg-max of the blurred image)");
+        if (args) check_frame_args("dh_predict_frames_hough_biwi", args, n);
+        if (offsets) check_offsets("dh_predict_frames_hough_biwi", offsets, n);
+        REQUIRE(n == 0 || out, "dh_predict_frames_hough_biwi: NULL out");
+        REQUIRE(c && f && (n == 0 || (blob && offsets && args)), "dh_predict_frames_hough_biwi: NULL argument");
+        c->cx->predict_frames_hough(*f->hf, nullptr, blob, offsets, n, w, h, DH_DEPTH_HOST, args, out, blur != 0, hough, hough_loc, from2d);
+    });
+}
 size_t dh_biwi_encode_bound(uint32_t w, uint32_t h) { return dh::rle_frame_bound(w, h); }
 int dh_biwi_encode_depth(const uint16_t* frames, uint32_t n, uint32_t w, uint32_t h, uint32_t threads, uint8_t* blob, size_t cap,
                          uint64_t* offsets, size_t* needed) {

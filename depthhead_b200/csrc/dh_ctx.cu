@@ -137,6 +137,7 @@ Context::~Context() {
     if (h_fs_) cudaFreeHost(h_fs_);
     if (h_counters_) cudaFreeHost(h_counters_);
     if (h_results_) cudaFreeHost(h_results_);
+    if (h_from2d_) cudaFreeHost(h_from2d_);
     if (h_result1_) cudaFreeHost(h_result1_);
     if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
     if (h_frame_k_) cudaFreeHost(h_frame_k_);
@@ -370,6 +371,7 @@ void Context::free_lane(Lane& L) {
     dev_free(L.img32);
     dev_free(L.img16);
     dev_free(L.img_keys);
+    dev_free(L.img_results);
     L.img_px = 0;
     dev_free(L.mask_plane);
     L.mask_px = 0;
@@ -854,6 +856,23 @@ void Context::predict_frames(const HostForest& hf, const uint16_t* depth, const 
     run_batch(hf, depth, blob, offsets, n, w, h, n ? args[0].K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
 }
 
+// dh_predict_frames_hough / _biwi: the poses of predict_frames, and what hough_image_frames computes with
+// K[i] = args[i].K, from the leaf words of the same traversal (run_pose_hough).  Chunks, lanes and image
+// scratch are those of the 2-D calls (image_chunk_cap), so that scratch stays bounded per lane.
+void Context::predict_frames_hough(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                                   uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out, bool blur,
+                                   uint16_t* hough, int hough_loc, dh_result* from2d) {
+    static const float kIdentity[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+    BackEnd be;
+    be.results = out;
+    be.args = args;
+    be.hough.blur = blur;
+    be.hough.image = hough;
+    be.hough.image_on_device = hough_loc == DH_DEPTH_DEVICE;
+    be.hough.from2d = from2d;
+    run_batch(hf, depth, blob, offsets, n, w, h, n ? args[0].K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
+}
+
 void check_biwi_offsets(const uint64_t* offsets, uint32_t n) {
     for (uint32_t i = 0; i < n; ++i) {
         if (offsets[i + 1] < offsets[i]) throw ModelError(DH_E_ARG, "Biwi offsets are not monotone at frame " + std::to_string(i));
@@ -971,17 +990,17 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     // Biwi input: the run-length expansion is latency-bound (one thread per frame walks the run
     // headers), so its chunks are larger: more frames in flight per launch
     uint32_t want_chunk = (blob && !chunk_frames_) ? std::min<uint32_t>(512u, n) : pick_chunk(n, depth_loc);
-    if (be.kind != BackEnd::kPose) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
+    if (be.image_scratch()) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
     const int n_lanes = timing_ ? 1 : (int)std::max<uint32_t>(1u, std::min<uint32_t>((uint32_t)max_lanes_, (n + want_chunk - 1) / want_chunk));
     ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
-    if (be.kind != BackEnd::kPose) ensure_image_scratch(n_lanes);
+    if (be.image_scratch()) ensure_image_scratch(n_lanes);
     if (be.kind == BackEnd::kPose && be.image && !be.image_on_device) ensure_mask_plane(n_lanes);
-    if (be.kind == BackEnd::kBlurred) ensure_blur_taps(hf);
+    if (be.kind == BackEnd::kBlurred || be.hough.blur) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
-    ensure_results(n);  // pinned staging for the results
+    ensure_results(n, be.hough.from2d != nullptr);  // pinned staging for the results
     if (be.args) ensure_frame_args(n);
     if (depth_loc != DH_DEPTH_DEVICE) ensure_staging(2);
     if (blob) ensure_biwi(offsets, n, F, 2);
@@ -1050,14 +1069,22 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     end_call();
     if (blob) check_biwi_status(n);
     if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
+    if (be.hough.from2d) std::memcpy(be.hough.from2d, h_from2d_, sizeof(dh_result) * n);
 }
 
-void Context::ensure_results(uint32_t n) {
+void Context::ensure_results(uint32_t n, bool from2d) {
     if (h_results_cap_ < n) {
         if (h_results_) cudaFreeHost(h_results_);
         h_results_ = nullptr;
         DH_CUDA(cudaHostAlloc((void**)&h_results_, sizeof(dh_result) * n, cudaHostAllocDefault));
         h_results_cap_ = n;
+    }
+    if (from2d && h_from2d_cap_ < n) {
+        if (h_from2d_) cudaFreeHost(h_from2d_);
+        h_from2d_ = nullptr;
+        h_from2d_cap_ = 0;
+        DH_CUDA(cudaHostAlloc((void**)&h_from2d_, sizeof(dh_result) * n, cudaHostAllocDefault));
+        h_from2d_cap_ = n;
     }
 }
 
@@ -1149,17 +1176,17 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     // the split adapts to how dense the frames are and how many cores the caller gave the workers.
     const bool hybrid = env_flag("DH_HOST_HYBRID", true) && !timing_ && max_lanes_ >= 2;
     uint32_t want_chunk = pick_chunk(n, DH_DEPTH_HOST);
-    if (be.kind != BackEnd::kPose) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
+    if (be.image_scratch()) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
     const int n_lanes = hybrid ? 2 : 1;
     ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
-    if (be.kind != BackEnd::kPose) ensure_image_scratch(n_lanes);
+    if (be.image_scratch()) ensure_image_scratch(n_lanes);
     if (be.kind == BackEnd::kPose && be.image && !be.image_on_device) ensure_mask_plane(n_lanes);
-    if (be.kind == BackEnd::kBlurred) ensure_blur_taps(hf);
+    if (be.kind == BackEnd::kBlurred || be.hough.blur) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
-    ensure_results(n);
+    ensure_results(n, be.hough.from2d != nullptr);
     if (be.args) ensure_frame_args(n);
     ensure_staging(hybrid ? 4 : 2);
     ensure_encode(n, F);
@@ -1350,6 +1377,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
             if (h_status_[i]) throw ModelError(DH_E_STATE, "internal error: frame " + std::to_string(i) + " did not survive the compressed host->device path");
     }
     if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
+    if (be.hough.from2d) std::memcpy(be.hough.from2d, h_from2d_, sizeof(dh_result) * n);
 }
 
 // ------------------------------------------------------------------------------------------------ tracks and seeded sequences
@@ -1805,7 +1833,7 @@ void Context::hough_image_frames(const HostForest& hf, const uint16_t* depth, co
     run_batch(hf, depth, blob, offsets, n, w, h, n ? K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
 }
 
-// u32 sums + two u16 planes per frame of a chunk, and the arg-max keys, on every lane of the call
+// u32 sums + two u16 planes per frame of a chunk, the arg-max keys and their poses, on every lane of the call
 void Context::ensure_image_scratch(int n_lanes) {
     const size_t frame_px = (size_t)sk_.w * sk_.h, need = (size_t)call_chunk_ * frame_px;
     for (int i = 0; i < std::max(1, std::min(n_lanes, kMaxLanes)); ++i) {
@@ -1815,10 +1843,12 @@ void Context::ensure_image_scratch(int n_lanes) {
         dev_free(L.img32);
         dev_free(L.img16);
         dev_free(L.img_keys);
+        dev_free(L.img_results);
         L.img_px = 0;
         dev_alloc(L.img32, need);
         dev_alloc(L.img16, 2 * need);
         dev_alloc(L.img_keys, (size_t)call_chunk_);
+        dev_alloc(L.img_results, (size_t)call_chunk_);
         L.img_px = need;
     }
 }
@@ -1849,8 +1879,59 @@ void Context::run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
         return;
     }
     if (be.image) run_pose_mask(L, b, f0, n, be);
+    if (be.hough.wanted()) run_pose_hough(L, b, f0, n, be.hough);
     run_back(L, b, n, iterations, be.args ? L.frame_k : nullptr);
     DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
+    if (be.hough.from2d) DH_CUDA(cudaMemcpyAsync(h_from2d_ + f0, L.img_results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
+}
+
+// The Hough image of a pose chunk, between its traversal and its patch gate as run_pose_mask: run_hough
+// as the 2-D calls run it (it reads the leaf words, the depth and the frames' K, none of which the pose
+// back end writes), without their counters launch (run_back counts every frame once).  Its from2d poses
+// go to the lane's img_results, since L.results is the pose back end's.  Device-bound images are written
+// in place; a host-bound image leaves through the lane's one deferred copy: the poses of both kinds go
+// to pinned memory with copies issued in stream order, so the image is the only deferred copy of the chunk.
+void Context::run_pose_hough(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd::Hough& hb) {
+    mark(DH_STAGE_VOTE);  // booked as the 2-D calls book their back end
+    uint16_t* image = run_hough(L, b, f0, n, hb.blur, hb.image, hb.image_on_device, hb.from2d ? L.img_results : nullptr, L.frame_k);
+    stage_check("2-D back end");
+    if (image && !hb.image_on_device) {
+        const size_t frame_px = (size_t)geom_.w * geom_.h;
+        L.pending_dst = hb.image + (size_t)f0 * frame_px;
+        L.pending_src = image;
+        L.pending_bytes = frame_px * n * sizeof(uint16_t);
+    }
+}
+
+// The Hough image of a chunk (frames f0 .. f0 + n - 1 of the batch) from the leaf words of its traversal:
+// the votes, then the raw image or its blur; with poses != nullptr the blurred image's arg-max and its pose
+// (predict_parameter_from2dhough) to poses [n] on the device.  The image goes to image + f0 frames when it
+// is on the device, else to the lane's second u16 plane.  Returns where the chunk's image is (nullptr:
+// image is nullptr, blurred from2d only).
+uint16_t* Context::run_hough(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, bool blur, uint16_t* image, bool image_on_device,
+                             dh_result* poses, const float* frame_k) {
+    const Geometry& g = geom_;
+    cudaStream_t st = L.stream;
+    const size_t frame_px = (size_t)g.w * g.h, px = frame_px * n;
+    uint16_t* out = image ? (image_on_device ? image + (size_t)f0 * frame_px : L.img16 + L.img_px) : nullptr;
+    DH_CUDA(cudaMemsetAsync(L.img32, 0, px * sizeof(uint32_t), st));
+    if (g.P) {
+        launch_hough_votes(b, g, fdev_, n, L.img32, st, frame_k);
+        launches_ += 1;
+    }
+    if (!blur) {
+        launch_narrow_u16(L.img32, out, px, st);
+        launches_ += 1;
+        return out;
+    }
+    if (poses) DH_CUDA(cudaMemsetAsync(L.img_keys, 0, sizeof(unsigned long long) * n, st));
+    launches_ += (uint64_t)launch_gaussian_blur(L.img32, L.img16, out, poses ? L.img_keys : nullptr, g.w, g.h, n, d_blur_taps_,
+                                                blur_radius_, st);
+    if (poses) {
+        launch_hough2d_pose(L.img_keys, b.depth, g, n, poses, st, frame_k);
+        launches_ += 1;
+    }
+    return out;
 }
 
 // The masks of a pose chunk, between its traversal and its patch gate (nothing after the traversal
@@ -1898,14 +1979,12 @@ void Context::run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
     cudaStream_t st = L.stream;
     const size_t frame_px = (size_t)g.w * g.h, px = frame_px * n;
     const float* frame_k = be.args ? L.frame_k : nullptr;  // masks project nothing
-    uint16_t* plane0 = L.img16;
-    uint16_t* plane1 = L.img16 + L.img_px;
     mark(DH_STAGE_VOTE);  // the whole 2-D back end is booked here
     void* image = nullptr;  // this chunk's image in device memory
     size_t elem = sizeof(uint16_t);
     if (be.kind == BackEnd::kMask) {
         elem = 1;
-        uint8_t* mask = be.image_on_device ? static_cast<uint8_t*>(be.image) + (size_t)f0 * frame_px : reinterpret_cast<uint8_t*>(plane1);
+        uint8_t* mask = be.image_on_device ? static_cast<uint8_t*>(be.image) + (size_t)f0 * frame_px : reinterpret_cast<uint8_t*>(L.img16 + L.img_px);
         DH_CUDA(cudaMemsetAsync(mask, 0, px, st));
         if (g.P) {
             launch_mask(b, g, fdev_, n, mask, st);
@@ -1913,24 +1992,8 @@ void Context::run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
         }
         image = mask;
     } else {
-        DH_CUDA(cudaMemsetAsync(L.img32, 0, px * sizeof(uint32_t), st));
-        if (g.P) {
-            launch_hough_votes(b, g, fdev_, n, L.img32, st, frame_k);
-            launches_ += 1;
-        }
-        if (be.image) image = be.image_on_device ? static_cast<uint16_t*>(be.image) + (size_t)f0 * frame_px : plane1;
-        if (be.kind == BackEnd::kVotes) {
-            launch_narrow_u16(L.img32, static_cast<uint16_t*>(image), px, st);
-            launches_ += 1;
-        } else {
-            if (be.results) DH_CUDA(cudaMemsetAsync(L.img_keys, 0, sizeof(unsigned long long) * n, st));
-            launches_ += (uint64_t)launch_gaussian_blur(L.img32, plane0, static_cast<uint16_t*>(image), be.results ? L.img_keys : nullptr,
-                                                        g.w, g.h, n, d_blur_taps_, blur_radius_, st);
-            if (be.results) {
-                launch_hough2d_pose(L.img_keys, b.depth, g, n, L.results, st, frame_k);
-                launches_ += 1;
-            }
-        }
+        image = run_hough(L, b, f0, n, be.kind == BackEnd::kBlurred, static_cast<uint16_t*>(be.image), be.image_on_device,
+                          be.results ? L.results : nullptr, frame_k);
     }
     stage_check("2-D back end");
     mark(DH_STAGE_D2H);

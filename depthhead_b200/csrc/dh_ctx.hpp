@@ -40,6 +40,7 @@ struct Lane {
     uint32_t* img32 = nullptr;      // [F][h][w] u32 vote sums
     uint16_t* img16 = nullptr;      // [2][F][h][w] horizontal blur, then the image handed out (mask: u8 in the second plane)
     unsigned long long* img_keys = nullptr;  // [F] arg-max keys of the from2d pass
+    dh_result* img_results = nullptr;        // [F] from2d poses of a pose pass (dh_predict_frames_hough; L.results holds its poses)
     size_t img_px = 0;              // F * h * w the image scratch holds
     // pose back end with host-bound masks (dh_predict_frames_mask): the u8 masks of a chunk, allocated by the first such call
     uint8_t* mask_plane = nullptr;  // [F][h][w]
@@ -68,6 +69,17 @@ struct BackEnd {
     void* image = nullptr;         // kMask: u8 [n][h][w]; kVotes / kBlurred: u16 [n][h][w] (kBlurred: may be nullptr);
                                    // kPose: u8 head masks [n][h][w] from the pose pass's own leaf words, or nullptr
     bool image_on_device = false;  // image points to device memory on the context's GPU
+    // kPose (dh_predict_frames_hough): the Hough image of the same frames from the pose pass's own leaf
+    // words, with the frames' own K; asked for iff image or from2d is set.  Never together with a mask.
+    struct Hough {
+        bool blur = false;              // build_hough_image, or the vote image before its blur
+        uint16_t* image = nullptr;      // u16 [n][h][w], or nullptr (blurred: from2d only)
+        bool image_on_device = false;
+        dh_result* from2d = nullptr;    // predict_parameter_from2dhough [n] (host memory; needs blur), or nullptr
+        bool wanted() const { return image || from2d; }
+    } hough;
+    // image back ends, and the pose back end with a Hough image, keep image scratch and cap their chunks by it
+    bool image_scratch() const { return kind != kPose || hough.wanted(); }
 };
 // Image back ends keep a u32 accumulator and two u16 planes per frame of a chunk (8 bytes per
 // pixel, 2.4 MB per VGA frame): their chunks hold at most this much image scratch per lane.
@@ -127,6 +139,11 @@ public:
     void predict_frames(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
                         uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out, uint8_t* mask = nullptr,
                         int mask_loc = DH_DEPTH_HOST);
+    // the same poses, and every frame's Hough image (blur: build_hough_image, else the raw votes) to
+    // [n][h][w] u16 at hough_loc and / or its predict_parameter_from2dhough to from2d [n] (dh_predict_frames_hough)
+    void predict_frames_hough(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                              uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out, bool blur,
+                              uint16_t* hough, int hough_loc, dh_result* from2d);
     // training: split scoring (dh_train.cu; houghforest.rs:250-295)
     TrainSet* trainset_create(const uint16_t* patches, uint64_t n, uint32_t sw, uint32_t sh, uint32_t rw, uint32_t rh,
                               const uint8_t* is_object, const float* offsets, const double* rotations);
@@ -182,7 +199,7 @@ private:
     void ensure_encode(uint32_t n, uint32_t F);
     void run_batch_encoded(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, const float K[9],
                            const BackEnd& be);
-    void ensure_results(uint32_t n);
+    void ensure_results(uint32_t n, bool from2d = false);
     void ensure_frame_args(uint32_t n);
     void ensure_image_scratch(int n_lanes);
     void ensure_mask_plane(int n_lanes);
@@ -190,8 +207,13 @@ private:
     // after run_front: the chunk's back end and the copies of its results (frames f0 .. f0 + n - 1 of the batch)
     void run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be);
     void run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be);
+    // the Hough image of a chunk (kVotes / kBlurred, and the pose back end's Hough destination)
+    uint16_t* run_hough(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, bool blur, uint16_t* image, bool image_on_device,
+                        dh_result* poses, const float* frame_k);
     // kPose with a mask destination: the chunk's masks from the leaf words its traversal left
     void run_pose_mask(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be);
+    // kPose with a Hough destination: the chunk's Hough image and from2d poses from the same leaf words
+    void run_pose_hough(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd::Hough& hb);
     void flush_pending(Lane& L);
     void free_scratch();
     TilePlan plan_tiles(const Geometry& g) const;
@@ -285,6 +307,8 @@ private:
     unsigned long long* h_counters_ = nullptr;
     dh_result* h_results_ = nullptr;      // batch results (grows with the batch; never referenced by a captured graph)
     size_t h_results_cap_ = 0;
+    dh_result* h_from2d_ = nullptr;       // from2d poses of dh_predict_frames_hough, beside the poses in h_results_ (grows likewise)
+    size_t h_from2d_cap_ = 0;
     dh_result* h_result1_ = nullptr;      // dh_predict's own fixed slot: the D2H copy node of its CUDA graph targets it
     // dh_predict_frames: every frame's FrameState (seeds) and K, K^-1, packed per chunk (grows with the batch)
     FrameState* h_frame_fs_ = nullptr;

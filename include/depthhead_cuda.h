@@ -33,6 +33,8 @@
  *                                                                                 dh_predict_frames_mask_biwi,
  *                                                                                 dh_predict_tracks_mask,
  *                                                                                 dh_predict_tracks_mask_biwi
+ *   examples/db_prediction.rs:140,154: pose and from2d of one Biwi frame        -> dh_predict_frames_hough,
+ *                                                                                 dh_predict_frames_hough_biwi
  *   src/db_reader/biwi.rs:27-60       read_cal (depth.cal -> IntrinsicMatrix)   -> dh_biwi_parse_cal
  *   src/db_reader/biwi.rs:63-77       read_gt (ground-truth pose file)          -> dh_biwi_parse_pose
  *   src/hough/houghforest.rs:250-295  HoughTreeFunctions::impurity (training)   -> dh_train_score_level
@@ -305,6 +307,42 @@ int dh_predict_tracks_mask_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* bl
                                 const uint64_t* seq_off, uint32_t w, uint32_t h, const dh_frame_args* seq_args, float min_seed_z,
                                 dh_result* out, uint8_t* mask, int mask_loc);
 
+/* Pose AND 2-D Hough result of the same frames from one traversal: what examples/db_prediction.rs:140,154
+ * asks of every Biwi frame (predict_parameter, then predict_parameter_from2dhough, with the K of the
+ * frame's folder).  The copy or decode of a frame, its box-sum image and its forest walk run once; the
+ * Hough image is built from the leaf words the pose pass found.  Arguments as dh_predict_frames /
+ * dh_predict_frames_biwi, plus those of dh_build_hough_image_frames with K[i] = args[i].K:
+ *   blur:     1 build_hough_image, 0 the vote image before its blur;
+ *   hough:    [n][h][w] u16 at hough_loc (DH_DEPTH_HOST or DH_DEPTH_DEVICE), or NULL.  Every pixel is
+ *             written, whatever the buffer held before;
+ *   from2d:   n results (host memory) of predict_parameter_from2dhough, or NULL.  The 2-D calls take no
+ *             seeds: the seeds of args act on out only.
+ * Contract:
+ *   - out equals, byte for byte over the whole dh_result array, dh_predict_frames / _frames_biwi with
+ *     the same arguments, at every chunk size;
+ *   - hough and from2d equal, byte for byte, dh_build_hough_image_frames / _biwi with K[i] = args[i].K
+ *     and the same blur;
+ *   - argument rules are those of both calls: with any frame to process a NULL out is DH_E_ARG, and so
+ *     are hough and from2d both NULL, from2d with blur = 0, blur other than 0 or 1, and a depth_loc or
+ *     hough_loc that is neither DH_DEPTH_HOST nor DH_DEPTH_DEVICE.  These checks happen before any
+ *     device work.  A caller who wants only one of the outputs has the existing calls;
+ *   - a damaged Biwi file gives the pose call's error: DH_E_ARG naming the lowest bad frame;
+ *   - n = 0 is a successful no-op;
+ *   - chunks are those of the 2-D calls: at most 256 MB / (8 w h + 8) frames (109 VGA frames), below
+ *     the chunk setting;
+ *   - counters [0]-[8], [10], [11] and dh_ctx_transfer_info equal the pose call's at the same chunks;
+ *     [9] (launches) is the pose call's at the same chunks plus, per chunk, the 2-D back end: 1 vote
+ *     launch (none for frames that hold no patch) + 1 narrowing (blur = 0) or 2 blur passes (blur = 1)
+ *     + 1 arg-max pose launch with from2d; no second front end and no second counters launch.  With
+ *     stage timing on, the 2-D back end is booked under DH_STAGE_VOTE.
+ * Synchronous. */
+int dh_predict_frames_hough(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                            int depth_loc, const dh_frame_args* args, dh_result* out,
+                            int blur, uint16_t* hough, int hough_loc, dh_result* from2d);
+int dh_predict_frames_hough_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
+                                 uint32_t w, uint32_t h, const dh_frame_args* args, dh_result* out,
+                                 int blur, uint16_t* hough, int hough_loc, dh_result* from2d);
+
 /* The writer for that format (the reference only reads it): n raw frames [n][h][w] u16 become n
  * files in ONE blob, file i at [offsets[i], offsets[i+1]) (offsets: n+1 entries, multiples of 16).
  * Runs are found at a granularity of 16 pixels: a group of 16 pixels with any non-zero pixel is
@@ -397,7 +435,8 @@ int dh_forest_to_json(const dh_forest* f, char* buf, size_t cap, size_t* needed)
  * TRAVERSE and D2H mean the same, and their whole back end (mask or vote image, blur, arg-max) is
  * booked under DH_STAGE_VOTE; GATE and MEANSHIFT stay 0.  The pose-and-mask calls
  * (dh_predict_frames_mask*, dh_predict_tracks_mask*) book their mask launch under DH_STAGE_VOTE too,
- * beside the seeds and cubes of the pose. */
+ * beside the seeds and cubes of the pose, and so do the pose-and-Hough calls (dh_predict_frames_hough*)
+ * their whole 2-D back end. */
 #define DH_STAGE_H2D 0
 #define DH_STAGE_SAT 1
 #define DH_STAGE_TRAVERSE 2
