@@ -25,6 +25,10 @@ import numpy as np
 
 from . import capi
 
+# predict_frames_heads: the votes a coarse cell needs to seed a further head.  Measured on the forest that
+# dh_train_learn grows from one-person synthetic frames (DESIGN.md §7 "Several heads per frame").
+DEFAULT_MIN_CELL_VOTES = 22000
+
 
 class IntrinsicMatrix:
     """types.rs:405-446.  Row-major 3x3 f32; the inverse is computed inside the library with the
@@ -478,6 +482,26 @@ class HoughPrediction:
         capi.check(capi.load().dh_predict_frames_hough(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(out), int(bool(blur)),
                                                        ip, iloc, capi.ptr(res)))
         return out, images, res
+
+    def predict_frames_heads(self, frames, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
+                             max_heads: int = 4, radius_mm: float = 150.0, min_cell_votes: int | None = None,
+                             ctx: Context | None = None, device_ptr: int | None = None, n: int | None = None, w: int | None = None,
+                             h: int | None = None):
+        """Up to max_heads heads of every frame (dh_predict_frames_heads, DESIGN.md §7): (capi.HEAD_DTYPE
+        [n, max_heads] in acceptance order, unused slots zero; uint32 [n] heads found, >= 1).  Head 0 is
+        predict_frames' result.  min_cell_votes None = DEFAULT_MIN_CELL_VOTES."""
+        _keep, p, loc, n, w, h = _as_frames(frames, device_ptr, n, w, h)
+        args = frame_args(n, intrinsics, midp_guess, rot_guess, has_midp, has_rot)
+        params = np.zeros(1, capi.HEADS_PARAMS_DTYPE)
+        params["max_heads"] = max_heads
+        params["min_cell_votes"] = DEFAULT_MIN_CELL_VOTES if min_cell_votes is None else min_cell_votes
+        params["radius_mm"] = radius_mm
+        ctx = ctx or default_context()
+        out = np.zeros((n, max(int(max_heads), 0)), capi.HEAD_DTYPE)
+        n_heads = np.zeros(n, np.uint32)
+        capi.check(capi.load().dh_predict_frames_heads(ctx._h, self._h, p, n, w, h, loc, capi.ptr(args), capi.ptr(params),
+                                                       capi.ptr(out), capi.ptr(n_heads)))
+        return out, n_heads
 
     def predict_tracks_with_mask(self, frames, lengths, intrinsics, midp_guess=None, rot_guess=None, has_midp=None, has_rot=None,
                                  min_seed_z: float = 500.0, ctx: Context | None = None, device_ptr: int | None = None,

@@ -43,6 +43,15 @@ FRAME_ARGS_DTYPE = np.dtype([("K", np.float32, 9), ("midp_guess", np.float32, 3)
 assert FRAME_ARGS_DTYPE.itemsize == 80
 
 
+# dh_heads_params / dh_head: dh_predict_frames_heads (16 and 72 bytes)
+HEADS_PARAMS_DTYPE = np.dtype([("max_heads", np.uint32), ("min_cell_votes", np.uint32), ("radius_mm", np.float32),
+                               ("_pad", np.uint32)], align=True)
+assert HEADS_PARAMS_DTYPE.itemsize == 16
+HEAD_DTYPE = np.dtype([("pose", RESULT_DTYPE), ("support", np.uint64), ("n_patches", np.uint32), ("seed_cell", np.uint32)],
+                      align=True)
+assert HEAD_DTYPE.itemsize == 72
+
+
 class dh_split_stats(C.Structure):
     _fields_ = [("n", C.c_uint32 * 2), ("n_pos", C.c_uint32 * 2), ("det_off", C.c_double * 2), ("det_rot", C.c_double * 2),
                 ("impurity", C.c_double)]
@@ -122,6 +131,7 @@ SIGNATURES = {
     "dh_predict_frames_mask_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp, _vp, C.c_int]),
     "dh_predict_tracks_mask": (C.c_int, [_vp, _vp, _vp, _u32, _vp, _u32, _u32, C.c_int, _vp, _f32, _vp, _vp, C.c_int]),
     "dh_predict_tracks_mask_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _vp, _u32, _u32, _vp, _f32, _vp, _vp, C.c_int]),
+    "dh_predict_frames_heads": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, C.c_int, _vp, _vp, _vp, _vp]),
     "dh_predict_frames_hough": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _u32, C.c_int, _vp, _vp, C.c_int, _vp, C.c_int, _vp]),
     "dh_predict_frames_hough_biwi": (C.c_int, [_vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp, C.c_int, _vp, C.c_int, _vp]),
     "dh_hough_image_raw": (C.c_int, [_vp, _vp, _vp, _u32, _u32, _vp, _vp]),

@@ -57,6 +57,15 @@ static_assert(sizeof(dh_frame_args) == 80 && offsetof(dh_frame_args, K) == 0 && 
                   offsetof(dh_frame_args, _pad) == 76,
               "dh_frame_args layout (mirrored by capi.FRAME_ARGS_DTYPE and the Rust shim)");
 
+static_assert(sizeof(dh_heads_params) == 16 && offsetof(dh_heads_params, max_heads) == 0 &&
+                  offsetof(dh_heads_params, min_cell_votes) == 4 && offsetof(dh_heads_params, radius_mm) == 8 &&
+                  offsetof(dh_heads_params, _pad) == 12,
+              "dh_heads_params layout (mirrored by capi.HEADS_PARAMS_DTYPE)");
+static_assert(sizeof(dh_head) == 72 && offsetof(dh_head, pose) == 0 && offsetof(dh_head, support) == 56 &&
+                  offsetof(dh_head, n_patches) == 64 && offsetof(dh_head, seed_cell) == 68,
+              "dh_head layout (mirrored by capi.HEAD_DTYPE)");
+static_assert(dh::kMaxHeads == 8, "dh_heads_params.max_heads allows 1..8");
+
 void check_frame_args(const char* fn, const dh_frame_args* args, uint32_t n, const char* what = "frame") {
     for (uint32_t i = 0; i < n; ++i)
         if (args[i].has_guess & ~3u)
@@ -393,6 +402,21 @@ int dh_predict_frames_hough_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* b
         REQUIRE(n == 0 || out, "dh_predict_frames_hough_biwi: NULL out");
         REQUIRE(c && f && (n == 0 || (blob && offsets && args)), "dh_predict_frames_hough_biwi: NULL argument");
         c->cx->predict_frames_hough(*f->hf, nullptr, blob, offsets, n, w, h, DH_DEPTH_HOST, args, out, blur != 0, hough, hough_loc, from2d);
+    });
+}
+int dh_predict_frames_heads(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                            const dh_frame_args* args, const dh_heads_params* params, dh_head* out, uint32_t* n_heads) {
+    return guarded([&] {
+        REQUIRE(depth_loc == DH_DEPTH_HOST || depth_loc == DH_DEPTH_DEVICE, "dh_predict_frames_heads: bad depth_loc");
+        REQUIRE(params, "dh_predict_frames_heads: NULL params");
+        REQUIRE(params->max_heads >= 1 && params->max_heads <= dh::kMaxHeads,
+                "dh_predict_frames_heads: max_heads must be 1..8, got " + std::to_string(params->max_heads));
+        REQUIRE(params->radius_mm > 0.0f, "dh_predict_frames_heads: radius_mm must be > 0 (and not NaN)");
+        REQUIRE(params->min_cell_votes >= 1, "dh_predict_frames_heads: min_cell_votes must be >= 1");
+        if (args) check_frame_args("dh_predict_frames_heads", args, n);
+        REQUIRE(n == 0 || (out && n_heads), "dh_predict_frames_heads: NULL out or n_heads");
+        REQUIRE(c && f && (n == 0 || (depth && args)), "dh_predict_frames_heads: NULL argument");
+        c->cx->predict_frames_heads(*f->hf, depth, n, w, h, depth_loc, args, *params, out, n_heads);
     });
 }
 size_t dh_biwi_encode_bound(uint32_t w, uint32_t h) { return dh::rle_frame_bound(w, h); }

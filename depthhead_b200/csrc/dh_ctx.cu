@@ -138,6 +138,8 @@ Context::~Context() {
     if (h_counters_) cudaFreeHost(h_counters_);
     if (h_results_) cudaFreeHost(h_results_);
     if (h_from2d_) cudaFreeHost(h_from2d_);
+    if (h_heads_) cudaFreeHost(h_heads_);
+    if (h_n_heads_) cudaFreeHost(h_n_heads_);
     if (h_result1_) cudaFreeHost(h_result1_);
     if (h_frame_fs_) cudaFreeHost(h_frame_fs_);
     if (h_frame_k_) cudaFreeHost(h_frame_k_);
@@ -375,6 +377,15 @@ void Context::free_lane(Lane& L) {
     L.img_px = 0;
     dev_free(L.mask_plane);
     L.mask_px = 0;
+    dev_free(L.heads_st);
+    dev_free(L.heads_grid);
+    dev_free(L.heads_fs);
+    dev_free(L.heads_res);
+    dev_free(L.heads_gated);
+    dev_free(L.heads_cubes);
+    dev_free(L.heads_out);
+    dev_free(L.heads_n);
+    L.heads_frames = 0;
     L.pending_bytes = 0;
     L.allocated = false;
     L.cubes_clean = false;
@@ -491,7 +502,8 @@ uint32_t Context::pick_chunk(uint32_t n_frames, int depth_loc) const {
     return std::max<uint32_t>(1u, std::min<uint32_t>(c, std::max<uint32_t>(n_frames, 1u)));
 }
 
-void Context::ensure_scratch(const HostForest& hf, uint32_t w, uint32_t h, uint32_t n_frames_hint, const float K[9], int n_lanes) {
+void Context::ensure_scratch(const HostForest& hf, uint32_t w, uint32_t h, uint32_t n_frames_hint, const float K[9], int n_lanes,
+                             bool heads) {
     const uint32_t sw = hf.subimage_width, sh = hf.subimage_height, stride = hf.stepwidth.load();
     if (stride == 0) throw ModelError(DH_E_SHAPE, "stepwidth 0: the reference's sliding window never advances");
     if (w < sw || h < sh)
@@ -505,7 +517,8 @@ void Context::ensure_scratch(const HostForest& hf, uint32_t w, uint32_t h, uint3
         const uint64_t npx = (w - sw + stride - 1) / stride, npy = (h - sh + stride - 1) / stride;
         const uint64_t PT = std::max<uint64_t>(npx * npy, 1) * (uint64_t)hf.n_trees;
         const uint64_t per_frame = (uint64_t)(h + 1) * ((w + 4) & ~3ull) * 4 + PT * 4 + npx * npy * 29 +
-                                   (uint64_t)w * h * 4 + 2ull * vote_box_cells() * 4 + 40000;
+                                   (uint64_t)w * h * 4 + 2ull * vote_box_cells() * 4 + 40000 +
+                                   (heads ? 2ull * vote_box_cells() * 4 + npx * npy * 16 + 4000 : 0ull);
         const uint64_t budget = 12ull << 30;
         cap = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(cap, budget / per_frame));
     }
@@ -600,6 +613,7 @@ FrameBuffers Context::buffers(const Lane& L, const uint16_t* depth) const {
     b.leaf_mask = leaf_codes_ ? kLeafIdMask : 0x7fffffffu;
     b.debug = debug_ ? 1u : 0u;
     b.clear_cubes = debug_ ? 0u : 1u;  // debug passes export the cubes after the call
+    b.support = 0;
     return b;
 }
 
@@ -873,6 +887,18 @@ void Context::predict_frames_hough(const HostForest& hf, const uint16_t* depth, 
     run_batch(hf, depth, blob, offsets, n, w, h, n ? args[0].K : kIdentity, blob ? DH_DEPTH_HOST : depth_loc, be);
 }
 
+// dh_predict_frames_heads: the pose pipeline of predict_frames, then the extra heads of every chunk (run_heads)
+void Context::predict_frames_heads(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                                   const dh_frame_args* args, const dh_heads_params& params, dh_head* out, uint32_t* n_heads) {
+    static const float kIdentity[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+    BackEnd be;
+    be.args = args;
+    be.heads = &params;
+    be.heads_out = out;
+    be.n_heads = n_heads;
+    run_batch(hf, depth, nullptr, nullptr, n, w, h, n ? args[0].K : kIdentity, depth_loc, be);
+}
+
 void check_biwi_offsets(const uint64_t* offsets, uint32_t n) {
     for (uint32_t i = 0; i < n; ++i) {
         if (offsets[i + 1] < offsets[i]) throw ModelError(DH_E_ARG, "Biwi offsets are not monotone at frame " + std::to_string(i));
@@ -992,15 +1018,17 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     uint32_t want_chunk = (blob && !chunk_frames_) ? std::min<uint32_t>(512u, n) : pick_chunk(n, depth_loc);
     if (be.image_scratch()) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
     const int n_lanes = timing_ ? 1 : (int)std::max<uint32_t>(1u, std::min<uint32_t>((uint32_t)max_lanes_, (n + want_chunk - 1) / want_chunk));
-    ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
+    ensure_scratch(hf, w, h, want_chunk, K, n_lanes, be.heads != nullptr);
     if (be.image_scratch()) ensure_image_scratch(n_lanes);
+    if (be.heads) ensure_heads_scratch(n_lanes);
     if (be.kind == BackEnd::kPose && be.image && !be.image_on_device) ensure_mask_plane(n_lanes);
     if (be.kind == BackEnd::kBlurred || be.hough.blur) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
     const uint32_t F = call_chunk_;
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
-    ensure_results(n, be.hough.from2d != nullptr);  // pinned staging for the results
+    ensure_results(n, be.hough.from2d != nullptr);
+    if (be.heads) ensure_heads_results(n, be.heads->max_heads);  // pinned staging for the results
     if (be.args) ensure_frame_args(n);
     if (depth_loc != DH_DEPTH_DEVICE) ensure_staging(2);
     if (blob) ensure_biwi(offsets, n, F, 2);
@@ -1070,6 +1098,10 @@ void Context::run_batch(const HostForest& hf, const uint16_t* depth, const uint8
     if (blob) check_biwi_status(n);
     if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
     if (be.hough.from2d) std::memcpy(be.hough.from2d, h_from2d_, sizeof(dh_result) * n);
+    if (be.heads) {
+        std::memcpy(be.heads_out, h_heads_, sizeof(dh_head) * n * be.heads->max_heads);
+        std::memcpy(be.n_heads, h_n_heads_, sizeof(uint32_t) * n);
+    }
 }
 
 void Context::ensure_results(uint32_t n, bool from2d) {
@@ -1178,8 +1210,9 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     uint32_t want_chunk = pick_chunk(n, DH_DEPTH_HOST);
     if (be.image_scratch()) want_chunk = std::min(want_chunk, image_chunk_cap(w, h));
     const int n_lanes = hybrid ? 2 : 1;
-    ensure_scratch(hf, w, h, want_chunk, K, n_lanes);
+    ensure_scratch(hf, w, h, want_chunk, K, n_lanes, be.heads != nullptr);
     if (be.image_scratch()) ensure_image_scratch(n_lanes);
+    if (be.heads) ensure_heads_scratch(n_lanes);
     if (be.kind == BackEnd::kPose && be.image && !be.image_on_device) ensure_mask_plane(n_lanes);
     if (be.kind == BackEnd::kBlurred || be.hough.blur) ensure_blur_taps(hf);
     const uint32_t iterations = hf.meanshift_iterations.load();
@@ -1187,6 +1220,7 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     const uint32_t n_chunks = (n + F - 1) / F;
     const size_t frame_px = (size_t)w * h;
     ensure_results(n, be.hough.from2d != nullptr);
+    if (be.heads) ensure_heads_results(n, be.heads->max_heads);
     if (be.args) ensure_frame_args(n);
     ensure_staging(hybrid ? 4 : 2);
     ensure_encode(n, F);
@@ -1378,6 +1412,10 @@ void Context::run_batch_encoded(const HostForest& hf, const uint16_t* depth, uin
     }
     if (be.results) std::memcpy(be.results, h_results_, sizeof(dh_result) * n);
     if (be.hough.from2d) std::memcpy(be.hough.from2d, h_from2d_, sizeof(dh_result) * n);
+    if (be.heads) {
+        std::memcpy(be.heads_out, h_heads_, sizeof(dh_head) * n * be.heads->max_heads);
+        std::memcpy(be.n_heads, h_n_heads_, sizeof(uint32_t) * n);
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ tracks and seeded sequences
@@ -1880,9 +1918,97 @@ void Context::run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32
     }
     if (be.image) run_pose_mask(L, b, f0, n, be);
     if (be.hough.wanted()) run_pose_hough(L, b, f0, n, be.hough);
-    run_back(L, b, n, iterations, be.args ? L.frame_k : nullptr);
+    if (be.heads) {
+        FrameBuffers bs = b;
+        bs.support = 1;  // head 0's support
+        run_back(L, bs, n, iterations, L.frame_k);
+        run_heads(L, bs, f0, n, iterations, be);
+    } else {
+        run_back(L, b, n, iterations, be.args ? L.frame_k : nullptr);
+    }
     DH_CUDA(cudaMemcpyAsync(h_results_ + f0, L.results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
     if (be.hough.from2d) DH_CUDA(cudaMemcpyAsync(h_from2d_ + f0, L.img_results, sizeof(dh_result) * n, cudaMemcpyDeviceToHost, L.stream));
+}
+
+// Extra heads of a pose chunk after its back end: round 0 writes head 0 (the chunk's results, the support of
+// their centre windows) and starts every frame's search, rounds 1 .. 2 (max_heads - 1) serve one try of every
+// frame still searching (launch_heads_round).  The launches do not wait for the GPU: frames that stopped
+// leave each kernel at once.
+void Context::run_heads(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be) {
+    const dh_heads_params& p = *be.heads;
+    cudaStream_t st = L.stream;
+    mark(DH_STAGE_MEANSHIFT);
+    HeadsBuffers hb{};
+    hb.st = L.heads_st;
+    hb.grid = L.heads_grid;
+    hb.fs = L.heads_fs;
+    hb.res = L.heads_res;
+    hb.gated = L.heads_gated;
+    hb.cubes = L.heads_cubes;
+    hb.out = L.heads_out;
+    hb.n_heads = L.heads_n;
+    hb.max_heads = p.max_heads;
+    hb.min_cell_votes = p.min_cell_votes;
+    hb.radius = p.radius_mm;
+    DH_CUDA(cudaMemsetAsync(L.heads_out, 0, sizeof(dh_head) * (size_t)n * p.max_heads, st));
+    DH_CUDA(cudaMemsetAsync(L.heads_fs, 0, sizeof(FrameState) * n, st));
+    const uint32_t rounds = 2u * (p.max_heads - 1u);
+    for (uint32_t r = 0; r <= rounds; ++r) {
+        launches_ += (uint64_t)launch_heads_round(b, hb, geom_, fdev_, n, r, iterations, n_sms_, L.frame_k, st);
+        stage_check("extra heads");
+    }
+    mark(DH_STAGE_D2H);
+    DH_CUDA(cudaMemcpyAsync(h_heads_ + (size_t)f0 * p.max_heads, L.heads_out, sizeof(dh_head) * (size_t)n * p.max_heads,
+                            cudaMemcpyDeviceToHost, st));
+    DH_CUDA(cudaMemcpyAsync(h_n_heads_ + f0, L.heads_n, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st));
+    DH_CUDA(cudaGetLastError());
+}
+
+void Context::ensure_heads_scratch(int n_lanes) {
+    const uint32_t F = sk_.frames;
+    const size_t P = std::max<uint32_t>(geom_.P, 1u);
+    for (int i = 0; i < std::max(1, std::min(n_lanes, kMaxLanes)); ++i) {
+        Lane& L = lanes_[i];
+        if (L.heads_frames >= F) continue;
+        DH_CUDA(cudaStreamSynchronize(stream_));
+        dev_free(L.heads_st);
+        dev_free(L.heads_grid);
+        dev_free(L.heads_fs);
+        dev_free(L.heads_res);
+        dev_free(L.heads_gated);
+        dev_free(L.heads_cubes);
+        dev_free(L.heads_out);
+        dev_free(L.heads_n);
+        L.heads_frames = 0;
+        dev_alloc(L.heads_st, F);
+        dev_alloc(L.heads_grid, (size_t)F * kPosGridCells);
+        dev_alloc(L.heads_fs, F);
+        dev_alloc(L.heads_res, F);
+        dev_alloc(L.heads_gated, (size_t)F * P);
+        dev_alloc(L.heads_cubes, (size_t)F * 2 * vote_box_cells());
+        DH_CUDA(cudaMemset(L.heads_cubes, 0, sizeof(uint32_t) * (size_t)F * 2 * vote_box_cells()));
+        dev_alloc(L.heads_out, (size_t)F * kMaxHeads);
+        dev_alloc(L.heads_n, F);
+        L.heads_frames = F;
+    }
+}
+
+void Context::ensure_heads_results(uint32_t n, uint32_t max_heads) {
+    const size_t need = (size_t)n * max_heads;
+    if (h_heads_cap_ < need) {
+        if (h_heads_) cudaFreeHost(h_heads_);
+        h_heads_ = nullptr;
+        h_heads_cap_ = 0;
+        DH_CUDA(cudaHostAlloc((void**)&h_heads_, sizeof(dh_head) * need, cudaHostAllocDefault));
+        h_heads_cap_ = need;
+    }
+    if (h_n_heads_cap_ < n) {
+        if (h_n_heads_) cudaFreeHost(h_n_heads_);
+        h_n_heads_ = nullptr;
+        h_n_heads_cap_ = 0;
+        DH_CUDA(cudaHostAlloc((void**)&h_n_heads_, sizeof(uint32_t) * n, cudaHostAllocDefault));
+        h_n_heads_cap_ = n;
+    }
 }
 
 // The Hough image of a pose chunk, between its traversal and its patch gate as run_pose_mask: run_hough

@@ -45,6 +45,16 @@ struct Lane {
     // pose back end with host-bound masks (dh_predict_frames_mask): the u8 masks of a chunk, allocated by the first such call
     uint8_t* mask_plane = nullptr;  // [F][h][w]
     size_t mask_px = 0;             // F * h * w it holds
+    // dh_predict_frames_heads: the tries of extra heads (HeadsBuffers), allocated by the first such call
+    HeadsState* heads_st = nullptr;   // [F]
+    uint32_t* heads_grid = nullptr;   // [F][400]
+    FrameState* heads_fs = nullptr;   // [F]
+    dh_result* heads_res = nullptr;   // [F]
+    float4* heads_gated = nullptr;    // [F][P]
+    uint32_t* heads_cubes = nullptr;  // [F][2][kBox^3], zero between tries
+    dh_head* heads_out = nullptr;     // [F][kMaxHeads]
+    uint32_t* heads_n = nullptr;      // [F]
+    uint32_t heads_frames = 0;        // F the above hold
     // a host-bound image copy of this lane's last chunk, issued before the lane's next chunk (a copy
     // to pageable memory blocks the host: deferred, it overlaps the other lane's kernels)
     void* pending_dst = nullptr;
@@ -80,6 +90,10 @@ struct BackEnd {
     } hough;
     // image back ends, and the pose back end with a Hough image, keep image scratch and cap their chunks by it
     bool image_scratch() const { return kind != kPose || hough.wanted(); }
+    // kPose (dh_predict_frames_heads): the extra heads of every frame after its pose (run_heads), or nullptr
+    const dh_heads_params* heads = nullptr;
+    dh_head* heads_out = nullptr;   // [n][max_heads] (host memory)
+    uint32_t* n_heads = nullptr;    // [n] (host memory)
 };
 // Image back ends keep a u32 accumulator and two u16 planes per frame of a chunk (8 bytes per
 // pixel, 2.4 MB per VGA frame): their chunks hold at most this much image scratch per lane.
@@ -144,6 +158,9 @@ public:
     void predict_frames_hough(const HostForest& hf, const uint16_t* depth, const uint8_t* blob, const uint64_t* offsets, uint32_t n,
                               uint32_t w, uint32_t h, int depth_loc, const dh_frame_args* args, dh_result* out, bool blur,
                               uint16_t* hough, int hough_loc, dh_result* from2d);
+    // up to params.max_heads heads of every frame (dh_predict_frames_heads): out [n][max_heads], n_heads [n] (host)
+    void predict_frames_heads(const HostForest& hf, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h, int depth_loc,
+                              const dh_frame_args* args, const dh_heads_params& params, dh_head* out, uint32_t* n_heads);
     // training: split scoring (dh_train.cu; houghforest.rs:250-295)
     TrainSet* trainset_create(const uint16_t* patches, uint64_t n, uint32_t sw, uint32_t sh, uint32_t rw, uint32_t rh,
                               const uint8_t* is_object, const float* offsets, const double* rotations);
@@ -186,7 +203,9 @@ public:
 private:
     void ensure_forest(const HostForest& hf);
     void free_forest();
-    void ensure_scratch(const HostForest& hf, uint32_t w, uint32_t h, uint32_t n_frames_hint, const float K[9], int n_lanes = 1);
+    // heads: the frames also keep the scratch of extra heads (ensure_heads_scratch), counted in the per-frame budget
+    void ensure_scratch(const HostForest& hf, uint32_t w, uint32_t h, uint32_t n_frames_hint, const float K[9], int n_lanes = 1,
+                        bool heads = false);
     void alloc_lane(Lane& L);
     void free_lane(Lane& L);
     void ensure_staging(int slots);
@@ -204,6 +223,10 @@ private:
     void ensure_image_scratch(int n_lanes);
     void ensure_mask_plane(int n_lanes);
     void ensure_blur_taps(const HostForest& hf);
+    void ensure_heads_scratch(int n_lanes);
+    void ensure_heads_results(uint32_t n, uint32_t max_heads);
+    // kPose with extra heads: the rounds of launch_heads_round after the chunk's back end, and the copies of its heads
+    void run_heads(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be);
     // after run_front: the chunk's back end and the copies of its results (frames f0 .. f0 + n - 1 of the batch)
     void run_chunk_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, uint32_t iterations, const BackEnd& be);
     void run_image_back(Lane& L, const FrameBuffers& b, uint32_t f0, uint32_t n, const BackEnd& be);
@@ -309,6 +332,9 @@ private:
     size_t h_results_cap_ = 0;
     dh_result* h_from2d_ = nullptr;       // from2d poses of dh_predict_frames_hough, beside the poses in h_results_ (grows likewise)
     size_t h_from2d_cap_ = 0;
+    dh_head* h_heads_ = nullptr;          // heads of dh_predict_frames_heads [n][max_heads] (grows likewise)
+    uint32_t* h_n_heads_ = nullptr;       // [n]
+    size_t h_heads_cap_ = 0, h_n_heads_cap_ = 0;
     dh_result* h_result1_ = nullptr;      // dh_predict's own fixed slot: the D2H copy node of its CUDA graph targets it
     // dh_predict_frames: every frame's FrameState (seeds) and K, K^-1, packed per chunk (grows with the batch)
     FrameState* h_frame_fs_ = nullptr;

@@ -1284,13 +1284,53 @@ __device__ Best block_argmax(const uint32_t* cells, int n, Best* s_red) {
     return r;
 }
 
+// Centre seed of coarse cell `cell` (prediction.rs:706-729, 750): z = mean of the non-zero depth in
+// the cell's pixels, the cell centre back-projected with kinv, truncated.  Whole CTA of kSeedThreads.
+__device__ __forceinline__ void cell_seed(const Geometry& g, const uint16_t* img, uint32_t cell, const float* kinv,
+                                          unsigned long long* s_sum, uint32_t* s_cnt, int32_t sm[3]) {
+    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    const uint32_t gpw = g.w / kGuessGridParts, gph = g.h / kGuessGridParts;
+    const uint32_t cgx = cell % kGuessGridParts, cgy = cell / kGuessGridParts;
+    unsigned long long zs = 0;
+    uint32_t zc = 0;
+    for (uint32_t i = tid; i < gpw * gph; i += kSeedThreads) {
+        const uint32_t v = img[(size_t)(gph * cgy + i / gpw) * g.w + gpw * cgx + i % gpw];
+        if (v > 0) {
+            zs += v;
+            zc += 1;
+        }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+        zs += __shfl_xor_sync(0xffffffffu, zs, d);
+        zc += __shfl_xor_sync(0xffffffffu, zc, d);
+    }
+    if (lane == 0) {
+        s_sum[warp] = zs;
+        s_cnt[warp] = zc;
+    }
+    __syncthreads();
+    zs = 0;
+    zc = 0;
+    for (int i = 0; i < kSeedThreads / 32; ++i) {
+        zs += s_sum[i];
+        zc += s_cnt[i];
+    }
+    const float meanz = zc > 0 ? (float)__ddiv_rn((double)zs, (double)zc) : 0.0f;
+    const float mxf = __fmul_rn(__fadd_rn((float)cgx, 0.5f), (float)gpw);  // :727-729
+    const float myf = __fmul_rn(__fadd_rn((float)cgy, 0.5f), (float)gph);
+    float m3[3];
+    img_to_space(kinv, mxf, myf, meanz, m3);
+    for (int k = 0; k < 3; ++k) sm[k] = __float2int_rz(m3[k]);  // :750
+}
+
 template <bool kFrameK>
 __global__ void __launch_bounds__(kSeedThreads) seed_kernel(FrameBuffers b, Geometry g, uint32_t iterations,
                                                             const float* __restrict__ frame_k) {
     __shared__ Best s_red[kSeedThreads / 32];
     __shared__ unsigned long long s_sum[kSeedThreads / 32];
     __shared__ uint32_t s_cnt[kSeedThreads / 32];
-    const uint32_t frame = blockIdx.x, tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    const uint32_t frame = blockIdx.x, tid = threadIdx.x;
     FrameState* fs = b.fs + frame;
     const uint32_t* grid = b.grids + (size_t)frame * (kPosGridCells + kRotGridCells);
     const uint32_t guessed = fs->has_guess;
@@ -1299,42 +1339,9 @@ __global__ void __launch_bounds__(kSeedThreads) seed_kernel(FrameBuffers b, Geom
     int32_t sm[3];
     {
         const Best bp = block_argmax(grid, kPosGridCells, s_red);
-        // z = mean of the non-zero depth in the winning grid part (prediction.rs:706-725)
-        const uint32_t gpw = g.w / kGuessGridParts, gph = g.h / kGuessGridParts;
-        const uint32_t cgx = bp.idx % kGuessGridParts, cgy = bp.idx / kGuessGridParts;
-        unsigned long long zs = 0;
-        uint32_t zc = 0;
-        const uint16_t* img = b.depth + (size_t)frame * g.h * g.w;
-        for (uint32_t i = tid; i < gpw * gph; i += kSeedThreads) {
-            const uint32_t v = img[(size_t)(gph * cgy + i / gpw) * g.w + gpw * cgx + i % gpw];
-            if (v > 0) {
-                zs += v;
-                zc += 1;
-            }
-        }
-#pragma unroll
-        for (int d = 16; d > 0; d >>= 1) {
-            zs += __shfl_xor_sync(0xffffffffu, zs, d);
-            zc += __shfl_xor_sync(0xffffffffu, zc, d);
-        }
-        if (lane == 0) {
-            s_sum[warp] = zs;
-            s_cnt[warp] = zc;
-        }
-        __syncthreads();
-        zs = 0;
-        zc = 0;
-        for (int i = 0; i < kSeedThreads / 32; ++i) {
-            zs += s_sum[i];
-            zc += s_cnt[i];
-        }
-        const float meanz = zc > 0 ? (float)__ddiv_rn((double)zs, (double)zc) : 0.0f;
-        const float mxf = __fmul_rn(__fadd_rn((float)cgx, 0.5f), (float)gpw);  // :727-729
-        const float myf = __fmul_rn(__fadd_rn((float)cgy, 0.5f), (float)gph);
-        float m3[3], kinv[9];
+        float kinv[9];
         if (kFrameK) load_mat3(frame_k + (size_t)frame * kFrameKFloats + 9, kinv);
-        img_to_space(kFrameK ? kinv : g.Kinv, mxf, myf, meanz, m3);
-        for (int k = 0; k < 3; ++k) sm[k] = __float2int_rz(m3[k]);  // :750
+        cell_seed(g, b.depth + (size_t)frame * g.h * g.w, bp.idx, kFrameK ? kinv : g.Kinv, s_sum, s_cnt, sm);
         if (guessed & 1u)  // prediction.rs:437-441
             for (int k = 0; k < 3; ++k) sm[k] = __float2int_rz(fs->midp_guess[k]);
     }
@@ -1467,15 +1474,17 @@ __device__ __forceinline__ void accumulate_pairs(const float4* __restrict__ gate
 }
 
 constexpr int kBuildThreads = 256;
+// kWhich: bit0 centre cube, bit1 rotation cube (3: the pose pass; 1 or 2: the tries of extra heads)
+template <uint32_t kWhich>
 __global__ void __launch_bounds__(kBuildThreads) box_build_kernel(FrameBuffers b, Geometry g, ForestDev f) {
     const uint32_t frame = blockIdx.y;
     const FrameState* fs = b.fs + frame;
-    if (!fs->box_valid[0]) return;  // meanshift_iterations == 0: the accumulators are never read
+    if (!fs->box_valid[kWhich == 2u ? 1 : 0]) return;  // meanshift_iterations == 0: the accumulators are never read
     const int32_t org_c[3] = {fs->box_org[0][0], fs->box_org[0][1], fs->box_org[0][2]};
     const int32_t org_r[3] = {fs->box_org[1][0], fs->box_org[1][1], fs->box_org[1][2]};
     uint32_t* cube_c = b.cubes + (size_t)(2u * frame) * kBoxCells;
     accumulate_pairs(b.gated + (size_t)frame * g.P, fs->n_gate, g.n_trees, b.leaf + (size_t)frame * g.n_trees * g.P, b.leaf_mask, g.P,
-                     blockIdx.x * (kBuildThreads / 32) + (threadIdx.x >> 5), gridDim.x * (kBuildThreads / 32), f, 3u, org_c,
+                     blockIdx.x * (kBuildThreads / 32) + (threadIdx.x >> 5), gridDim.x * (kBuildThreads / 32), f, kWhich, org_c,
                      cube_c, org_r, cube_c + kBoxCells);
 }
 
@@ -1536,8 +1545,10 @@ __device__ __noinline__ void rebuild_cube(const float4* __restrict__ gated, uint
 // the ranking, the non-zero ones are written as (cell, value) at their rank, and the summands are then
 // computed densely, one thread per non-zero cell (walking all 250 chunks of 32 cells with only the
 // non-zero lanes working took 53 % of the kernel's instructions, measured).
+// which_only: 2 = both accumulators of every frame (item = 2 * frame + which); 0 or 1 = that accumulator of
+// every frame (item = frame), and only of frames whose FrameState::active has its bit (tries of extra heads).
 __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b, Geometry g, ForestDev f, uint32_t iterations,
-                                                                  uint32_t n_items) {
+                                                                  uint32_t n_items, uint32_t which_only) {
     extern __shared__ __align__(16) uint8_t ms_smem[];
     uint2* s_list = reinterpret_cast<uint2*>(ms_smem);       // [kMsSegment] (ord, value) of the non-zero cells by rank
     float(*s_terms)[kMsSegment] = reinterpret_cast<float(*)[kMsSegment]>(ms_smem + kMsSegment * 8);  // [4][kMsSegment]
@@ -1549,6 +1560,7 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
     __shared__ int32_t s_pos[3], s_org[3];
     __shared__ uint32_t s_flags, s_done;
     __shared__ uint32_t s_item;
+    __shared__ unsigned long long s_sup[kMsWarps];
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
     // cube offsets of this thread's window cells ord = j * kMsThreads + tid, two per word, computed
     // once and parked in shared memory (eight registers less across the rounds)
@@ -1567,9 +1579,17 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
     // one by their index, the following ones as they become free (a launch of one CTA per accumulator ran
     // 2.3 rounds of CTAs and paid for three).
     for (uint32_t item = blockIdx.x; item < n_items;) {
-    const uint32_t frame = item >> 1, which = item & 1u;
+    const uint32_t frame = which_only < 2u ? item : item >> 1, which = which_only < 2u ? which_only : item & 1u;
     FrameState* fs = b.fs + frame;
-    uint32_t* box = b.cubes + (size_t)item * kBoxCells;
+    uint32_t* box = b.cubes + (size_t)(2u * frame + which) * kBoxCells;
+    if (which_only < 2u && !((fs->active >> which) & 1u)) {  // this frame's search has stopped, or its try was dropped
+        if (tid == 0) s_item = gridDim.x + atomicAdd(&b.fs[0].work_next, 1u);
+        __syncthreads();
+        item = s_item;
+        __syncthreads();
+        continue;
+    }
+    const bool built = fs->box_valid[which] != 0u;  // box_build_kernel filled the cube around box_org
     if (tid == 0) {
         s_flags = 0;
         s_done = 0;
@@ -1735,6 +1755,45 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
         }
     }
     __syncthreads();
+    if (b.support && which == 0u) {
+        // the u32 cells of the final window: the cube holds them unless the last update (or the cycle stop) left it
+        const int32_t pos[3] = {s_pos[0], s_pos[1], s_pos[2]};
+        int32_t org[3] = {s_org[0], s_org[1], s_org[2]};
+        bool inside = built;
+        for (int k = 0; k < 3; ++k) {
+            const long long lo = (long long)pos[k] - 10 - org[k], hi = (long long)pos[k] + 9 - org[k];
+            if (lo < 0 || hi >= kBox) inside = false;
+        }
+        if (!inside) {
+            ++rebuilds;
+            __syncthreads();
+            for (int k = 0; k < 3; ++k) org[k] = (int32_t)((uint32_t)pos[k] - (uint32_t)(kBox / 2));
+            if (tid == 0)
+                for (int k = 0; k < 3; ++k) s_org[k] = org[k];
+            rebuild_cube(b.gated + (size_t)frame * g.P, fs->n_gate, g.n_trees, b.leaf + (size_t)frame * g.n_trees * g.P, b.leaf_mask, g.P,
+                         f.leaf_info, f.leaf_box, f.offsets, f.rot_bins, which, org[0], org[1], org[2], box);
+        }
+        const uint32_t base = ((uint32_t)((long long)pos[0] - 10 - org[0]) * kBox + (uint32_t)((long long)pos[1] - 10 - org[1])) * kBox +
+                              (uint32_t)((long long)pos[2] - 10 - org[2]);
+        unsigned long long sum = 0;
+#pragma unroll
+        for (int j = 0; j < kMsLoads; j += 2) {
+            const uint32_t pk = s_offp[(j >> 1) * kMsThreads + tid];
+            const uint32_t o0 = pk & 0xffffu, o1 = pk >> 16;
+            if (o0 != kMsNoCell) sum += __ldcg(box + base + o0);
+            if (o1 != kMsNoCell) sum += __ldcg(box + base + o1);
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
+        if (lane == 0) s_sup[warp] = sum;
+        __syncthreads();
+        if (tid == 0) {
+            unsigned long long t = 0;
+            for (int i = 0; i < kMsWarps; ++i) t += s_sup[i];
+            fs->support = t;
+        }
+        __syncthreads();
+    }
     if (b.clear_cubes) {
         // leave the cube empty for the next pass over this scratch: 128 KB of stores that overlap the
         // other CTAs' rounds instead of one memset of every cube in front of the vote stage
@@ -1754,6 +1813,225 @@ __global__ void __launch_bounds__(kMsThreads, 3) meanshift_kernel(FrameBuffers b
     item = s_item;
     __syncthreads();
     }
+}
+
+// ================================================================ K4d: extra heads (dh_predict_frames_heads)
+// Rules: DESIGN.md §7 "Several heads per frame"; oracle: orc_predict_heads.  One CTA per frame for the
+// seed and patch kernels; the cubes and mean-shift of a try are box_build_kernel and meanshift_kernel on the
+// try's buffers (HeadsBuffers), one accumulator of each frame per launch.
+constexpr int kHeadsThreads = kSeedThreads;
+
+// the try's centre as integers: the mean-shift position that store_result wrote as floats (exact below 2^24)
+__device__ __forceinline__ void centre_of(const dh_result& r, int32_t c[3]) {
+    for (int k = 0; k < 3; ++k) c[k] = (int32_t)r.mid_point[k];
+}
+
+// Try `round` >= 1: suppress the previous try in the working grid, then seed this one from its first maximum.
+__global__ void __launch_bounds__(kHeadsThreads) heads_seed_kernel(FrameBuffers b, HeadsBuffers hb, Geometry g, uint32_t round,
+                                                                  uint32_t iterations, const float* __restrict__ frame_k) {
+    __shared__ uint32_t s_grid[kPosGridCells];
+    __shared__ Best s_red[kHeadsThreads / 32];
+    __shared__ unsigned long long s_sum[kHeadsThreads / 32];
+    __shared__ uint32_t s_cnt[kHeadsThreads / 32];
+    __shared__ float s_uvr[3];
+    const uint32_t frame = blockIdx.x, tid = threadIdx.x;
+    HeadsState* st = hb.st + frame;
+    FrameState* fs = hb.fs + frame;
+    if (frame == 0 && tid == 0) hb.fs[0].work_next = 0;  // the centre mean-shift launch hands out its items afresh
+    if (!st->searching) {
+        if (tid == 0) {
+            fs->active = 0;
+            fs->box_valid[0] = fs->box_valid[1] = 0;
+        }
+        return;
+    }
+    const uint32_t* src = round == 1 ? b.grids + (size_t)frame * (kPosGridCells + kRotGridCells) : hb.grid + (size_t)frame * kPosGridCells;
+    for (int i = tid; i < kPosGridCells; i += kHeadsThreads) s_grid[i] = src[i];
+    const float* Kf = frame_k + (size_t)frame * kFrameKFloats;
+    if (tid == 0) {
+        // the previous try's centre in the image: space_to_img clamped like coarse_pos_cell, and R in pixels at its depth
+        const dh_result& prev = round == 1 ? b.results[frame] : hb.res[frame];
+        float K[9], p2[2];
+        load_mat3(Kf, K);
+        const float p3[3] = {prev.mid_point[0], prev.mid_point[1], prev.mid_point[2]};
+        space_to_img(K, p3, p2);
+        const float mx = (p2[0] > 0.0f) ? p2[0] : 0.0f, my = (p2[1] > 0.0f) ? p2[1] : 0.0f;
+        s_uvr[0] = (mx < (float)(g.w - 1)) ? mx : (float)(g.w - 1);
+        s_uvr[1] = (my < (float)(g.h - 1)) ? my : (float)(g.h - 1);
+        const float z = p3[2];
+        s_uvr[2] = z > 0.0f ? __fdiv_rn(__fmul_rn(hb.radius, K[0]), z) : 0.0f;
+    }
+    __syncthreads();
+    {
+        const float u = s_uvr[0], v = s_uvr[1], r = s_uvr[2], rr = __fmul_rn(r, r);
+        const uint32_t gpw = g.w / kGuessGridParts, gph = g.h / kGuessGridParts;
+        for (int i = tid; i < kPosGridCells; i += kHeadsThreads) {
+            const uint32_t gx = (uint32_t)i % kGuessGridParts, gy = (uint32_t)i / kGuessGridParts;
+            // nearest point of the closed cell rectangle, squared distance without fused operations
+            const float nx = fminf(fmaxf(u, (float)(gx * gpw)), (float)((gx + 1) * gpw));
+            const float ny = fminf(fmaxf(v, (float)(gy * gph)), (float)((gy + 1) * gph));
+            const float dx = __fsub_rn(u, nx), dy = __fsub_rn(v, ny);
+            if (__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)) <= rr) s_grid[i] = 0;
+        }
+    }
+    __syncthreads();
+    if (tid == 0 && st->seed_cell < (uint32_t)kPosGridCells) s_grid[st->seed_cell] = 0;
+    __syncthreads();
+    const Best best = block_argmax(s_grid, kPosGridCells, s_red);  // first maximum, as the reference's arg-max
+    if (best.val < hb.min_cell_votes) {
+        if (tid == 0) {
+            st->searching = 0;
+            fs->active = 0;
+            fs->box_valid[0] = fs->box_valid[1] = 0;
+        }
+        return;
+    }
+    int32_t sm[3];
+    float kinv[9];
+    load_mat3(Kf + 9, kinv);
+    cell_seed(g, b.depth + (size_t)frame * g.h * g.w, best.idx, kinv, s_sum, s_cnt, sm);
+    for (int i = tid; i < kPosGridCells; i += kHeadsThreads) hb.grid[(size_t)frame * kPosGridCells + i] = s_grid[i];
+    if (tid == 0) {
+        st->seed_cell = best.idx;
+        for (int k = 0; k < 3; ++k) {
+            fs->seed_mid[k] = sm[k];
+            fs->box_org[0][k] = (int32_t)((uint32_t)sm[k] - (uint32_t)(kBox / 2));
+        }
+        fs->box_valid[0] = iterations > 0 ? 1u : 0u;
+        fs->box_valid[1] = 0;
+        fs->active = 1u;
+        fs->n_gate = b.fs[frame].n_gate;  // the centre cube (and its rebuilds) take every gated patch
+    }
+}
+
+// After the centre of try `round` (round 0: head 0, the pass's own result): the duplicate test, the gated
+// patches within R of the centre, and (round >= 1) their coarse rotation grid and the rotation seed.
+constexpr int kHeadsPatchSmem = kRotGridCells * 4;
+__global__ void __launch_bounds__(kHeadsThreads) heads_patch_kernel(FrameBuffers b, HeadsBuffers hb, Geometry g, ForestDev f,
+                                                                   uint32_t round, uint32_t iterations) {
+    extern __shared__ __align__(16) uint32_t s_rot[];  // [8000] coarse rotation grid of the kept patches
+    __shared__ Best s_red[kHeadsThreads / 32];
+    __shared__ uint32_t s_kept;
+    const uint32_t frame = blockIdx.x, tid = threadIdx.x, lane = tid & 31u;
+    HeadsState* st = hb.st + frame;
+    FrameState* fs = hb.fs + frame;
+    if (frame == 0 && tid == 0) hb.fs[0].work_next = 0;  // the rotation mean-shift launch hands out its items afresh
+    if (round > 0 && !(fs->active & 1u)) return;
+    const dh_result& r = round == 0 ? b.results[frame] : hb.res[frame];
+    int32_t c[3];
+    centre_of(r, c);
+    if (round > 0) {
+        // a centre within R of an accepted head is a duplicate: integer squared distance against floor(R)^2
+        const long long fr = (long long)floorf(hb.radius), lim = fr * fr;
+        bool dup = false;
+        for (uint32_t a = 0; a < st->n_acc; ++a) {
+            const long long dx = (long long)c[0] - st->centre[a][0], dy = (long long)c[1] - st->centre[a][1],
+                            dz = (long long)c[2] - st->centre[a][2];
+            if (dx * dx + dy * dy + dz * dz <= lim) dup = true;
+        }
+        if (dup) {
+            if (tid == 0) {
+                fs->active = 0;
+                fs->box_valid[1] = 0;
+            }
+            return;
+        }
+    }
+    if (tid == 0) s_kept = 0;
+    if (round > 0)
+        for (int i = tid; i < kRotGridCells; i += kHeadsThreads) s_rot[i] = 0;
+    __syncthreads();
+    // gated patches within R of the centre: f32 differences, ((dx^2 + dy^2) + dz^2) <= R^2 without fused operations
+    const float cx = r.mid_point[0], cy = r.mid_point[1], cz = r.mid_point[2], rr = __fmul_rn(hb.radius, hb.radius);
+    const uint32_t ngate = b.fs[frame].n_gate;
+    const float4* gated = b.gated + (size_t)frame * g.P;
+    float4* kept = hb.gated + (size_t)frame * g.P;
+    for (uint32_t i0 = 0; i0 < ngate; i0 += kHeadsThreads) {
+        const uint32_t i = i0 + tid;
+        bool in = false;
+        float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (i < ngate) {
+            p = gated[i];
+            const float dx = __fsub_rn(p.x, cx), dy = __fsub_rn(p.y, cy), dz = __fsub_rn(p.z, cz);
+            in = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)) <= rr;
+        }
+        const uint32_t m = __ballot_sync(0xffffffffu, in);
+        uint32_t base = 0;
+        if (lane == 0 && m) base = atomicAdd(&s_kept, (uint32_t)__popc(m));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (in && round > 0) kept[base + __popc(m & ((1u << lane) - 1u))] = p;
+    }
+    __syncthreads();
+    const uint32_t nkept = s_kept;
+    if (round == 0) {
+        // head 0: the pass's result, its support and seed cell; the search starts from it
+        uint32_t cell = 0xffffffffu;
+        if (!(b.fs[frame].has_guess & 1u)) cell = block_argmax(b.grids + (size_t)frame * (kPosGridCells + kRotGridCells), kPosGridCells, s_red).idx;
+        if (tid == 0) {
+            dh_head h;
+            h.pose = r;
+            h.support = b.fs[frame].support;
+            h.n_patches = nkept;
+            h.seed_cell = cell;
+            hb.out[(size_t)frame * hb.max_heads] = h;
+            hb.n_heads[frame] = 1;
+            for (int k = 0; k < 3; ++k) st->centre[0][k] = c[k];
+            st->n_acc = 1;
+            st->searching = hb.max_heads > 1u ? 1u : 0u;
+            st->seed_cell = cell;
+            st->n_patches = nkept;
+        }
+        return;
+    }
+    // the kept patches' rotation votes into the coarse grid: the leaves' static cell lists (leaf_gate_kernel)
+    const uint32_t T = g.n_trees;
+    const int32_t* leaf_f = b.leaf + (size_t)frame * T * g.P;
+    for (uint32_t i = tid; i < nkept * T; i += kHeadsThreads) {
+        const uint32_t t = i / nkept;
+        const float4 p = kept[i - t * nkept];
+        const int32_t L = (int32_t)((uint32_t)leaf_f[(size_t)t * g.P + __float_as_uint(p.w)] & b.leaf_mask);
+        const LeafInfo li = f.leaf_info[L];
+        if ((li.flags & kLeafVotes) && (li.flags & kLeafRotOk)) {
+            const uint32_t n = li.flags >> kLeafRotCellsShift;
+            for (uint32_t j = 0; j < n; ++j) {
+                const uint32_t e = __ldg(f.rot_cells + li.vote_start + j);
+                atomicAdd(&s_rot[e & ((1u << kRotCellBits) - 1u)], li.valtoadd * (e >> kRotCellBits));
+            }
+        }
+    }
+    __syncthreads();
+    const Best br = block_argmax(s_rot, kRotGridCells, s_red);  // prediction.rs:733-742 on these patches
+    if (tid == 0) {
+        const uint32_t rc[3] = {br.idx % 20u, (br.idx % 400u) / 20u, br.idx / 400u};
+        for (int k = 0; k < 3; ++k) {
+            const double deg = __ddiv_rn(__dadd_rn(__dmul_rn((double)rc[k], 360.0), 180.0), (double)kGuessGridParts);
+            fs->seed_rot[k] = __double2int_rz(__ddiv_rn(__dmul_rn(deg, (double)kRotGridParts), 360.0));
+            fs->box_org[1][k] = (int32_t)((uint32_t)fs->seed_rot[k] - (uint32_t)(kBox / 2));
+        }
+        fs->box_valid[1] = iterations > 0 ? 1u : 0u;
+        fs->active = 2u;
+        fs->n_gate = nkept;  // the rotation cube (and its rebuilds) take the kept patches, in hb.gated
+        for (int k = 0; k < 3; ++k) st->centre[st->n_acc][k] = c[k];
+        st->n_patches = nkept;
+    }
+}
+
+// The accepted try of this round becomes the frame's next head.
+__global__ void __launch_bounds__(128) heads_commit_kernel(HeadsBuffers hb, uint32_t n) {
+    const uint32_t frame = blockIdx.x * blockDim.x + threadIdx.x;
+    if (frame >= n) return;
+    HeadsState* st = hb.st + frame;
+    const FrameState* fs = hb.fs + frame;
+    if (!(fs->active & 2u)) return;
+    dh_head h;
+    h.pose = hb.res[frame];
+    h.support = fs->support;
+    h.n_patches = st->n_patches;
+    h.seed_cell = st->seed_cell;
+    hb.out[(size_t)frame * hb.max_heads + st->n_acc] = h;
+    st->n_acc += 1;
+    hb.n_heads[frame] = st->n_acc;
+    if (st->n_acc >= hb.max_heads) st->searching = 0;
 }
 
 // float -> bfloat16 bit pattern, rounded towards -inf / +inf (exact for values a bfloat16 holds; inf stays inf)
@@ -2613,7 +2891,7 @@ int launch_seed_and_cubes(const FrameBuffers& b, const Geometry& g, const Forest
     const uint32_t per_frame =
         std::max<uint32_t>(1u, std::min<uint32_t>(64u, (g.P * g.n_trees / 8u + kBuildThreads - 1) / kBuildThreads));
     dim3 gr(per_frame, n_frames);
-    box_build_kernel<<<gr, kBuildThreads, 0, s>>>(b, g, f);
+    box_build_kernel<3u><<<gr, kBuildThreads, 0, s>>>(b, g, f);
     return 2;
 }
 
@@ -2625,8 +2903,52 @@ int launch_meanshift(const FrameBuffers& b, const Geometry& g, const ForestDev& 
     // persistent CTAs: three per SM (registers; measured 0.247 -> 0.239 ms against one CTA per accumulator)
     const uint32_t n_items = 2u * n_frames;
     const uint32_t grid = std::min<uint32_t>(n_items, 3u * (uint32_t)std::max(n_sms, 1));
-    meanshift_kernel<<<grid, kMsThreads, kMsSmemBytes, s>>>(b, g, f, iterations, n_items);
+    meanshift_kernel<<<grid, kMsThreads, kMsSmemBytes, s>>>(b, g, f, iterations, n_items, 2u);
     return 1;
+}
+
+int launch_heads_round(const FrameBuffers& b, const HeadsBuffers& hb, const Geometry& g, const ForestDev& f, uint32_t n_frames,
+                       uint32_t round, uint32_t iterations, int n_sms, const float* frame_k, cudaStream_t s) {
+    static SmemConfig configured;
+    if (configured.raise((uint32_t)kHeadsPatchSmem))
+        cudaFuncSetAttribute(heads_patch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHeadsPatchSmem);
+    if (round == 0) {
+        heads_patch_kernel<<<n_frames, kHeadsThreads, kHeadsPatchSmem, s>>>(b, hb, g, f, 0u, iterations);
+        return 1;
+    }
+    // the try's view of the pass: its own frame states, cubes and results; the gated patches of the centre
+    // cube are the pass's, those of the rotation cube the ones within R
+    FrameBuffers t = b;
+    t.fs = hb.fs;
+    t.cubes = hb.cubes;
+    t.results = hb.res;
+    t.ms_trace = nullptr;
+    t.clear_cubes = 1;
+    t.support = 1;
+    const uint32_t per_frame =
+        std::max<uint32_t>(1u, std::min<uint32_t>(64u, (g.P * g.n_trees / 8u + kBuildThreads - 1) / kBuildThreads));
+    const uint32_t grid = std::min<uint32_t>(n_frames, 3u * (uint32_t)std::max(n_sms, 1));
+    static SmemConfig ms_configured;
+    if (ms_configured.raise((uint32_t)kMsSmemBytes))
+        cudaFuncSetAttribute(meanshift_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMsSmemBytes);
+    int launches = 0;
+    heads_seed_kernel<<<n_frames, kHeadsThreads, 0, s>>>(b, hb, g, round, iterations, frame_k);
+    ++launches;
+    if (g.P && iterations) {
+        box_build_kernel<1u><<<dim3(per_frame, n_frames), kBuildThreads, 0, s>>>(t, g, f);
+        ++launches;
+    }
+    meanshift_kernel<<<grid, kMsThreads, kMsSmemBytes, s>>>(t, g, f, iterations, n_frames, 0u);
+    heads_patch_kernel<<<n_frames, kHeadsThreads, kHeadsPatchSmem, s>>>(b, hb, g, f, round, iterations);
+    launches += 2;
+    t.gated = hb.gated;
+    if (g.P && iterations) {
+        box_build_kernel<2u><<<dim3(per_frame, n_frames), kBuildThreads, 0, s>>>(t, g, f);
+        ++launches;
+    }
+    meanshift_kernel<<<grid, kMsThreads, kMsSmemBytes, s>>>(t, g, f, iterations, n_frames, 1u);
+    heads_commit_kernel<<<(n_frames + 127) / 128, 128, 0, s>>>(hb, n_frames);
+    return launches + 2;
 }
 
 void launch_leaf_gates(const double* leaf_prob, const uint32_t* vote_start, const uint32_t* n_votes,

@@ -31,7 +31,8 @@ struct alignas(16) FrameState {
     float midp_guess[3];
     double rot_guess[3];
     uint32_t work_next;       // frame 0's: accumulators handed out to the persistent mean-shift CTAs beyond the first round
-    uint32_t _pad[3];
+    uint32_t active;          // extra heads (launch_heads_round): bit w = accumulator w of this frame's try runs its mean-shift
+    unsigned long long support;  // FrameBuffers::support: u32 cells of the centre accumulator in the final 20^3 window
 };
 
 struct Geometry {
@@ -103,6 +104,7 @@ struct FrameBuffers {
     uint32_t debug;         // 1: compute the seed grids even when the caller supplied seeds
     uint32_t clear_cubes;   // 1: meanshift_kernel zeroes its accumulator cube when it is done with it (the next
                             // pass finds the cubes empty without a memset of all of them)
+    uint32_t support;       // 1: meanshift_kernel sums the final window of every centre accumulator into FrameState::support
 };
 
 // Leaf words: the walk stores ~child of the node it left; with probability codes in the uniform node
@@ -149,6 +151,34 @@ int launch_gaussian_blur(const uint32_t* in, uint16_t* tmp, uint16_t* out, unsig
                          uint32_t n_frames, const float* k, int radius, cudaStream_t s);
 void launch_hough2d_pose(const unsigned long long* keys, const uint16_t* depth, const Geometry& g, uint32_t n_frames, dh_result* out,
                          cudaStream_t s, const float* frame_k = nullptr);
+// dh_predict_frames_heads: the extra heads of a pose pass (DESIGN.md §7), in rounds after run_back.  Round 0
+// writes head 0 (the pass's own result) and starts the search; round k >= 1 serves try k of every frame that is
+// still searching: its seed from the working grid, centre cube and mean-shift, the patches within R of the
+// centre, their rotation grid, cube and mean-shift, and the head if it is accepted.
+constexpr uint32_t kMaxHeads = 8;
+struct HeadsState {
+    int32_t centre[kMaxHeads][3];  // accepted heads' centres (the mid_points as integers)
+    uint32_t n_acc;                // heads accepted so far
+    uint32_t searching;            // 0: no further try
+    uint32_t seed_cell;            // coarse cell of the current try, 0xffffffff for a caller seed
+    uint32_t n_patches;            // gated patches within R of the current try's centre
+};
+struct HeadsBuffers {
+    HeadsState* st;       // [F]
+    uint32_t* grid;       // [F][400] working copy of the frame's position grid
+    FrameState* fs;       // [F] seeds, cube origins, mean-shift state and support of the current try
+    dh_result* res;       // [F] pose of the current try
+    float4* gated;        // [F][P] gated patches within R of the current try's centre
+    uint32_t* cubes;      // [F][2][kBox^3] the try's accumulator cubes (left empty by the mean-shift CTAs)
+    dh_head* out;         // [F][max_heads]
+    uint32_t* n_heads;    // [F]
+    uint32_t max_heads, min_cell_votes;
+    float radius;         // R (mm)
+};
+// b: the pass's buffers (b.support set, so FrameState::support holds head 0's); frame_k as in launch_gate_coarse
+// (the heads call always has per-frame intrinsics).  Returns the launches made.
+int launch_heads_round(const FrameBuffers& b, const HeadsBuffers& hb, const Geometry& g, const ForestDev& f, uint32_t n_frames,
+                       uint32_t round, uint32_t iterations, int n_sms, const float* frame_k, cudaStream_t s);
 void launch_seq_guess(FrameState* fs, const dh_result* prev, uint32_t n, float min_seed_z, cudaStream_t s);
 
 // dh_predict_tracks: one slot of a pass (frame = global frame index, track = its track, prev = the

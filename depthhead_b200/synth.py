@@ -22,6 +22,41 @@ KINECT_K = np.array([[560.0, 0.0, 320.0], [0.0, 560.0, 240.0], [0.0, 0.0, 1.0]],
 
 
 # ----------------------------------------------------------------------------- frames
+def _draw_person(img, hx, hy, hz, rng, mask=None):
+    """A torso slab and a head ellipsoid centred at (hx, hy, hz) mm into img [h, w] (nearer surfaces are the
+    caller's order: a later person overwrites), the head's pixels set to 255 in mask if given."""
+    h, w = img.shape
+    fx, fy, cx, cy = 560.0 * w / 640.0, 560.0 * h / 480.0, w / 2.0, h / 2.0
+    # torso slab: below the head, slightly behind the head centre
+    tz = hz + 40.0
+    u0, u1 = int(cx + (hx - 230) * fx / tz), int(cx + (hx + 230) * fx / tz)
+    v0, v1 = int(cy + (hy + 115) * fy / tz), h
+    u0, u1, v0, v1 = max(u0, 0), min(u1, w), max(v0, 0), min(v1, h)
+    if u1 > u0 and v1 > v0:
+        uu = np.arange(u0, u1)[None, :]
+        vv = np.arange(v0, v1)[:, None]
+        shape = tz + 0.00008 * ((uu - (u0 + u1) / 2.0) ** 2) * tz / fx + 0.02 * (vv - v0)
+        img[v0:v1, u0:u1] = np.clip(shape + rng.uniform(-3, 3, shape.shape), 1, 65535).astype(np.uint16)
+    # head ellipsoid (orthographic approximation around the head centre)
+    a, b, c = 75.0, 100.0, 90.0
+    ru, rv = int(a * fx / hz) + 2, int(b * fy / hz) + 2
+    uc, vc = cx + hx * fx / hz, cy + hy * fy / hz
+    u0, u1 = max(int(uc - ru), 0), min(int(uc + ru) + 1, w)
+    v0, v1 = max(int(vc - rv), 0), min(int(vc + rv) + 1, h)
+    if u1 > u0 and v1 > v0:
+        uu = np.arange(u0, u1)[None, :]
+        vv = np.arange(v0, v1)[:, None]
+        X = (uu - cx) * hz / fx - hx
+        Y = (vv - cy) * hz / fy - hy
+        q = 1.0 - (X / a) ** 2 - (Y / b) ** 2
+        inside = q > 0
+        d = hz - c * np.sqrt(np.where(inside, q, 0.0)) + rng.uniform(-3, 3, q.shape)
+        reg = img[v0:v1, u0:u1]
+        reg[inside] = np.clip(d, 1, 65535).astype(np.uint16)[inside]
+        if mask is not None:
+            mask[v0:v1, u0:u1][inside] = 255
+
+
 def make_frames(n: int, seed: int = 0, w: int = 640, h: int = 480, sequence: bool = False,
                 start_index: int = 0, with_truth: bool = False):
     """n synthetic depth frames [n,h,w] u16.  One "person": a head ellipsoid (semi-axes
@@ -35,7 +70,6 @@ def make_frames(n: int, seed: int = 0, w: int = 640, h: int = 480, sequence: boo
     out = np.zeros((n, h, w), np.uint16)
     centres = np.zeros((n, 3), np.float32)
     masks = np.zeros((n, h, w), np.uint8) if with_truth else None
-    fx, fy, cx, cy = 560.0 * w / 640.0, 560.0 * h / 480.0, w / 2.0, h / 2.0
     for i in range(n):
         gi = start_index + i
         if sequence:
@@ -52,44 +86,38 @@ def make_frames(n: int, seed: int = 0, w: int = 640, h: int = 480, sequence: boo
         if hc is None:
             hc = rng.uniform([-150, -80, 700], [150, 40, 1200])
         hx, hy, hz = float(hc[0]), float(hc[1]), float(hc[2])
-        img = out[i]
-        # torso slab: below the head, slightly behind the head centre
-        tz = hz + 40.0
-        u0, u1 = int(cx + (hx - 230) * fx / tz), int(cx + (hx + 230) * fx / tz)
-        v0, v1 = int(cy + (hy + 115) * fy / tz), h
-        u0, u1, v0, v1 = max(u0, 0), min(u1, w), max(v0, 0), min(v1, h)
-        if u1 > u0 and v1 > v0:
-            uu = np.arange(u0, u1)[None, :]
-            vv = np.arange(v0, v1)[:, None]
-            shape = tz + 0.00008 * ((uu - (u0 + u1) / 2.0) ** 2) * tz / fx + 0.02 * (vv - v0)
-            img[v0:v1, u0:u1] = np.clip(shape + rng.uniform(-3, 3, shape.shape), 1, 65535).astype(np.uint16)
-        # head ellipsoid (orthographic approximation around the head centre)
-        a, b, c = 75.0, 100.0, 90.0
-        ru, rv = int(a * fx / hz) + 2, int(b * fy / hz) + 2
-        uc, vc = cx + hx * fx / hz, cy + hy * fy / hz
-        u0, u1 = max(int(uc - ru), 0), min(int(uc + ru) + 1, w)
-        v0, v1 = max(int(vc - rv), 0), min(int(vc + rv) + 1, h)
-        if u1 > u0 and v1 > v0:
-            uu = np.arange(u0, u1)[None, :]
-            vv = np.arange(v0, v1)[:, None]
-            X = (uu - cx) * hz / fx - hx
-            Y = (vv - cy) * hz / fy - hy
-            q = 1.0 - (X / a) ** 2 - (Y / b) ** 2
-            inside = q > 0
-            d = hz - c * np.sqrt(np.where(inside, q, 0.0)) + rng.uniform(-3, 3, q.shape)
-            reg = img[v0:v1, u0:u1]
-            reg[inside] = np.clip(d, 1, 65535).astype(np.uint16)[inside]
-            if with_truth:
-                masks[i, v0:v1, u0:u1][inside] = 255
+        _draw_person(out[i], hx, hy, hz, rng, masks[i] if with_truth else None)
         centres[i] = (hx, hy, hz)
         # dropout: 1-2 % of pixels to 0
         frac = rng.uniform(0.01, 0.02)
         drop = rng.random((h, w)) < frac
-        img[drop] = 0
+        out[i][drop] = 0
     if with_truth:
         rots = np.stack([centres[:, 0] / 8.0, centres[:, 1] / 4.0, (centres[:, 2] - 950.0) / 16.0], 1).astype(np.float32)
         return out, centres, rots, masks
     return out
+
+
+def make_person_frames(n: int, seed: int = 0, w: int = 640, h: int = 480, persons=None):
+    """n frames [n,h,w] u16 with 1-3 "persons" each (make_frames' person), side by side at different depths,
+    and their true head centres: (frames, centres [n,3,3] f32 mm with NaN rows for absent persons, counts [n]).
+    persons: None = 1-3 drawn per frame, an int = that many in every frame.  Person k stands in its own
+    lateral slot (heads at least 400 mm apart); the nearer persons are drawn last, 1-2 % dropout as make_frames."""
+    out = np.zeros((n, h, w), np.uint16)
+    centres = np.full((n, 3, 3), np.nan, np.float32)
+    counts = np.zeros(n, np.int32)
+    slots = {1: [0.0], 2: [-260.0, 260.0], 3: [-440.0, 0.0, 440.0]}
+    for i in range(n):
+        rng = np.random.default_rng([seed, 104729, i])
+        k = int(rng.integers(1, 4)) if persons is None else int(persons)
+        hc = np.stack([np.asarray(slots[k]) + rng.uniform(-40, 40, k), rng.uniform(-80, 40, k), rng.uniform(800, 1300, k)], 1)
+        for j in np.argsort(-hc[:, 2]):
+            _draw_person(out[i], float(hc[j, 0]), float(hc[j, 1]), float(hc[j, 2]), rng)
+        centres[i, :k] = hc
+        counts[i] = k
+        drop = rng.random((h, w)) < rng.uniform(0.01, 0.02)
+        out[i][drop] = 0
+    return out, centres, counts
 
 
 # ----------------------------------------------------------------------------- forest

@@ -343,6 +343,34 @@ int dh_predict_frames_hough_biwi(dh_ctx* c, const dh_forest* f, const uint8_t* b
                                  uint32_t w, uint32_t h, const dh_frame_args* args, dh_result* out,
                                  int blur, uint16_t* hough, int hough_loc, dh_result* from2d);
 
+/* Several heads per frame (DESIGN.md §7 "Several heads per frame"): more seeds into the votes the pose
+ * pass already cast.  After head 0 (the pose of dh_predict_frames), every try suppresses the coarse
+ * 20x20 cells within the projected radius R of its centre, seeds the next try at the first maximum of
+ * what is left (a cell of at least min_cell_votes), and runs mean-shift from it in the frame's centre
+ * accumulator.  A centre within R of an accepted head is dropped; at most 2 (max_heads - 1) tries follow
+ * head 0.  The rotation of head k >= 1 comes from the gated patches within R of its centre only; head 0
+ * keeps the frame-wide rotation of dh_predict_frames. */
+typedef struct dh_heads_params {
+    uint32_t max_heads;       /* 1..8 */
+    uint32_t min_cell_votes;  /* a further seed needs a coarse-grid cell with at least this many votes (>= 1) */
+    float radius_mm;          /* head radius R (> 0): suppression, duplicate test, vote attribution */
+    uint32_t _pad;
+} dh_heads_params;            /* 16 bytes */
+typedef struct dh_head {
+    dh_result pose;           /* head 0 is dh_predict_frames' result, bit for bit */
+    uint64_t support;         /* sum of the u32 centre-accumulator cells in the final 20^3 window (-10..+9) */
+    uint32_t n_patches;       /* gated patches whose p3 lies within R of mid_point */
+    uint32_t seed_cell;       /* coarse 20x20 cell the head was seeded from (gy*20+gx); 0xffffffff for a caller seed */
+} dh_head;                    /* 72 bytes */
+/* Frames and arguments as dh_predict_frames (host or device frames, the same chunked pipeline); heads of
+ * frame i in acceptance order to out[i * max_heads + k] (host), their count (>= 1) to n_heads[i] (host);
+ * unused slots are zeroed.  DH_E_ARG, naming the field, for a NULL params, max_heads 0 or > 8,
+ * radius_mm <= 0 or NaN, min_cell_votes 0, and a has_guess with bits other than 0-1.  Synchronous;
+ * n = 0 is a successful no-op. */
+int dh_predict_frames_heads(dh_ctx* c, const dh_forest* f, const uint16_t* depth, uint32_t n, uint32_t w, uint32_t h,
+                            int depth_loc, const dh_frame_args* args, const dh_heads_params* params, dh_head* out,
+                            uint32_t* n_heads);
+
 /* The writer for that format (the reference only reads it): n raw frames [n][h][w] u16 become n
  * files in ONE blob, file i at [offsets[i], offsets[i+1]) (offsets: n+1 entries, multiples of 16).
  * Runs are found at a granularity of 16 pixels: a group of 16 pixels with any non-zero pixel is
